@@ -8,6 +8,7 @@ arm; both pinned to the TestKajita2003 datrefs), 320-tap preview window.  A "ste
 one preview step = one OneIterationOfPreview call for both axes (PreviewControl.cpp:324-374).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            the CUDA path through the C ABI
+                  [--dump-outputs DIR]                           + the last timed pass's outputs as DIR/*.npy
   python bench.py --impl reference [...]                         the reference's CPU path on the host cores: its own
                                                                  PreviewControl object code (oracle/_ref), one process per core
 
@@ -963,6 +964,23 @@ def wieber_leg(ctx, wg, args, rank, want_cpu, hbm_peak):
     return res, kern
 
 
+DUMP_ROWS = 1 << 19          # preview steps sampled by --dump-outputs: 512 Ki rows of CoM + ZMP = 32 MB
+
+
+def dump_preview_outputs(out_dir, dcom, dzmp, ds, B, n):
+    """--dump-outputs: what the last timed pass hands its caller, as float64 .npy files - the CoM [n][6] and ZMP [n][2]
+    rows at a fixed, seeded sample of the n preview steps (every row when n <= DUMP_ROWS), the sampled row indices, and
+    the final [B][8] state of every walk.  The workload is seeded, so two builds can be compared file by file."""
+    os.makedirs(out_dir, exist_ok=True)
+    com = dcom.download(np.float64, (n, 6))
+    zmp = dzmp.download(np.float64, (n, 2))
+    rows = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    np.save(os.path.join(out_dir, "preview_com.npy"), com[rows])
+    np.save(os.path.join(out_dir, "preview_zmp.npy"), zmp[rows])
+    np.save(os.path.join(out_dir, "preview_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "preview_state.npy"), ds.download(np.float64, (B, 8)))
+
+
 def run_cuda(args):
     rank, local_rank, world = dist_env()
     import jrl_walkgen_b200 as wg
@@ -1026,6 +1044,9 @@ def run_cuda(args):
     launches = ctx.launches
     prof = ctx.prof_end()
     sum_mode, fit_resid = ctx.preview_sum_info()
+    if args.dump_outputs and rank == 0:
+        # before the direct-sum leg below reuses the same output buffers
+        dump_preview_outputs(args.dump_outputs, dcom, dzmp, ds, B, n)
 
     # ---- the same pass with the preview sum evaluated directly (the 320-tap FIR of preview_fused_kernel, FP64-pipe bound):
     # the kernel the recursive evaluation replaced as the default, timed beside it on the same inputs
@@ -1310,7 +1331,11 @@ def main():
     ap.add_argument("--e2e-passes", type=int, default=48)
     ap.add_argument("--sweep-instances", type=int, default=1000000)
     ap.add_argument("--sweep-periods", type=int, default=100)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the CoM / ZMP / state outputs of the last timed pass as DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl cuda)")
     # stdout carries the ONE JSON line and nothing else: libraries that print to file descriptor 1 on their own (NCCL announces
     # its version there when the box sets NCCL_DEBUG) are sent to stderr for the run; emit_line() puts the descriptor back
     global _STDOUT_FD

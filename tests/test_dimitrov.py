@@ -1,13 +1,16 @@
 """Dimitrov2008 path (support polygons -> constraint matrices -> PLDP -> LIPM): oracle pins (CPU) and CUDA parity (GPU).
 
 Pins (SURVEY 8c: the reference ships no test or datref for this generator - parity unpinned by golden vectors):
-  * the convex hull and BuildLinearConstraintInequalities restatements against the reference's OWN object code
-    (ConvexHull.cpp, FootConstraintsAsLinearSystem.cpp compiled where they lie into oracle/_ref) - bitwise;
-  * the receding-horizon loop against the same loop driven through the reference's own PLDPSolver object - bitwise;
+  * the convex hull and BuildLinearConstraintInequalities restatements against what the reference's OWN object code
+    (ConvexHull.cpp, FootConstraintsAsLinearSystem.cpp) returns on the same inputs - bitwise, stored in
+    tests/golden/dimitrov_ref.npz (tests/golden/make_dimitrov_ref.py);
+  * the receding-horizon loop against the same loop driven through the reference's own PLDPSolver object - bitwise (stored
+    solutions for the straight walk; the whole-generator cases run that object from oracle/_ref);
   * size-independent properties: every previewed CoP lies in its support polygon, the solution is the constrained
     optimum of the reference's cost.
 """
 import ctypes as C
+import os
 
 import numpy as np
 import pytest
@@ -20,6 +23,7 @@ import zmpdisc_oracle as zo
 PROFILES = ("StraightWalking", "Circle", "PbFlorentSeq1", "PbFlorentSeq2")
 needs_ref = pytest.mark.skipif(ol.ref() is None or not hasattr(ol.ref(), "ref_fcals_build"),
                                reason="oracle/_ref (reference object code) not built")
+REF = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "dimitrov_ref.npz"))
 
 
 def feet_of(name):
@@ -38,41 +42,22 @@ def assert_same_lci(a, b):
 # ------------------------------------------------------------------------------------------------
 # CPU
 # ------------------------------------------------------------------------------------------------
-@needs_ref
 def test_oracle_convex_hull_equals_reference_object_code():
-    rng = np.random.default_rng(7)
-    for trial in range(400):
-        kind = trial % 4
-        if kind == 0:      # two feet, same heading (collinear corners: 4 or 6 vertices)
-            th = rng.uniform(-0.5, 0.5) if trial % 8 else 0.0
-            feet = [(rng.uniform(-0.2, 0.2), 0.095, th), (rng.uniform(-0.2, 0.2), -0.095, th)]
-        elif kind == 1:    # two feet, different headings (up to 8 vertices)
-            feet = [(rng.uniform(-0.2, 0.2), 0.095, rng.uniform(-0.6, 0.6)), (rng.uniform(-0.2, 0.2), -0.095, rng.uniform(-0.6, 0.6))]
-        else:
-            feet = None
-        if feet:
-            pts = []
-            for (x, y, th) in feet:
-                c, s = np.cos(th), np.sin(th)
-                for lx, ly in ((1, -1), (1, 1), (-1, 1), (-1, -1)):
-                    pts.append((x + lx * 0.085 * c - ly * 0.03 * s, y + lx * 0.085 * s + ly * 0.03 * c))
-            pts = np.array(pts)
-        else:
-            pts = rng.uniform(-1, 1, (rng.integers(3, 9), 2))
-            if kind == 3:
-                pts = np.round(pts * 4) / 4      # many exact ties and collinear triples
-                if len(np.unique(pts, axis=0)) < 3:
-                    continue
-        a, b = do.hull(pts), do.ref_hull(pts)
+    """400 seeded point sets (tests/golden/make_dimitrov_ref.py): two feet with the same or different headings (collinear
+    corners, up to 8 vertices), random points, and points with exact ties and collinear triples."""
+    for trial in range(len(REF["hull"])):
+        pts = REF["hull_points"][trial, :REF["hull_npts"][trial]]
+        a, b = do.hull(pts), REF["hull"][trial, :REF["hull_count"][trial]]
         assert a.tobytes() == b.tobytes(), (trial, pts, a, b)
 
 
-@needs_ref
 @pytest.mark.parametrize("name", PROFILES)
 def test_oracle_fcals_equals_reference_object_code_on_the_kajita_profiles(name):
     left, right, lt, _ = feet_of(name)
     a = do.fcals(left, right, lt)
-    b = do.ref_fcals(left, right, lt)
+    b = np.zeros(len(REF["fcals_%s_rows" % name]), dtype=do.LCI)   # the reference reports no first_sample / state / rc
+    for k in ("rows", "similar", "A", "B", "center", "t_start", "t_end"):
+        b[k] = REF["fcals_%s_%s" % (name, k)]
     assert_same_lci(a, b)
     assert (a["rc"] == 0).all()
     # structure: the walk opens and closes in double support, polygons tile the clock without gaps
@@ -105,11 +90,11 @@ def test_oracle_constants_match_independent_numpy_construction():
     np.testing.assert_allclose(K.iPu, Kn.iPu, rtol=1e-6, atol=1e-6)
 
 
-@needs_ref
 def test_oracle_loop_equals_the_loop_driven_through_the_reference_pldp_object():
     """BuildZMPTrajectoryFromFootTrajectory, PLDP branch: the oracle's loop against the same loop with the solve done by
-    the reference's PLDPSolver object (hot-start memory inside the object, as in the reference): X bitwise, period by
-    period, up to the period at which the reference's solver would print "PB ON constraint" and call exit(0)."""
+    the reference's PLDPSolver object (hot-start memory inside the object, as in the reference; its solutions stored):
+    X bitwise, period by period, up to the period at which the reference's solver would print "PB ON constraint" and call
+    exit(0)."""
     left, right, lt, _ = feet_of("StraightWalking")
     par = do.default_params()
     out = do.run(left, right, lt, par)
@@ -121,28 +106,20 @@ def test_oracle_loop_equals_the_loop_driven_through_the_reference_pldp_object():
     assert (per["rc"][:17] == 0).all() and (per["status"][:17] == 0).all()
     K = do.Constants(par)
     P = do.fcals(left, right, lt, par)
-    ref = po.RefPLDP(K)
-    removed, starting = 0, True
     st = 0.0
     for li in range(17):
         xk = per["xk"][li].copy()
         pb = do.build_constraints(K, P, st, xk)
         assert pb["m"] == per["m"][li] and pb["n_first"] == per["n_first"][li]
         assert st == per["t_start"][li]
-        packed = {"m": np.array([pb["m"]]), "DPu": pb["DPu"][None], "DPx": pb["DPx"][None], "D": pb["D"][None],
-                  "ZMPRef": pb["ZMPRef"][None], "XkYk": pb["XkYk"][None]}
-        rc, X = ref.solve(packed, 0, starting=starting, n_removed=removed)
-        assert rc == 0
+        X = REF["loop_X"][li]
         jx = 0.0
         jy = 0.0
         for j in range(16):          # the reference's sequential sum (:1382-1400)
             jx += K.iLQ[j, 0] * X[j]
             jy += K.iLQ[j, 0] * X[j + 16]
         assert jx == per["jerk_x"][li] and jy == per["jerk_y"][li], li
-        starting = False
-        removed = pb["n_first"]
         st += par.T
-    ref.close()
 
 
 REF_OBJECT_CASES = ("StraightWalking", "StraightWalking@500", "StraightWalking@900", "Circle@200", "Circle@300", "Circle@640",

@@ -28,7 +28,9 @@ def _worker(rank, world, port, q):
 
 
 def test_two_ranks_shard_and_reduce_over_gloo():
-    import torch.multiprocessing as mp
+    # torch is imported by the spawned ranks only: in a test process where the library has already dlopen'ed the system's
+    # libnccl.so.2 (test_multi_gpu), importing torch here would bind libtorch_cuda to that older NCCL and fail
+    import multiprocessing as mp
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
     port = 29500 + (os.getpid() % 2000)

@@ -1,18 +1,18 @@
 """Pins for the PLDP / OptCholesky oracle (oracle/oracle_pldp.cpp) - all CPU.
 
 The reference ships no test or golden data for PLDPSolver (SURVEY 8c: parity unpinned by golden vectors); the pin is
-the reference's OWN object code (oracle/_ref: PLDPSolver.cpp / OptCholesky.cpp compiled from /root/reference) on
-identical inputs.  OptCholesky additionally reproduces the reference's only test, tests/TestOptCholesky.cpp
+what the reference's OWN object code (PLDPSolver.cpp / OptCholesky.cpp) returns on identical seeded inputs, stored in
+tests/golden/pldp_ref.npz (tests/golden/make_pldp_ref.py) and compared bitwise.  OptCholesky additionally reproduces the reference's only test, tests/TestOptCholesky.cpp
 (||A A^T - L L^T||_F <= 1e-6 on a 12 x 15 uniform matrix, rows added one by one; then full Cholesky + inverse).
 """
-import ctypes as C
+import os
 
 import numpy as np
-import pytest
 
-import oracle_lib as ol
 import pldp_oracle as po
 from jrl_walkgen_b200 import workloads as W
+
+REF = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "pldp_ref.npz"))
 
 
 def test_oracle_optcholesky_reproduces_testoptcholesky():
@@ -33,9 +33,6 @@ def test_oracle_optcholesky_reproduces_testoptcholesky():
 
 
 def test_oracle_optcholesky_equals_reference_object_code():
-    ref = ol.ref()
-    if ref is None:
-        pytest.skip("oracle/_ref not built on this machine")
     rng = np.random.default_rng(1)
     for mode, nb, cu in ((0, 12, 15), (1, 20, 32)):
         if mode == 0:
@@ -44,31 +41,20 @@ def test_oracle_optcholesky_equals_reference_object_code():
             A = rng.uniform(-1.0, 1.0, size=(cu, nb + 1))           # column-major, leading dimension nb + 1
         A = np.ascontiguousarray(A)
         rows = rng.permutation(nb)[:10].astype(np.int32)
-        L = np.zeros((nb, nb)); Lr = np.zeros((nb, nb))
+        L = np.zeros((nb, nb))
         po.lib().oracle_optcholesky_add_rows(mode, nb, cu, nb, A.ctypes.data, rows.ctypes.data, 0, 10, L.ctypes.data)
-        ref.ref_optcholesky_new.restype = C.c_void_p
-        h = ref.ref_optcholesky_new(nb, cu, mode)
-        ref.ref_optcholesky_set_A(C.c_void_p(h), A.ctypes.data_as(C.c_void_p), nb)
-        ref.ref_optcholesky_set_L(C.c_void_p(h), Lr.ctypes.data_as(C.c_void_p))
-        for r in rows:
-            ref.ref_optcholesky_add(C.c_void_p(h), int(r))
-        assert np.array_equal(L, Lr)                                # bitwise
-        ref.ref_optcholesky_delete(C.c_void_p(h))
+        assert np.array_equal(L, REF["optchol_L%d" % mode])         # bitwise
 
 
 def test_oracle_pldp_equals_reference_object_code_cold_and_hot():
     """Cold start and a hot-started sequence: X bitwise equal to the reference's PLDPSolver (the 1.3 ms wall-clock cap
     of the reference does not bind on these ~50 us problems)."""
-    if ol.ref() is None:
-        pytest.skip("oracle/_ref not built on this machine")
     K, pb = W.pldp_batch(40, seed=3)
     n_act = []
     for b in range(20):
-        ref2 = po.RefPLDP(K)                                        # fresh solver: no hot-start memory
-        rc, Xr = ref2.solve(pb, b, starting=True)
-        ref2.close()
+        Xr = REF["cold_X"][b]                                       # fresh solver: no hot-start memory
         X, info, act = po.oracle_solve(K, pb, b, hot=None, starting=True)
-        assert rc == 0 and info[0] == 0 and info[1] == 0
+        assert info[0] == 0 and info[1] == 0
         assert np.array_equal(X, Xr), (b, np.abs(X - Xr).max())
         n_act.append(info[3])
     assert max(n_act) >= 3                                          # constraints do get activated
@@ -80,7 +66,6 @@ def test_oracle_pldp_equals_reference_object_code_cold_and_hot():
         polys = W._support_polygons(rng, K.N, K.T, count=K.N + 25)
         xk_r = np.zeros(6); xk_r[0], xk_r[3] = polys[0][0]
         xk_o = xk_r.copy()
-        ref = po.RefPLDP(K)
         hot = np.zeros(1, dtype=po.STATE)
         n_removed = 0
         for t in range(25):
@@ -92,10 +77,10 @@ def test_oracle_pldp_equals_reference_object_code_cold_and_hot():
                 # negative and the reference calls exit(0) (:822-828).  The oracle reports status 2 instead; the
                 # reference must not be driven there inside the test process.
                 overshoot += 1
+                assert np.isnan(REF["hot_X"][seq, t]).all()
                 break
-            pr = W.pldp_pack(K, [W.pldp_problem_from(K, polys[t:t + K.N], xk_r)])
-            rc, Xr = ref.solve(pr, 0, starting=(t == 0), n_removed=n_removed)
-            assert rc == 0 and info[0] == 0 and info[1] == 0
+            Xr = REF["hot_X"][seq, t]
+            assert info[0] == 0 and info[1] == 0
             assert np.array_equal(X, Xr), (seq, t, np.abs(X - Xr).max())
             compared += 1
             kept += int(hot["n_prev"][0])
@@ -111,8 +96,6 @@ def test_oracle_pldp_similar_constraints_semantics_equal_reference_object_code()
         guarantees): reference object == oracle with the flags == oracle without them, bitwise - the reuse is bit-neutral;
     (b) backward flags that do NOT match the matrix: the reference reuses -tmp1 of the other row anyway; the oracle
         restates that exactly (bitwise equal X and activation order), and the result differs from the flag-less solve."""
-    if ol.ref() is None:
-        pytest.skip("oracle/_ref not built on this machine")
     K, pb = W.pldp_batch(24, seed=11)
     differ = 0
     for b in range(24):
@@ -121,8 +104,8 @@ def test_oracle_pldp_similar_constraints_semantics_equal_reference_object_code()
         assert (sim_ok[:m] != 0).sum() == m // 2
         X0, i0, a0 = po.oracle_solve(K, pb, b, starting=True)
         X1, i1, a1 = po.oracle_solve(K, pb, b, starting=True, similar=sim_ok)
-        ref = po.RefPLDP(K); rc, Xr = ref.solve(pb, b, starting=True, similar=sim_ok); ref.close()
-        assert rc == 0 and np.array_equal(X1, Xr) and np.array_equal(X0, X1) and np.array_equal(a0, a1)
+        Xr = REF["similar_X"][b]
+        assert np.array_equal(X1, Xr) and np.array_equal(X0, X1) and np.array_equal(a0, a1)
         rng = np.random.default_rng([11, b])
         sim_bad = np.zeros(128, dtype=np.int32)
         for li in range(1, m):
@@ -130,9 +113,10 @@ def test_oracle_pldp_similar_constraints_semantics_equal_reference_object_code()
                 sim_bad[li] = -int(rng.integers(1, min(li, 5) + 1))
         X2, i2, a2 = po.oracle_solve(K, pb, b, starting=True, similar=sim_bad)
         if i2[1] != 0:
-            continue          # a wrong reuse can drive the step length negative: the reference would exit(0) - and take
-                              # the test process with it - so it is only called where the oracle predicts a clean solve
-        ref = po.RefPLDP(K); rc, Xr2 = ref.solve(pb, b, starting=True, similar=sim_bad); ref.close()
+            assert REF["similar_bad_rc"][b] == -1
+            continue          # a wrong reuse can drive the step length negative: the reference would exit(0) there, so
+                              # it has a stored solve only where the oracle predicts a clean one
+        Xr2, rc = REF["similar_bad_X"][b], REF["similar_bad_rc"][b]
         assert np.array_equal(X2, Xr2, equal_nan=True) and rc == i2[0], (b, np.abs(X2 - Xr2).max())
         differ += int(not np.array_equal(X2, X0))
     assert differ >= 2

@@ -19,7 +19,8 @@ import oracle_lib as ol
 import preview_ref as pr
 import zmpdisc_oracle as zo
 
-pytestmark = pytest.mark.skipif(pr.lib() is None, reason="oracle/_ref/libwalkgen_ref.so (reference object code) not built")
+needs_ref = pytest.mark.skipif(pr.lib() is None, reason="oracle/_ref/libwalkgen_ref.so (reference object code) not built")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "preview_ref.npz")
 
 TOL_COM = 1e-9     # m; north_star asks 1e-6 m for CoM/ZMP trajectories
 CONFIGS = [(0.005, 1.6, 0.814, 1), (0.005, 1.6, 0.807709, 1), (0.01, 1.6, 0.814, 0), (0.005, 0.8, 0.75, 1)]
@@ -45,6 +46,20 @@ def straight_walking_zmpref():
     return z
 
 
+def gpu_preview_inputs():
+    """The StraightWalking ZMP reference and 64 seeded random walks, with their seeded initial states."""
+    rng = np.random.default_rng(21)
+    walks = [straight_walking_zmpref()] + [synth_walk(rng, int(L)) for L in rng.integers(900, 5200, size=64)]
+    st0 = rng.normal(scale=0.01, size=(len(walks), 8)); st0[0] = 0.0
+    return walks, st0
+
+
+def sample_rows(steps, b, count):
+    """Fixed, seeded sample of `count` preview steps of walk b (its first and last step included), sorted."""
+    r = 1 + np.random.default_rng([21, b]).choice(steps - 2, size=count - 2, replace=False)
+    return np.sort(np.concatenate([[0, steps - 1], r]).astype(np.int64))
+
+
 def ref_with_gains(g, T, Tp, zc):
     rp = pr.RefPreview(1, False)
     rp.set_gains(T, Tp, zc, g.Kx, g.Ks, g.F)
@@ -54,6 +69,7 @@ def ref_with_gains(g, T, Tp, zc):
 # ------------------------------------------------------------------------------------------------
 # CPU: restatement vs reference object code
 # ------------------------------------------------------------------------------------------------
+@needs_ref
 @pytest.mark.parametrize("T,Tp,zc,mode", CONFIGS)
 def test_reference_gains_vs_oracle_and_product(T, Tp, zc, mode):
     """ComputeOptimalWeights of the reference (generalized Schur form through dgges_) against the oracle's Riccati
@@ -76,6 +92,7 @@ def test_reference_gains_vs_oracle_and_product(T, Tp, zc, mode):
     assert np.array_equal(g["A"], np.array(p.A[:])) and np.array_equal(g["B"], np.array(p.B[:]))
 
 
+@needs_ref
 def test_reference_gains_through_plugin_commands():
     """:samplingperiod / :previewcontroltime / :comheight with automatic weights (PreviewControl.cpp:512-548)."""
     if not pr.lapack_available():
@@ -89,6 +106,7 @@ def test_reference_gains_through_plugin_commands():
     assert g["NL"] == 320 and abs(g["Ks"] - o.Ks) <= 2e-9 * o.Ks
 
 
+@needs_ref
 @pytest.mark.parametrize("simulation", [True, False])
 @pytest.mark.parametrize("use_lindex", [False, True])
 def test_oracle_recursion_is_bitwise_the_reference(simulation, use_lindex):
@@ -111,6 +129,7 @@ def test_oracle_recursion_is_bitwise_the_reference(simulation, use_lindex):
     rp.close()
 
 
+@needs_ref
 def test_oracle_1d_variants_are_bitwise_the_reference():
     """OneIterationOfPreview1D: deque overload (:376-421) and vector overload with its wrap-around branch (:423-484)."""
     o = ol.OracleGains(0.005, 1.6, 0.814, 1)
@@ -142,6 +161,7 @@ def test_oracle_1d_variants_are_bitwise_the_reference():
     rp.close()
 
 
+@needs_ref
 def test_read_precomputed_file_goes_through_float(tmp_path):
     """ReadPrecomputedFile parses every gain into a `float` (PreviewControl.cpp:157-176): a 17-digit file comes back
     rounded to single precision.  The product's PreviewControl::ReadPrecomputedFile mirror does the same
@@ -179,23 +199,27 @@ def _gpu_run(ctx, gains, offsets, z, st0, simulation=True):
 def test_gpu_preview_vs_reference_object(ctx, own_gains, shape):
     """The batch preview kernels (shape -1: the default choice for this batch size; 0: preview_rec_kernel at 64 x 8; 2:
     preview_rec_warp_kernel, the one a batch of thousands of walks runs through; 3: 256 x 2, small batches) against PreviewControl::OneIterationOfPreview of the reference object on the StraightWalking
-    ZMP reference and 64 random walks.  own_gains=False: both sides use the product's gains (pins the recursion);
-    own_gains=True: the reference computes its own gains through dgges_ (pins gains + recursion end to end)."""
+    ZMP reference and 64 random walks.  own_gains=False: both sides use the product's gains (pins the recursion; the
+    reference's output is stored, at 96 seeded steps of every walk, in tests/golden/preview_ref.npz); own_gains=True: the
+    reference object computes its own gains through dgges_ (pins gains + recursion end to end); where oracle/_ref is not
+    built, the oracle's recursion on the oracle's own gains (Riccati fixed point, independent of the product's doubling solve,
+    2e-9 relative from dgges_) stands in for it."""
     import jrl_walkgen_b200 as wg
     T, Tp, zc = 0.005, 1.6, 0.807709
     gains = wg.preview_gains(T, Tp, zc, 1)
-    rp = pr.RefPreview(1, False)
-    if own_gains:
+    rp = og = None
+    if own_gains and pr.lib() is not None:
         if not pr.lapack_available():
             pytest.skip("no LAPACK with dgges_ in this image")
+        rp = pr.RefPreview(1, False)
         rp.compute_weights(T, Tp, zc, 1)
+    elif own_gains:
+        og = ol.OracleGains(T, Tp, zc, 1)
     else:
-        rp.set_gains(T, Tp, zc, np.array(gains.Kx[:]), gains.Ks, np.array(gains.F[:gains.NL]))
-    rng = np.random.default_rng(21)
-    walks = [straight_walking_zmpref()] + [synth_walk(rng, int(L)) for L in rng.integers(900, 5200, size=64)]
+        gold = np.load(GOLDEN)
+    walks, st0 = gpu_preview_inputs()
     offsets = np.concatenate([[0], np.cumsum([len(w) for w in walks])]).astype(np.int64)
     z = np.concatenate(walks)
-    st0 = rng.normal(scale=0.01, size=(len(walks), 8)); st0[0] = 0.0
     ctx.preview_set_cta_shape(shape)
     for simulation in (True, False):
         try:
@@ -204,40 +228,48 @@ def test_gpu_preview_vs_reference_object(ctx, own_gains, shape):
             ctx.preview_set_cta_shape(-1)
             raise
         worst = 0.0
+        tag = "sim" if simulation else "nosim"
         for b, w in enumerate(walks):
-            sr = st0[b].copy()
-            com_r, zmp_r, steps = rp.run(w, sr, simulation)
+            steps = len(w) - 320 + 1
             o = int(offsets[b])
-            assert steps == len(w) - 320 + 1
-            e = max(np.abs(com[o:o + steps, [0, 3]] - com_r[:steps, [0, 3]]).max(),
-                    np.abs(zmp[o:o + steps] - zmp_r[:steps]).max())
+            if rp is not None or og is not None:
+                sr = st0[b].copy()
+                com_r, zmp_r, steps_r = rp.run(w, sr, simulation) if rp is not None else \
+                    ol.oracle_preview_batch(og, [0, len(w)], w, sr, simulation)
+                assert steps_r == steps
+                rows = np.arange(steps)
+                com_r, zmp_r = com_r[:steps, [0, 3]], zmp_r[:steps]
+            else:
+                rows = sample_rows(steps, b, 96)
+                assert np.array_equal(rows, gold[tag + "_rows"][b])
+                com_r, zmp_r, sr = gold[tag + "_com_x_y"][b], gold[tag + "_zmp"][b], gold[tag + "_state"][b]
+            e = max(np.abs(com[o + rows][:, [0, 3]] - com_r).max(), np.abs(zmp[o + rows] - zmp_r).max())
             worst = max(worst, e)
             assert np.allclose(st[b, :6], sr[:6], atol=1e-8, rtol=0)
         assert worst < (TOL_COM if simulation else 1e-7), worst
     ctx.preview_set_cta_shape(-1)
-    rp.close()
+    if rp is not None:
+        rp.close()
 
 
 @pytest.mark.gpu
 def test_gpu_one_iteration_vs_reference_object(ctx):
     """wg_preview_one_iteration (the per-tick call of the class mirror) over 200 consecutive ticks of the
-    StraightWalking reference == the reference object, tick by tick."""
+    StraightWalking reference == the reference object (its output stored in tests/golden/preview_ref.npz), tick by tick."""
     import jrl_walkgen_b200 as wg
     gains = wg.preview_gains(0.005, 1.6, 0.807709, 1)
     ctx.preview_set_gains(gains)
-    rp = pr.RefPreview(1, False)
-    rp.set_gains(0.005, 1.6, 0.807709, np.array(gains.Kx[:]), gains.Ks, np.array(gains.F[:gains.NL]))
     z = straight_walking_zmpref()[600:600 + 320 + 200]
-    st = np.zeros(8)
-    com_r, zmp_r, steps = rp.run(z, st)
+    gold = np.load(GOLDEN)
+    com_r, zmp_r = gold["one_iteration_com"], gold["one_iteration_zmp"]
     x = np.zeros(3); y = np.zeros(3); sx = sy = 0.0
     for k in range(200):
         x, y, sx, sy, zx, zy = ctx.preview_one_iteration(x, y, sx, sy, z[k:k + 320])
         assert np.abs(x - com_r[k, :3]).max() < 1e-9 and np.abs(y - com_r[k, 3:]).max() < 1e-9
         assert abs(zx - zmp_r[k, 0]) < 1e-9 and abs(zy - zmp_r[k, 1]) < 1e-9
-    rp.close()
 
 
+@needs_ref
 @pytest.mark.gpu
 def test_cpp_mirror_1d_variants_and_precomputed_file_vs_reference_object(tmp_path):
     """The host class mirror (PreviewControl::ReadPrecomputedFile, OneIterationOfPreview1D deque and vector overloads

@@ -4,7 +4,9 @@ reference's OWN object code: src/ZMPRefTrajectoryGeneration/ZMPQPWithConstraint.
 reference's).  The reference holds no golden data for this generator.
   * CPU: the restatement oracle/oracle_wieber.cpp (with the reference's ql0001_) against that object: polygons and the
     whole CoM / ZMP output, bitwise.
-  * GPU: wg_wieber_run_batch against the same object at north_star's tolerance (1e-6 m on CoM / ZMP).
+  * GPU: wg_wieber_run_batch against the same object at north_star's tolerance (1e-6 m on CoM / ZMP).  Where oracle/_ref is
+    not built, the GPU tests compare with wieber_oracle.OracleWieber instead, which reproduces that object's trajectory to
+    1e-7 m; the tests of the reference object itself need oracle/_ref.
 """
 import ctypes as C
 
@@ -16,8 +18,8 @@ import dimitrov_oracle as do
 import wieber_oracle as wo
 import zmpdisc_oracle as zo
 
-pytestmark = pytest.mark.skipif(ol.ref() is None or not hasattr(ol.ref(), "ref_wieber_new"),
-                                reason="oracle/_ref/libwalkgen_ref.so (reference object code) not built")
+HAVE_REF = ol.ref() is not None and hasattr(ol.ref(), "ref_wieber_new")
+needs_ref = pytest.mark.skipif(not HAVE_REF, reason="oracle/_ref/libwalkgen_ref.so (reference object code) not built")
 
 
 def short_walk(nsteps=4, sx=0.2):
@@ -28,11 +30,12 @@ def short_walk(nsteps=4, sx=0.2):
 
 @pytest.fixture(scope="module")
 def ref_gen():
-    r = wo.RefWieber()
+    r = wo.RefWieber() if HAVE_REF else wo.OracleWieber()
     yield r
     r.close()
 
 
+@needs_ref
 def test_polygons_are_those_of_the_reference_generator(ref_gen):
     """BuildLinearConstraintInequalities of ZMPQPWithConstraint == oracle_fcals_build (rows A, B and the time windows), bitwise,
     on the four TestKajita2003 profiles."""
@@ -47,6 +50,7 @@ def test_polygons_are_those_of_the_reference_generator(ref_gen):
         assert np.array_equal(lci["t_start"], times[:, 0]) and np.array_equal(lci["t_end"], times[:, 1]), name
 
 
+@needs_ref
 def test_restatement_matches_reference_object_bitwise(ref_gen):
     """BuildZMPTrajectoryFromFootTrajectory on a four-step walk: every CoM / ZMP sample the loop writes."""
     w = short_walk(4)
@@ -103,6 +107,7 @@ def test_gpu_wieber_generator_matches_reference_object(ctx, ref_gen, materialize
           f"active-set changes per QP {out['qp_iterations'].sum() / out['periods_done'].sum():.1f}")
 
 
+@needs_ref
 def test_reference_qld_regularises_the_hessian_and_the_rule_is_restated():
     """Finding of this pin: the Wieber2006 Hessian (beta PPu'PPu + alpha VPu'VPu, 75 samples of 20 ms) has eigenvalues down to
     3e-10 (cond 5e11).  ql0001_ does not factorise it as given: ql0002_ adds a multiple of I until every Cholesky pivot exceeds

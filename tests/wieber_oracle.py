@@ -85,3 +85,29 @@ class RefWieber:
         n = self.r.ref_wieber_polygons(self.h, len(L), ol.dptr(L), ol.dptr(R), st.ctypes.data_as(IP), ol.dptr(t), cx, cy, cap, 8,
                                        ol.dptr(rows), ol.dptr(times), nr.ctypes.data_as(IP))
         return rows[:n], times[:n], nr[:n]
+
+
+class OracleWieber:
+    """Stand-in for RefWieber.run where oracle/_ref is not built: the restatement oracle/oracle_wieber.cpp (bitwise the
+    reference object when both use the reference's ql0001_) with its QP solved in extended precision on the Hessian plus
+    QLD's diagonal boost (wg_qld_diagonal_boost, QLD's rule restated).  That chain reproduces the reference object's
+    trajectory to 1e-7 m (CoM) / 1e-8 m (ZMP): test_reference_qld_regularises_the_hessian_and_the_rule_is_restated."""
+
+    def __init__(self):
+        from jrl_walkgen_b200 import _capi
+        Cf = np.asfortranarray(constants()[0])
+        self.boost = _capi.load().wg_qld_diagonal_boost(2 * N_DEFAULT, 2 * N_DEFAULT, Cf.ctypes.data, 1e-8)
+
+    def close(self):
+        pass
+
+    def run(self, walk):
+        o = _ora()
+        o.oracle_wieber_set_boost.argtypes = [C.c_double]
+        o.oracle_wieber_set_solver(2); o.oracle_wieber_set_boost(self.boost)
+        try:
+            k, com, zz, _ = run(walk)
+        finally:
+            o.oracle_wieber_set_solver(0); o.oracle_wieber_set_boost(0.0)
+        return (0 if k > 0 else -1), com, zz
+
