@@ -541,7 +541,10 @@ int wg_optcholesky_full_batch(wg_ctx *ctx, int mem, int B, int n, const double *
  * bounds, then n upper bounds (qld.cpp:520-536).  One CTA per QP; dual active-set method in range-space form (qld.cu).
  * ifail: 0 ok; 1 iteration limit 40 (m + n) (QLD :459); 2 C not positive definite and eps = 0 (with eps > 0 the diagonal is
  * boosted as QLD does, :809-918); 3 more than n active rows; 5 bad dimensions; 10 + j: constraint j (1-based) cannot be satisfied
- * together with the active ones (QLD's ifail > 10).  On failure x is the unconstrained minimiser.
+ * together with the active ones (QLD's ifail > 10).  On failure x is the unconstrained minimiser.  A row of zeros is
+ * inconsistent (10 + j) when b_j < 0 (inequality) or b_j != 0 (equality), and ignored with u_j = 0 otherwise.  Equality rows
+ * that depend on earlier ones are skipped when consistent (their multipliers are then not unique: the solver returns one
+ * choice) and reported as 10 + j when not.
  * ---------------------------------------------------------------------------------------------- */
 #define WG_QLD_MAX_N 160
 #define WG_QLD_MAX_M 1024
@@ -560,7 +563,7 @@ typedef struct wg_qld_batch {
   long long b_stride;
   const double *xl, *xu;      /* [B][n] each, or both NULL (no bounds; the reference passes -1e8 / +1e8)          */
   double *x;                  /* [B][n]        out                                                               */
-  double *u;                  /* [B][u_stride] out, or NULL                                                      */
+  double *u;                  /* [B][u_stride] out, or NULL; entries past m (+ 2n) of each row are set to 0        */
   long long u_stride;         /* >= mmax (+ 2 n when bounds are given)                                           */
   int32_t *ifail;             /* [B]           out                                                               */
   int32_t *iterations;        /* [B]           out (active-set changes), or NULL                                 */
@@ -575,7 +578,8 @@ typedef struct wg_qld_batch {
  * found by its 2 x 2 minor test and by doubling steps until every Cholesky pivot exceeds vsmall = eps (the accuracy argument
  * of ql0001_, 1e-8 in every call of the reference).  For a well conditioned C diag is 0; for the reference's generators
  * (eigenvalues down to 2e-9) it is not, and ql0001_'s results are those of the regularised problem - pass the reference's eps
- * to reproduce them, 0 to solve the problem as stated.  wg_qld_shared_boost returns the diag that was added. */
+ * to reproduce them, 0 to solve the problem as stated.  wg_qld_shared_boost returns the diag that was added.  The Wieber2006
+ * generator keeps its Hessian apart: running it does not replace the one installed here. */
 int wg_qld_set_shared_hessian(wg_ctx *ctx, int n, int nmax, const double *C, double eps);
 double wg_qld_shared_boost(wg_ctx *ctx);
 /* The rule alone (host arithmetic, no device): the multiple of I that ql0001_(eps) adds to C before factorising it. */
@@ -588,7 +592,8 @@ int wg_qld_solve_batch(wg_ctx *ctx, int mem, int B, const wg_qld_batch *batch);
  * i.e. a half-plane normal (A0, A1) applied to previewed sample `sample[r]` of the lower-triangular Toeplitz map uz from the
  * jerks to the CoP.  A0, A1, sample: [B][row_stride] (row_stride >= mmax), uz_dev: N DEVICE doubles; batch->A is ignored.  The
  * m x n matrix (360 KB per Wieber QP) is neither materialised nor streamed: the violation scan works on the N points Uz x.
- * Device memory only (mem = WG_MEM_DEVICE).  Same results as the dense entry on the materialised matrix up to rounding. */
+ * Device memory only (mem = WG_MEM_DEVICE).  Same results as the dense entry on the materialised matrix up to rounding.
+ * sample[r] is not validated: a value >= N is read as N - 1. */
 int wg_qld_solve_batch_ranked(wg_ctx *ctx, int mem, int B, const wg_qld_batch *batch, const double *A0, const double *A1,
                               const unsigned char *sample, long long row_stride, const double *uz_dev, int N);
 

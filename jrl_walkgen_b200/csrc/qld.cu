@@ -30,11 +30,17 @@ namespace {
 constexpr int QT = 256;              // threads per CTA
 constexpr int QW = QT / 32;
 
+// A Hessian shared by every QP of a batch, factorised once on the host.
+struct SharedHessian {
+  double *d_hinv = nullptr;          // [n*n] X = L^-1 in symmetric storage
+  double *d_c = nullptr;             // [n*n] the Hessian itself, symmetric dense
+  int n = 0;
+  double boost = 0.0;                // the multiple of I QLD's rule added to it
+};
+
 struct QldState {
-  double *d_hinv_shared = nullptr;   // [n*n] inverse of the shared Hessian
-  double *d_c_shared = nullptr;      // [n*n] the shared Hessian itself (refinement step), symmetric dense
-  int shared_n = 0;
-  double shared_boost = 0.0;         // the multiple of I QLD's rule added to the shared Hessian
+  SharedHessian caller;              // wg_qld_set_shared_hessian
+  SharedHessian generator;           // the Wieber2006 generator's own (wgi_qld_set_generator_hessian): a caller's stays put
   // per-call scratch
   double *d_hinv = nullptr; size_t cap_hinv = 0;     // [B][n*n] per-QP inverses
   double *d_work = nullptr; size_t cap_work = 0;     // per-CTA Z (n x qcap) and T (packed)
@@ -303,6 +309,7 @@ __device__ __forceinline__ void rows_partial(const double *__restrict__ A, int m
 
 struct QldArgs {
   int B, n, nmax, mmax, qcap;
+  int pstride;                              // stride of the QW partial row sums in shared memory: >= mmax, and QW pstride >= 4N (RANKED)
   const int *m, *me;
   const double *C; long long c_stride;      // per-QP Hessians (refinement), or the shared one with stride 0
   const double *S; long long h_stride;      // X = L^-1 in symmetric storage; stride 0: shared
@@ -338,14 +345,14 @@ qld_kernel(QldArgs P)
   __shared__ int redi[QW];
   __shared__ int s_b;
   const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
-  const int n = P.n, qcap = P.qcap, mmax = P.mmax;
+  const int n = P.n, qcap = P.qcap, mmax = P.mmax, pstride = P.pstride;
   const bool bounds = (P.xl != nullptr) && (P.xu != nullptr);
   const int mtot_max = mmax + (bounds ? 2 * n : 0);
   double *x = reinterpret_cast<double *>(smem_raw);
   double *v = x + n, *v0 = v + n, *ap = v0 + n, *yp = ap + n, *yd = yp + n;
   double *inrm = yd + n;
-  double *part = inrm + mtot_max;                                         // QW x mmax partial row sums
-  double *u = part + (size_t)QW * mmax, *g = u + qcap, *w = g + qcap, *r = w + qcap;
+  double *part = inrm + mtot_max;                                         // QW x pstride partial row sums
+  double *u = part + (size_t)QW * pstride, *g = u + qcap, *w = g + qcap, *r = w + qcap;
   int *Wc = reinterpret_cast<int *>(r + qcap);
   int *slot = Wc + qcap, *freeslot = slot + qcap;
   signed char *sgn = reinterpret_cast<signed char *>(freeslot + qcap);   // sign of an active (equality) row
@@ -370,7 +377,8 @@ qld_kernel(QldArgs P)
     const double *S = P.S + (size_t)b * P.h_stride;
     const double *Cm = P.C ? P.C + (size_t)b * P.c_stride : nullptr;
     const double *xl = bounds ? P.xl + (size_t)b * n : nullptr, *xu = bounds ? P.xu + (size_t)b * n : nullptr;
-    int fail = 0, iters = 0, q = 0, neq = 0;
+    // neq: equality rows processed (added, or skipped as redundant); qeq: equality rows in the active set, positions 0..qeq-1
+    int fail = 0, iters = 0, q = 0, neq = 0, qeq = 0;
     if (m < 0 || m > mmax || me < 0 || me > m) fail = 5;                  // QLD ifail 5: wrong dimensions
     if (!fail && P.hfail && P.hfail[P.h_stride ? b : 0]) fail = 2;
     const int mtot = fail ? 0 : m + (bounds ? 2 * n : 0);
@@ -383,7 +391,7 @@ qld_kernel(QldArgs P)
       for (int i = t; i < N; i += QT) uzs[i] = P.uz[i];
       __syncthreads();
       for (int i = t; i < N; i += QT) { double a = 0.0; for (int k = 0; k <= i; ++k) a = fma(uzs[k], uzs[k], a); rn2[i] = a; }
-    } else if (!fail) rows_partial(A, mmax, m, n, nullptr, part, mmax, warp, lane);
+    } else if (!fail) rows_partial(A, mmax, m, n, nullptr, part, pstride, warp, lane);
     __syncthreads();
     for (int i = t; i < n; i += QT) { v0[i] = -v0[i]; v[i] = v0[i]; }
     for (int rr = t; rr < mtot; rr += QT) {
@@ -393,10 +401,12 @@ qld_kernel(QldArgs P)
         else {
           s = 0.0;
 #pragma unroll
-          for (int wq = 0; wq < QW; ++wq) s += part[(size_t)wq * mmax + rr];
+          for (int wq = 0; wq < QW; ++wq) s += part[(size_t)wq * pstride + rr];
         }
       }
-      inrm[rr] = s > 0.0 ? rsqrt(s) : 0.0;
+      // a zero row is scaled by 1, so that its violation is b itself: with b < 0 it is picked, found dependent on any active
+      // set and reported as inconsistent (ifail 10 + j); with b >= 0 it is never violated
+      inrm[rr] = s > 0.0 ? rsqrt(s) : 1.0;
       act[rr] = 0;
     }
     __syncthreads();
@@ -440,7 +450,7 @@ qld_kernel(QldArgs P)
             for (; k <= i; ++k) a0 = fma(uzs[i - k], xa[k], a0);
             pts[e] = (a0 + a1) + (a2 + a3);
           }
-        } else rows_partial(A, mmax, m, n, x, part, mmax, warp, lane);
+        } else rows_partial(A, mmax, m, n, x, part, pstride, warp, lane);
         __syncthreads();
         for (int rr = t; rr < mtot; rr += QT) {
           if (act[rr] || rr < me) continue;          // equalities are all taken above
@@ -452,7 +462,7 @@ qld_kernel(QldArgs P)
             } else {
               s = 0.0;
 #pragma unroll
-              for (int wq = 0; wq < QW; ++wq) s += part[(size_t)wq * mmax + rr];
+              for (int wq = 0; wq < QW; ++wq) s += part[(size_t)wq * pstride + rr];
             }
             const double bb = bv[rr];
             s += bb;
@@ -536,7 +546,7 @@ qld_kernel(QldArgs P)
           double s = 0.0;
           for (int rr = j; rr < q; ++rr) s = fma(T[tri(rr) + j], w[rr], s);
           r[j] = s;
-          if (s > 0.0 && j >= neq) {                        // equality rows are never dropped
+          if (s > 0.0 && j >= qeq) {                        // equality rows are never dropped
             const double tj = u[j] / s;
             if (tj < t1) { t1 = tj; l = j; }
           }
@@ -569,7 +579,7 @@ qld_kernel(QldArgs P)
           for (int i = t; i < n; i += QT) Y[(size_t)sl * n + i] = yd[i] * idd;
           if (t == 0) { T[tri(q) + q] = idd; Wc[q] = p; slot[q] = sl; u[q] = up; sgn[q] = (signed char)sign; act[p] = 1; }
           --nfree; ++q;
-          if (neq < me) ++neq;
+          if (neq < me) { ++neq; ++qeq; }
           added = true;
           __syncthreads();
           break;
@@ -651,8 +661,7 @@ qld_kernel(QldArgs P)
     for (int i = t; i < n; i += QT) P.x[(size_t)b * n + i] = x[i];
     if (P.u) {
       double *uo = P.u + (size_t)b * P.u_stride;
-      const int mu = max(m, 0) + 2 * n;
-      for (int k = t; k < mu && k < P.u_stride; k += QT) uo[k] = 0.0;
+      for (int k = t; k < P.u_stride; k += QT) uo[k] = 0.0;             // the whole row: no stale values past m + 2n
       __syncthreads();
       if (!fail)
         for (int k = t; k < q; k += QT) {
@@ -669,10 +678,10 @@ qld_kernel(QldArgs P)
   }
 }
 
-size_t qld_smem_bytes(int n, int mmax, int qcap, bool bounds)
+size_t qld_smem_bytes(int n, int mmax, int pstride, int qcap, bool bounds)
 {
   const size_t mtot = (size_t)mmax + (bounds ? 2 * (size_t)n : 0);
-  size_t s = sizeof(double) * (6 * (size_t)n + mtot + (size_t)QW * mmax + 4 * (size_t)qcap) + sizeof(int) * 3 * (size_t)qcap + qcap + mtot;
+  size_t s = sizeof(double) * (6 * (size_t)n + mtot + (size_t)QW * pstride + 4 * (size_t)qcap) + sizeof(int) * 3 * (size_t)qcap + qcap + mtot;
   return (s + 15) & ~(size_t)15;
 }
 
@@ -691,7 +700,8 @@ void wg_qld_release(wg_ctx *ctx)
 {
   if (!ctx->qld) return;
   QldState *st = static_cast<QldState *>(ctx->qld);
-  cudaFree(st->d_hinv_shared); cudaFree(st->d_c_shared); cudaFree(st->d_hinv); cudaFree(st->d_work); cudaFree(st->d_next);
+  for (SharedHessian *h : {&st->caller, &st->generator}) { cudaFree(h->d_hinv); cudaFree(h->d_c); }
+  cudaFree(st->d_hinv); cudaFree(st->d_work); cudaFree(st->d_next);
   cudaFree(st->d_fail); cudaFree(st->d_stage);
   delete st;
   ctx->qld = nullptr;
@@ -753,18 +763,15 @@ static double qld_diagonal_boost(int n, int nmax, const double *C, double vsmall
   return diag;
 }
 
-extern "C" {
-
-int wg_qld_set_shared_hessian(wg_ctx *ctx, int n, int nmax, const double *C_in, double eps)
+// Factorise C (+ QLD's boost) into slot h.  The slot keeps its previous Hessian when C is refused.
+static int install_shared_hessian(wg_ctx *ctx, SharedHessian &h, int n, int nmax, const double *C_in, double eps)
 {
   if (!ctx || n <= 0 || n > WG_QLD_MAX_N || nmax < n || !C_in) return WG_ERR_INVALID;
   wg_device_guard guard(ctx->device);
-  QldState *st = state_of(ctx);
   const double boost = qld_diagonal_boost(n, nmax, C_in, eps);
   std::vector<double> Cb(C_in, C_in + (size_t)nmax * n);
   for (int i = 0; i < n; ++i) Cb[(size_t)i * nmax + i] += boost;
   const double *C = Cb.data();
-  st->shared_boost = boost;
   // the inverse in extended precision on the host: once per Hessian, and the generators' Hessians (sums of products of
   // integrator matrices over 75 samples) are badly conditioned
   typedef long double LD;
@@ -772,7 +779,7 @@ int wg_qld_set_shared_hessian(wg_ctx *ctx, int n, int nmax, const double *C_in, 
   for (int j = 0; j < n; ++j) {
     LD p = C[(size_t)j * nmax + j];
     for (int k = 0; k < j; ++k) p -= L[(size_t)j * n + k] * L[(size_t)j * n + k];
-    if (!(p > 0)) return wg_fail(ctx, WG_ERR_INVALID, "wg_qld_set_shared_hessian: C is not positive definite");
+    if (!(p > 0)) return wg_fail(ctx, WG_ERR_INVALID, "shared Hessian: C is not positive definite");
     const LD l = sqrtl(p);
     L[(size_t)j * n + j] = l;
     for (int i = j + 1; i < n; ++i) {
@@ -796,17 +803,29 @@ int wg_qld_set_shared_hessian(wg_ctx *ctx, int n, int nmax, const double *C_in, 
       Cs[(size_t)a * n + b] = Cs[(size_t)b * n + a] = C[(size_t)b * nmax + a];
     }
   WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  if (st->shared_n != n) {
-    cudaFree(st->d_hinv_shared); cudaFree(st->d_c_shared);
-    st->d_hinv_shared = st->d_c_shared = nullptr; st->shared_n = 0;
-    WG_CUDA(ctx, cudaMalloc(&st->d_hinv_shared, sizeof(double) * n * n));
-    WG_CUDA(ctx, cudaMalloc(&st->d_c_shared, sizeof(double) * n * n));
-    st->shared_n = n;
+  if (h.n != n) {
+    cudaFree(h.d_hinv); cudaFree(h.d_c);
+    h.d_hinv = h.d_c = nullptr; h.n = 0;
+    WG_CUDA(ctx, cudaMalloc(&h.d_hinv, sizeof(double) * n * n));
+    WG_CUDA(ctx, cudaMalloc(&h.d_c, sizeof(double) * n * n));
+    h.n = n;
   }
-  WG_CUDA(ctx, cudaMemcpy(st->d_hinv_shared, H.data(), sizeof(double) * n * n, cudaMemcpyHostToDevice));
-  WG_CUDA(ctx, cudaMemcpy(st->d_c_shared, Cs.data(), sizeof(double) * n * n, cudaMemcpyHostToDevice));
-  ctx->qld_shared_owner = nullptr;    // a generator that installs its own Hessian claims it after this call
+  WG_CUDA(ctx, cudaMemcpy(h.d_hinv, H.data(), sizeof(double) * n * n, cudaMemcpyHostToDevice));
+  WG_CUDA(ctx, cudaMemcpy(h.d_c, Cs.data(), sizeof(double) * n * n, cudaMemcpyHostToDevice));
+  h.boost = boost;
   return WG_OK;
+}
+
+extern "C" {
+
+int wg_qld_set_shared_hessian(wg_ctx *ctx, int n, int nmax, const double *C, double eps)
+{
+  return ctx ? install_shared_hessian(ctx, state_of(ctx)->caller, n, nmax, C, eps) : WG_ERR_INVALID;
+}
+
+int wgi_qld_set_generator_hessian(wg_ctx *ctx, int n, int nmax, const double *C, double eps)
+{
+  return ctx ? install_shared_hessian(ctx, state_of(ctx)->generator, n, nmax, C, eps) : WG_ERR_INVALID;
 }
 
 double wg_qld_diagonal_boost(int n, int nmax, const double *C, double eps)
@@ -815,11 +834,12 @@ double wg_qld_diagonal_boost(int n, int nmax, const double *C, double eps)
   return qld_diagonal_boost(n, nmax, C, eps);
 }
 
-double wg_qld_shared_boost(wg_ctx *ctx) { return ctx && ctx->qld ? static_cast<QldState *>(ctx->qld)->shared_boost : 0.0; }
+double wg_qld_shared_boost(wg_ctx *ctx) { return ctx && ctx->qld ? static_cast<QldState *>(ctx->qld)->caller.boost : 0.0; }
 
 struct RankedRows { const double *A0, *A1; const unsigned char *samp; long long row_stride; const double *uz; int N; };
 
-static int qld_solve_impl(wg_ctx *ctx, int mem, int B, const wg_qld_batch *q, const RankedRows *rk)
+// generator: shared_hessian = 1 means the generator's Hessian (wgi_qld_set_generator_hessian), not the caller's
+static int qld_solve_impl(wg_ctx *ctx, int mem, int B, const wg_qld_batch *q, const RankedRows *rk, bool generator)
 {
   if (!ctx || !q || B < 0) return WG_ERR_INVALID;
   if (B == 0) return WG_OK;
@@ -832,7 +852,8 @@ static int qld_solve_impl(wg_ctx *ctx, int mem, int B, const wg_qld_batch *q, co
     return WG_ERR_INVALID;
   wg_device_guard guard(ctx->device);
   QldState *st = state_of(ctx);
-  if (q->shared_hessian && (st->shared_n != n || !st->d_hinv_shared))
+  const SharedHessian &sh = generator ? st->generator : st->caller;
+  if (q->shared_hessian && (sh.n != n || !sh.d_hinv))
     return wg_fail(ctx, WG_ERR_NOT_READY, "wg_qld_set_shared_hessian not called for this n");
   const bool bounds = q->xl != nullptr;
   const size_t nb = (size_t)B;
@@ -895,8 +916,8 @@ static int qld_solve_impl(wg_ctx *ctx, int mem, int B, const wg_qld_batch *q, co
   a.d = d.d; a.A = d.A; a.a_stride = q->a_stride; a.b = d.b; a.b_stride = q->b_stride;
   a.xl = d.xl; a.xu = d.xu; a.x = d.x; a.u = d.u; a.u_stride = q->u_stride; a.ifail = d.ifail; a.iterations = d.iterations;
   if (q->shared_hessian) {
-    a.S = st->d_hinv_shared; a.h_stride = 0; a.hfail = nullptr;
-    a.C = st->d_c_shared; a.c_stride = 0;
+    a.S = sh.d_hinv; a.h_stride = 0; a.hfail = nullptr;
+    a.C = sh.d_c; a.c_stride = 0;
   } else {
     if ((rc = ensure(ctx, reinterpret_cast<void **>(&st->d_hinv), &st->cap_hinv, sizeof(double) * nb * n * n)) != WG_OK) return rc;
     if ((rc = ensure(ctx, reinterpret_cast<void **>(&st->d_fail), &st->cap_fail, sizeof(int) * nb)) != WG_OK) return rc;
@@ -906,7 +927,9 @@ static int qld_solve_impl(wg_ctx *ctx, int mem, int B, const wg_qld_batch *q, co
   }
   a.A0 = a.A1 = nullptr; a.samp = nullptr; a.row_stride = 0; a.uz = nullptr; a.N = 0;
   if (rk) { a.A0 = rk->A0; a.A1 = rk->A1; a.samp = rk->samp; a.row_stride = rk->row_stride; a.uz = rk->uz; a.N = rk->N; }
-  const size_t smem = qld_smem_bytes(n, std::max(mmax, rk ? (4 * rk->N + QW - 1) / QW : 0), a.qcap, bounds);
+  // the partial row sums are also the ranked kernel's 4N doubles of points, uz and row norms: the multipliers start after both
+  a.pstride = std::max(mmax, rk ? (4 * rk->N + QW - 1) / QW : 0);
+  const size_t smem = qld_smem_bytes(n, mmax, a.pstride, a.qcap, bounds);
   if (smem > 200 * 1024) return wg_fail(ctx, WG_ERR_INVALID, "wg_qld_solve_batch: problem too large for shared memory");
   if (rk) WG_SMEM_ATTR(ctx, WG_ATTR_DENSEQP_RANKED, qld_kernel<true>, smem);
   else WG_SMEM_ATTR(ctx, WG_ATTR_DENSEQP, qld_kernel<false>, smem);
@@ -930,13 +953,20 @@ static int qld_solve_impl(wg_ctx *ctx, int mem, int B, const wg_qld_batch *q, co
   return WG_OK;
 }
 
-int wg_qld_solve_batch(wg_ctx *ctx, int mem, int B, const wg_qld_batch *q) { return qld_solve_impl(ctx, mem, B, q, nullptr); }
+int wg_qld_solve_batch(wg_ctx *ctx, int mem, int B, const wg_qld_batch *q) { return qld_solve_impl(ctx, mem, B, q, nullptr, false); }
 
 int wg_qld_solve_batch_ranked(wg_ctx *ctx, int mem, int B, const wg_qld_batch *q, const double *A0, const double *A1,
                               const unsigned char *sample, long long row_stride, const double *uz_dev, int N)
 {
   RankedRows rk = {A0, A1, sample, row_stride, uz_dev, N};
-  return qld_solve_impl(ctx, mem, B, q, &rk);
+  return qld_solve_impl(ctx, mem, B, q, &rk, false);
+}
+
+int wgi_qld_solve_generator(wg_ctx *ctx, int B, const wg_qld_batch *q, const double *A0, const double *A1,
+                            const unsigned char *sample, long long row_stride, const double *uz_dev, int N)
+{
+  RankedRows rk = {A0, A1, sample, row_stride, uz_dev, N};
+  return qld_solve_impl(ctx, WG_MEM_DEVICE, B, q, A0 ? &rk : nullptr, true);
 }
 
 }  // extern "C"

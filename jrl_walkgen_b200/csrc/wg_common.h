@@ -56,7 +56,6 @@ struct wg_ctx {
   void *dimitrov = nullptr;
   // dense QP solver (qld.cu) and the Wieber2006 generator on top of it (wieber.cu)
   void *qld = nullptr;
-  const void *qld_shared_owner = nullptr;   // which generator's Hessian wg_qld_set_shared_hessian holds (nullptr: a caller's)
   void *wieber = nullptr;
 };
 
@@ -132,6 +131,12 @@ struct wgi_kajita_view {
 extern "C" int wgi_kajita_discretize_device(wg_ctx *ctx, wg_kajita_plan *pl, double **zmpref, wg_foot_sample **left,
                                             wg_foot_sample **right, int32_t **types, wgi_kajita_view *view);
 extern "C" const void *wgi_pldp_device_consts(wg_ctx *ctx);   // PldpConsts on the device, or nullptr
+// The dense QP solver with the Wieber2006 generator's own shared Hessian, kept apart from the one a caller installs with
+// wg_qld_set_shared_hessian.  wgi_qld_solve_generator: device memory; A0 = nullptr selects the dense rows of batch->A, else
+// the rank-structured rows of wg_qld_solve_batch_ranked.
+extern "C" int wgi_qld_set_generator_hessian(wg_ctx *ctx, int n, int nmax, const double *C, double eps);
+extern "C" int wgi_qld_solve_generator(wg_ctx *ctx, int B, const wg_qld_batch *q, const double *A0, const double *A1,
+                                       const unsigned char *sample, long long row_stride, const double *uz_dev, int N);
 
 struct wg_device_guard {
   int prev = -1;

@@ -356,8 +356,7 @@ int wg_wieber_set_params(wg_ctx *ctx, const wg_wieber_params *p)
   WbHost *H = wb_of(ctx);
   int rc = make_constants(*p, H, H->Ccm);
   if (rc != WG_OK) return rc;
-  if ((rc = wg_qld_set_shared_hessian(ctx, 2 * p->N, 2 * p->N, H->Ccm.data(), p->qld_eps)) != WG_OK) return rc;
-  ctx->qld_shared_owner = H;
+  if ((rc = wgi_qld_set_generator_hessian(ctx, 2 * p->N, 2 * p->N, H->Ccm.data(), p->qld_eps)) != WG_OK) return rc;
   H->par = *p;
   if (!H->d) WG_CUDA(ctx, cudaMalloc(&H->d, sizeof(WbConsts)));
   WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -389,12 +388,6 @@ int wg_wieber_run_batch(wg_ctx *ctx, wg_kajita_plan *plan, int mem, double *com_
   const bool host = mem == WG_MEM_HOST;
   const wg_wieber_params &par = H->par;
   const int N = par.N, nv = 2 * N, ld = 8 * N + 1;
-  // the shared Hessian of the dense solver may have been replaced by another caller of wg_qld_set_shared_hessian
-  if (ctx->qld_shared_owner != H) {
-    int rch = wg_qld_set_shared_hessian(ctx, nv, nv, H->Ccm.data(), H->par.qld_eps);
-    if (rch != WG_OK) return rch;
-    ctx->qld_shared_owner = H;
-  }
   // ---- GetZMPDiscretization (:1355-1364)
   double *d_zmp = host ? nullptr : zmp_out;
   wg_foot_sample *d_left = host ? nullptr : left, *d_right = host ? nullptr : right;
@@ -469,8 +462,7 @@ int wg_wieber_run_batch(wg_ctx *ctx, wg_kajita_plan *plan, int mem, double *com_
                                                      d_zmp, d_walks, d_m, d_Px, d_Pu, d_D, d_A0, d_A1, d_samp);
     wg_prof_stop(ctx);
     WG_LAUNCHED(ctx);
-    if (dense) rc = wg_qld_solve_batch(ctx, WG_MEM_DEVICE, B, &q);
-    else rc = wg_qld_solve_batch_ranked(ctx, WG_MEM_DEVICE, B, &q, d_A0, d_A1, d_samp, ld, d_uz, N);
+    rc = wgi_qld_solve_generator(ctx, B, &q, d_A0, d_A1, d_samp, ld, d_uz, N);     // d_A0 = nullptr in dense mode
     if (rc != WG_OK) return rc;
     wg_prof_start(ctx, WG_K_WIEBER);
     wieber_post_kernel<<<grid, WB_T, 0, ctx->stream>>>(B, H->d, V.d_samp_off, d_m, d_Px, d_Pu, d_X, d_ifail, d_it, d_walks,
