@@ -1067,7 +1067,7 @@ static int mpc_launch(wg_ctx *ctx, MpcState *m, int B, int nsteps, wg_herdt_mpc_
   static const int split = getenv("WG_HERDT_MPC_SPLIT") ? atoi(getenv("WG_HERDT_MPC_SPLIT")) : 1;
   if (split) return mpc_launch_split(ctx, m, B, nsteps, states, vel_ref, ticks, steps, qp_in);
   const size_t smem = (sizeof(herdt::Work) + sizeof(MpcWarp) + sizeof(double) * herdt::TRI) * MPC_WARPS;
-  WG_SMEM_ATTR(ctx, WG_ATTR_HERDT_MPC, herdt_mpc_kernel, smem);
+  WG_SMEM_ATTR(ctx, herdt_mpc_kernel, smem);
   int per_sm = (int)((227 * 1024) / (smem + 1024));
   if (per_sm < 1) per_sm = 1;
   int blocks = (B + MPC_WARPS - 1) / MPC_WARPS;

@@ -247,7 +247,7 @@ static int herdt_launch(wg_ctx *ctx, HerdtState *st, int B, const wg_herdt_qp_in
                         const herdt::LaunchOpts &opt = herdt::LaunchOpts())
 {
   const size_t smem = sizeof(herdt::Work) * QP_WARPS;
-  WG_SMEM_ATTR(ctx, WG_ATTR_HERDT_QP, herdt_qp_kernel, smem);
+  WG_SMEM_ATTR(ctx, herdt_qp_kernel, smem);
   int per_sm = (int)((227 * 1024) / (smem + 1024));
   if (per_sm < 1) per_sm = 1;
   int blocks = (B + QP_WARPS - 1) / QP_WARPS;

@@ -364,7 +364,7 @@ static int pldp_solve_impl(wg_ctx *ctx, int mem, int B, const wg_pldp_batch *pb,
     int a_cap = (stage && !ranked) ? (int)((pb->dpu_stride + 1) & ~1LL) : 0;
     size_t smem = sizeof(double) * (size_t)a_cap * PLDP_WARPS;
     if (smem > 190 * 1024) { a_cap = 0; smem = 0; }
-    WG_SMEM_ATTR(ctx, WG_ATTR_PLDP, pldp_kernel<false>, smem);
+    WG_SMEM_ATTR(ctx, pldp_kernel<false>, smem);
     const int per_sm = smem ? (int)((227 * 1024) / (smem + (sizeof(PldpWarp) + 1100) * PLDP_WARPS + 1024)) : (ranked ? 4 : 8);
     if (grid > ctx->sm_count * (per_sm > 0 ? per_sm : 1)) grid = ctx->sm_count * (per_sm > 0 ? per_sm : 1);
     if (!p->d_next) WG_CUDA(ctx, cudaMalloc(&p->d_next, sizeof(int)));

@@ -35,6 +35,7 @@
 #include <vector>
 #include <cmath>
 #include <algorithm>
+#include <type_traits>
 
 // ---------------------------------------------------------------------------------------------
 // Host: gains by structure-preserving doubling (SDA) for the DARE
@@ -392,13 +393,169 @@ __device__ __forceinline__ double preview_tick(Axis &a, double f, double pk)
   return z;
 }
 
-__device__ __forceinline__ void scan_combine(Axis &c, const double *__restrict__ P, double n0, double n1, double n2,
-                                             double n3)
+__device__ __forceinline__ Axis axis_zero()
 {
-  c.x0 = fma(P[0], n0, fma(P[1], n1, fma(P[2], n2, fma(P[3], n3, c.x0))));
-  c.x1 = fma(P[4], n0, fma(P[5], n1, fma(P[6], n2, fma(P[7], n3, c.x1))));
-  c.x2 = fma(P[8], n0, fma(P[9], n1, fma(P[10], n2, fma(P[11], n3, c.x2))));
-  c.s = fma(P[12], n0, fma(P[13], n1, fma(P[14], n2, fma(P[15], n3, c.s))));
+  Axis a;
+  a.x0 = a.x1 = a.x2 = a.s = 0.0;
+  return a;
+}
+__device__ __forceinline__ void operator+=(Axis &a, const Axis &b)
+{
+  a.x0 += b.x0; a.x1 += b.x1; a.x2 += b.x2; a.s += b.s;
+}
+// c += g a, component by component
+__device__ __forceinline__ void axpy(Axis &c, const double *g, double a)
+{
+  c.x0 = fma(g[0], a, c.x0); c.x1 = fma(g[1], a, c.x1);
+  c.x2 = fma(g[2], a, c.x2); c.s = fma(g[3], a, c.s);
+}
+__device__ __forceinline__ Axis shfl_up(const Axis &a, int d)
+{
+  Axis r;
+  r.x0 = __shfl_up_sync(0xffffffffu, a.x0, d); r.x1 = __shfl_up_sync(0xffffffffu, a.x1, d);
+  r.x2 = __shfl_up_sync(0xffffffffu, a.x2, d); r.s = __shfl_up_sync(0xffffffffu, a.s, d);
+  return r;
+}
+__device__ __forceinline__ Axis shfl_down(const Axis &a, int d)
+{
+  Axis r;
+  r.x0 = __shfl_down_sync(0xffffffffu, a.x0, d); r.x1 = __shfl_down_sync(0xffffffffu, a.x1, d);
+  r.x2 = __shfl_down_sync(0xffffffffu, a.x2, d); r.s = __shfl_down_sync(0xffffffffu, a.s, d);
+  return r;
+}
+// The two records of 8 doubles: a walk's state {x,dx,ddx,y,dy,ddy,sx,sy} (state arrays, s_carry) and a scan total
+// {x axis, y axis} (s_tot, s_totb, s_halo).
+__device__ __forceinline__ void load_state(const double *q, Axis &x, Axis &y)
+{
+  x.x0 = q[0]; x.x1 = q[1]; x.x2 = q[2]; x.s = q[6];
+  y.x0 = q[3]; y.x1 = q[4]; y.x2 = q[5]; y.s = q[7];
+}
+__device__ __forceinline__ void store_state(double *q, const Axis &x, const Axis &y)
+{
+  q[0] = x.x0; q[1] = x.x1; q[2] = x.x2; q[6] = x.s;
+  q[3] = y.x0; q[4] = y.x1; q[5] = y.x2; q[7] = y.s;
+}
+__device__ __forceinline__ void load_pair(const double *q, Axis &x, Axis &y)
+{
+  x.x0 = q[0]; x.x1 = q[1]; x.x2 = q[2]; x.s = q[3];
+  y.x0 = q[4]; y.x1 = q[5]; y.x2 = q[6]; y.s = q[7];
+}
+__device__ __forceinline__ void store_pair(double *q, const Axis &x, const Axis &y)
+{
+  q[0] = x.x0; q[1] = x.x1; q[2] = x.x2; q[3] = x.s;
+  q[4] = y.x0; q[5] = y.x1; q[6] = y.x2; q[7] = y.s;
+}
+
+// c += P n, P a row-major 4 x 4 matrix
+__device__ __forceinline__ void scan_combine(Axis &c, const double *__restrict__ P, const Axis &n)
+{
+  c.x0 = fma(P[0], n.x0, fma(P[1], n.x1, fma(P[2], n.x2, fma(P[3], n.s, c.x0))));
+  c.x1 = fma(P[4], n.x0, fma(P[5], n.x1, fma(P[6], n.x2, fma(P[7], n.s, c.x1))));
+  c.x2 = fma(P[8], n.x0, fma(P[9], n.x1, fma(P[10], n.x2, fma(P[11], n.s, c.x2))));
+  c.s = fma(P[12], n.x0, fma(P[13], n.x1, fma(P[14], n.x2, fma(P[15], n.s, c.s))));
+}
+
+// ---- Phases shared by the kernels below (the phase numbers are those of their comments).
+// (2a) local aggregate: the cart-table state after a thread's FIR_R ticks started from zero, as the linear map of its inputs
+// (preview sums ax / ay, ZMP reference pk); the thread that owns the tile's first tick (carry_in) adds M^8 x the carried state,
+// which it also returns in (inx, iny).
+template <bool SIM>
+__device__ __forceinline__ void local_aggregate(const double *ax, const double *ay, const double2 *pk, bool carry_in,
+                                                const double *s_carry, const double (*Pm)[16], Axis &cx, Axis &cy,
+                                                Axis &inx, Axis &iny)
+{
+  cx = axis_zero(); cy = axis_zero();
+  inx = cx; iny = cy;
+  const double(*Gm)[4] = c_pc.G[SIM ? 1 : 0];
+  const double(*Hm)[4] = c_pc.H[SIM ? 1 : 0];
+#pragma unroll
+  for (int r = 0; r < FIR_R; ++r) {
+    axpy(cx, Gm[r], ax[r]);
+    axpy(cy, Gm[r], ay[r]);
+    if (SIM) {
+      axpy(cx, Hm[r], pk[r].x);
+      axpy(cy, Hm[r], pk[r].y);
+    }
+  }
+  if (carry_in) {
+    load_state(s_carry, inx, iny);
+    scan_combine(cx, Pm[0], inx);
+    scan_combine(cy, Pm[0], iny);
+  }
+}
+
+// (2b) Kogge-Stone scan UP the lanes of a warp: c_t += M^(8d) c_{t-d}
+__device__ __forceinline__ void scan_up(Axis &cx, Axis &cy, int lane, const double (*Pm)[16])
+{
+#pragma unroll
+  for (int l = 0; l < 5; ++l) {
+    const int d = 1 << l;
+    const Axis a = shfl_up(cx, d), b = shfl_up(cy, d);
+    if (lane >= d) {
+      scan_combine(cx, Pm[l], a);
+      scan_combine(cy, Pm[l], b);
+    }
+  }
+}
+
+// (1b) local pass: ax[r], ay[r] = the part of f of tick 8t + r that comes from this thread's own 8 samples and their partners NL
+// further on; (bx, by) = the thread's total, W at tick 8t for a zero state at tick 8t + 8; pk = the thread's own ZMP reference
+// (the `ZMPPositions[lindex]` of the integrator).  The ring of samples has CAP slots; the kernel's slot mapping comes in as
+// own(j) = sample j of the thread (slot own0 + j) and ring(i) = the sample in slot i.
+template <bool SIM, class Own, class Ring>
+__device__ __forceinline__ void local_pass(Own own, Ring ring, int own0, int NL, int CAP, double *ax, double *ay, double2 *pk,
+                                           Axis &bx, Axis &by)
+{
+  bx = axis_zero();
+  by = bx;
+#pragma unroll
+  for (int r = 0; r < FIR_R; ++r) { ax[r] = 0.0; ay[r] = 0.0; }
+#pragma unroll
+  for (int j = 0; j < FIR_R; ++j) {
+    const double2 a = own(j);
+    int fi = own0 + j + NL;
+    if (fi >= CAP) fi -= CAP;
+    const double2 f = ring(fi);
+    pk[j] = SIM ? a : make_double2(0.0, 0.0);
+#pragma unroll
+    for (int r = 0; r <= j; ++r) {
+      ax[r] = fma(c_pc.RF0[j - r], a.x, ax[r]); ax[r] = fma(c_pc.RFN[j - r], f.x, ax[r]);
+      ay[r] = fma(c_pc.RF0[j - r], a.y, ay[r]); ay[r] = fma(c_pc.RFN[j - r], f.y, ay[r]);
+    }
+    bx.x0 = fma(c_pc.RV[j][0], a.x, bx.x0); bx.x0 = fma(c_pc.RVN[j][0], f.x, bx.x0);
+    bx.x1 = fma(c_pc.RV[j][1], a.x, bx.x1); bx.x1 = fma(c_pc.RVN[j][1], f.x, bx.x1);
+    bx.x2 = fma(c_pc.RV[j][2], a.x, bx.x2); bx.x2 = fma(c_pc.RVN[j][2], f.x, bx.x2);
+    bx.s = fma(c_pc.RV[j][3], a.x, bx.s); bx.s = fma(c_pc.RVN[j][3], f.x, bx.s);
+    by.x0 = fma(c_pc.RV[j][0], a.y, by.x0); by.x0 = fma(c_pc.RVN[j][0], f.y, by.x0);
+    by.x1 = fma(c_pc.RV[j][1], a.y, by.x1); by.x1 = fma(c_pc.RVN[j][1], f.y, by.x1);
+    by.x2 = fma(c_pc.RV[j][2], a.y, by.x2); by.x2 = fma(c_pc.RVN[j][2], f.y, by.x2);
+    by.s = fma(c_pc.RV[j][3], a.y, by.s); by.s = fma(c_pc.RVN[j][3], f.y, by.s);
+  }
+}
+
+// (1c) Kogge-Stone scan DOWN the lanes of a warp: c_t += L^(8d) c_{t+d}
+__device__ __forceinline__ void scan_down(Axis &bx, Axis &by, int lane)
+{
+#pragma unroll
+  for (int l = 0; l < 5; ++l) {
+    const int d = 1 << l;
+    const Axis a = shfl_down(bx, d), b = shfl_down(by, d);
+    if (lane + d < 32) {
+      scan_combine(bx, c_pc.RP[l], a);
+      scan_combine(by, c_pc.RP[l], b);
+    }
+  }
+}
+
+// (1d) f of tick r += (w' L^(8 - r)) . W_in, W_in = (ix, iy) the true W at the thread's end
+__device__ __forceinline__ void add_window(double *ax, double *ay, const Axis &ix, const Axis &iy)
+{
+#pragma unroll
+  for (int r = 0; r < FIR_R; ++r) {
+    const double *g = c_pc.RW[FIR_R - r];
+    ax[r] = fma(g[0], ix.x0, fma(g[1], ix.x1, fma(g[2], ix.x2, fma(g[3], ix.s, ax[r]))));
+    ay[r] = fma(g[0], iy.x0, fma(g[1], iy.x1, fma(g[2], iy.x2, fma(g[3], iy.s, ay[r]))));
+  }
 }
 
 // ADD: second stage of ZMPPreviewControlWithMultiBodyZMP (SecondStageOfControl, ZMPPreviewControlWithMultiBodyZMP.cpp:317-376):
@@ -474,53 +631,10 @@ preview_fused_kernel(const int *__restrict__ order, const int64_t *__restrict__ 
     // ---- (2a) local aggregate: state after this thread's 8 ticks started from zero, as the linear map of its
     //      inputs (thread 0 adds M^8 x the carried state)
     Axis cx, cy, inx, iny;
-    cx.x0 = cx.x1 = cx.x2 = cx.s = 0.0;
-    cy.x0 = cy.x1 = cy.x2 = cy.s = 0.0;
-    inx = cx; iny = cy;
-    {
-      const double(*Gm)[4] = c_pc.G[SIM ? 1 : 0];
-      const double(*Hm)[4] = c_pc.H[SIM ? 1 : 0];
-#pragma unroll
-      for (int r = 0; r < FIR_R; ++r) {
-        cx.x0 = fma(Gm[r][0], ax[r], cx.x0); cx.x1 = fma(Gm[r][1], ax[r], cx.x1);
-        cx.x2 = fma(Gm[r][2], ax[r], cx.x2); cx.s = fma(Gm[r][3], ax[r], cx.s);
-        cy.x0 = fma(Gm[r][0], ay[r], cy.x0); cy.x1 = fma(Gm[r][1], ay[r], cy.x1);
-        cy.x2 = fma(Gm[r][2], ay[r], cy.x2); cy.s = fma(Gm[r][3], ay[r], cy.s);
-        if (SIM) {
-          cx.x0 = fma(Hm[r][0], pk[r].x, cx.x0); cx.x1 = fma(Hm[r][1], pk[r].x, cx.x1);
-          cx.x2 = fma(Hm[r][2], pk[r].x, cx.x2); cx.s = fma(Hm[r][3], pk[r].x, cx.s);
-          cy.x0 = fma(Hm[r][0], pk[r].y, cy.x0); cy.x1 = fma(Hm[r][1], pk[r].y, cy.x1);
-          cy.x2 = fma(Hm[r][2], pk[r].y, cy.x2); cy.s = fma(Hm[r][3], pk[r].y, cy.s);
-        }
-      }
-      if (t == 0) {
-        inx.x0 = s_carry[0]; inx.x1 = s_carry[1]; inx.x2 = s_carry[2]; inx.s = s_carry[6];
-        iny.x0 = s_carry[3]; iny.x1 = s_carry[4]; iny.x2 = s_carry[5]; iny.s = s_carry[7];
-        scan_combine(cx, Pm[0], inx.x0, inx.x1, inx.x2, inx.s);
-        scan_combine(cy, Pm[0], iny.x0, iny.x1, iny.x2, iny.s);
-      }
-    }
+    local_aggregate<SIM>(ax, ay, pk, t == 0, s_carry, Pm, cx, cy, inx, iny);
     // ---- (2b) Kogge-Stone scan over threads: c_t += M^(8d) c_{t-d}
-#pragma unroll
-    for (int l = 0; l < 5; ++l) {
-      const int d = 1 << l;
-      const double a0 = __shfl_up_sync(0xffffffffu, cx.x0, d), a1 = __shfl_up_sync(0xffffffffu, cx.x1, d);
-      const double a2 = __shfl_up_sync(0xffffffffu, cx.x2, d), a3 = __shfl_up_sync(0xffffffffu, cx.s, d);
-      const double b0 = __shfl_up_sync(0xffffffffu, cy.x0, d), b1 = __shfl_up_sync(0xffffffffu, cy.x1, d);
-      const double b2 = __shfl_up_sync(0xffffffffu, cy.x2, d), b3 = __shfl_up_sync(0xffffffffu, cy.s, d);
-      if (lane >= d) {
-        scan_combine(cx, Pm[l], a0, a1, a2, a3);
-        scan_combine(cy, Pm[l], b0, b1, b2, b3);
-      }
-    }
-    // The shuffle levels give a scan segmented per warp.  Carry across warps: T_w = total of warp w (lane 31),
-    // state entering warp w: W_w = M^256 W_{w-1} + T_{w-1}, W_0 = 0 (the carried tile state is inside thread 0's
-    // local pass); lane j then adds M^(8 (j+1)) W_w, built from the bits of j+1 with the same constant matrices.
-    if (lane == 31) {
-      double *n = s_tot[t >> 5];
-      n[0] = cx.x0; n[1] = cx.x1; n[2] = cx.x2; n[3] = cx.s;
-      n[4] = cy.x0; n[5] = cy.x1; n[6] = cy.x2; n[7] = cy.s;
-    }
+    scan_up(cx, cy, lane, Pm);
+    if (lane == 31) store_pair(s_tot[t >> 5], cx, cy);
     __syncthreads();
     // ---- (2c) true start state of this thread = inclusive result of thread t-1
     Axis sx, sy;
@@ -534,8 +648,8 @@ preview_fused_kernel(const int *__restrict__ order, const int64_t *__restrict__ 
         Axis nx, ny;
         nx.x0 = n[0]; nx.x1 = n[1]; nx.x2 = n[2]; nx.s = n[3];
         ny.x0 = n[4]; ny.x1 = n[5]; ny.x2 = n[6]; ny.s = n[7];
-        scan_combine(nx, Pm[5], vx.x0, vx.x1, vx.x2, vx.s);
-        scan_combine(ny, Pm[5], vy.x0, vy.x1, vy.x2, vy.s);
+        scan_combine(nx, Pm[5], vx);
+        scan_combine(ny, Pm[5], vy);
         vx = nx; vy = ny;
       }
       const Axis wx_in = vx, wy_in = vy;
@@ -546,8 +660,8 @@ preview_fused_kernel(const int *__restrict__ order, const int64_t *__restrict__ 
             Axis zx, zy;
             zx.x0 = zx.x1 = zx.x2 = zx.s = 0.0;
             zy.x0 = zy.x1 = zy.x2 = zy.s = 0.0;
-            scan_combine(zx, Pm[l], vx.x0, vx.x1, vx.x2, vx.s);
-            scan_combine(zy, Pm[l], vy.x0, vy.x1, vy.x2, vy.s);
+            scan_combine(zx, Pm[l], vx);
+            scan_combine(zy, Pm[l], vy);
             vx = zx; vy = zy;
           }
         }
@@ -618,10 +732,7 @@ preview_fused_kernel(const int *__restrict__ order, const int64_t *__restrict__ 
         __syncwarp();
       }
     }
-    if (k0 <= last && last < k0 + FIR_R) {   // the thread that ran the tile's last valid tick carries the state
-      s_carry[0] = sx.x0; s_carry[1] = sx.x1; s_carry[2] = sx.x2; s_carry[6] = sx.s;
-      s_carry[3] = sy.x0; s_carry[4] = sy.x1; s_carry[5] = sy.x2; s_carry[7] = sy.s;
-    }
+    if (k0 <= last && last < k0 + FIR_R) store_state(s_carry, sx, sy);   // the thread that ran the tile's last valid tick carries the state
   }
   __syncthreads();
   if (t < 8) state[8 * (size_t)b + t] = s_carry[t];
@@ -763,57 +874,15 @@ preview_rec_kernel(const int *__restrict__ order, const int64_t *__restrict__ of
       if ((lane & 3) == 0) s_halo[w][((lane & 16) ? 4 : 0) + ((lane & 8) ? 2 : 0) + ((lane & 4) ? 1 : 0)] = k1;
     }
 
-    // ---- (1b) local pass: ax[r], ay[r] = the part of f of tick 8t + r that comes from this thread's own 8 samples and
-    //      their partners NL further on; (bx, by) = the thread's total, W at tick 8t for a zero state at tick 8t + 8
+    // ---- (1b) local pass
     double ax[FIR_R], ay[FIR_R];
-    double2 pk[FIR_R];                          // the thread's own ZMP reference (the `ZMPPositions[lindex]` of the integrator)
+    double2 pk[FIR_R];
     Axis bx, by;
-    bx.x0 = bx.x1 = bx.x2 = bx.s = 0.0;
-    by = bx;
-    {
-      const double2 *own = sp + pad9(own0);
-#pragma unroll
-      for (int r = 0; r < FIR_R; ++r) { ax[r] = 0.0; ay[r] = 0.0; }
-#pragma unroll
-      for (int j = 0; j < FIR_R; ++j) {
-        const double2 a = own[j];
-        int fi = own0 + j + NL;
-        if (fi >= CAP) fi -= CAP;
-        const double2 f = sp[pad9(fi)];
-        pk[j] = SIM ? a : make_double2(0.0, 0.0);
-#pragma unroll
-        for (int r = 0; r <= j; ++r) {
-          ax[r] = fma(c_pc.RF0[j - r], a.x, ax[r]); ax[r] = fma(c_pc.RFN[j - r], f.x, ax[r]);
-          ay[r] = fma(c_pc.RF0[j - r], a.y, ay[r]); ay[r] = fma(c_pc.RFN[j - r], f.y, ay[r]);
-        }
-        bx.x0 = fma(c_pc.RV[j][0], a.x, bx.x0); bx.x0 = fma(c_pc.RVN[j][0], f.x, bx.x0);
-        bx.x1 = fma(c_pc.RV[j][1], a.x, bx.x1); bx.x1 = fma(c_pc.RVN[j][1], f.x, bx.x1);
-        bx.x2 = fma(c_pc.RV[j][2], a.x, bx.x2); bx.x2 = fma(c_pc.RVN[j][2], f.x, bx.x2);
-        bx.s = fma(c_pc.RV[j][3], a.x, bx.s); bx.s = fma(c_pc.RVN[j][3], f.x, bx.s);
-        by.x0 = fma(c_pc.RV[j][0], a.y, by.x0); by.x0 = fma(c_pc.RVN[j][0], f.y, by.x0);
-        by.x1 = fma(c_pc.RV[j][1], a.y, by.x1); by.x1 = fma(c_pc.RVN[j][1], f.y, by.x1);
-        by.x2 = fma(c_pc.RV[j][2], a.y, by.x2); by.x2 = fma(c_pc.RVN[j][2], f.y, by.x2);
-        by.s = fma(c_pc.RV[j][3], a.y, by.s); by.s = fma(c_pc.RVN[j][3], f.y, by.s);
-      }
-    }
-    // ---- (1c) Kogge-Stone scan DOWN the tile: c_t += L^(8d) c_{t+d} (segmented per warp)
-#pragma unroll
-    for (int l = 0; l < 5; ++l) {
-      const int d = 1 << l;
-      const double a0 = __shfl_down_sync(FULL, bx.x0, d), a1 = __shfl_down_sync(FULL, bx.x1, d);
-      const double a2 = __shfl_down_sync(FULL, bx.x2, d), a3 = __shfl_down_sync(FULL, bx.s, d);
-      const double b0 = __shfl_down_sync(FULL, by.x0, d), b1 = __shfl_down_sync(FULL, by.x1, d);
-      const double b2 = __shfl_down_sync(FULL, by.x2, d), b3 = __shfl_down_sync(FULL, by.s, d);
-      if (lane + d < 32) {
-        scan_combine(bx, c_pc.RP[l], a0, a1, a2, a3);
-        scan_combine(by, c_pc.RP[l], b0, b1, b2, b3);
-      }
-    }
-    if (lane == 0) {
-      double *n = s_totb[w];
-      n[0] = bx.x0; n[1] = bx.x1; n[2] = bx.x2; n[3] = bx.s;
-      n[4] = by.x0; n[5] = by.x1; n[6] = by.x2; n[7] = by.s;
-    }
+    const double2 *own = sp + pad9(own0);
+    local_pass<SIM>([&](int j) { return own[j]; }, [&](int i) { return sp[pad9(i)]; }, own0, NL, CAP, ax, ay, pk, bx, by);
+    // ---- (1c) Kogge-Stone scan DOWN the tile (segmented per warp)
+    scan_down(bx, by, lane);
+    if (lane == 0) store_pair(s_totb[w], bx, by);
     __syncthreads();      // every read of the tile buffer is done: it becomes the store staging area below
     {
       // state entering this warp from above: V_(NW-1) = W at the tile's end, V_(u-1) = T_u + L^256 V_u
@@ -830,8 +899,8 @@ preview_rec_kernel(const int *__restrict__ order, const int64_t *__restrict__ of
         Axis nx, ny;
         nx.x0 = n[0]; nx.x1 = n[1]; nx.x2 = n[2]; nx.s = n[3];
         ny.x0 = n[4]; ny.x1 = n[5]; ny.x2 = n[6]; ny.s = n[7];
-        scan_combine(nx, c_pc.RP[5], vx.x0, vx.x1, vx.x2, vx.s);
-        scan_combine(ny, c_pc.RP[5], vy.x0, vy.x1, vy.x2, vy.s);
+        scan_combine(nx, c_pc.RP[5], vx);
+        scan_combine(ny, c_pc.RP[5], vy);
         vx = nx; vy = ny;
       }
       // true W at this thread's end (tick 8t + 8) = inclusive result of lane + 1 (nothing for lane 31) + (L^8)^(31-lane) V
@@ -846,64 +915,19 @@ preview_rec_kernel(const int *__restrict__ order, const int64_t *__restrict__ of
         double Pl[16];
 #pragma unroll
         for (int e = 0; e < 8; ++e) { const double2 q = __ldg(lp + e); Pl[2 * e] = q.x; Pl[2 * e + 1] = q.y; }
-        scan_combine(ix, Pl, vx.x0, vx.x1, vx.x2, vx.s);
-        scan_combine(iy, Pl, vy.x0, vy.x1, vy.x2, vy.s);
+        scan_combine(ix, Pl, vx);
+        scan_combine(iy, Pl, vy);
       }
-      // ---- (1d) f of tick r += (w' L^(8 - r)) . W_in
-#pragma unroll
-      for (int r = 0; r < FIR_R; ++r) {
-        const double *g = c_pc.RW[FIR_R - r];
-        ax[r] = fma(g[0], ix.x0, fma(g[1], ix.x1, fma(g[2], ix.x2, fma(g[3], ix.s, ax[r]))));
-        ay[r] = fma(g[0], iy.x0, fma(g[1], iy.x1, fma(g[2], iy.x2, fma(g[3], iy.s, ay[r]))));
-      }
+      // ---- (1d)
+      add_window(ax, ay, ix, iy);
     }
 
     // ---- (2a) local aggregate of the cart-table recursion (as preview_fused_kernel)
     Axis cx, cy, inx, iny;
-    cx.x0 = cx.x1 = cx.x2 = cx.s = 0.0;
-    cy.x0 = cy.x1 = cy.x2 = cy.s = 0.0;
-    inx = cx; iny = cy;
-    {
-      const double(*Gm)[4] = c_pc.G[SIM ? 1 : 0];
-      const double(*Hm)[4] = c_pc.H[SIM ? 1 : 0];
-#pragma unroll
-      for (int r = 0; r < FIR_R; ++r) {
-        cx.x0 = fma(Gm[r][0], ax[r], cx.x0); cx.x1 = fma(Gm[r][1], ax[r], cx.x1);
-        cx.x2 = fma(Gm[r][2], ax[r], cx.x2); cx.s = fma(Gm[r][3], ax[r], cx.s);
-        cy.x0 = fma(Gm[r][0], ay[r], cy.x0); cy.x1 = fma(Gm[r][1], ay[r], cy.x1);
-        cy.x2 = fma(Gm[r][2], ay[r], cy.x2); cy.s = fma(Gm[r][3], ay[r], cy.s);
-        if (SIM) {
-          cx.x0 = fma(Hm[r][0], pk[r].x, cx.x0); cx.x1 = fma(Hm[r][1], pk[r].x, cx.x1);
-          cx.x2 = fma(Hm[r][2], pk[r].x, cx.x2); cx.s = fma(Hm[r][3], pk[r].x, cx.s);
-          cy.x0 = fma(Hm[r][0], pk[r].y, cy.x0); cy.x1 = fma(Hm[r][1], pk[r].y, cy.x1);
-          cy.x2 = fma(Hm[r][2], pk[r].y, cy.x2); cy.s = fma(Hm[r][3], pk[r].y, cy.s);
-        }
-      }
-      if (t == 0) {
-        inx.x0 = s_carry[0]; inx.x1 = s_carry[1]; inx.x2 = s_carry[2]; inx.s = s_carry[6];
-        iny.x0 = s_carry[3]; iny.x1 = s_carry[4]; iny.x2 = s_carry[5]; iny.s = s_carry[7];
-        scan_combine(cx, Pm[0], inx.x0, inx.x1, inx.x2, inx.s);
-        scan_combine(cy, Pm[0], iny.x0, iny.x1, iny.x2, iny.s);
-      }
-    }
-    // ---- (2b) Kogge-Stone scan UP the tile: c_t += M^(8d) c_{t-d}
-#pragma unroll
-    for (int l = 0; l < 5; ++l) {
-      const int d = 1 << l;
-      const double a0 = __shfl_up_sync(FULL, cx.x0, d), a1 = __shfl_up_sync(FULL, cx.x1, d);
-      const double a2 = __shfl_up_sync(FULL, cx.x2, d), a3 = __shfl_up_sync(FULL, cx.s, d);
-      const double b0 = __shfl_up_sync(FULL, cy.x0, d), b1 = __shfl_up_sync(FULL, cy.x1, d);
-      const double b2 = __shfl_up_sync(FULL, cy.x2, d), b3 = __shfl_up_sync(FULL, cy.s, d);
-      if (lane >= d) {
-        scan_combine(cx, Pm[l], a0, a1, a2, a3);
-        scan_combine(cy, Pm[l], b0, b1, b2, b3);
-      }
-    }
-    if (lane == 31) {
-      double *n = s_tot[w];
-      n[0] = cx.x0; n[1] = cx.x1; n[2] = cx.x2; n[3] = cx.s;
-      n[4] = cy.x0; n[5] = cy.x1; n[6] = cy.x2; n[7] = cy.s;
-    }
+    local_aggregate<SIM>(ax, ay, pk, t == 0, s_carry, Pm, cx, cy, inx, iny);
+    // ---- (2b) Kogge-Stone scan UP the tile
+    scan_up(cx, cy, lane, Pm);
+    if (lane == 31) store_pair(s_tot[w], cx, cy);
     __syncthreads();
     // ---- (2c) true start state of this thread = inclusive result of thread t-1
     Axis sx, sy;
@@ -916,8 +940,8 @@ preview_rec_kernel(const int *__restrict__ order, const int64_t *__restrict__ of
         Axis nx, ny;
         nx.x0 = n[0]; nx.x1 = n[1]; nx.x2 = n[2]; nx.s = n[3];
         ny.x0 = n[4]; ny.x1 = n[5]; ny.x2 = n[6]; ny.s = n[7];
-        scan_combine(nx, Pm[5], vx.x0, vx.x1, vx.x2, vx.s);
-        scan_combine(ny, Pm[5], vy.x0, vy.x1, vy.x2, vy.s);
+        scan_combine(nx, Pm[5], vx);
+        scan_combine(ny, Pm[5], vy);
         vx = nx; vy = ny;
       }
       const Axis wx_in = vx, wy_in = vy;
@@ -928,26 +952,24 @@ preview_rec_kernel(const int *__restrict__ order, const int64_t *__restrict__ of
             Axis zx, zy;
             zx.x0 = zx.x1 = zx.x2 = zx.s = 0.0;
             zy.x0 = zy.x1 = zy.x2 = zy.s = 0.0;
-            scan_combine(zx, Pm[l], vx.x0, vx.x1, vx.x2, vx.s);
-            scan_combine(zy, Pm[l], vy.x0, vy.x1, vy.x2, vy.s);
+            scan_combine(zx, Pm[l], vx);
+            scan_combine(zy, Pm[l], vy);
             vx = zx; vy = zy;
           }
         }
         cx.x0 += vx.x0; cx.x1 += vx.x1; cx.x2 += vx.x2; cx.s += vx.s;
         cy.x0 += vy.x0; cy.x1 += vy.x1; cy.x2 += vy.x2; cy.s += vy.s;
       }
-      sx.x0 = __shfl_up_sync(FULL, cx.x0, 1); sx.x1 = __shfl_up_sync(FULL, cx.x1, 1);
-      sx.x2 = __shfl_up_sync(FULL, cx.x2, 1); sx.s = __shfl_up_sync(FULL, cx.s, 1);
-      sy.x0 = __shfl_up_sync(FULL, cy.x0, 1); sy.x1 = __shfl_up_sync(FULL, cy.x1, 1);
-      sy.x2 = __shfl_up_sync(FULL, cy.x2, 1); sy.s = __shfl_up_sync(FULL, cy.s, 1);
+      sx.x0 = __shfl_up_sync(0xffffffffu, cx.x0, 1); sx.x1 = __shfl_up_sync(0xffffffffu, cx.x1, 1);
+      sx.x2 = __shfl_up_sync(0xffffffffu, cx.x2, 1); sx.s = __shfl_up_sync(0xffffffffu, cx.s, 1);
+      sy.x0 = __shfl_up_sync(0xffffffffu, cy.x0, 1); sy.x1 = __shfl_up_sync(0xffffffffu, cy.x1, 1);
+      sy.x2 = __shfl_up_sync(0xffffffffu, cy.x2, 1); sy.s = __shfl_up_sync(0xffffffffu, cy.s, 1);
       if (lane == 0) {
         if (w == 0) { sx = inx; sy = iny; }
         else { sx = wx_in; sy = wy_in; }
       }
     }
-    // ---- (2d) final pass.  Every thread stores its own rows straight from registers: two ticks are 96 B of CoM and 32 B of
-    //      ZMP, i.e. four whole 32-byte sectors, written with 256-bit stores (STG.256) when the rows of this trajectory start
-    //      on a 32-byte boundary and with 128-bit stores otherwise; no staging, no index arithmetic per store.
+    // ---- (2d) final pass, rows stored straight from registers
     const int k0 = start + FIR_R * t;
     const int last = min(start + FIR_TILE, nsteps) - 1;   // last valid tick of this tile
     {
@@ -999,10 +1021,7 @@ preview_rec_kernel(const int *__restrict__ order, const int64_t *__restrict__ of
         }
       }
     }
-    if (k0 <= last && last < k0 + FIR_R) {   // the thread that ran the tile's last valid tick carries the state
-      s_carry[0] = sx.x0; s_carry[1] = sx.x1; s_carry[2] = sx.x2; s_carry[6] = sx.s;
-      s_carry[3] = sy.x0; s_carry[4] = sy.x1; s_carry[5] = sy.x2; s_carry[7] = sy.s;
-    }
+    if (k0 <= last && last < k0 + FIR_R) store_state(s_carry, sx, sy);   // the thread that ran the tile's last valid tick carries the state
     base += FIR_TILE;
     if (base >= CAP) base -= CAP;
   }
@@ -1127,34 +1146,10 @@ preview_rec_warp_kernel(const int *__restrict__ order, const int64_t *__restrict
     double ax[FIR_R], ay[FIR_R];
     double2 pk[FIR_R];
     Axis bx, by;
-    bx.x0 = bx.x1 = bx.x2 = bx.s = 0.0;
-    by = bx;
     {
       const double2 *own = sp + own0;          // own0 is a multiple of 8: sample j of the block sits at j ^ ((own0 >> 3) & 7)
       const int osw = (own0 >> 3) & 7;
-#pragma unroll
-      for (int r = 0; r < FIR_R; ++r) { ax[r] = 0.0; ay[r] = 0.0; }
-#pragma unroll
-      for (int j = 0; j < FIR_R; ++j) {
-        const double2 a = own[j ^ osw];
-        int fi = own0 + j + NL;
-        if (fi >= CAP) fi -= CAP;
-        const double2 f = sp[swz8(fi)];
-        pk[j] = SIM ? a : make_double2(0.0, 0.0);
-#pragma unroll
-        for (int r = 0; r <= j; ++r) {
-          ax[r] = fma(c_pc.RF0[j - r], a.x, ax[r]); ax[r] = fma(c_pc.RFN[j - r], f.x, ax[r]);
-          ay[r] = fma(c_pc.RF0[j - r], a.y, ay[r]); ay[r] = fma(c_pc.RFN[j - r], f.y, ay[r]);
-        }
-        bx.x0 = fma(c_pc.RV[j][0], a.x, bx.x0); bx.x0 = fma(c_pc.RVN[j][0], f.x, bx.x0);
-        bx.x1 = fma(c_pc.RV[j][1], a.x, bx.x1); bx.x1 = fma(c_pc.RVN[j][1], f.x, bx.x1);
-        bx.x2 = fma(c_pc.RV[j][2], a.x, bx.x2); bx.x2 = fma(c_pc.RVN[j][2], f.x, bx.x2);
-        bx.s = fma(c_pc.RV[j][3], a.x, bx.s); bx.s = fma(c_pc.RVN[j][3], f.x, bx.s);
-        by.x0 = fma(c_pc.RV[j][0], a.y, by.x0); by.x0 = fma(c_pc.RVN[j][0], f.y, by.x0);
-        by.x1 = fma(c_pc.RV[j][1], a.y, by.x1); by.x1 = fma(c_pc.RVN[j][1], f.y, by.x1);
-        by.x2 = fma(c_pc.RV[j][2], a.y, by.x2); by.x2 = fma(c_pc.RVN[j][2], f.y, by.x2);
-        by.s = fma(c_pc.RV[j][3], a.y, by.s); by.s = fma(c_pc.RVN[j][3], f.y, by.s);
-      }
+      local_pass<SIM>([&](int j) { return own[j ^ osw]; }, [&](int i) { return sp[swz8(i)]; }, own0, NL, CAP, ax, ay, pk, bx, by);
     }
     __syncwarp();          // every read of this tile's samples is done; s_halo is written
     // the slots of the tile's own samples are dead: they receive what the next tile adds, samples [start + CAP, start + CAP + TILE)
@@ -1172,92 +1167,30 @@ preview_rec_warp_kernel(const int *__restrict__ order, const int64_t *__restrict
     }
     // ---- (1c) lane 31 takes W at the tile's end, then Kogge-Stone DOWN the tile: c_t += L^(8d) c_{t+d}
     Axis ix, iy;                               // W at tick 8 lane + 8 (the end of this lane's ticks)
-    ix.x0 = s_halo[0]; ix.x1 = s_halo[1]; ix.x2 = s_halo[2]; ix.s = s_halo[3];
-    iy.x0 = s_halo[4]; iy.x1 = s_halo[5]; iy.x2 = s_halo[6]; iy.s = s_halo[7];
+    load_pair(s_halo, ix, iy);
     if (lane == 31) {
-      scan_combine(bx, c_pc.RP[0], ix.x0, ix.x1, ix.x2, ix.s);
-      scan_combine(by, c_pc.RP[0], iy.x0, iy.x1, iy.x2, iy.s);
+      scan_combine(bx, c_pc.RP[0], ix);
+      scan_combine(by, c_pc.RP[0], iy);
     }
-#pragma unroll
-    for (int l = 0; l < 5; ++l) {
-      const int d = 1 << l;
-      const double a0 = __shfl_down_sync(FULL, bx.x0, d), a1 = __shfl_down_sync(FULL, bx.x1, d);
-      const double a2 = __shfl_down_sync(FULL, bx.x2, d), a3 = __shfl_down_sync(FULL, bx.s, d);
-      const double b0 = __shfl_down_sync(FULL, by.x0, d), b1 = __shfl_down_sync(FULL, by.x1, d);
-      const double b2 = __shfl_down_sync(FULL, by.x2, d), b3 = __shfl_down_sync(FULL, by.s, d);
-      if (lane + d < 32) {
-        scan_combine(bx, c_pc.RP[l], a0, a1, a2, a3);
-        scan_combine(by, c_pc.RP[l], b0, b1, b2, b3);
-      }
-    }
+    scan_down(bx, by, lane);
     {
-      const double a0 = __shfl_down_sync(FULL, bx.x0, 1), a1 = __shfl_down_sync(FULL, bx.x1, 1);
-      const double a2 = __shfl_down_sync(FULL, bx.x2, 1), a3 = __shfl_down_sync(FULL, bx.s, 1);
-      const double b0 = __shfl_down_sync(FULL, by.x0, 1), b1 = __shfl_down_sync(FULL, by.x1, 1);
-      const double b2 = __shfl_down_sync(FULL, by.x2, 1), b3 = __shfl_down_sync(FULL, by.s, 1);
-      if (lane != 31) {
-        ix.x0 = a0; ix.x1 = a1; ix.x2 = a2; ix.s = a3;
-        iy.x0 = b0; iy.x1 = b1; iy.x2 = b2; iy.s = b3;
-      }
+      const Axis a = shfl_down(bx, 1), b = shfl_down(by, 1);
+      if (lane != 31) { ix = a; iy = b; }
     }
-    // ---- (1d) f of tick r += (w' L^(8 - r)) . W_in
-#pragma unroll
-    for (int r = 0; r < FIR_R; ++r) {
-      const double *g = c_pc.RW[FIR_R - r];
-      ax[r] = fma(g[0], ix.x0, fma(g[1], ix.x1, fma(g[2], ix.x2, fma(g[3], ix.s, ax[r]))));
-      ay[r] = fma(g[0], iy.x0, fma(g[1], iy.x1, fma(g[2], iy.x2, fma(g[3], iy.s, ay[r]))));
-    }
+    // ---- (1d)
+    add_window(ax, ay, ix, iy);
 
     // ---- (2a) local aggregate of the cart-table recursion; lane 0 takes the carried state
     Axis cx, cy, inx, iny;
-    cx.x0 = cx.x1 = cx.x2 = cx.s = 0.0;
-    cy.x0 = cy.x1 = cy.x2 = cy.s = 0.0;
-    inx = cx; iny = cy;
-    {
-      const double(*Gm)[4] = c_pc.G[SIM ? 1 : 0];
-      const double(*Hm)[4] = c_pc.H[SIM ? 1 : 0];
-#pragma unroll
-      for (int r = 0; r < FIR_R; ++r) {
-        cx.x0 = fma(Gm[r][0], ax[r], cx.x0); cx.x1 = fma(Gm[r][1], ax[r], cx.x1);
-        cx.x2 = fma(Gm[r][2], ax[r], cx.x2); cx.s = fma(Gm[r][3], ax[r], cx.s);
-        cy.x0 = fma(Gm[r][0], ay[r], cy.x0); cy.x1 = fma(Gm[r][1], ay[r], cy.x1);
-        cy.x2 = fma(Gm[r][2], ay[r], cy.x2); cy.s = fma(Gm[r][3], ay[r], cy.s);
-        if (SIM) {
-          cx.x0 = fma(Hm[r][0], pk[r].x, cx.x0); cx.x1 = fma(Hm[r][1], pk[r].x, cx.x1);
-          cx.x2 = fma(Hm[r][2], pk[r].x, cx.x2); cx.s = fma(Hm[r][3], pk[r].x, cx.s);
-          cy.x0 = fma(Hm[r][0], pk[r].y, cy.x0); cy.x1 = fma(Hm[r][1], pk[r].y, cy.x1);
-          cy.x2 = fma(Hm[r][2], pk[r].y, cy.x2); cy.s = fma(Hm[r][3], pk[r].y, cy.s);
-        }
-      }
-      if (lane == 0) {
-        inx.x0 = s_carry[0]; inx.x1 = s_carry[1]; inx.x2 = s_carry[2]; inx.s = s_carry[6];
-        iny.x0 = s_carry[3]; iny.x1 = s_carry[4]; iny.x2 = s_carry[5]; iny.s = s_carry[7];
-        scan_combine(cx, Pm[0], inx.x0, inx.x1, inx.x2, inx.s);
-        scan_combine(cy, Pm[0], iny.x0, iny.x1, iny.x2, iny.s);
-      }
-    }
-    // ---- (2b) Kogge-Stone scan UP the tile: c_t += M^(8d) c_{t-d}
-#pragma unroll
-    for (int l = 0; l < 5; ++l) {
-      const int d = 1 << l;
-      const double a0 = __shfl_up_sync(FULL, cx.x0, d), a1 = __shfl_up_sync(FULL, cx.x1, d);
-      const double a2 = __shfl_up_sync(FULL, cx.x2, d), a3 = __shfl_up_sync(FULL, cx.s, d);
-      const double b0 = __shfl_up_sync(FULL, cy.x0, d), b1 = __shfl_up_sync(FULL, cy.x1, d);
-      const double b2 = __shfl_up_sync(FULL, cy.x2, d), b3 = __shfl_up_sync(FULL, cy.s, d);
-      if (lane >= d) {
-        scan_combine(cx, Pm[l], a0, a1, a2, a3);
-        scan_combine(cy, Pm[l], b0, b1, b2, b3);
-      }
-    }
+    local_aggregate<SIM>(ax, ay, pk, lane == 0, s_carry, Pm, cx, cy, inx, iny);
+    // ---- (2b) Kogge-Stone scan UP the tile
+    scan_up(cx, cy, lane, Pm);
     // ---- (2c) true start state of this lane = inclusive result of lane - 1
-    Axis sx, sy;
-    sx.x0 = __shfl_up_sync(FULL, cx.x0, 1); sx.x1 = __shfl_up_sync(FULL, cx.x1, 1);
-    sx.x2 = __shfl_up_sync(FULL, cx.x2, 1); sx.s = __shfl_up_sync(FULL, cx.s, 1);
-    sy.x0 = __shfl_up_sync(FULL, cy.x0, 1); sy.x1 = __shfl_up_sync(FULL, cy.x1, 1);
-    sy.x2 = __shfl_up_sync(FULL, cy.x2, 1); sy.s = __shfl_up_sync(FULL, cy.s, 1);
+    Axis sx = shfl_up(cx, 1), sy = shfl_up(cy, 1);
     if (lane == 0) { sx = inx; sy = iny; }
     __syncwarp();                              // s_carry and s_halo have been read
-    // ---- (2d) final pass, rows stored straight from registers (256-bit stores, see preview_rec_kernel)
+    // ---- (2d) final pass, rows stored straight from registers, CoM pairs through the bulk-copy engine (16-byte alignment is
+    //      all it asks)
     const int k0 = start + FIR_R * lane;
     const int last = min(start + RW_TILE, nsteps) - 1;   // last valid tick of this tile
     {
@@ -1324,10 +1257,7 @@ preview_rec_warp_kernel(const int *__restrict__ order, const int64_t *__restrict
         }
       }
     }
-    if (k0 <= last && last < k0 + FIR_R) {   // the lane that ran the tile's last valid tick carries the state
-      s_carry[0] = sx.x0; s_carry[1] = sx.x1; s_carry[2] = sx.x2; s_carry[6] = sx.s;
-      s_carry[3] = sy.x0; s_carry[4] = sy.x1; s_carry[5] = sy.x2; s_carry[7] = sy.s;
-    }
+    if (k0 <= last && last < k0 + FIR_R) store_state(s_carry, sx, sy);   // the lane that ran the tile's last valid tick carries the state
     base += RW_TILE;
     if (base >= CAP) base -= CAP;
   }
@@ -1536,124 +1466,59 @@ double rec_setup(const wg_preview_gains_t &g, PreviewConsts &pc, std::vector<dou
 
 }  // namespace
 
-// One CTA shape of the fused kernel: THREADS threads (tile = 8 x THREADS ticks), at least MIN_CTAS resident per SM.
-template <int THREADS, int MIN_CTAS>
-static int preview_launch_shape(wg_ctx *ctx, wg_preview_plan *pl, const int *d_order, int count, const double *d_zmp,
-                                double *d_state, double *d_com, double *d_zmpout, int simulation,
-                                const double *d_com_add = nullptr, bool pos_only = false)
+// One launch of a preview kernel: the 96 KB check, the gains of this context in the device's __constant__ block, the
+// shared-memory opt-in and the profiler bracket.
+template <class... P, class... A>
+static int preview_launch(wg_ctx *ctx, void (*kern)(P...), int count, int threads, size_t smem, const char *too_large,
+                          A... args)
 {
-  const int NLpad = (pl->NL + FIR_R - 1) / FIR_R * FIR_R;
-  const int span = FIR_R * THREADS + NLpad;
-  // the tile buffer doubles as the store staging area (320 double2 per warp)
-  const size_t smem = sizeof(double2) * std::max<size_t>((size_t)(span + (span >> 3) + 2), (size_t)(THREADS / 32) * 320);
-  if (smem > 96 * 1024) return wg_fail(ctx, WG_ERR_INVALID, "preview window too large for the FIR tile");
-  constexpr int slot = WG_ATTR_PREVIEW_0 + (THREADS == 128 ? 0 : THREADS == 32 ? 2 : 4);
-  if (simulation) WG_SMEM_ATTR(ctx, slot, (preview_fused_kernel<true, THREADS, MIN_CTAS>), smem);
-  else WG_SMEM_ATTR(ctx, slot + 1, (preview_fused_kernel<false, THREADS, MIN_CTAS>), smem);
-  const double2 *pz = reinterpret_cast<const double2 *>(d_zmp);
+  if (smem > 96 * 1024) return wg_fail(ctx, WG_ERR_INVALID, too_large);
   std::lock_guard<std::mutex> lock(g_pv_mutex);
   { const int rc = preview_bind(ctx); if (rc != WG_OK) return rc; }
-  if (pos_only) {             // CoM position only: d_zmpout is the [total][2] position array
-    if (simulation) {
-      WG_SMEM_ATTR(ctx, WG_ATTR_PREVIEW_POS_0 + 2 * (THREADS == 128 ? 0 : THREADS == 32 ? 1 : 2), (preview_fused_kernel<true, THREADS, MIN_CTAS, false, true>), smem);
-    } else {
-      WG_SMEM_ATTR(ctx, WG_ATTR_PREVIEW_POS_0 + 2 * (THREADS == 128 ? 0 : THREADS == 32 ? 1 : 2) + 1, (preview_fused_kernel<false, THREADS, MIN_CTAS, false, true>), smem);
-    }
-    wg_prof_start(ctx, WG_K_PREVIEW_FUSED);
-    if (simulation)
-      preview_fused_kernel<true, THREADS, MIN_CTAS, false, true><<<count, THREADS, smem, ctx->stream>>>(d_order, pl->d_offsets, pz, d_state, nullptr, d_zmpout);
-    else
-      preview_fused_kernel<false, THREADS, MIN_CTAS, false, true><<<count, THREADS, smem, ctx->stream>>>(d_order, pl->d_offsets, pz, d_state, nullptr, d_zmpout);
-    wg_prof_stop(ctx);
-    WG_LAUNCHED(ctx);
-    return WG_OK;
-  }
-  if (d_com_add && d_com) {   // second stage: always with the integrated error (Simulation = true, :343-347)
-    WG_SMEM_ATTR(ctx, WG_ATTR_PREVIEW_ADD_0 + (THREADS == 128 ? 0 : THREADS == 32 ? 1 : 2), (preview_fused_kernel<true, THREADS, MIN_CTAS, true>), smem);
-    wg_prof_start(ctx, WG_K_PREVIEW_FUSED);
-    preview_fused_kernel<true, THREADS, MIN_CTAS, true><<<count, THREADS, smem, ctx->stream>>>(d_order, pl->d_offsets, pz, d_state, d_com, d_zmpout, d_com_add);
-    wg_prof_stop(ctx);
-    WG_LAUNCHED(ctx);
-    return WG_OK;
-  }
+  WG_SMEM_ATTR(ctx, kern, smem);
   wg_prof_start(ctx, WG_K_PREVIEW_FUSED);
-  if (simulation)
-    preview_fused_kernel<true, THREADS, MIN_CTAS><<<count, THREADS, smem, ctx->stream>>>(d_order, pl->d_offsets, pz, d_state, d_com, d_zmpout);
-  else
-    preview_fused_kernel<false, THREADS, MIN_CTAS><<<count, THREADS, smem, ctx->stream>>>(d_order, pl->d_offsets, pz, d_state, d_com, d_zmpout);
+  kern<<<count, threads, smem, ctx->stream>>>(args...);
   wg_prof_stop(ctx);
   WG_LAUNCHED(ctx);
   return WG_OK;
 }
 
-// The recursive kernel in the same CTA shapes.
-template <int THREADS, int MIN_CTAS>
-static int preview_launch_rec(wg_ctx *ctx, wg_preview_plan *pl, const int *d_order, int count, const double *d_zmp,
-                              double *d_state, double *d_com, double *d_zmpout, int simulation,
-                              const double *d_com_add, bool pos_only)
+// The kernel of variant <SIM, ADD, POS> in the family (direct sum, recursive, recursive one-warp) and CTA shape that
+// wgi_preview_launch_range chose, with the dynamic shared memory that shape needs.
+template <bool SIM, bool ADD, bool POS>
+static int preview_launch_variant(wg_ctx *ctx, wg_preview_plan *pl, bool recursive, int shape, const int *d_order, int count,
+                                  const double2 *pz, double *d_state, double *d_com, double *d_zmpout, const double *d_com_add)
 {
   const int NLpad = (pl->NL + FIR_R - 1) / FIR_R * FIR_R;
-  const int cap = 2 * FIR_R * THREADS + NLpad;     // ring of two tiles + the window
-  const size_t smem = sizeof(double2) * (size_t)(cap + (cap >> 3) + 2);
-  if (smem > 96 * 1024) return wg_fail(ctx, WG_ERR_INVALID, "preview window too large for the tile");
-  constexpr int slot = WG_ATTR_PREVIEW_REC_0 + 5 * (THREADS == 128 ? 0 : THREADS == 32 ? 1 : THREADS == 64 ? 2 : 3);
-  const double2 *pz = reinterpret_cast<const double2 *>(d_zmp);
+  const int64_t *off = pl->d_offsets;
+  if (!recursive) {
+    // tile = 8 x threads ticks; the tile buffer doubles as the store staging area (320 double2 per warp)
+    auto smem = [&](int threads) {
+      const int span = FIR_R * threads + NLpad;
+      return sizeof(double2) * std::max<size_t>((size_t)(span + (span >> 3) + 2), (size_t)(threads / 32) * 320);
+    };
+    const char *msg = "preview window too large for the FIR tile";
+    switch (shape) {
+    case 1: return preview_launch(ctx, preview_fused_kernel<SIM, 128, 4, ADD, POS>, count, 128, smem(128), msg, d_order, off, pz, d_state, d_com, d_zmpout, d_com_add);
+    case 2: return preview_launch(ctx, preview_fused_kernel<SIM, 32, 16, ADD, POS>, count, 32, smem(32), msg, d_order, off, pz, d_state, d_com, d_zmpout, d_com_add);
+    default: return preview_launch(ctx, preview_fused_kernel<SIM, 64, 8, ADD, POS>, count, 64, smem(64), msg, d_order, off, pz, d_state, d_com, d_zmpout, d_com_add);
+    }
+  }
   const double2 *E = reinterpret_cast<const double2 *>(ctx->preview_rec_dev);
+  const char *msg = "preview window too large for the tile";
+  if (shape == 2)   // swizzled ring + 32 staging slots of 400 B
+    return preview_launch(ctx, preview_rec_warp_kernel<SIM, ADD, POS>, count, 32, sizeof(double2) * (size_t)(RW_TILE + NLpad + 25 * 32),
+                          msg, d_order, off, pz, d_state, d_com, d_zmpout, d_com_add, E);
+  auto smem = [&](int threads) {   // ring of two tiles + the window
+    const int cap = 2 * FIR_R * threads + NLpad;
+    return sizeof(double2) * (size_t)(cap + (cap >> 3) + 2);
+  };
   const double2 *lp = E + 2 * (size_t)NLpad;
-  std::lock_guard<std::mutex> lock(g_pv_mutex);
-  { const int rc = preview_bind(ctx); if (rc != WG_OK) return rc; }
-#define WG_REC_LAUNCH(SLOT, SIMF, ADDF, POSF, COM, ADDP)                                                                \
-  do {                                                                                                                 \
-    WG_SMEM_ATTR(ctx, slot + (SLOT), (preview_rec_kernel<SIMF, THREADS, MIN_CTAS, ADDF, POSF>), smem);                   \
-    wg_prof_start(ctx, WG_K_PREVIEW_FUSED);                                                                            \
-    preview_rec_kernel<SIMF, THREADS, MIN_CTAS, ADDF, POSF><<<count, THREADS, smem, ctx->stream>>>(                     \
-        d_order, pl->d_offsets, pz, d_state, COM, d_zmpout, ADDP, E, lp);                                              \
-    wg_prof_stop(ctx);                                                                                                 \
-    WG_LAUNCHED(ctx);                                                                                                  \
-    return WG_OK;                                                                                                      \
-  } while (0)
-  if (pos_only) {
-    if (simulation) WG_REC_LAUNCH(0, true, false, true, nullptr, nullptr);
-    else WG_REC_LAUNCH(1, false, false, true, nullptr, nullptr);
+  switch (shape) {
+  case 1: return preview_launch(ctx, preview_rec_kernel<SIM, 128, 4, ADD, POS>, count, 128, smem(128), msg, d_order, off, pz, d_state, d_com, d_zmpout, d_com_add, E, lp);
+  case 3: return preview_launch(ctx, preview_rec_kernel<SIM, 256, 2, ADD, POS>, count, 256, smem(256), msg, d_order, off, pz, d_state, d_com, d_zmpout, d_com_add, E, lp);
+  default: return preview_launch(ctx, preview_rec_kernel<SIM, 64, 8, ADD, POS>, count, 64, smem(64), msg, d_order, off, pz, d_state, d_com, d_zmpout, d_com_add, E, lp);
   }
-  if (d_com_add && d_com) WG_REC_LAUNCH(2, true, true, false, d_com, d_com_add);
-  if (simulation) WG_REC_LAUNCH(3, true, false, false, d_com, nullptr);
-  else WG_REC_LAUNCH(4, false, false, false, d_com, nullptr);
-#undef WG_REC_LAUNCH
-}
-
-// The recursive kernel, one warp per trajectory.
-static int preview_launch_recw(wg_ctx *ctx, wg_preview_plan *pl, const int *d_order, int count, const double *d_zmp,
-                               double *d_state, double *d_com, double *d_zmpout, int simulation,
-                               const double *d_com_add, bool pos_only)
-{
-  const int NLpad = (pl->NL + FIR_R - 1) / FIR_R * FIR_R;
-  const int cap = RW_TILE + NLpad;
-  const size_t smem = sizeof(double2) * (size_t)(cap + 25 * 32);     // swizzled ring + 32 staging slots of 400 B
-  if (smem > 96 * 1024) return wg_fail(ctx, WG_ERR_INVALID, "preview window too large for the tile");
-  constexpr int slot = WG_ATTR_PREVIEW_REC_0 + 5;
-  const double2 *pz = reinterpret_cast<const double2 *>(d_zmp);
-  const double2 *E = reinterpret_cast<const double2 *>(ctx->preview_rec_dev);
-  std::lock_guard<std::mutex> lock(g_pv_mutex);
-  { const int rc = preview_bind(ctx); if (rc != WG_OK) return rc; }
-#define WG_RECW_LAUNCH(SLOT, SIMF, ADDF, POSF, COM, ADDP)                                                               \
-  do {                                                                                                                 \
-    WG_SMEM_ATTR(ctx, slot + (SLOT), (preview_rec_warp_kernel<SIMF, ADDF, POSF>), smem);                                \
-    wg_prof_start(ctx, WG_K_PREVIEW_FUSED);                                                                            \
-    preview_rec_warp_kernel<SIMF, ADDF, POSF><<<count, 32, smem, ctx->stream>>>(d_order, pl->d_offsets, pz, d_state,    \
-                                                                                 COM, d_zmpout, ADDP, E);              \
-    wg_prof_stop(ctx);                                                                                                 \
-    WG_LAUNCHED(ctx);                                                                                                  \
-    return WG_OK;                                                                                                      \
-  } while (0)
-  if (pos_only) {
-    if (simulation) WG_RECW_LAUNCH(0, true, false, true, nullptr, nullptr);
-    else WG_RECW_LAUNCH(1, false, false, true, nullptr, nullptr);
-  }
-  if (d_com_add && d_com) WG_RECW_LAUNCH(2, true, true, false, d_com, d_com_add);
-  if (simulation) WG_RECW_LAUNCH(3, true, false, false, d_com, nullptr);
-  else WG_RECW_LAUNCH(4, false, false, false, d_com, nullptr);
-#undef WG_RECW_LAUNCH
 }
 
 extern "C" {
@@ -1865,19 +1730,18 @@ int wgi_preview_launch_range(wg_ctx *ctx, wg_preview_plan *pl, const int *d_orde
   }
   if (ctx->preview_sum_mode == WG_PREVIEW_SUM_RECURSIVE && !ctx->preview_rec_ok)
     return wg_fail(ctx, WG_ERR_INVALID, "WG_PREVIEW_SUM_RECURSIVE: the window weights of this context are not of the form w' L^i v");
-  if (recursive) {
-    switch (shape) {
-    case 1: return preview_launch_rec<128, 4>(ctx, pl, d_order, count, d_zmp, d_state, d_com, d_zmpout, simulation, d_com_add, pos_only != 0);
-    case 2: return preview_launch_recw(ctx, pl, d_order, count, d_zmp, d_state, d_com, d_zmpout, simulation, d_com_add, pos_only != 0);
-    case 3: return preview_launch_rec<256, 2>(ctx, pl, d_order, count, d_zmp, d_state, d_com, d_zmpout, simulation, d_com_add, pos_only != 0);
-    default: return preview_launch_rec<64, 8>(ctx, pl, d_order, count, d_zmp, d_state, d_com, d_zmpout, simulation, d_com_add, pos_only != 0);
-    }
-  }
-  switch (shape) {
-  case 1: return preview_launch_shape<128, 4>(ctx, pl, d_order, count, d_zmp, d_state, d_com, d_zmpout, simulation, d_com_add, pos_only != 0);
-  case 2: return preview_launch_shape<32, 16>(ctx, pl, d_order, count, d_zmp, d_state, d_com, d_zmpout, simulation, d_com_add, pos_only != 0);
-  default: return preview_launch_shape<64, 8>(ctx, pl, d_order, count, d_zmp, d_state, d_com, d_zmpout, simulation, d_com_add, pos_only != 0);
-  }
+  // variant: position only (the CoM (x, y) pair leaves through the ZMP path), the second stage (always with the integrated
+  // error, ZMPPreviewControlWithMultiBodyZMP.cpp:343-347), or the plain run
+  const double2 *pz = reinterpret_cast<const double2 *>(d_zmp);
+  auto launch = [&](auto sim, auto add, auto pos) {
+    return preview_launch_variant<sim, add, pos>(ctx, pl, recursive, shape, d_order, count, pz, d_state, pos ? nullptr : d_com,
+                                                 d_zmpout, add ? d_com_add : nullptr);
+  };
+  const std::true_type T{};
+  const std::false_type F{};
+  if (pos_only) return simulation ? launch(T, F, T) : launch(F, F, T);
+  if (d_com_add && d_com) return launch(T, T, F);
+  return simulation ? launch(T, F, F) : launch(F, F, F);
 }
 
 static int preview_run(wg_ctx *ctx, wg_preview_plan *pl, int mem, const double *zmpref_xy, double *state,

@@ -931,8 +931,8 @@ static int qld_solve_impl(wg_ctx *ctx, int mem, int B, const wg_qld_batch *q, co
   a.pstride = std::max(mmax, rk ? (4 * rk->N + QW - 1) / QW : 0);
   const size_t smem = qld_smem_bytes(n, mmax, a.pstride, a.qcap, bounds);
   if (smem > 200 * 1024) return wg_fail(ctx, WG_ERR_INVALID, "wg_qld_solve_batch: problem too large for shared memory");
-  if (rk) WG_SMEM_ATTR(ctx, WG_ATTR_DENSEQP_RANKED, qld_kernel<true>, smem);
-  else WG_SMEM_ATTR(ctx, WG_ATTR_DENSEQP, qld_kernel<false>, smem);
+  if (rk) WG_SMEM_ATTR(ctx, qld_kernel<true>, smem);
+  else WG_SMEM_ATTR(ctx, qld_kernel<false>, smem);
   int per_sm = (int)std::min<size_t>(2, (220 * 1024) / (smem + 1024));
   if (per_sm < 1) per_sm = 1;
   const int blocks = std::max(1, std::min(B, ctx->sm_count * per_sm));

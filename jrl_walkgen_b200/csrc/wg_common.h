@@ -9,8 +9,6 @@
 
 #define WG_VERSION ((0 << 16) | (1 << 8) | 0)
 
-struct wg_preview_consts;  // preview.cu
-
 // Kernel ids of the per-kernel CUDA-event profiler (wg_prof_*): bench.py reads the average launch
 // duration of each kernel over the timed region from these.
 enum { WG_K_PREVIEW_FIR = 0, WG_K_PREVIEW_RECUR = 1, WG_K_HERDT_QP = 2, WG_K_HERDT_MPC = 3, WG_K_PLDP = 4,
@@ -37,7 +35,6 @@ struct wg_ctx {
   // preview control
   bool preview_ready = false;
   wg_preview_gains_t preview_gains;
-  double *d_previewF = nullptr;  // device copy of F padded with zeros
   std::vector<unsigned char> preview_image;   // host image of the kernels' __constant__ block (PreviewConsts + taps)
   unsigned long long preview_gen = 0;         // bumped by wg_preview_set_gains
   void *preview_tick = nullptr;               // buffers of wg_preview_one_iteration (preview.cu)
@@ -100,18 +97,13 @@ inline void wg_prof_stop(wg_ctx *ctx)
 }
 
 // cudaFuncAttributeMaxDynamicSharedMemorySize is a per-DEVICE, per-function attribute: keep the largest value set so far
-// per (device, slot) instead of in function-local statics (a second context on another GPU must set it again, a second
-// context on the same GPU must not lower it).  Slots: one per kernel instantiation that needs more than 48 KB.
-enum { WG_ATTR_PREVIEW_0 = 0, /* .. 5: {sim, nosim} x 3 CTA shapes */ WG_ATTR_HERDT_QP = 6, WG_ATTR_HERDT_MPC = 7,
-       WG_ATTR_PLDP = 8, WG_ATTR_PLDP_RANKED = 9, WG_ATTR_ZMPDISC = 10, WG_ATTR_DIMITROV = 11, WG_ATTR_DENSEQP = 12,
-       WG_ATTR_PREVIEW_ADD_0 = 13, /* .. 15: second-stage variant x 3 CTA shapes */
-       WG_ATTR_PREVIEW_POS_0 = 16, /* .. 21: position-only variant {sim, nosim} x 3 CTA shapes */ WG_ATTR_DENSEQP_RANKED = 22,
-       WG_ATTR_PREVIEW_REC_0 = 24, /* .. 43: recursive preview kernel, 5 variants x 4 CTA shapes */ WG_ATTR_SLOTS = 48 };
-extern "C" int wgi_smem_attr(wg_ctx *ctx, int slot, const void *func, size_t bytes);
-#define WG_SMEM_ATTR(ctx, slot, func, bytes)                                              \
-  do {                                                                                    \
-    int rc__ = wgi_smem_attr((ctx), (slot), reinterpret_cast<const void *>(func), (bytes)); \
-    if (rc__ != WG_OK) return rc__;                                                       \
+// per (device, kernel) instead of in function-local statics (a second context on another GPU must set it again, a second
+// context on the same GPU must not lower it).  Kernels that need at most 48 KB are left alone.
+extern "C" int wgi_smem_attr(wg_ctx *ctx, const void *func, size_t bytes);
+#define WG_SMEM_ATTR(ctx, func, bytes)                                              \
+  do {                                                                              \
+    int rc__ = wgi_smem_attr((ctx), reinterpret_cast<const void *>(func), (bytes)); \
+    if (rc__ != WG_OK) return rc__;                                                 \
   } while (0)
 
 // preview.cu internals used by zmpdisc.cu (the footsteps -> CoM pipeline): launch the fused preview kernel over `count`

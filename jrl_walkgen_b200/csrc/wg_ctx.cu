@@ -10,21 +10,23 @@ extern void wg_dimitrov_release(wg_ctx *ctx);
 extern void wg_qld_release(wg_ctx *ctx);
 extern void wg_wieber_release(wg_ctx *ctx);
 
+#include <map>
 #include <mutex>
+#include <utility>
 
 namespace {
 std::mutex g_attr_mutex;
-size_t g_attr_smem[64][WG_ATTR_SLOTS];   // zero-initialised: largest dynamic shared memory size set per (device, slot)
+std::map<std::pair<int, const void *>, size_t> g_attr_smem;   // largest dynamic shared memory size set per (device, kernel)
 }
 
-extern "C" int wgi_smem_attr(wg_ctx *ctx, int slot, const void *func, size_t bytes)
+extern "C" int wgi_smem_attr(wg_ctx *ctx, const void *func, size_t bytes)
 {
   if (bytes <= 48 * 1024) return WG_OK;   // the default limit needs no opt-in
-  if (ctx->device < 0 || ctx->device >= 64 || slot < 0 || slot >= WG_ATTR_SLOTS) return WG_ERR_INVALID;
   std::lock_guard<std::mutex> lock(g_attr_mutex);
-  if (bytes > g_attr_smem[ctx->device][slot]) {
+  size_t &set = g_attr_smem[{ctx->device, func}];
+  if (bytes > set) {
     WG_CUDA(ctx, cudaFuncSetAttribute(func, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-    g_attr_smem[ctx->device][slot] = bytes;
+    set = bytes;
   }
   return WG_OK;
 }
@@ -71,7 +73,6 @@ int wg_ctx_destroy(wg_ctx *ctx)
   wg_wieber_release(ctx);
   wg_qld_release(ctx);
   wg_pldp_release(ctx);
-  if (ctx->d_previewF) cudaFree(ctx->d_previewF);
   for (cudaEvent_t e : ctx->prof.ev) cudaEventDestroy(e);
   cudaEventDestroy(ctx->ev0);
   cudaEventDestroy(ctx->ev1);

@@ -804,7 +804,7 @@ static int zd_launch(wg_ctx *ctx, wg_kajita_plan *pl, int b0, int b1, const Out 
   if (b1 <= b0) return WG_OK;
   const size_t smem = sizeof(double2) * (size_t)ZD_WARPS * (pl->K.cap + 2 * ZD_HIST + ZD_HEAD);
   if (smem > 200 * 1024) return wg_fail(ctx, WG_ERR_INVALID, "step segment too long for the shared-memory buffer");
-  WG_SMEM_ATTR(ctx, WG_ATTR_ZMPDISC, zmpdisc_kernel, smem);
+  WG_SMEM_ATTR(ctx, zmpdisc_kernel, smem);
   const int walks = b1 - b0;
   const int grid = std::max(1, std::min((walks + ZD_WARPS - 1) / ZD_WARPS, ctx->sm_count * 3));
   // the whole batch uses the global longest-first order, a chunk [b0, b1) the per-chunk one (both are permutations of
