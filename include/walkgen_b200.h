@@ -680,6 +680,56 @@ int wg_zmpdisc_run_batch(wg_ctx *ctx, wg_kajita_plan *plan, int mem, double *zmp
 int wg_kajita_run_batch(wg_ctx *ctx, wg_kajita_plan *plan, int mem, double *state, double *com_out, double *zmp_out,
                         double *zmpref_xy, wg_foot_sample *left, wg_foot_sample *right, int simulation);
 
+/* On-line form: B walks whose footsteps arrive while they run, each walk's state kept on the device between runs.
+ *   replaces ZMPDiscretization::InitOnLine (src/ZMPRefTrajectoryGeneration/ZMPDiscretization.cpp:319-513),
+ *            ZMPDiscretization::OnLineAddFoot (:573-1020) and ZMPDiscretization::EndPhaseOfTheWalking (:1129-1300),
+ *            each driving the preview loop over the new part of the ZMP FIFO                               [device]
+ * Each run emits what one append scheduled.  For walk b, flags[b] selects:
+ *   WG_STREAM_START   (re)start the walk (InitOnLine); its state is dropped.  The append's first step is the support-foot
+ *                     step (step 0 of a plan's list): the run emits the 2*NL lead-in, then one segment per further step.
+ *                     The preview state of the walk is zeroed.  init_feet_host[b] as in wg_kajita_plan_create.
+ *   (no flag)         each appended step is one OnLineAddFoot and emits its segment.
+ *   WG_STREAM_FINISH  after this append's steps, EndPhaseOfTheWalking (n_end + 3*NL samples); the walk closes.
+ * A walk with no steps and no flags is untouched.  START|FINISH on a whole step list is exactly one walk of a plan: the
+ * samples a walk emits over all its runs, concatenated, are bitwise what wg_zmpdisc_run_batch gives for its whole list.
+ *
+ * wg_kajita_stream_append plans the next run on the host (the step timings size it) and starts an asynchronous H2D copy
+ * of its steps; steps, offsets and flags are host arrays (step_offsets [B+1], walk b appends steps [off[b], off[b+1]) of
+ * steps_host; flags_host [B] may be NULL for no flags).  Refused with WG_ERR_INVALID, every walk left unchanged: steps for a
+ * walk that is not open and has no START; START with zero steps or with init_feet_host == NULL; FINISH on a closed walk;
+ * a step timing that wg_kajita_plan_create refuses; an append while the previous one has not been run.
+ *
+ * wg_kajita_stream_run executes the pending append (a run with none pending does nothing).  Outputs live in `mem` and
+ * each may be NULL; their rows:
+ *   zmpref_xy [][2], zmp_theta [], left [], right [], step_type [][3]: walk b's new samples are rows [so[b], so[b+1]),
+ *       compact and in order (so = wg_kajita_stream_sample_offsets).
+ *   com_out [][6], zmp_out [][2]: walk b's com_counts[b] new preview steps are the first rows of [co[b], co[b+1])
+ *       (co = wg_kajita_stream_com_offsets).  Row j is the walk's preview step steps_previewed_before + j, the row
+ *       wg_kajita_run_batch writes at offsets[b] + steps_previewed_before + j.  Rows past the count: untouched with
+ *       WG_MEM_DEVICE, zero with WG_MEM_HOST.  A walk's preview consumes its samples as they arrive: after a run it has
+ *       previewed max(0, samples_emitted - NL + 1) steps, so FINISH completes the walk's preview.
+ * with_preview = 1 needs preview gains on the context (WG_ERR_NOT_READY otherwise) and keeps their NL: a run after gains of
+ * another NL were set is refused with WG_ERR_NOT_READY.  Gains of the same NL and the sum mode are read at run time, as
+ * wg_kajita_run_batch does.  With with_preview = 0 the stream is the front end only and com_out / zmp_out must be NULL.
+ * The offsets returned below describe the pending append (or the last one run); they stay valid until the next append.
+ * In steady state a run allocates nothing and creates no stream or event; buffers grow when a run needs more. */
+typedef struct wg_kajita_stream wg_kajita_stream;
+enum { WG_STREAM_START = 1, WG_STREAM_FINISH = 2 };
+int wg_kajita_stream_create(wg_ctx *ctx, const wg_zmpdisc_params *p, int B, int with_preview, wg_kajita_stream **out);
+int wg_kajita_stream_destroy(wg_kajita_stream *s);
+int wg_kajita_stream_append(wg_kajita_stream *s, const int64_t *step_offsets_host, const wg_rel_step *steps_host,
+                            const int32_t *flags_host, const double *init_feet_host);
+const int64_t *wg_kajita_stream_sample_offsets(const wg_kajita_stream *s);  /* B+1: rows of the samples the run emits */
+const int64_t *wg_kajita_stream_com_offsets(const wg_kajita_stream *s);     /* B+1: rows reserved for its preview steps */
+const int64_t *wg_kajita_stream_com_counts(const wg_kajita_stream *s);      /* B: preview steps each walk gets          */
+int wg_kajita_stream_run(wg_kajita_stream *s, int mem, double *zmpref_xy, double *zmp_theta, wg_foot_sample *left,
+                         wg_foot_sample *right, int32_t *step_type, double *com_out, double *zmp_out, int simulation);
+/* After the last run: preview_state [B][8] (in `mem`; as wg_preview_run_batch's state) and, in host arrays of B entries,
+ * the samples each walk emitted and the preview steps it ran since its START, and whether it is open.  Any may be NULL.
+ * With WG_MEM_HOST the call waits for the stream. */
+int wg_kajita_stream_state(wg_kajita_stream *s, int mem, double *preview_state, int64_t *samples_emitted,
+                           int64_t *steps_previewed, int32_t *open);
+
 /* ------------------------------------------------------------------------------------------------
  * Dimitrov2008 front to back: feet trajectories -> support polygons -> per-period constraint matrices ->
  * PLDP solve -> LIPM, closed loop on the device (one warp owns one walk for its whole duration)

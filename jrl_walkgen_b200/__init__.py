@@ -24,7 +24,8 @@ REL_STEP_DTYPE, KAJITA_FOOT_DTYPE = _capi.kajita_dtypes()
 LCI_DTYPE, DIMITROV_PERIOD_DTYPE = _capi.dimitrov_dtypes()
 DimitrovParams = _capi.DimitrovParams
 
-__all__ = ["MultiContext", "LCI_DTYPE", "DIMITROV_PERIOD_DTYPE", "DimitrovParams", "dimitrov_default_params", "Context", "PreviewPlan", "KajitaPlan", "zmpdisc_default_params", "REL_STEP_DTYPE", "KAJITA_FOOT_DTYPE", "preview_gains", "herdt_default_params", "herdt_mpc_default_params", "HerdtParams", "HerdtMpcParams",
+__all__ = ["MultiContext", "LCI_DTYPE", "DIMITROV_PERIOD_DTYPE", "DimitrovParams", "dimitrov_default_params", "Context", "PreviewPlan", "KajitaPlan", "KajitaStream",
+           "STREAM_START", "STREAM_FINISH", "zmpdisc_default_params", "REL_STEP_DTYPE", "KAJITA_FOOT_DTYPE", "preview_gains", "herdt_default_params", "herdt_mpc_default_params", "HerdtParams", "HerdtMpcParams",
            "PLDP_STATE_DTYPE", "PLDP_INFO_DTYPE", "FOOT_DTYPE", "TICK_DTYPE", "MPC_STATE_DTYPE", "MPC_STEP_DTYPE", "TICKS_PER_STEP", "QP_INPUT_DTYPE",
            "QP_OUTPUT_DTYPE", "ACTIVE_SET_DTYPE", "WalkgenError", "device_count",
            "MODE_WITH_INITIALPOS", "MODE_WITHOUT_INITIALPOS", "WG_MEM_HOST", "WG_MEM_DEVICE"]
@@ -213,6 +214,10 @@ class Context:
     def kajita_plan(self, step_offsets, steps, init_feet, params=None) -> "KajitaPlan":
         """The step stacks of B walks, resident on the GPU (wg_kajita_plan_create)."""
         return KajitaPlan(self, step_offsets, steps, init_feet, params)
+
+    def kajita_stream(self, B, params=None, with_preview=True) -> "KajitaStream":
+        """B walks whose footsteps arrive while they run (wg_kajita_stream_create)."""
+        return KajitaStream(self, B, params, with_preview)
 
     def preview_one_iteration(self, x, y, sx, sy, window_xy, simulation=True):
         """PreviewControl::OneIterationOfPreview for one instance (host buffers)."""
@@ -601,6 +606,72 @@ class KajitaPlan:
     def destroy(self):
         if self.h:
             self.ctx.lib.wg_kajita_plan_destroy(self.h)
+            self.h = None
+
+
+STREAM_START, STREAM_FINISH = 1, 2
+
+
+class KajitaStream:
+    """On-line Kajita2003 generator for B walks: InitOnLine / OnLineAddFoot / EndPhaseOfTheWalking, batched, with the
+    preview loop consuming each walk's new ZMP reference (wg_kajita_stream_*).  One append plans one run."""
+
+    def __init__(self, ctx: Context, B, params=None, with_preview=True):
+        self.ctx = ctx
+        self.B = int(B)
+        self.params = params if params is not None else zmpdisc_default_params()
+        self.with_preview = bool(with_preview)
+        h = C.c_void_p()
+        ctx._check(ctx.lib.wg_kajita_stream_create(ctx.h, C.byref(self.params), self.B, int(self.with_preview), C.byref(h)))
+        self.h = h
+        self.sample_offsets = np.zeros(self.B + 1, dtype=np.int64)
+        self.com_offsets = np.zeros(self.B + 1, dtype=np.int64)
+        self.com_counts = np.zeros(self.B, dtype=np.int64)
+
+    def append(self, step_offsets, steps, flags=None, init_feet=None):
+        """Plan the next run: walk b appends steps[step_offsets[b]:step_offsets[b+1]] with flags[b] (STREAM_START /
+        STREAM_FINISH).  Refreshes sample_offsets, com_offsets and com_counts (the row layout of the run)."""
+        off = np.ascontiguousarray(step_offsets, dtype=np.int64)
+        assert len(off) == self.B + 1
+        steps = np.ascontiguousarray(steps, dtype=REL_STEP_DTYPE)
+        fl = None if flags is None else np.ascontiguousarray(flags, dtype=np.int32)
+        feet = None if init_feet is None else np.ascontiguousarray(init_feet, dtype=np.float64).reshape(self.B, 6)
+        lib = self.ctx.lib
+        self.ctx._check(lib.wg_kajita_stream_append(self.h, off.ctypes.data_as(_capi.c_i64_p), steps.ctypes.data if len(steps) else None,
+                                                    _ptr(fl), _ptr(feet)))
+        self.sample_offsets = np.ctypeslib.as_array(lib.wg_kajita_stream_sample_offsets(self.h), shape=(self.B + 1,)).copy()
+        self.com_offsets = np.ctypeslib.as_array(lib.wg_kajita_stream_com_offsets(self.h), shape=(self.B + 1,)).copy()
+        self.com_counts = np.ctypeslib.as_array(lib.wg_kajita_stream_com_counts(self.h), shape=(self.B,)).copy()
+        return self.sample_offsets, self.com_offsets, self.com_counts
+
+    def host_outputs(self, com=True):
+        """Zeroed host arrays sized for the planned run: zmpref, zmp_theta, left, right, step_type (and com_out, zmp_out)."""
+        n, m = int(self.sample_offsets[-1]), int(self.com_offsets[-1])
+        out = dict(zmpref_xy=np.zeros((n, 2)), zmp_theta=np.zeros(n), left=np.zeros(n, dtype=KAJITA_FOOT_DTYPE),
+                   right=np.zeros(n, dtype=KAJITA_FOOT_DTYPE), step_type=np.zeros((n, 3), dtype=np.int32))
+        if com and self.with_preview:
+            out.update(com_out=np.zeros((m, 6)), zmp_out=np.zeros((m, 2)))
+        return out
+
+    def run(self, zmpref_xy=None, zmp_theta=None, left=None, right=None, step_type=None, com_out=None, zmp_out=None,
+            simulation=True, mem=WG_MEM_HOST):
+        """Run the planned append (wg_kajita_stream_run); any output may be None."""
+        self.ctx._check(self.ctx.lib.wg_kajita_stream_run(self.h, mem, _ptr(zmpref_xy), _ptr(zmp_theta), _ptr(left), _ptr(right),
+                                                          _ptr(step_type), _ptr(com_out), _ptr(zmp_out), int(simulation)))
+
+    def state(self, preview_state=None, mem=WG_MEM_HOST):
+        """-> (preview_state [B][8] or None, samples_emitted [B], steps_previewed [B], open [B])."""
+        if preview_state is None and self.with_preview and mem == WG_MEM_HOST:
+            preview_state = np.zeros((self.B, 8))
+        emitted = np.zeros(self.B, dtype=np.int64); previewed = np.zeros(self.B, dtype=np.int64)
+        is_open = np.zeros(self.B, dtype=np.int32)
+        self.ctx._check(self.ctx.lib.wg_kajita_stream_state(self.h, mem, _ptr(preview_state), _ptr(emitted), _ptr(previewed),
+                                                            _ptr(is_open)))
+        return preview_state, emitted, previewed, is_open
+
+    def destroy(self):
+        if self.h:
+            self.ctx.lib.wg_kajita_stream_destroy(self.h)
             self.h = None
 
 

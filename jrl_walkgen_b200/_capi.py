@@ -319,6 +319,15 @@ SIGNATURES = {
                                        C.c_void_p]),
     "wg_kajita_run_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                       C.c_void_p, C.c_void_p, C.c_int]),
+    "wg_kajita_stream_create": (C.c_int, [C.c_void_p, C.POINTER(ZmpDiscParams), C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
+    "wg_kajita_stream_destroy": (C.c_int, [C.c_void_p]),
+    "wg_kajita_stream_append": (C.c_int, [C.c_void_p, c_i64_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "wg_kajita_stream_sample_offsets": (c_i64_p, [C.c_void_p]),
+    "wg_kajita_stream_com_offsets": (c_i64_p, [C.c_void_p]),
+    "wg_kajita_stream_com_counts": (c_i64_p, [C.c_void_p]),
+    "wg_kajita_stream_run": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_void_p, C.c_int]),
+    "wg_kajita_stream_state": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "wg_dimitrov_default_params": (None, [C.POINTER(DimitrovParams)]),
     "wg_dimitrov_set_params": (C.c_int, [C.c_void_p, C.POINTER(DimitrovParams)] + [C.c_void_p] * 6),
     "wg_dimitrov_period_count": (C.c_int64, [C.POINTER(DimitrovParams), C.c_int64]),

@@ -1698,6 +1698,23 @@ int wg_preview_plan_destroy(wg_preview_plan *pl)
   return WG_OK;
 }
 
+// Internal (zmpdisc.cu, wg_kajita_stream): give the plan's B trajectories new offsets, in its own device array.  The copy is
+// asynchronous on the context stream: offsets_host must stay unchanged until the stream has passed it.
+int wgi_preview_plan_set_offsets(wg_preview_plan *pl, const int64_t *offsets_host)
+{
+  wg_ctx *ctx = pl->ctx;
+  int64_t total_steps = 0;
+  for (int b = 0; b < pl->B; ++b) {
+    const int64_t L = offsets_host[b + 1] - offsets_host[b];
+    if (L >= pl->NL) total_steps += L - pl->NL + 1;
+  }
+  pl->total_samples = pl->B > 0 ? offsets_host[pl->B] : 0;
+  pl->total_steps = total_steps;
+  if (pl->B > 0)
+    WG_CUDA(ctx, cudaMemcpyAsync(pl->d_offsets, offsets_host, sizeof(int64_t) * (pl->B + 1), cudaMemcpyHostToDevice, ctx->stream));
+  return WG_OK;
+}
+
 int64_t wg_preview_plan_total_steps(const wg_preview_plan *pl) { return pl ? pl->total_steps : 0; }
 int64_t wg_preview_plan_total_samples(const wg_preview_plan *pl) { return pl ? pl->total_samples : 0; }
 

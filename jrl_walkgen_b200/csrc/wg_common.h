@@ -111,6 +111,8 @@ extern "C" int wgi_smem_attr(wg_ctx *ctx, const void *func, size_t bytes);
 extern "C" int wgi_preview_launch_range(wg_ctx *ctx, wg_preview_plan *pl, const int *d_order, int count,
                                         const double *d_zmp, double *d_state, double *d_com, double *d_zmpout,
                                         int simulation, const double *d_com_add = nullptr, int pos_only = 0);
+// Replace the offsets of a plan's B trajectories (same B, no allocation); the copy is asynchronous on the context stream.
+extern "C" int wgi_preview_plan_set_offsets(wg_preview_plan *pl, const int64_t *offsets_host);
 
 // zmpdisc.cu / pldp.cu internals used by dimitrov.cu
 struct wgi_kajita_view {
