@@ -437,8 +437,7 @@ int wg_herdt_mpc_stats(wg_ctx *ctx, int B, const wg_herdt_mpc_state *d_states, d
  *   steps   : [B][nsteps] or NULL     per-period summaries
  *   qp_in   : [B] or NULL             the QP input of each instance's LAST period (workload capture)
  * Instances whose on-line mode ended (:stoppg + preview horizon elapsed) are left untouched.
- * A period is three kernel launches (FSM + QP record, the solver of wg_herdt_qp_solve_batch, interpolation + state update);
- * the environment variable WG_HERDT_MPC_SPLIT=0 selects the single fused kernel instead (same results, slower on large batches). */
+ * A period is three kernel launches (FSM + QP record, the solver of wg_herdt_qp_solve_batch, interpolation + state update). */
 int wg_herdt_mpc_run_batch(wg_ctx *ctx, int mem, int B, int nsteps, wg_herdt_mpc_state *states,
                            const double *vel_ref, wg_herdt_tick *ticks, wg_herdt_mpc_step *steps,
                            wg_herdt_qp_input *qp_in);

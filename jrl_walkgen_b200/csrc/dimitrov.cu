@@ -72,18 +72,6 @@ DimHost *dim_of(wg_ctx *ctx)
   return static_cast<DimHost *>(ctx->dimitrov);
 }
 
-int dm_ensure(wg_ctx *ctx, DimHost *p, int slot, size_t bytes)
-{
-  if (p->cap[slot] >= bytes && p->buf[slot]) return WG_OK;
-  WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  cudaFree(p->buf[slot]);
-  p->buf[slot] = nullptr; p->cap[slot] = 0;
-  if (slot == 12) p->order_plan = nullptr;
-  WG_CUDA(ctx, cudaMalloc(&p->buf[slot], bytes ? bytes : 8));
-  p->cap[slot] = bytes;
-  return WG_OK;
-}
-
 // ---------------------------------------------------------------------------------------------------------------
 // Convex hull and half-plane form (device; one thread)
 // ---------------------------------------------------------------------------------------------------------------
@@ -707,7 +695,7 @@ extern "C" int wgi_fcals_launch(wg_ctx *ctx, int B, const int64_t *d_samp_off, c
   if (!H->ready) H->par.sampling_period = sampling_period;     // clock table only
   int rc = ensure_clock(ctx, H, max_n);
   if (rc != WG_OK) return rc;
-  if ((rc = dm_ensure(ctx, H, 13, sizeof(DimConsts))) != WG_OK) return rc;
+  if ((rc = wgi_grow_scratch(ctx, &H->buf[13], &H->cap[13], sizeof(DimConsts))) != WG_OK) return rc;
   DimConsts alt;
   std::memset(&alt, 0, sizeof alt);
   alt.hw = hw; alt.hh = hh; alt.merge_rows = 0;
@@ -789,9 +777,9 @@ int wg_convex_hull_batch(wg_ctx *ctx, int mem, int B, int n, const double *xy, d
   const size_t nb = (size_t)B;
   if (mem == WG_MEM_HOST) {
     int rc;
-    if ((rc = dm_ensure(ctx, H, 0, sizeof(double) * 2 * n * nb)) != WG_OK) return rc;
-    if ((rc = dm_ensure(ctx, H, 1, sizeof(double) * 16 * nb)) != WG_OK) return rc;
-    if ((rc = dm_ensure(ctx, H, 2, sizeof(int32_t) * nb)) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, &H->buf[0], &H->cap[0], sizeof(double) * 2 * n * nb)) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, &H->buf[1], &H->cap[1], sizeof(double) * 16 * nb)) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, &H->buf[2], &H->cap[2], sizeof(int32_t) * nb)) != WG_OK) return rc;
     WG_CUDA(ctx, cudaMemcpyAsync(H->buf[0], xy, sizeof(double) * 2 * n * nb, cudaMemcpyHostToDevice, ctx->stream));
     dxy = static_cast<const double *>(H->buf[0]); dh = static_cast<double *>(H->buf[1]); dc = static_cast<int32_t *>(H->buf[2]);
   } else if (mem != WG_MEM_DEVICE) return WG_ERR_INVALID;
@@ -825,17 +813,17 @@ int wg_fcals_build_batch(wg_ctx *ctx, int mem, int B, const int64_t *sample_offs
   int rc;
   if ((rc = ensure_clock(ctx, H, (size_t)max_n)) != WG_OK) return rc;
   const size_t ns = (size_t)sample_offsets[B], nl = (size_t)lci_offsets[B], nb = (size_t)B;
-  if ((rc = dm_ensure(ctx, H, 3, sizeof(int64_t) * 2 * (nb + 1))) != WG_OK) return rc;
+  if ((rc = wgi_grow_scratch(ctx, &H->buf[3], &H->cap[3], sizeof(int64_t) * 2 * (nb + 1))) != WG_OK) return rc;
   int64_t *d_so = static_cast<int64_t *>(H->buf[3]), *d_lo = d_so + (nb + 1);
   WG_CUDA(ctx, cudaMemcpyAsync(d_so, sample_offsets, sizeof(int64_t) * (nb + 1), cudaMemcpyHostToDevice, ctx->stream));
   WG_CUDA(ctx, cudaMemcpyAsync(d_lo, lci_offsets, sizeof(int64_t) * (nb + 1), cudaMemcpyHostToDevice, ctx->stream));
   const wg_foot_sample *dl = left, *dr = right; const int32_t *dt = step_type; wg_lci *dp = lci; int32_t *dn = n_lci;
   if (mem == WG_MEM_HOST) {
-    if ((rc = dm_ensure(ctx, H, 4, sizeof(wg_foot_sample) * ns)) != WG_OK) return rc;
-    if ((rc = dm_ensure(ctx, H, 5, sizeof(wg_foot_sample) * ns)) != WG_OK) return rc;
-    if ((rc = dm_ensure(ctx, H, 6, sizeof(int32_t) * 3 * ns)) != WG_OK) return rc;
-    if ((rc = dm_ensure(ctx, H, 7, sizeof(wg_lci) * std::max<size_t>(nl, 1))) != WG_OK) return rc;
-    if ((rc = dm_ensure(ctx, H, 8, sizeof(int32_t) * nb)) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, &H->buf[4], &H->cap[4], sizeof(wg_foot_sample) * ns)) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, &H->buf[5], &H->cap[5], sizeof(wg_foot_sample) * ns)) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, &H->buf[6], &H->cap[6], sizeof(int32_t) * 3 * ns)) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, &H->buf[7], &H->cap[7], sizeof(wg_lci) * std::max<size_t>(nl, 1))) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, &H->buf[8], &H->cap[8], sizeof(int32_t) * nb)) != WG_OK) return rc;
     WG_CUDA(ctx, cudaMemcpyAsync(H->buf[4], left, sizeof(wg_foot_sample) * ns, cudaMemcpyHostToDevice, ctx->stream));
     WG_CUDA(ctx, cudaMemcpyAsync(H->buf[5], right, sizeof(wg_foot_sample) * ns, cudaMemcpyHostToDevice, ctx->stream));
     WG_CUDA(ctx, cudaMemcpyAsync(H->buf[6], step_type, sizeof(int32_t) * 3 * ns, cudaMemcpyHostToDevice, ctx->stream));
@@ -900,9 +888,9 @@ int wg_dimitrov_run_batch(wg_ctx *ctx, wg_kajita_plan *plan, int mem, double *co
   if ((rc = ensure_clock(ctx, H, (size_t)max_n)) != WG_OK) return rc;
   const size_t nl = (size_t)lci_off[B];
   const size_t npr = periods ? (size_t)period_offsets[B] : 0;
-  if ((rc = dm_ensure(ctx, H, 3, sizeof(int64_t) * 2 * (nb + 1))) != WG_OK) return rc;
-  if ((rc = dm_ensure(ctx, H, 7, sizeof(wg_lci) * nl)) != WG_OK) return rc;
-  if ((rc = dm_ensure(ctx, H, 8, sizeof(int32_t) * 3 * nb)) != WG_OK) return rc;
+  if ((rc = wgi_grow_scratch(ctx, &H->buf[3], &H->cap[3], sizeof(int64_t) * 2 * (nb + 1))) != WG_OK) return rc;
+  if ((rc = wgi_grow_scratch(ctx, &H->buf[7], &H->cap[7], sizeof(wg_lci) * nl)) != WG_OK) return rc;
+  if ((rc = wgi_grow_scratch(ctx, &H->buf[8], &H->cap[8], sizeof(int32_t) * 3 * nb)) != WG_OK) return rc;
   int64_t *d_lo = static_cast<int64_t *>(H->buf[3]), *d_po = d_lo + (nb + 1);
   wg_lci *d_lci = static_cast<wg_lci *>(H->buf[7]);
   int32_t *d_nlci = static_cast<int32_t *>(H->buf[8]), *d_status = d_nlci + nb, *d_done = d_status + nb;
@@ -913,8 +901,15 @@ int wg_dimitrov_run_batch(wg_ctx *ctx, wg_kajita_plan *plan, int mem, double *co
   int32_t *d_st = status ? status : d_status, *d_dn = periods_done ? periods_done : d_done;
   if (host) {
     d_com = nullptr;
-    if (com_out) { if ((rc = dm_ensure(ctx, H, 9, sizeof(double) * 6 * ns)) != WG_OK) return rc; d_com = static_cast<double *>(H->buf[9]); }
-    if (periods) { if ((rc = dm_ensure(ctx, H, 10, sizeof(wg_dimitrov_period) * std::max<size_t>(npr, 1))) != WG_OK) return rc; d_per = static_cast<wg_dimitrov_period *>(H->buf[10]); }
+    if (com_out) {
+      if ((rc = wgi_grow_scratch(ctx, &H->buf[9], &H->cap[9], sizeof(double) * 6 * ns)) != WG_OK) return rc;
+      d_com = static_cast<double *>(H->buf[9]);
+    }
+    if (periods) {
+      if ((rc = wgi_grow_scratch(ctx, &H->buf[10], &H->cap[10], sizeof(wg_dimitrov_period) * std::max<size_t>(npr, 1))) != WG_OK)
+        return rc;
+      d_per = static_cast<wg_dimitrov_period *>(H->buf[10]);
+    }
     d_st = d_status; d_dn = d_done;
   }
   if (d_com) WG_CUDA(ctx, cudaMemsetAsync(d_com, 0, sizeof(double) * 6 * ns, ctx->stream));
@@ -923,11 +918,13 @@ int wg_dimitrov_run_batch(wg_ctx *ctx, wg_kajita_plan *plan, int mem, double *co
   if ((rc = launch_fcals(ctx, H, B, V.d_samp_off, d_left, d_right, d_types, d_lo, d_lci, d_nlci)) != WG_OK) return rc;
   // ---- the loop
   const int grid = std::max(1, std::min((B + DM_WARPS - 1) / DM_WARPS, ctx->sm_count * 3));
-  if ((rc = dm_ensure(ctx, H, 11, 64)) != WG_OK) return rc;
+  if ((rc = wgi_grow_scratch(ctx, &H->buf[11], &H->cap[11], 64)) != WG_OK) return rc;
   int *d_next = static_cast<int *>(H->buf[11]);
   WG_CUDA(ctx, cudaMemsetAsync(d_next, 0, sizeof(int), ctx->stream));
   // longest-processing-time-first order (the sample count is a faithful proxy of the period count); uploaded once per plan
-  if ((rc = dm_ensure(ctx, H, 12, sizeof(int) * nb)) != WG_OK) return rc;
+  const size_t order_cap = H->cap[12];
+  if ((rc = wgi_grow_scratch(ctx, &H->buf[12], &H->cap[12], sizeof(int) * nb)) != WG_OK) return rc;
+  if (H->cap[12] != order_cap) H->order_plan = nullptr;   // a new buffer holds no order yet
   if (H->order_plan != plan || H->order_B != B || H->order_total != (int64_t)ns) {
     std::vector<int> order(B);
     for (int b = 0; b < B; ++b) order[b] = b;

@@ -15,15 +15,14 @@ struct HerdtState {
   Consts *d_consts = nullptr;
   bool ready = false;
   // staging for WG_MEM_HOST calls
-  wg_herdt_qp_input *d_in = nullptr;
-  wg_herdt_qp_output *d_out = nullptr;
-  int cap = 0;
+  wg_herdt_qp_input *d_in = nullptr; size_t cap_in = 0;
+  wg_herdt_qp_output *d_out = nullptr; size_t cap_out = 0;
   int *d_next = nullptr;          // work counter of herdt_qp_kernel
   double *d_T = nullptr; size_t cap_T = 0;   // per-warp T slices
-  wg_herdt_active_set *d_act = nullptr; int cap_act = 0;   // staging of the warm-start sets (WG_MEM_HOST)
+  wg_herdt_active_set *d_act = nullptr; size_t cap_act = 0;   // staging of the warm-start sets (WG_MEM_HOST)
   // WG_MEM_HOST pipeline: upload / download streams and per-chunk events
   cudaStream_t up = nullptr, down = nullptr;
-  cudaEvent_t ev_up[8] = {nullptr}, ev_k[8] = {nullptr}, ev0 = nullptr;
+  cudaEvent_t ev_up[2] = {nullptr}, ev_k[2] = {nullptr}, ev0 = nullptr;
 };
 
 HerdtState *state_of(wg_ctx *ctx)
@@ -192,7 +191,7 @@ void wg_herdt_release(wg_ctx *ctx)
   cudaFree(st->d_consts); cudaFree(st->d_in); cudaFree(st->d_out); cudaFree(st->d_next); cudaFree(st->d_T); cudaFree(st->d_act);
   if (st->up) cudaStreamDestroy(st->up);
   if (st->down) cudaStreamDestroy(st->down);
-  for (int c = 0; c < 8; ++c) { if (st->ev_up[c]) cudaEventDestroy(st->ev_up[c]); if (st->ev_k[c]) cudaEventDestroy(st->ev_k[c]); }
+  for (int c = 0; c < 2; ++c) { if (st->ev_up[c]) cudaEventDestroy(st->ev_up[c]); if (st->ev_k[c]) cudaEventDestroy(st->ev_k[c]); }
   if (st->ev0) cudaEventDestroy(st->ev0);
   delete st;
   ctx->herdt = nullptr;
@@ -254,13 +253,8 @@ static int herdt_launch(wg_ctx *ctx, HerdtState *st, int B, const wg_herdt_qp_in
   const int cap = ctx->sm_count * per_sm;
   if (blocks > cap) blocks = cap;   // persistent: a multiple of the SM count, grid-stride over instances
   if (!st->d_next) WG_CUDA(ctx, cudaMalloc(&st->d_next, sizeof(int)));
-  const size_t needT = (size_t)blocks * QP_WARPS * herdt::TRI;
-  if (st->cap_T < needT) {
-    WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    cudaFree(st->d_T); st->d_T = nullptr; st->cap_T = 0;
-    WG_CUDA(ctx, cudaMalloc(&st->d_T, sizeof(double) * needT));
-    st->cap_T = needT;
-  }
+  int rc = wgi_grow_scratch(ctx, reinterpret_cast<void **>(&st->d_T), &st->cap_T, sizeof(double) * blocks * QP_WARPS * herdt::TRI);
+  if (rc != WG_OK) return rc;
   WG_CUDA(ctx, cudaMemsetAsync(st->d_next, 0, sizeof(int), ctx->stream));
   wg_prof_start(ctx, WG_K_HERDT_QP);
   herdt_qp_kernel<<<blocks, QP_WARPS * 32, smem, ctx->stream>>>(B, st->d_consts, d_in, d_out, st->d_next, st->d_T, opt);
@@ -278,27 +272,22 @@ int wg_herdt_qp_solve_batch(wg_ctx *ctx, int mem, int B, const wg_herdt_qp_input
   wg_device_guard guard(ctx->device);
   if (mem == WG_MEM_DEVICE) return herdt_launch(ctx, st, B, in, out);
   if (mem != WG_MEM_HOST) return WG_ERR_INVALID;
-  if (st->cap < B) {
-    WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    cudaFree(st->d_in); cudaFree(st->d_out);
-    st->d_in = nullptr; st->d_out = nullptr; st->cap = 0;
-    WG_CUDA(ctx, cudaMalloc(&st->d_in, sizeof(wg_herdt_qp_input) * (size_t)B));
-    WG_CUDA(ctx, cudaMalloc(&st->d_out, sizeof(wg_herdt_qp_output) * (size_t)B));
-    st->cap = B;
-  }
-  // two or three large chunks (small launches waste the tail of the persistent grid: 8 chunks of 2048 measured 18 % SLOWER than
+  int rc;
+  if ((rc = wgi_grow_scratch(ctx, reinterpret_cast<void **>(&st->d_in), &st->cap_in, sizeof(wg_herdt_qp_input) * (size_t)B)) != WG_OK ||
+      (rc = wgi_grow_scratch(ctx, reinterpret_cast<void **>(&st->d_out), &st->cap_out, sizeof(wg_herdt_qp_output) * (size_t)B)) != WG_OK)
+    return rc;
+  // at most two large chunks (small launches waste the tail of the persistent grid: 8 chunks of 2048 measured 18 % SLOWER than
   // the unpipelined call): the upload of chunk c+1 and the download of chunk c-1 overlap the kernel of chunk c
   if (!st->up) {
     WG_CUDA(ctx, cudaStreamCreateWithFlags(&st->up, cudaStreamNonBlocking));
     WG_CUDA(ctx, cudaStreamCreateWithFlags(&st->down, cudaStreamNonBlocking));
-    for (int c = 0; c < 8; ++c) {
+    for (int c = 0; c < 2; ++c) {
       WG_CUDA(ctx, cudaEventCreateWithFlags(&st->ev_up[c], cudaEventDisableTiming));
       WG_CUDA(ctx, cudaEventCreateWithFlags(&st->ev_k[c], cudaEventDisableTiming));
     }
     WG_CUDA(ctx, cudaEventCreateWithFlags(&st->ev0, cudaEventDisableTiming));
   }
-  static const int want = getenv("WG_HERDT_CHUNKS") ? atoi(getenv("WG_HERDT_CHUNKS")) : 2;
-  const int nch = std::max(1, std::min(std::min(8, want), B / 4096));
+  const int nch = std::max(1, std::min(2, B / 4096));
   WG_CUDA(ctx, cudaEventRecord(st->ev0, ctx->stream));
   WG_CUDA(ctx, cudaStreamWaitEvent(st->up, st->ev0, 0));
   for (int c = 0; c < nch; ++c) {
@@ -306,8 +295,7 @@ int wg_herdt_qp_solve_batch(wg_ctx *ctx, int mem, int B, const wg_herdt_qp_input
     WG_CUDA(ctx, cudaMemcpyAsync(st->d_in + b0, in + b0, sizeof(wg_herdt_qp_input) * (b1 - b0), cudaMemcpyHostToDevice, st->up));
     WG_CUDA(ctx, cudaEventRecord(st->ev_up[c], st->up));
     WG_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, st->ev_up[c], 0));
-    int rc = herdt_launch(ctx, st, (int)(b1 - b0), st->d_in + b0, st->d_out + b0);
-    if (rc != WG_OK) return rc;
+    if ((rc = herdt_launch(ctx, st, (int)(b1 - b0), st->d_in + b0, st->d_out + b0)) != WG_OK) return rc;
     WG_CUDA(ctx, cudaEventRecord(st->ev_k[c], ctx->stream));
     WG_CUDA(ctx, cudaStreamWaitEvent(st->down, st->ev_k[c], 0));
     WG_CUDA(ctx, cudaMemcpyAsync(out + b0, st->d_out + b0, sizeof(wg_herdt_qp_output) * (b1 - b0), cudaMemcpyDeviceToHost, st->down));
@@ -334,27 +322,19 @@ int wg_herdt_qp_solve_batch_warm(wg_ctx *ctx, int mem, int B, const wg_herdt_qp_
     return herdt_launch(ctx, st, B, in, out, opt);
   }
   if (mem != WG_MEM_HOST) return WG_ERR_INVALID;
-  if (st->cap < B) {
-    WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    cudaFree(st->d_in); cudaFree(st->d_out);
-    st->d_in = nullptr; st->d_out = nullptr; st->cap = 0;
-    WG_CUDA(ctx, cudaMalloc(&st->d_in, sizeof(wg_herdt_qp_input) * (size_t)B));
-    WG_CUDA(ctx, cudaMalloc(&st->d_out, sizeof(wg_herdt_qp_output) * (size_t)B));
-    st->cap = B;
-  }
-  if (st->cap_act < B) {
-    WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    cudaFree(st->d_act); st->d_act = nullptr; st->cap_act = 0;
-    WG_CUDA(ctx, cudaMalloc(&st->d_act, sizeof(wg_herdt_active_set) * (size_t)B));
-    st->cap_act = B;
-  }
+  int rc;
+  if ((rc = wgi_grow_scratch(ctx, reinterpret_cast<void **>(&st->d_in), &st->cap_in, sizeof(wg_herdt_qp_input) * (size_t)B)) != WG_OK ||
+      (rc = wgi_grow_scratch(ctx, reinterpret_cast<void **>(&st->d_out), &st->cap_out, sizeof(wg_herdt_qp_output) * (size_t)B)) != WG_OK)
+    return rc;
+  if ((rc = wgi_grow_scratch(ctx, reinterpret_cast<void **>(&st->d_act), &st->cap_act, sizeof(wg_herdt_active_set) * (size_t)B)) != WG_OK)
+    return rc;
   WG_CUDA(ctx, cudaMemcpyAsync(st->d_in, in, sizeof(wg_herdt_qp_input) * (size_t)B, cudaMemcpyHostToDevice, ctx->stream));
   if (guess) {
     WG_CUDA(ctx, cudaMemcpyAsync(st->d_act, guess, sizeof(wg_herdt_active_set) * (size_t)B, cudaMemcpyHostToDevice, ctx->stream));
     opt.guess = reinterpret_cast<const unsigned char *>(st->d_act);
   }
   opt.active_out = reinterpret_cast<unsigned char *>(st->d_act);
-  int rc = herdt_launch(ctx, st, B, st->d_in, st->d_out, opt);
+  rc = herdt_launch(ctx, st, B, st->d_in, st->d_out, opt);
   if (rc != WG_OK) return rc;
   WG_CUDA(ctx, cudaMemcpyAsync(out, st->d_out, sizeof(wg_herdt_qp_output) * (size_t)B, cudaMemcpyDeviceToHost, ctx->stream));
   if (active_out)

@@ -342,8 +342,8 @@ static __device__ __noinline__ void warm_start(Work &s, double *__restrict__ T, 
 
 // Build and solve the QP of the instance in s.in.  On return s.jr / s.ff hold the solution, s.u / s.W / q the
 // multipliers of the active rows.  All 32 lanes of the warp must call.
-// T: [TRI] doubles of scratch for the inverse Cholesky factor of the active Gram matrix, private to the warp (shared or
-// global memory: the open-loop kernel keeps it in global memory to fit 16 warps/SM).
+// T: [TRI] doubles of scratch for the inverse Cholesky factor of the active Gram matrix, private to the warp, in global
+// memory (herdt_qp_kernel keeps it there to fit 16 warps/SM).
 __device__ inline Result solve_warp(Work &s, const Consts &C, int lane, int &q_out, double *__restrict__ T,
                                     const wg_herdt_active_set *__restrict__ hint = nullptr, int hint_age = 1)
 {

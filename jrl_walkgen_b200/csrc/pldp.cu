@@ -247,17 +247,6 @@ PldpHost *pldp_of(wg_ctx *ctx)
   return static_cast<PldpHost *>(ctx->pldp);
 }
 
-int ensure(wg_ctx *ctx, PldpHost *p, int slot, size_t bytes)
-{
-  if (p->cap[slot] >= bytes) return WG_OK;
-  WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  cudaFree(p->buf[slot]);
-  p->buf[slot] = nullptr; p->cap[slot] = 0;
-  WG_CUDA(ctx, cudaMalloc(&p->buf[slot], bytes ? bytes : 8));
-  p->cap[slot] = bytes;
-  return WG_OK;
-}
-
 int grid_for(wg_ctx *ctx, int B, int warps) { int g = (B + warps - 1) / warps; int cap = ctx->sm_count * 8; return g < cap ? (g > 0 ? g : 1) : cap; }
 
 }  // namespace
@@ -411,13 +400,13 @@ static int pldp_solve_impl(wg_ctx *ctx, int mem, int B, const wg_pldp_batch *pb,
       {8, pb->starting, pb->starting ? sizeof(int) : 0, (const void **)&d.starting}};
   for (const Item &it : in) {
     if (!it.src) continue;
-    int rc = ensure(ctx, p, it.slot, it.per * nb);
+    int rc = wgi_grow_scratch(ctx, &p->buf[it.slot], &p->cap[it.slot], it.per * nb);
     if (rc != WG_OK) return rc;
     *it.dst = p->buf[it.slot];
   }
   // outputs + hot-start state share one allocation: X | info | hot
   const size_t ox = 0, oi = ox + sizeof(double) * PLDP_U * nb, oh = oi + sizeof(wg_pldp_info) * nb;
-  int rc = ensure(ctx, p, 9, oh + sizeof(wg_pldp_state) * nb);
+  int rc = wgi_grow_scratch(ctx, &p->buf[9], &p->cap[9], oh + sizeof(wg_pldp_state) * nb);
   if (rc != WG_OK) return rc;
   char *base = static_cast<char *>(p->buf[9]);
   d.X = reinterpret_cast<double *>(base + ox);
@@ -484,9 +473,9 @@ int wg_optcholesky_add_rows_batch(wg_ctx *ctx, int mem, int B, int mode, int nb_
   const size_t nb = (size_t)B;
   if (mem == WG_MEM_HOST) {
     int rc;
-    if ((rc = ensure(ctx, p, 2, sizeof(double) * (size_t)a_stride * nb)) != WG_OK) return rc;
-    if ((rc = ensure(ctx, p, 6, sizeof(int) * (size_t)rows_stride * nb)) != WG_OK) return rc;
-    if ((rc = ensure(ctx, p, 9, sizeof(double) * (size_t)l_stride * nb)) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, &p->buf[2], &p->cap[2], sizeof(double) * (size_t)a_stride * nb)) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, &p->buf[6], &p->cap[6], sizeof(int) * (size_t)rows_stride * nb)) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, &p->buf[9], &p->cap[9], sizeof(double) * (size_t)l_stride * nb)) != WG_OK) return rc;
     WG_CUDA(ctx, cudaMemcpyAsync(p->buf[2], A, sizeof(double) * (size_t)a_stride * nb, cudaMemcpyHostToDevice, ctx->stream));
     WG_CUDA(ctx, cudaMemcpyAsync(p->buf[6], rows, sizeof(int) * (size_t)rows_stride * nb, cudaMemcpyHostToDevice, ctx->stream));
     WG_CUDA(ctx, cudaMemcpyAsync(p->buf[9], L, sizeof(double) * (size_t)l_stride * nb, cudaMemcpyHostToDevice, ctx->stream));
@@ -516,8 +505,8 @@ int wg_optcholesky_full_batch(wg_ctx *ctx, int mem, int B, int n, const double *
   const double *dA = A; double *dL = L, *diL = iL;
   if (mem == WG_MEM_HOST) {
     int rc;
-    if ((rc = ensure(ctx, p, 2, bytes)) != WG_OK) return rc;
-    if ((rc = ensure(ctx, p, 9, 2 * bytes)) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, &p->buf[2], &p->cap[2], bytes)) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, &p->buf[9], &p->cap[9], 2 * bytes)) != WG_OK) return rc;
     if (A) WG_CUDA(ctx, cudaMemcpyAsync(p->buf[2], A, bytes, cudaMemcpyHostToDevice, ctx->stream));
     dL = static_cast<double *>(p->buf[9]); diL = iL ? dL + (size_t)n * n * B : nullptr;
     WG_CUDA(ctx, cudaMemcpyAsync(dL, L, bytes, cudaMemcpyHostToDevice, ctx->stream));

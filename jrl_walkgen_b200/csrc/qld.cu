@@ -56,17 +56,6 @@ QldState *state_of(wg_ctx *ctx)
   return static_cast<QldState *>(ctx->qld);
 }
 
-int ensure(wg_ctx *ctx, void **p, size_t *cap, size_t bytes)
-{
-  if (*cap >= bytes) return WG_OK;
-  WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  cudaFree(*p);
-  *p = nullptr; *cap = 0;
-  WG_CUDA(ctx, cudaMalloc(p, bytes));
-  *cap = bytes;
-  return WG_OK;
-}
-
 __device__ __forceinline__ int tri(int i) { return (i * (i + 1)) >> 1; }
 
 __device__ __forceinline__ double warp_sum(double v)
@@ -879,7 +868,7 @@ static int qld_solve_impl(wg_ctx *ctx, int mem, int B, const wg_qld_batch *q, co
     const size_t o_u = off; off += al(szu);
     const size_t o_f = off; off += al(sz_m);
     const size_t o_it = off; off += al(sz_m);
-    if ((rc = ensure(ctx, &st->d_stage, &st->cap_stage, off)) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, &st->d_stage, &st->cap_stage, off)) != WG_OK) return rc;
     char *base = static_cast<char *>(st->d_stage);
     auto up = [&](size_t o, const void *src, size_t bytes) -> cudaError_t {
       return bytes ? cudaMemcpyAsync(base + o, src, bytes, cudaMemcpyHostToDevice, ctx->stream) : cudaSuccess;
@@ -919,8 +908,8 @@ static int qld_solve_impl(wg_ctx *ctx, int mem, int B, const wg_qld_batch *q, co
     a.S = sh.d_hinv; a.h_stride = 0; a.hfail = nullptr;
     a.C = sh.d_c; a.c_stride = 0;
   } else {
-    if ((rc = ensure(ctx, reinterpret_cast<void **>(&st->d_hinv), &st->cap_hinv, sizeof(double) * nb * n * n)) != WG_OK) return rc;
-    if ((rc = ensure(ctx, reinterpret_cast<void **>(&st->d_fail), &st->cap_fail, sizeof(int) * nb)) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, reinterpret_cast<void **>(&st->d_hinv), &st->cap_hinv, sizeof(double) * nb * n * n)) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, reinterpret_cast<void **>(&st->d_fail), &st->cap_fail, sizeof(int) * nb)) != WG_OK) return rc;
     if ((rc = hinv_launch(ctx, B, n, nmax, d.C, (long long)nmax * n, st->d_hinv, st->d_fail, q->eps)) != WG_OK) return rc;
     a.S = st->d_hinv; a.h_stride = (long long)n * n; a.hfail = st->d_fail;
     a.C = d.C; a.c_stride = (long long)nmax * n;
@@ -937,7 +926,9 @@ static int qld_solve_impl(wg_ctx *ctx, int mem, int B, const wg_qld_batch *q, co
   if (per_sm < 1) per_sm = 1;
   const int blocks = std::max(1, std::min(B, ctx->sm_count * per_sm));
   a.work_stride = (long long)n * a.qcap + (long long)a.qcap * (a.qcap + 1) / 2;
-  if ((rc = ensure(ctx, reinterpret_cast<void **>(&st->d_work), &st->cap_work, sizeof(double) * (size_t)blocks * a.work_stride)) != WG_OK) return rc;
+  if ((rc = wgi_grow_scratch(ctx, reinterpret_cast<void **>(&st->d_work), &st->cap_work,
+                             sizeof(double) * (size_t)blocks * a.work_stride)) != WG_OK)
+    return rc;
   a.work = st->d_work;
   if (!st->d_next) WG_CUDA(ctx, cudaMalloc(&st->d_next, sizeof(int)));
   a.next = st->d_next;

@@ -106,6 +106,11 @@ extern "C" int wgi_smem_attr(wg_ctx *ctx, const void *func, size_t bytes);
     if (rc__ != WG_OK) return rc__;                                                 \
   } while (0)
 
+// Grow-only device scratch: make *buf hold at least `bytes` (8 for a zero-byte request), *cap being its size in bytes.  A
+// buffer that must grow is freed after the context stream drains (earlier launches may still read it); on return *buf is
+// never null.
+extern "C" int wgi_grow_scratch(wg_ctx *ctx, void **buf, size_t *cap, size_t bytes);
+
 // preview.cu internals used by zmpdisc.cu (the footsteps -> CoM pipeline): launch the fused preview kernel over `count`
 // trajectories listed in the device array d_order.
 extern "C" int wgi_preview_launch_range(wg_ctx *ctx, wg_preview_plan *pl, const int *d_order, int count,

@@ -31,6 +31,18 @@ extern "C" int wgi_smem_attr(wg_ctx *ctx, const void *func, size_t bytes)
   return WG_OK;
 }
 
+extern "C" int wgi_grow_scratch(wg_ctx *ctx, void **buf, size_t *cap, size_t bytes)
+{
+  bytes = std::max<size_t>(bytes, 8);
+  if (*buf && *cap >= bytes) return WG_OK;
+  WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  cudaFree(*buf);
+  *buf = nullptr; *cap = 0;
+  WG_CUDA(ctx, cudaMalloc(buf, bytes));
+  *cap = bytes;
+  return WG_OK;
+}
+
 extern "C" {
 
 int wg_version(void) { return WG_VERSION; }

@@ -61,17 +61,6 @@ WbHost *wb_of(wg_ctx *ctx)
   return static_cast<WbHost *>(ctx->wieber);
 }
 
-int wb_ensure(wg_ctx *ctx, WbHost *p, int slot, size_t bytes)
-{
-  if (p->cap[slot] >= bytes && p->buf[slot]) return WG_OK;
-  WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  cudaFree(p->buf[slot]);
-  p->buf[slot] = nullptr; p->cap[slot] = 0;
-  WG_CUDA(ctx, cudaMalloc(&p->buf[slot], bytes ? bytes : 8));
-  p->cap[slot] = bytes;
-  return WG_OK;
-}
-
 // ---------------------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(WB_T)
 wieber_pre_kernel(int B, const WbConsts *__restrict__ Kp, const int64_t *__restrict__ samp_off,
@@ -420,15 +409,15 @@ int wg_wieber_run_batch(wg_ctx *ctx, wg_kajita_plan *plan, int mem, double *com_
     WG_CUDA(ctx, cudaMemcpy(H->d_start, H->start_h.data(), sizeof(double) * H->start_h.size(), cudaMemcpyHostToDevice));
   }
   const size_t nl = (size_t)lci_off[B];
-  if ((rc = wb_ensure(ctx, H, 0, sizeof(int64_t) * (nb + 1))) != WG_OK) return rc;
-  if ((rc = wb_ensure(ctx, H, 1, sizeof(wg_lci) * nl)) != WG_OK) return rc;
-  if ((rc = wb_ensure(ctx, H, 2, sizeof(int32_t) * 4 * nb)) != WG_OK) return rc;
-  if ((rc = wb_ensure(ctx, H, 3, sizeof(WbWalk) * nb)) != WG_OK) return rc;
-  if ((rc = wb_ensure(ctx, H, 4, sizeof(double) * nb * ld)) != WG_OK) return rc;
+  if ((rc = wgi_grow_scratch(ctx, &H->buf[0], &H->cap[0], sizeof(int64_t) * (nb + 1))) != WG_OK) return rc;
+  if ((rc = wgi_grow_scratch(ctx, &H->buf[1], &H->cap[1], sizeof(wg_lci) * nl)) != WG_OK) return rc;
+  if ((rc = wgi_grow_scratch(ctx, &H->buf[2], &H->cap[2], sizeof(int32_t) * 4 * nb)) != WG_OK) return rc;
+  if ((rc = wgi_grow_scratch(ctx, &H->buf[3], &H->cap[3], sizeof(WbWalk) * nb)) != WG_OK) return rc;
+  if ((rc = wgi_grow_scratch(ctx, &H->buf[4], &H->cap[4], sizeof(double) * nb * ld)) != WG_OK) return rc;
   const bool dense = par.materialize_pu != 0;
-  if (dense) { if ((rc = wb_ensure(ctx, H, 5, sizeof(double) * nb * ld * nv)) != WG_OK) return rc; }
-  else { if ((rc = wb_ensure(ctx, H, 9, (sizeof(double) * 2 + 1) * nb * ld + 64)) != WG_OK) return rc; }
-  if ((rc = wb_ensure(ctx, H, 6, sizeof(double) * nb * nv * 2)) != WG_OK) return rc;
+  if (dense) { if ((rc = wgi_grow_scratch(ctx, &H->buf[5], &H->cap[5], sizeof(double) * nb * ld * nv)) != WG_OK) return rc; }
+  else { if ((rc = wgi_grow_scratch(ctx, &H->buf[9], &H->cap[9], (sizeof(double) * 2 + 1) * nb * ld + 64)) != WG_OK) return rc; }
+  if ((rc = wgi_grow_scratch(ctx, &H->buf[6], &H->cap[6], sizeof(double) * nb * nv * 2)) != WG_OK) return rc;
   int64_t *d_lo = static_cast<int64_t *>(H->buf[0]);
   wg_lci *d_lci = static_cast<wg_lci *>(H->buf[1]);
   int32_t *d_nlci = static_cast<int32_t *>(H->buf[2]), *d_m = d_nlci + nb, *d_ifail = d_m + nb, *d_it = d_ifail + nb;
@@ -441,7 +430,10 @@ int wg_wieber_run_batch(wg_ctx *ctx, wg_kajita_plan *plan, int mem, double *com_
   WG_CUDA(ctx, cudaMemcpyAsync(d_lo, lci_off.data(), sizeof(int64_t) * (nb + 1), cudaMemcpyHostToDevice, ctx->stream));
   WG_CUDA(ctx, cudaMemsetAsync(d_walks, 0, sizeof(WbWalk) * nb, ctx->stream));
   double *d_com = com_out;
-  if (host && com_out) { if ((rc = wb_ensure(ctx, H, 7, sizeof(double) * 6 * ns)) != WG_OK) return rc; d_com = static_cast<double *>(H->buf[7]); }
+  if (host && com_out) {
+    if ((rc = wgi_grow_scratch(ctx, &H->buf[7], &H->cap[7], sizeof(double) * 6 * ns)) != WG_OK) return rc;
+    d_com = static_cast<double *>(H->buf[7]);
+  }
   if (d_com) WG_CUDA(ctx, cudaMemsetAsync(d_com, 0, sizeof(double) * 6 * ns, ctx->stream));
   // ---- BuildLinearConstraintInequalities (:229-502)
   const double *d_clock = nullptr;
@@ -474,7 +466,7 @@ int wg_wieber_run_batch(wg_ctx *ctx, wg_kajita_plan *plan, int mem, double *com_
   int32_t *d_status = status, *d_done = periods_done;
   long long *d_iter = qp_iterations;
   if (host) {
-    if ((rc = wb_ensure(ctx, H, 8, (sizeof(int32_t) * 2 + sizeof(long long)) * nb)) != WG_OK) return rc;
+    if ((rc = wgi_grow_scratch(ctx, &H->buf[8], &H->cap[8], (sizeof(int32_t) * 2 + sizeof(long long)) * nb)) != WG_OK) return rc;
     d_iter = static_cast<long long *>(H->buf[8]);
     d_status = reinterpret_cast<int32_t *>(d_iter + nb); d_done = d_status + nb;
   }
