@@ -1045,13 +1045,28 @@ preview_rec_kernel(const int *__restrict__ order, const int64_t *__restrict__ of
 //     (400-byte stride: conflict-free 128-bit stores) and hands them over with ONE cp.async.bulk request per tile.  A warp-wide
 //     256-bit store of this row layout touches 32 different 128-byte lines, and the LSU tag stage - not HBM - was what the stores
 //     cost; measured on configs[1]: 39.2 G steps/s with direct stores, 42.4 with one request per tick pair (16 warps/SM), 43.8 per
-//     four ticks (13 warps/SM), 47.2 per tile (22 KB of shared memory per warp: 10 warps/SM, 138 registers, no spills).  The
-//     request is issued lane by lane (UBLKCP takes uniform registers: a 10-instruction loop per lane), which is why fewer, larger
-//     requests win against occupancy.  The ZMP pair (one sector per lane) stays a 256-bit store: a second request per lane costs
-//     more than it saves (measured 38.7 G steps/s at 8 warps/SM).
+//     four ticks (13 warps/SM), 47.2 per tile (22 KB of shared memory per warp: 10 warps/SM, 140 registers, no spills).
+//     UBLKCP takes its operands in uniform registers, so a request issued by every lane for its own slot becomes a
+//     ~10-instruction loop per lane (11 % of the kernel's instructions).  Instead, after the warp has staged the tile, ONE
+//     elected lane issues all 32 requests: lane i's request depends only on i and the tile, its operands are warp-uniform, and
+//     a whole tile's 32 requests unroll to ~5 instructions each (0.310 -> 0.298 ms per launch on configs[1]).  The ZMP pair (one
+//     sector per lane) stays a 256-bit store: a second request per lane costs more than it saves (38.7 G steps/s at 8 warps/SM).
 // ---------------------------------------------------------------------------------------------
 constexpr int RW_TILE = FIR_R * 32;
 constexpr int RW_U = 5;                        // halo samples per lane fetched together
+
+// shared -> global through the bulk-copy engine (cp.async.bulk, UBLKCP): 16-byte aligned addresses and size
+__device__ __forceinline__ void bulk_store(double *dst, unsigned src_smem, unsigned bytes)
+{
+  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;\n" ::"l"(dst), "r"(src_smem), "r"(bytes) : "memory");
+}
+// true in exactly one lane of the (converged) warp: what the compiler needs to issue a request once, not once per lane
+__device__ __forceinline__ bool elect_one()
+{
+  unsigned r;
+  asm volatile("{\n .reg .pred p;\n elect.sync _|p, 0xffffffff;\n selp.u32 %0, 1, 0, p;\n}\n" : "=r"(r));
+  return r != 0;
+}
 
 template <bool SIM, bool ADD = false, bool POS = false>
 __global__ void __launch_bounds__(32, 10)
@@ -1200,6 +1215,10 @@ preview_rec_warp_kernel(const int *__restrict__ order, const int64_t *__restrict
       const bool c32 = ((reinterpret_cast<uintptr_t>(gc) | (ADD ? reinterpret_cast<uintptr_t>(ga) : 0)) & 31) == 0;
       const bool z32 = (reinterpret_cast<uintptr_t>(gz) & 31) == 0;
       const bool bulk = com != nullptr;        // CoM pairs through the bulk-copy engine (16-byte alignment is all it asks)
+      if (bulk) {                              // the previous tile's requests have read the staging slots
+        asm volatile("cp.async.bulk.wait_group.read 0;\n" ::: "memory");
+        __syncwarp();
+      }
 #pragma unroll
       for (int j = 0; j < FIR_R / 2; ++j) {
         const int r0 = 2 * j, r1 = 2 * j + 1;
@@ -1222,16 +1241,8 @@ preview_rec_warp_kernel(const int *__restrict__ order, const int64_t *__restrict
             }
             if (bulk) {
               double2 *sg = stage + 6 * j;
-              if (j == 0) asm volatile("cp.async.bulk.wait_group.read 0;\n" ::: "memory");   // the previous tile has left the slot
               sg[0] = make_double2(a0, a1); sg[1] = make_double2(a2, a3); sg[2] = make_double2(a4, a5);
               sg[3] = make_double2(b0, b1); sg[4] = make_double2(b2, b3); sg[5] = make_double2(b4, b5);
-              if (j == FIR_R / 2 - 1 || k0 + r1 + 2 > last) {      // all eight ticks staged, or the next pair will not be a whole pair
-                asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");
-                const unsigned sa = (unsigned)__cvta_generic_to_shared(stage);
-                const unsigned bytes = 96u * (unsigned)(j + 1);
-                asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;\n" ::"l"(gc), "r"(sa), "r"(bytes) : "memory");
-                asm volatile("cp.async.bulk.commit_group;\n" ::: "memory");
-              }
             } else {
               st32g(gc + 6 * r0, a0, a1, a2, a3, c32);
               st32g(gc + 6 * r0 + 4, a4, a5, b0, b1, c32);
@@ -1254,6 +1265,26 @@ preview_rec_warp_kernel(const int *__restrict__ order, const int64_t *__restrict
             g2[0] = make_double2(a0, a1); g2[1] = make_double2(a2, a3); g2[2] = make_double2(a4, a5);
           }
           if (zmp) *reinterpret_cast<double2 *>(gz + 2 * r0) = POS ? make_double2(sx.x0, sy.x0) : make_double2(zx0, zy0);
+        }
+      }
+      // one lane hands every lane's whole tick pairs to the bulk-copy engine: lane i's request depends on i and on the tile only,
+      // so its operands are warp-uniform and each request is one UBLKCP (issued from every lane, each request costs a
+      // ~10-instruction loop over the lanes, 11 % of the kernel's instructions)
+      if (bulk) {
+        asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");
+        __syncwarp();
+        if (elect_one()) {
+          const int nt = last - start + 1;     // valid ticks of this tile
+          double *g = com + 6 * (size_t)(o + start);
+          const unsigned sa = (unsigned)__cvta_generic_to_shared(sp + CAP);
+          if (nt >= RW_TILE) {                 // a whole tile: 32 requests of 384 B, constant offsets
+#pragma unroll
+            for (int i = 0; i < 32; ++i) bulk_store(g + 6 * FIR_R * i, sa + 400u * i, 96u * (FIR_R / 2));
+          } else {
+            for (int i = 0; i < 32 && FIR_R * i + 1 < nt; ++i)   // lane i's whole tick pairs
+              bulk_store(g + 6 * FIR_R * i, sa + 400u * i, 96u * (unsigned)min(FIR_R / 2, (nt - FIR_R * i) / 2));
+          }
+          asm volatile("cp.async.bulk.commit_group;\n" ::: "memory");
         }
       }
     }
