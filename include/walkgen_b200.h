@@ -443,6 +443,60 @@ int wg_herdt_mpc_run_batch(wg_ctx *ctx, int mem, int B, int nsteps, wg_herdt_mpc
                            wg_herdt_qp_input *qp_in);
 
 /* ------------------------------------------------------------------------------------------------
+ * Herdt2010 on-line generator, one 5 ms control tick at a time, for B robots
+ *   replaces PatternGeneratorInterface::RunOneStepOfTheControlLoop, Herdt branch (PatternGeneratorInterfacePrivate.cpp:1246-1336):
+ *            ZMPVelocityReferencedQP::OnLine (ZMPVelocityReferencedQP.cpp:324-458) and the pop of the four deques by
+ *            CoMAndFootOnlyStrategy::OneGlobalStepOfControl (CoMAndFootOnlyStrategy.cpp:56-124);
+ *            :HerdtOnline (InitOnLine), :setVelReference (Reference()) and :stoppg between ticks.
+ * Every robot keeps its own clock, deques and commands, so robots started at different ticks and commanded at different
+ * ticks advance together.  One tick of robot b is what one RunOneStepOfTheControlLoop does for that robot alone:
+ *   - its command of this tick is applied (WG_CMD_VEL writes new_ref, WG_CMD_STOP sets ending_phase);
+ *   - its clock advances by Ts;
+ *   - while on line, the end-of-on-line test runs, and when clock + 1e-5 > upper_time_limit one QP period fires (the
+ *     same device code as wg_herdt_mpc_run_batch): the back element of the deques takes the new feet, then the period's
+ *     samples 1..19 and the state's com_back / foot[.][2] sample are appended;
+ *   - one element is popped into rows[t][b] and running[t][b] = 1; when the deques are empty the robot stops for good
+ *     (running[t][b] = 0 from then on, until it is started again).
+ * A robot that is not started, or has stopped, is not advanced and ignores its commands: its running entry is 0 and its row
+ * is untouched with WG_MEM_DEVICE, zero with WG_MEM_HOST.
+ *
+ * Memory: the deques of a robot are a ring of WG_HERDT_ONLINE_QUEUE wg_herdt_tick rows in device memory.  A robot holds at
+ * most 29 rows before a pop (8 buffered at the start plus 20 at the first tick; 9 + 20 at each later QP instant); a QP
+ * instant that would overflow the ring (possible only after the states were edited) stops the robot's on-line mode with
+ * last_fail = -1 instead.  Per robot: 7424 B of queue, 1000 B of state, 5120 B of staged period rows, 1760 B of QP records:
+ * about 15.3 GB for 10^6 robots.
+ * Parameters come from wg_herdt_set_params / wg_herdt_mpc_set_params and are read at tick time; without them start and tick
+ * return WG_ERR_NOT_READY.  A tick is four kernel launches whatever number of robots fire; with WG_MEM_DEVICE it does not
+ * synchronise, and once its buffers exist it allocates nothing.
+ * ---------------------------------------------------------------------------------------------- */
+#define WG_HERDT_ONLINE_QUEUE 29
+enum { WG_CMD_VEL = 1, WG_CMD_STOP = 2 };
+
+typedef struct wg_herdt_command {      /* one robot, one tick; applied before that tick                          */
+  double vel[3];                       /* WG_CMD_VEL: :setVelReference dx dy dyaw (new_ref)                      */
+  int32_t flags;                       /* WG_CMD_VEL | WG_CMD_STOP (:stoppg); 0 = no command                     */
+  int32_t pad_;
+} wg_herdt_command;                    /* 32 bytes */
+
+typedef struct wg_herdt_online wg_herdt_online;
+int wg_herdt_online_create(wg_ctx *ctx, int B, wg_herdt_online **out);
+int wg_herdt_online_destroy(wg_herdt_online *h);
+/* :HerdtOnline for the n robots idx_host[0..n): state as wg_herdt_mpc_init15 (robot idx[i] reads init15_host +
+ * i*init_stride; stride 0 broadcasts), deques = the 8 buffered start samples (TimeBuffer_/Ts, the state's com_back and
+ * feet), clock restarted at 0.  Robots not listed keep running.  Refused with WG_ERR_INVALID, nothing changed: n < 0,
+ * init_stride < 0, an index out of [0, B) or repeated, NULL arrays with n > 0.  Waits for the context stream. */
+int wg_herdt_online_start(wg_herdt_online *h, int n, const int32_t *idx_host, const double *init15_host, int init_stride);
+/* nticks control ticks for every started robot.  In `mem`, each may be NULL:
+ *   commands [nticks][B]   command of robot b before tick t
+ *   rows     [nticks][B]   the popped COMState / ZMPPosition / feet
+ *   running  [nticks][B]   1 = RunOneStepOfTheControlLoop returned true
+ * Refused with WG_ERR_INVALID, nothing changed: nticks < 0 or an unknown mem. */
+int wg_herdt_online_tick(wg_herdt_online *h, int mem, int nticks, const wg_herdt_command *commands, wg_herdt_tick *rows,
+                         int8_t *running);
+/* The B state records in DEVICE memory (plain data, editable between calls as wg_herdt_mpc_run_batch's are). */
+wg_herdt_mpc_state *wg_herdt_online_states(wg_herdt_online *h);
+
+/* ------------------------------------------------------------------------------------------------
  * Dimitrov PLDP solver and OptCholesky, batched (QP_N = 16: control vector of 2N = 32 entries)
  *   replaces PLDPSolver::PLDPSolver / SolveProblem / ComputeInitialSolution / ComputeProjectedDescentDirection /
  *            ComputeAlpha / StoreCurrentZMPSolution   (src/Mathematics/PLDPSolver.cpp:56-135, :287-1032)

@@ -22,9 +22,15 @@ ACTIVE_SET_DTYPE = _capi.herdt_active_set_dtype()
 PLDP_STATE_DTYPE, PLDP_INFO_DTYPE = _capi.pldp_dtypes()
 REL_STEP_DTYPE, KAJITA_FOOT_DTYPE = _capi.kajita_dtypes()
 LCI_DTYPE, DIMITROV_PERIOD_DTYPE = _capi.dimitrov_dtypes()
+HERDT_COMMAND_DTYPE = _capi.herdt_command_dtype()
+CMD_VEL, CMD_STOP = _capi.WG_CMD_VEL, _capi.WG_CMD_STOP
+HERDT_ONLINE_QUEUE = _capi.HERDT_ONLINE_QUEUE
+# init15 of the TestHerdt2010 start at rest: CoM (x, dx, ddx, y, dy, ddy, z), trunk yaw and rate, left and right foot (x, y, theta)
+HERDT_INIT15 = (0.0316055, 0.0, 0.0, 0.0, 0.0, 0.0, 0.7116911, 0.0, 0.0, 0.0, 0.09, 0.0, 0.0, -0.09, 0.0)
 DimitrovParams = _capi.DimitrovParams
 
-__all__ = ["MultiContext", "LCI_DTYPE", "DIMITROV_PERIOD_DTYPE", "DimitrovParams", "dimitrov_default_params", "Context", "PreviewPlan", "KajitaPlan", "KajitaStream",
+__all__ = ["MultiContext", "LCI_DTYPE", "DIMITROV_PERIOD_DTYPE", "DimitrovParams", "dimitrov_default_params", "Context", "PreviewPlan", "KajitaPlan", "KajitaStream", "HerdtOnline",
+           "HERDT_COMMAND_DTYPE", "CMD_VEL", "CMD_STOP", "HERDT_ONLINE_QUEUE", "HERDT_INIT15",
            "STREAM_START", "STREAM_FINISH", "zmpdisc_default_params", "REL_STEP_DTYPE", "KAJITA_FOOT_DTYPE", "preview_gains", "herdt_default_params", "herdt_mpc_default_params", "HerdtParams", "HerdtMpcParams",
            "PLDP_STATE_DTYPE", "PLDP_INFO_DTYPE", "FOOT_DTYPE", "TICK_DTYPE", "MPC_STATE_DTYPE", "MPC_STEP_DTYPE", "TICKS_PER_STEP", "QP_INPUT_DTYPE",
            "QP_OUTPUT_DTYPE", "ACTIVE_SET_DTYPE", "WalkgenError", "device_count",
@@ -362,6 +368,10 @@ class Context:
         self._check(self.lib.wg_herdt_mpc_run_batch(self.h, WG_MEM_DEVICE, int(B), int(nsteps), _ptr(d_states),
                                                     _ptr(d_vel_ref), _ptr(d_ticks), _ptr(d_steps), _ptr(d_qp_in)))
 
+    def herdt_online(self, B) -> "HerdtOnline":
+        """B robots driven one 5 ms control tick at a time (wg_herdt_online_create)."""
+        return HerdtOnline(self, B)
+
 
     # ---- Dimitrov PLDP / OptCholesky ------------------------------------------------------------
     def pldp_set_constants(self, iPu, Px, Pu):
@@ -672,6 +682,66 @@ class KajitaStream:
     def destroy(self):
         if self.h:
             self.ctx.lib.wg_kajita_stream_destroy(self.h)
+            self.h = None
+
+
+class HerdtOnline:
+    """On-line Herdt2010 generator for B robots: RunOneStepOfTheControlLoop batched, each robot with its own start tick,
+    commands (:setVelReference, :stoppg) and deques (wg_herdt_online_*)."""
+
+    def __init__(self, ctx: Context, B):
+        self.ctx = ctx
+        self.B = int(B)
+        h = C.c_void_p()
+        ctx._check(ctx.lib.wg_herdt_online_create(ctx.h, self.B, C.byref(h)))
+        self.h = h
+
+    def start(self, idx, init15=HERDT_INIT15):
+        """:HerdtOnline for the robots idx; init15: one start configuration (broadcast) or an array [len(idx)][15]."""
+        idx = np.ascontiguousarray(idx, dtype=np.int32).reshape(-1)
+        init = np.ascontiguousarray(init15, dtype=np.float64)
+        stride = 0 if init.ndim == 1 else 15
+        assert init.size == 15 or init.shape == (len(idx), 15)
+        self.ctx._check(self.ctx.lib.wg_herdt_online_start(self.h, len(idx), idx.ctypes.data, init.ctypes.data, stride))
+
+    def tick(self, nticks, commands=None, rows=True, running=True):
+        """nticks ticks on host arrays: commands [nticks][B] of HERDT_COMMAND_DTYPE or None -> (rows [nticks][B] of
+        TICK_DTYPE, running [nticks][B] int8), each None when not asked for."""
+        n = int(nticks)
+        cmd = None if commands is None else np.ascontiguousarray(commands, dtype=HERDT_COMMAND_DTYPE)
+        assert cmd is None or cmd.shape == (n, self.B)
+        r = np.zeros((n, self.B), dtype=TICK_DTYPE) if rows else None
+        run = np.zeros((n, self.B), dtype=np.int8) if running else None
+        self.ctx._check(self.ctx.lib.wg_herdt_online_tick(self.h, WG_MEM_HOST, n, _ptr(cmd), _ptr(r), _ptr(run)))
+        return r, run
+
+    def tick_device(self, nticks, d_commands=None, d_rows=None, d_running=None):
+        """Device-resident form (asynchronous on the context stream)."""
+        self.ctx._check(self.ctx.lib.wg_herdt_online_tick(self.h, WG_MEM_DEVICE, int(nticks), _ptr(d_commands), _ptr(d_rows),
+                                                          _ptr(d_running)))
+
+    @property
+    def d_states(self) -> int:
+        """Device address of the B MPC_STATE_DTYPE records."""
+        return self.ctx.lib.wg_herdt_online_states(self.h)
+
+    def states(self):
+        """Host copy of the B state records."""
+        out = np.zeros(self.B, dtype=MPC_STATE_DTYPE)
+        self.ctx._check(self.ctx.lib.wg_memcpy_d2h(self.ctx.h, out.ctypes.data, self.d_states, out.nbytes))
+        self.ctx.sync()
+        return out
+
+    def set_states(self, states):
+        """Write B state records (e.g. a copy from states(), edited) back to the device."""
+        st = np.ascontiguousarray(states, dtype=MPC_STATE_DTYPE)
+        assert st.shape == (self.B,)
+        self.ctx._check(self.ctx.lib.wg_memcpy_h2d(self.ctx.h, self.d_states, st.ctypes.data, st.nbytes))
+        self.ctx.sync()
+
+    def destroy(self):
+        if self.h:
+            self.ctx.lib.wg_herdt_online_destroy(self.h)
             self.h = None
 
 

@@ -224,6 +224,19 @@ def herdt_mpc_dtypes():
     return foot, tick, state, step
 
 
+HERDT_ONLINE_QUEUE = 29
+WG_CMD_VEL = 1
+WG_CMD_STOP = 2
+
+
+def herdt_command_dtype():
+    """numpy mirror of wg_herdt_command (32 B)."""
+    np = _np()
+    d = np.dtype([("vel", "f8", 3), ("flags", "i4"), ("pad_", "i4")])
+    assert d.itemsize == 32
+    return d
+
+
 # name -> (restype, argtypes); also the list checked against include/walkgen_b200.h by the tests
 SIGNATURES = {
     "wg_version": (C.c_int, []),
@@ -343,6 +356,11 @@ SIGNATURES = {
     "wg_herdt_mpc_stats": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "wg_herdt_mpc_run_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                          C.c_void_p, C.c_void_p]),
+    "wg_herdt_online_create": (C.c_int, [C.c_void_p, C.c_int, C.POINTER(C.c_void_p)]),
+    "wg_herdt_online_destroy": (C.c_int, [C.c_void_p]),
+    "wg_herdt_online_start": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
+    "wg_herdt_online_tick": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "wg_herdt_online_states": (C.c_void_p, [C.c_void_p]),
 }
 
 _lib = None
