@@ -496,6 +496,48 @@ int wg_herdt_online_tick(wg_herdt_online *h, int mem, int nticks, const wg_herdt
 /* The B state records in DEVICE memory (plain data, editable between calls as wg_herdt_mpc_run_batch's are). */
 wg_herdt_mpc_state *wg_herdt_online_states(wg_herdt_online *h);
 
+/* Whole robots: save, restore and copy, for checkpoints, lookahead branches and migration between handles, processes or GPUs.
+ *
+ * A robot of wg_herdt_online is its state record, its deques and its {count, running} slot: everything the next tick of that
+ * robot reads.  The rest of a handle is per-tick scratch that is dead between calls: the staged period rows, the QP records
+ * and outputs and the per-robot fire flags are written for the robots that fire before they are read, within one tick.  The
+ * generator parameters (wg_herdt_set_params, wg_herdt_mpc_set_params) belong to the context, not to the robot: a record is
+ * only meaningful under the parameters it was saved with, and no call checks that.
+ *
+ * The record is CANONICAL: the ring is rotated so that the front row is rows[0], and rows[count..) are zero.  Two robots with
+ * the same history since their start save to bitwise-equal records whatever number of ticks their rings have turned.
+ *
+ * In every call the index arrays are HOST pointers; NULL means robots 0..n-1 and needs n <= B of that handle.  Every call
+ * runs on the context stream, in order with ticks; a refused call returns WG_ERR_INVALID and changes no robot.  Device record
+ * arrays must be 16-byte aligned (records move as 16-byte words: a warp moves two rows per instruction).
+ *
+ * wg_herdt_online_save: robot idx[i] -> out[i]; indices in [0, B), repeats allowed.  WG_MEM_DEVICE: one launch, no
+ *   synchronisation, no allocation once the index scratch exists.  WG_MEM_HOST: the same launch, a D2H copy, a synchronise.
+ * wg_herdt_online_restore: in[i] -> robot idx[i]; indices in [0, B) and unique.  The ring is written with its head at row 0.
+ *   Records come from outside the program, so all n are validated before any robot changes: 0 <= count <= 29, running is 0
+ *   or 1, and running == 0 implies count == 0 (a robot stops only when its deques are empty, an unstarted robot holds none).
+ *   The state record itself is not validated, as with wg_herdt_online_states.  WG_MEM_HOST: the records are checked on the
+ *   host, then one H2D copy, one launch and a synchronise.  WG_MEM_DEVICE: a check kernel writes one flag, the call reads it
+ *   (one synchronise), then the restore launch: two launches and one synchronise, the price of the all-or-nothing rule.
+ * wg_herdt_online_copy: robot src_idx[i] of src -> robot dst_idx[i] of dst, device to device: state, slot and ring verbatim,
+ *   one launch, no synchronisation, no validation of data (a live handle already keeps the invariant).  src_idx may repeat
+ *   (fork one robot into K); dst_idx must be unique.  Refused: handles of two contexts, an index out of range, dst == src with
+ *   an index that is both a source and a destination, n < 0, n above B for a NULL index array.
+ * save and restore also refuse: n < 0, an index out of range (restore: or repeated), n above B for a NULL index array, a
+ * NULL record array with n > 0, an unknown mem, device records that are not 16-byte aligned. */
+typedef struct wg_herdt_online_robot {
+  wg_herdt_tick rows[WG_HERDT_ONLINE_QUEUE]; /* the deques, FRONT FIRST (rows[0] is popped next); rows[count..) zero     */
+  wg_herdt_mpc_state state;
+  int32_t count;                             /* rows held, 0..WG_HERDT_ONLINE_QUEUE                                   */
+  int32_t running;                           /* 1: started and not yet stopped (PGI m_Running)                        */
+  int32_t pad_[4];
+} wg_herdt_online_robot;                     /* 8448 bytes: a multiple of 16, rows at offset 0                        */
+
+int wg_herdt_online_save(wg_herdt_online *h, int mem, int n, const int32_t *idx, wg_herdt_online_robot *out);
+int wg_herdt_online_restore(wg_herdt_online *h, int mem, int n, const int32_t *idx, const wg_herdt_online_robot *in);
+int wg_herdt_online_copy(wg_herdt_online *dst, int n, const int32_t *dst_idx, const wg_herdt_online *src,
+                         const int32_t *src_idx);
+
 /* ------------------------------------------------------------------------------------------------
  * Dimitrov PLDP solver and OptCholesky, batched (QP_N = 16: control vector of 2N = 32 entries)
  *   replaces PLDPSolver::PLDPSolver / SolveProblem / ComputeInitialSolution / ComputeProjectedDescentDirection /

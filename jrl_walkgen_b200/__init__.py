@@ -25,12 +25,13 @@ LCI_DTYPE, DIMITROV_PERIOD_DTYPE = _capi.dimitrov_dtypes()
 HERDT_COMMAND_DTYPE = _capi.herdt_command_dtype()
 CMD_VEL, CMD_STOP = _capi.WG_CMD_VEL, _capi.WG_CMD_STOP
 HERDT_ONLINE_QUEUE = _capi.HERDT_ONLINE_QUEUE
+ONLINE_ROBOT_DTYPE = _capi.herdt_online_robot_dtype()
 # init15 of the TestHerdt2010 start at rest: CoM (x, dx, ddx, y, dy, ddy, z), trunk yaw and rate, left and right foot (x, y, theta)
 HERDT_INIT15 = (0.0316055, 0.0, 0.0, 0.0, 0.0, 0.0, 0.7116911, 0.0, 0.0, 0.0, 0.09, 0.0, 0.0, -0.09, 0.0)
 DimitrovParams = _capi.DimitrovParams
 
 __all__ = ["MultiContext", "LCI_DTYPE", "DIMITROV_PERIOD_DTYPE", "DimitrovParams", "dimitrov_default_params", "Context", "PreviewPlan", "KajitaPlan", "KajitaStream", "HerdtOnline",
-           "HERDT_COMMAND_DTYPE", "CMD_VEL", "CMD_STOP", "HERDT_ONLINE_QUEUE", "HERDT_INIT15",
+           "HERDT_COMMAND_DTYPE", "CMD_VEL", "CMD_STOP", "HERDT_ONLINE_QUEUE", "ONLINE_ROBOT_DTYPE", "HERDT_INIT15",
            "STREAM_START", "STREAM_FINISH", "zmpdisc_default_params", "REL_STEP_DTYPE", "KAJITA_FOOT_DTYPE", "preview_gains", "herdt_default_params", "herdt_mpc_default_params", "HerdtParams", "HerdtMpcParams",
            "PLDP_STATE_DTYPE", "PLDP_INFO_DTYPE", "FOOT_DTYPE", "TICK_DTYPE", "MPC_STATE_DTYPE", "MPC_STEP_DTYPE", "TICKS_PER_STEP", "QP_INPUT_DTYPE",
            "QP_OUTPUT_DTYPE", "ACTIVE_SET_DTYPE", "WalkgenError", "device_count",
@@ -48,6 +49,10 @@ def _ptr(a):
         return C.c_void_p(a.ptr)
     assert a.flags["C_CONTIGUOUS"]
     return a.ctypes.data_as(C.c_void_p)
+
+
+def _indices(idx):
+    return None if idx is None else np.ascontiguousarray(idx, dtype=np.int32).reshape(-1)
 
 
 def herdt_default_params(sole_length=0.25, sole_width=0.14) -> HerdtParams:
@@ -738,6 +743,36 @@ class HerdtOnline:
         assert st.shape == (self.B,)
         self.ctx._check(self.ctx.lib.wg_memcpy_h2d(self.ctx.h, self.d_states, st.ctypes.data, st.nbytes))
         self.ctx.sync()
+
+    def save(self, idx=None):
+        """-> host records [n] of ONLINE_ROBOT_DTYPE of the robots idx (all B when None): wg_herdt_online_save."""
+        ia = _indices(idx)
+        out = np.zeros(self.B if ia is None else len(ia), dtype=ONLINE_ROBOT_DTYPE)
+        self.ctx._check(self.ctx.lib.wg_herdt_online_save(self.h, WG_MEM_HOST, len(out), _ptr(ia), out.ctypes.data))
+        return out
+
+    def restore(self, records, idx=None):
+        """Write host records (ONLINE_ROBOT_DTYPE) into the robots idx (0..len(records)-1 when None); all or nothing."""
+        rec = np.ascontiguousarray(records, dtype=ONLINE_ROBOT_DTYPE).reshape(-1)
+        ia = _indices(idx)
+        assert ia is None or len(ia) == len(rec)
+        self.ctx._check(self.ctx.lib.wg_herdt_online_restore(self.h, WG_MEM_HOST, len(rec), _ptr(ia), rec.ctypes.data))
+
+    def save_device(self, n, d_out, idx=None):
+        """Device-resident save of n robots into d_out (asynchronous on the context stream)."""
+        self.ctx._check(self.ctx.lib.wg_herdt_online_save(self.h, WG_MEM_DEVICE, int(n), _ptr(_indices(idx)), _ptr(d_out)))
+
+    def restore_device(self, n, d_in, idx=None):
+        """Device-resident restore of n records from d_in (waits for the check of the records)."""
+        self.ctx._check(self.ctx.lib.wg_herdt_online_restore(self.h, WG_MEM_DEVICE, int(n), _ptr(_indices(idx)), _ptr(d_in)))
+
+    def copy_from(self, src: "HerdtOnline", src_idx=None, dst_idx=None):
+        """Robot src_idx[i] of src -> robot dst_idx[i] of this handle, on the device (wg_herdt_online_copy); n is the
+        length of the index arrays given, B of this handle when neither is."""
+        si, di = _indices(src_idx), _indices(dst_idx)
+        n = len(di) if di is not None else (len(si) if si is not None else self.B)
+        assert si is None or len(si) == n
+        self.ctx._check(self.ctx.lib.wg_herdt_online_copy(self.h, n, _ptr(di), src.h, _ptr(si)))
 
     def destroy(self):
         if self.h:

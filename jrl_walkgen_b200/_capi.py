@@ -237,6 +237,16 @@ def herdt_command_dtype():
     return d
 
 
+def herdt_online_robot_dtype():
+    """numpy mirror of wg_herdt_online_robot (8448 B): one whole robot of wg_herdt_online, deques front first."""
+    np = _np()
+    _, tick, state, _ = herdt_mpc_dtypes()
+    d = np.dtype([("rows", tick, (HERDT_ONLINE_QUEUE,)), ("state", state), ("count", "i4"), ("running", "i4"),
+                  ("pad_", "i4", 4)])
+    assert d.itemsize == 8448 and d.fields["rows"][1] == 0
+    return d
+
+
 # name -> (restype, argtypes); also the list checked against include/walkgen_b200.h by the tests
 SIGNATURES = {
     "wg_version": (C.c_int, []),
@@ -361,6 +371,9 @@ SIGNATURES = {
     "wg_herdt_online_start": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
     "wg_herdt_online_tick": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "wg_herdt_online_states": (C.c_void_p, [C.c_void_p]),
+    "wg_herdt_online_save": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "wg_herdt_online_restore": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
+    "wg_herdt_online_copy": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
 }
 
 _lib = None

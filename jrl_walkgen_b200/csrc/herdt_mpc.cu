@@ -760,6 +760,113 @@ online_merge_pop_kernel(int B, const wg_herdt_mpc_state *__restrict__ states, co
   }
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Whole robots (wg_herdt_online_save / restore / copy): one warp per robot.  Rows move as 16-byte words, so one warp
+// instruction moves two 256-byte rows.  A state record sits at a 1000-byte stride in the handle, only 8-byte aligned, so it
+// moves as 8-byte words; in a record it starts the 1024-byte tail {state, count, running, pad}, which is stored as 16-byte
+// words.
+// ---------------------------------------------------------------------------------------------------------------
+constexpr int ROW_V4 = (int)(sizeof(wg_herdt_tick) / 16);                 // 16
+constexpr int RING_V4 = QCAP * ROW_V4;                                    // 464
+constexpr int RING_ITERS = (RING_V4 + 31) / 32;                           // 15: unrolled, so a lane has all its loads in flight
+constexpr int STATE_LL = (int)(sizeof(wg_herdt_mpc_state) / 8);           // 125
+constexpr int TAIL_V2 = (int)((sizeof(wg_herdt_online_robot) - offsetof(wg_herdt_online_robot, state)) / 16);   // 64
+static_assert(sizeof(wg_herdt_online_robot) == 8448 && offsetof(wg_herdt_online_robot, rows) == 0, "record layout");
+static_assert(offsetof(wg_herdt_online_robot, state) == QCAP * sizeof(wg_herdt_tick), "record layout");
+static_assert(offsetof(wg_herdt_online_robot, count) == offsetof(wg_herdt_online_robot, state) + 8 * STATE_LL &&
+              offsetof(wg_herdt_online_robot, running) == offsetof(wg_herdt_online_robot, count) + 4, "record tail layout");
+
+// the canonical record of robot idx[i] (robot i when idx is NULL): ring from its head, zero past count
+__global__ void __launch_bounds__(MPC_WARPS * 32)
+online_save_kernel(int n, const int32_t *__restrict__ idx, const wg_herdt_mpc_state *__restrict__ states,
+                   const wg_herdt_tick *__restrict__ queue, const OnlineSlot *__restrict__ slots,
+                   wg_herdt_online_robot *__restrict__ out)
+{
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int i = blockIdx.x * MPC_WARPS + warp; i < n; i += gridDim.x * MPC_WARPS) {
+    const int b = idx ? idx[i] : i;
+    const OnlineSlot s = slots[b];
+    const uint4 *q = reinterpret_cast<const uint4 *>(queue + (size_t)b * QCAP);
+    uint4 *o = reinterpret_cast<uint4 *>(out + i);
+#pragma unroll
+    for (int k = 0; k < RING_ITERS; ++k) {
+      const int e = lane + 32 * k, r = e / ROW_V4;
+      if (e < RING_V4) o[e] = (r < s.count) ? q[((s.head + r) % QCAP) * ROW_V4 + e % ROW_V4] : make_uint4(0u, 0u, 0u, 0u);
+    }
+    const long long *st = reinterpret_cast<const long long *>(states + b);
+    const long long slot = (long long)(((unsigned long long)(unsigned)s.running << 32) | (unsigned)s.count);
+    longlong2 *t = reinterpret_cast<longlong2 *>(o + RING_V4);
+    for (int e = lane; e < TAIL_V2; e += 32) {
+      const int k = 2 * e;
+      longlong2 v;
+      v.x = (k < STATE_LL) ? st[k] : (k == STATE_LL ? slot : 0);
+      v.y = (k + 1 < STATE_LL) ? st[k + 1] : (k + 1 == STATE_LL ? slot : 0);
+      t[e] = v;
+    }
+  }
+}
+
+// Record in[i] -> robot idx[i] (robot i when idx is NULL), head 0.  The records were validated before this launch.
+__global__ void __launch_bounds__(MPC_WARPS * 32)
+online_restore_kernel(int n, const int32_t *__restrict__ idx, const wg_herdt_online_robot *__restrict__ in,
+                      wg_herdt_mpc_state *__restrict__ states, wg_herdt_tick *__restrict__ queue, OnlineSlot *__restrict__ slots)
+{
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int i = blockIdx.x * MPC_WARPS + warp; i < n; i += gridDim.x * MPC_WARPS) {
+    const int b = idx ? idx[i] : i;
+    const uint4 *src = reinterpret_cast<const uint4 *>(in + i);
+    uint4 *q = reinterpret_cast<uint4 *>(queue + (size_t)b * QCAP);
+#pragma unroll
+    for (int k = 0; k < RING_ITERS; ++k) {
+      const int e = lane + 32 * k;
+      if (e < RING_V4) q[e] = src[e];
+    }
+    long long *st = reinterpret_cast<long long *>(states + b);
+    const longlong2 *t = reinterpret_cast<const longlong2 *>(src + RING_V4);
+    for (int e = lane; e < TAIL_V2; e += 32) {
+      const int k = 2 * e;
+      const longlong2 v = t[e];
+      if (k < STATE_LL) st[k] = v.x;
+      if (k + 1 < STATE_LL) st[k + 1] = v.y;
+    }
+    if (lane == 0) { OnlineSlot s; s.head = 0; s.count = in[i].count; s.running = in[i].running; s.pad_ = 0; slots[b] = s; }
+  }
+}
+
+// The invariant the tick kernels keep, over n records from outside the program: *bad = 1 when any record breaks it
+__global__ void __launch_bounds__(MPC_WARPS * 32)
+online_restore_check_kernel(int n, const wg_herdt_online_robot *__restrict__ in, int *__restrict__ bad)
+{
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const int c = in[i].count, r = in[i].running;
+    if (c < 0 || c > QCAP || (r != 0 && r != 1) || (r == 0 && c != 0)) *bad = 1;
+  }
+}
+
+// Robot sidx[i] of one handle -> robot didx[i] of another (or of the same, the two index sets disjoint), verbatim
+__global__ void __launch_bounds__(MPC_WARPS * 32)
+online_copy_kernel(int n, const int32_t *__restrict__ didx, const int32_t *__restrict__ sidx,
+                   const wg_herdt_mpc_state *__restrict__ s_states, const wg_herdt_tick *__restrict__ s_queue,
+                   const OnlineSlot *__restrict__ s_slots, wg_herdt_mpc_state *__restrict__ d_states,
+                   wg_herdt_tick *__restrict__ d_queue, OnlineSlot *__restrict__ d_slots)
+{
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int i = blockIdx.x * MPC_WARPS + warp; i < n; i += gridDim.x * MPC_WARPS) {
+    const int d = didx ? didx[i] : i, s = sidx ? sidx[i] : i;
+    const uint4 *sq = reinterpret_cast<const uint4 *>(s_queue + (size_t)s * QCAP);
+    uint4 *dq = reinterpret_cast<uint4 *>(d_queue + (size_t)d * QCAP);
+#pragma unroll
+    for (int k = 0; k < RING_ITERS; ++k) {
+      const int e = lane + 32 * k;
+      if (e < RING_V4) dq[e] = sq[e];
+    }
+    const long long *ss = reinterpret_cast<const long long *>(s_states + s);
+    long long *ds = reinterpret_cast<long long *>(d_states + d);
+    for (int e = lane; e < STATE_LL; e += 32) ds[e] = ss[e];
+    if (lane == 0) d_slots[d] = s_slots[s];
+  }
+}
+
 }  // namespace
 
 const herdt::Consts *wg_herdt_device_consts(wg_ctx *ctx);
@@ -1016,13 +1123,55 @@ struct wg_herdt_online {
   // staging of start (init states, indices) and of WG_MEM_HOST ticks (commands, rows, running)
   void *d_init = nullptr, *d_idx = nullptr, *d_cmd = nullptr, *d_rows = nullptr, *d_run = nullptr;
   size_t cap_init = 0, cap_idx = 0, cap_cmd = 0, cap_rows = 0, cap_run = 0;
+  // staging of WG_MEM_HOST robot records, and the flag of the device-record check
+  void *d_robots = nullptr, *d_flag = nullptr;
+  size_t cap_robots = 0, cap_flag = 0;
 };
 
 static void online_free(wg_herdt_online *h)
 {
   cudaFree(h->d_states); cudaFree(h->d_queue); cudaFree(h->d_slots); cudaFree(h->d_staged);
   cudaFree(h->d_init); cudaFree(h->d_idx); cudaFree(h->d_cmd); cudaFree(h->d_rows); cudaFree(h->d_run);
+  cudaFree(h->d_robots); cudaFree(h->d_flag);
   delete h;
+}
+
+// Robot indices from the host: NULL = 0..n-1 (needs n <= B); otherwise in [0, B), and unique when `unique`.  Sets mark[b]
+// (B entries, zero on entry) for every robot b named.
+static bool online_indices_ok(int B, int n, const int32_t *idx, bool unique, std::vector<char> &mark)
+{
+  if (!idx) {
+    if (n > B) return false;
+    for (int i = 0; i < n; ++i) mark[i] = 1;
+    return true;
+  }
+  for (int i = 0; i < n; ++i) {
+    const int32_t b = idx[i];
+    if (b < 0 || b >= B || (unique && mark[b])) return false;
+    mark[b] = 1;
+  }
+  return true;
+}
+
+// Upload up to two host index arrays into the handle's index scratch; a NULL array stays NULL.
+static int online_upload_indices(wg_herdt_online *h, int n, const int32_t *a, const int32_t *b, const int32_t **da,
+                                 const int32_t **db)
+{
+  wg_ctx *ctx = h->ctx;
+  const size_t bytes = sizeof(int32_t) * (size_t)n;
+  int rc;
+  if ((a || b) && (rc = wgi_grow_scratch(ctx, &h->d_idx, &h->cap_idx, bytes * ((a && b) ? 2 : 1))) != WG_OK) return rc;
+  int32_t *d = static_cast<int32_t *>(h->d_idx);
+  *da = nullptr;
+  if (db) *db = nullptr;
+  if (a) { WG_CUDA(ctx, cudaMemcpyAsync(d, a, bytes, cudaMemcpyHostToDevice, ctx->stream)); *da = d; d += n; }
+  if (b) { WG_CUDA(ctx, cudaMemcpyAsync(d, b, bytes, cudaMemcpyHostToDevice, ctx->stream)); *db = d; }
+  return WG_OK;
+}
+
+static int online_blocks(wg_ctx *ctx, int n)
+{
+  return std::max(1, std::min((n + MPC_WARPS - 1) / MPC_WARPS, ctx->sm_count * 16));
 }
 
 static int online_ticks(wg_herdt_online *h, MpcState *m, int nticks, const wg_herdt_command *cmd, wg_herdt_tick *rows,
@@ -1156,6 +1305,110 @@ int wg_herdt_online_tick(wg_herdt_online *h, int mem, int nticks, const wg_herdt
   if (rows) WG_CUDA(ctx, cudaMemcpyAsync(rows, h->d_rows, sizeof(wg_herdt_tick) * n, cudaMemcpyDeviceToHost, ctx->stream));
   if (running) WG_CUDA(ctx, cudaMemcpyAsync(running, h->d_run, sizeof(int8_t) * n, cudaMemcpyDeviceToHost, ctx->stream));
   WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return WG_OK;
+}
+
+int wg_herdt_online_save(wg_herdt_online *h, int mem, int n, const int32_t *idx, wg_herdt_online_robot *out)
+{
+  if (!h || n < 0 || (n > 0 && !out) || (mem != WG_MEM_HOST && mem != WG_MEM_DEVICE)) return WG_ERR_INVALID;
+  wg_ctx *ctx = h->ctx;
+  if (mem == WG_MEM_DEVICE && reinterpret_cast<uintptr_t>(out) % 16)
+    return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_save: device records must be 16-byte aligned");
+  std::vector<char> mark((size_t)h->B, 0);
+  if (!online_indices_ok(h->B, n, idx, false, mark))
+    return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_save: index out of range, or n > B without indices");
+  if (n == 0) return WG_OK;
+  wg_device_guard guard(ctx->device);
+  const size_t bytes = sizeof(wg_herdt_online_robot) * (size_t)n;
+  int rc;
+  if (mem == WG_MEM_HOST && (rc = wgi_grow_scratch(ctx, &h->d_robots, &h->cap_robots, bytes)) != WG_OK) return rc;
+  wg_herdt_online_robot *d_out = mem == WG_MEM_HOST ? static_cast<wg_herdt_online_robot *>(h->d_robots) : out;
+  const int32_t *d_idx;
+  if ((rc = online_upload_indices(h, n, idx, nullptr, &d_idx, nullptr)) != WG_OK) return rc;
+  wg_prof_start(ctx, WG_K_HERDT_MPC);
+  online_save_kernel<<<online_blocks(ctx, n), MPC_WARPS * 32, 0, ctx->stream>>>(n, d_idx, h->d_states, h->d_queue, h->d_slots,
+                                                                                d_out);
+  wg_prof_stop(ctx);
+  WG_LAUNCHED(ctx);
+  if (mem == WG_MEM_DEVICE) return WG_OK;
+  WG_CUDA(ctx, cudaMemcpyAsync(out, d_out, bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return WG_OK;
+}
+
+static bool online_record_ok(const wg_herdt_online_robot &r)
+{
+  return r.count >= 0 && r.count <= QCAP && (r.running == 0 || r.running == 1) && (r.running == 1 || r.count == 0);
+}
+
+int wg_herdt_online_restore(wg_herdt_online *h, int mem, int n, const int32_t *idx, const wg_herdt_online_robot *in)
+{
+  if (!h || n < 0 || (n > 0 && !in) || (mem != WG_MEM_HOST && mem != WG_MEM_DEVICE)) return WG_ERR_INVALID;
+  wg_ctx *ctx = h->ctx;
+  if (mem == WG_MEM_DEVICE && reinterpret_cast<uintptr_t>(in) % 16)
+    return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_restore: device records must be 16-byte aligned");
+  std::vector<char> mark((size_t)h->B, 0);
+  if (!online_indices_ok(h->B, n, idx, true, mark))
+    return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_restore: index out of range or repeated, or n > B without indices");
+  if (mem == WG_MEM_HOST)
+    for (int i = 0; i < n; ++i)
+      if (!online_record_ok(in[i])) return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_restore: invalid count / running");
+  if (n == 0) return WG_OK;
+  wg_device_guard guard(ctx->device);
+  const size_t bytes = sizeof(wg_herdt_online_robot) * (size_t)n;
+  const int blocks = online_blocks(ctx, n);
+  int rc;
+  const wg_herdt_online_robot *d_in = in;
+  if (mem == WG_MEM_HOST) {
+    if ((rc = wgi_grow_scratch(ctx, &h->d_robots, &h->cap_robots, bytes)) != WG_OK) return rc;
+    d_in = static_cast<const wg_herdt_online_robot *>(h->d_robots);
+    WG_CUDA(ctx, cudaMemcpyAsync(h->d_robots, in, bytes, cudaMemcpyHostToDevice, ctx->stream));
+  } else {
+    if ((rc = wgi_grow_scratch(ctx, &h->d_flag, &h->cap_flag, sizeof(int))) != WG_OK) return rc;
+    int *flag = static_cast<int *>(h->d_flag), bad = 0;
+    WG_CUDA(ctx, cudaMemsetAsync(flag, 0, sizeof(int), ctx->stream));
+    wg_prof_start(ctx, WG_K_HERDT_MPC);
+    online_restore_check_kernel<<<std::max(1, std::min((n + MPC_WARPS * 32 - 1) / (MPC_WARPS * 32), ctx->sm_count * 16)),
+                                  MPC_WARPS * 32, 0, ctx->stream>>>(n, in, flag);
+    wg_prof_stop(ctx);
+    WG_LAUNCHED(ctx);
+    WG_CUDA(ctx, cudaMemcpyAsync(&bad, flag, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (bad) return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_restore: invalid count / running");
+  }
+  const int32_t *d_idx;
+  if ((rc = online_upload_indices(h, n, idx, nullptr, &d_idx, nullptr)) != WG_OK) return rc;
+  wg_prof_start(ctx, WG_K_HERDT_MPC);
+  online_restore_kernel<<<blocks, MPC_WARPS * 32, 0, ctx->stream>>>(n, d_idx, d_in, h->d_states, h->d_queue, h->d_slots);
+  wg_prof_stop(ctx);
+  WG_LAUNCHED(ctx);
+  if (mem == WG_MEM_HOST) WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return WG_OK;
+}
+
+int wg_herdt_online_copy(wg_herdt_online *dst, int n, const int32_t *dst_idx, const wg_herdt_online *src,
+                         const int32_t *src_idx)
+{
+  if (!dst || !src || n < 0) return WG_ERR_INVALID;
+  wg_ctx *ctx = dst->ctx;
+  if (src->ctx != ctx) return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_copy: handles of two contexts");
+  std::vector<char> dmark((size_t)dst->B, 0), smark((size_t)src->B, 0);
+  if (!online_indices_ok(dst->B, n, dst_idx, true, dmark) || !online_indices_ok(src->B, n, src_idx, false, smark))
+    return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_copy: index out of range, repeated destination, or n > B without indices");
+  if (dst == src)
+    for (int b = 0; b < dst->B; ++b)
+      if (dmark[b] && smark[b]) return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_copy: a robot is both source and destination");
+  if (n == 0) return WG_OK;
+  wg_device_guard guard(ctx->device);
+  const int32_t *d_didx, *d_sidx;
+  const int rc = online_upload_indices(dst, n, dst_idx, src_idx, &d_didx, &d_sidx);
+  if (rc != WG_OK) return rc;
+  wg_prof_start(ctx, WG_K_HERDT_MPC);
+  online_copy_kernel<<<online_blocks(ctx, n), MPC_WARPS * 32, 0, ctx->stream>>>(n, d_didx, d_sidx, src->d_states, src->d_queue,
+                                                                                src->d_slots, dst->d_states, dst->d_queue,
+                                                                                dst->d_slots);
+  wg_prof_stop(ctx);
+  WG_LAUNCHED(ctx);
   return WG_OK;
 }
 
