@@ -825,6 +825,65 @@ int wg_kajita_stream_run(wg_kajita_stream *s, int mem, double *zmpref_xy, double
 int wg_kajita_stream_state(wg_kajita_stream *s, int mem, double *preview_state, int64_t *samples_emitted,
                            int64_t *steps_previewed, int32_t *open);
 
+/* Whole walks: save, restore and copy, for checkpoints, rewinds, footstep lookahead branches and migration between streams,
+ * processes or GPUs.
+ *
+ * A walk of wg_kajita_stream is a fixed-size record plus its preview carry, the last NL-1 unconsumed ZMP samples (rows of
+ * double[2]; carry[n][NL-1][2] for n walks, none in a stream without preview).  Together they are everything the walk's next
+ * run reads.  The zmpdisc parameters and preview gains belong to the context, not to the walk: a record is only meaningful
+ * under the ones it was saved with, and no call checks that beyond NL and with_preview.
+ *
+ * The record is CANONICAL: two walks with the same history since their START save to the same bytes.  Carry rows
+ * [count, NL-1) are zero, count = samples_emitted - steps_previewed; a walk never started saves as all zeros; pad_ is zero.
+ * samples_emitted is what wg_kajita_stream_state reports.
+ *
+ * In every call the index arrays are HOST pointers; NULL means walks 0..n-1 and needs n <= B of that stream.  Every call
+ * runs on the context stream, in order with appends and runs.  A refused call returns WG_ERR_INVALID and changes no walk,
+ * on the device or on the host.  All three are refused while an append is pending on a stream involved (its plan was made
+ * from the walks' present counters); they leave the offsets of the last run (wg_kajita_stream_sample_offsets, ...) as they
+ * are.  Device arrays must be 16-byte aligned.  carry must be non-NULL (n > 0) in a stream with preview and NULL in one
+ * without.
+ *
+ * wg_kajita_stream_save: walk idx[i] -> walks[i], carry[i]; indices in [0, B), repeats allowed.  WG_MEM_DEVICE: one H2D
+ *   copy of the indices and the walks' host-side counters, one launch, no synchronisation.  WG_MEM_HOST: the same, then the
+ *   D2H copies and a synchronise.
+ * wg_kajita_stream_restore: walks[i], carry[i] -> walk idx[i]; indices in [0, B) and unique.  Records come from outside the
+ *   program, so all n are validated before any walk changes: open is 0 or 1, samples_emitted >= 0, open == 1 implies
+ *   samples_emitted > 0, and steps_previewed == max(0, samples_emitted - (NL-1)) with preview, 0 without: the invariants
+ *   every run keeps.  The walk state proper (support frame, feet, last step, filter history, preview state) is not
+ *   validated, as wg_kajita_stream_state's preview state is not.  Carry rows past count are written as zero, the walk's
+ *   status as 0.  WG_MEM_HOST: the records are checked on the host, then the H2D copies, one launch and a synchronise.
+ *   WG_MEM_DEVICE: a check kernel validates the records and returns their counters with one D2H copy (one synchronise:
+ *   the host plans appends from them), then the restore launch: two launches and one synchronise.
+ * wg_kajita_stream_copy: walk src_idx[i] of src -> walk dst_idx[i] of dst, device to device: record, preview state and
+ *   carry verbatim, the host-side counters on the host; one launch, no synchronisation, no validation of data (a live
+ *   stream keeps the invariants).  src_idx may repeat (fork one walk into K); dst_idx must be unique.  Refused: streams of
+ *   two contexts, streams whose with_preview or NL differ, an index out of range, dst == src with an index that is both a
+ *   source and a destination.
+ * All three also refuse n < 0 and n above B for a NULL index array; save and restore refuse a NULL walks array with n > 0
+ * and an unknown mem. */
+typedef struct wg_kajita_stream_walk {
+  double support[6];           /* m_CurrentSupportFootPosition: r00 r01 r10 r11 tx ty                              */
+  double prev_support[2];      /* translation of the previous support foot                                         */
+  wg_foot_sample left, right;  /* feet after the last sample emitted                                               */
+  double zmp_theta;            /* theta of FinalZMPPositions.back() (degrees)                                       */
+  int64_t samples_emitted;     /* since the walk's START                                                            */
+  double final0[2];            /* FinalZMPPositions[0]                                                              */
+  wg_rel_step last;            /* last step appended: rel0 of the next OnLineAddFoot / EndPhaseOfTheWalking        */
+  double hist[16][2];          /* last 16 filtered ZMP samples, as the generator keeps them                        */
+  double preview_state[8];     /* as wg_preview_run_batch's state; zero in a stream without preview                 */
+  int64_t steps_previewed;     /* since START                                                                       */
+  int32_t open;                /* 1: started, not finished                                                          */
+  int32_t pad_;
+} wg_kajita_stream_walk;       /* 576 bytes, a multiple of 16 */
+
+int wg_kajita_stream_carry_rows(const wg_kajita_stream *s);   /* NL-1 with preview, 0 without */
+int wg_kajita_stream_save(wg_kajita_stream *s, int mem, int n, const int32_t *idx, wg_kajita_stream_walk *walks, double *carry);
+int wg_kajita_stream_restore(wg_kajita_stream *s, int mem, int n, const int32_t *idx, const wg_kajita_stream_walk *walks,
+                             const double *carry);
+int wg_kajita_stream_copy(wg_kajita_stream *dst, int n, const int32_t *dst_idx, const wg_kajita_stream *src,
+                          const int32_t *src_idx);
+
 /* ------------------------------------------------------------------------------------------------
  * Dimitrov2008 front to back: feet trajectories -> support polygons -> per-period constraint matrices ->
  * PLDP solve -> LIPM, closed loop on the device (one warp owns one walk for its whole duration)

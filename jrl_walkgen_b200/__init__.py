@@ -21,6 +21,7 @@ TICKS_PER_STEP = _capi.HERDT_TICKS_PER_STEP
 ACTIVE_SET_DTYPE = _capi.herdt_active_set_dtype()
 PLDP_STATE_DTYPE, PLDP_INFO_DTYPE = _capi.pldp_dtypes()
 REL_STEP_DTYPE, KAJITA_FOOT_DTYPE = _capi.kajita_dtypes()
+KAJITA_STREAM_WALK_DTYPE = _capi.kajita_stream_walk_dtype()
 LCI_DTYPE, DIMITROV_PERIOD_DTYPE = _capi.dimitrov_dtypes()
 HERDT_COMMAND_DTYPE = _capi.herdt_command_dtype()
 CMD_VEL, CMD_STOP = _capi.WG_CMD_VEL, _capi.WG_CMD_STOP
@@ -32,7 +33,7 @@ DimitrovParams = _capi.DimitrovParams
 
 __all__ = ["MultiContext", "LCI_DTYPE", "DIMITROV_PERIOD_DTYPE", "DimitrovParams", "dimitrov_default_params", "Context", "PreviewPlan", "KajitaPlan", "KajitaStream", "HerdtOnline",
            "HERDT_COMMAND_DTYPE", "CMD_VEL", "CMD_STOP", "HERDT_ONLINE_QUEUE", "ONLINE_ROBOT_DTYPE", "HERDT_INIT15",
-           "STREAM_START", "STREAM_FINISH", "zmpdisc_default_params", "REL_STEP_DTYPE", "KAJITA_FOOT_DTYPE", "preview_gains", "herdt_default_params", "herdt_mpc_default_params", "HerdtParams", "HerdtMpcParams",
+           "STREAM_START", "STREAM_FINISH", "zmpdisc_default_params", "REL_STEP_DTYPE", "KAJITA_FOOT_DTYPE", "KAJITA_STREAM_WALK_DTYPE", "preview_gains", "herdt_default_params", "herdt_mpc_default_params", "HerdtParams", "HerdtMpcParams",
            "PLDP_STATE_DTYPE", "PLDP_INFO_DTYPE", "FOOT_DTYPE", "TICK_DTYPE", "MPC_STATE_DTYPE", "MPC_STEP_DTYPE", "TICKS_PER_STEP", "QP_INPUT_DTYPE",
            "QP_OUTPUT_DTYPE", "ACTIVE_SET_DTYPE", "WalkgenError", "device_count",
            "MODE_WITH_INITIALPOS", "MODE_WITHOUT_INITIALPOS", "WG_MEM_HOST", "WG_MEM_DEVICE"]
@@ -639,6 +640,7 @@ class KajitaStream:
         h = C.c_void_p()
         ctx._check(ctx.lib.wg_kajita_stream_create(ctx.h, C.byref(self.params), self.B, int(self.with_preview), C.byref(h)))
         self.h = h
+        self.carry_rows = int(ctx.lib.wg_kajita_stream_carry_rows(h))   # NL-1 with preview, 0 without
         self.sample_offsets = np.zeros(self.B + 1, dtype=np.int64)
         self.com_offsets = np.zeros(self.B + 1, dtype=np.int64)
         self.com_counts = np.zeros(self.B, dtype=np.int64)
@@ -683,6 +685,43 @@ class KajitaStream:
         self.ctx._check(self.ctx.lib.wg_kajita_stream_state(self.h, mem, _ptr(preview_state), _ptr(emitted), _ptr(previewed),
                                                             _ptr(is_open)))
         return preview_state, emitted, previewed, is_open
+
+    def save(self, idx=None):
+        """-> (walks [n] of KAJITA_STREAM_WALK_DTYPE, carry [n][carry_rows][2] or None without preview) of the walks idx
+        (all B when None): wg_kajita_stream_save."""
+        ia = _indices(idx)
+        n = self.B if ia is None else len(ia)
+        walks = np.zeros(n, dtype=KAJITA_STREAM_WALK_DTYPE)
+        carry = np.zeros((n, self.carry_rows, 2)) if self.with_preview else None
+        self.ctx._check(self.ctx.lib.wg_kajita_stream_save(self.h, WG_MEM_HOST, n, _ptr(ia), walks.ctypes.data, _ptr(carry)))
+        return walks, carry
+
+    def restore(self, walks, carry, idx=None):
+        """Write host records and carry rows into the walks idx (0..len(walks)-1 when None); all or nothing."""
+        rec = np.ascontiguousarray(walks, dtype=KAJITA_STREAM_WALK_DTYPE).reshape(-1)
+        c = None if carry is None else np.ascontiguousarray(carry, dtype=np.float64)
+        assert c is None or c.shape == (len(rec), self.carry_rows, 2)
+        ia = _indices(idx)
+        assert ia is None or len(ia) == len(rec)
+        self.ctx._check(self.ctx.lib.wg_kajita_stream_restore(self.h, WG_MEM_HOST, len(rec), _ptr(ia), rec.ctypes.data, _ptr(c)))
+
+    def save_device(self, n, d_walks, d_carry, idx=None):
+        """Device-resident save of n walks into d_walks, d_carry (None without preview); asynchronous on the context stream."""
+        self.ctx._check(self.ctx.lib.wg_kajita_stream_save(self.h, WG_MEM_DEVICE, int(n), _ptr(_indices(idx)), _ptr(d_walks),
+                                                           _ptr(d_carry)))
+
+    def restore_device(self, n, d_walks, d_carry, idx=None):
+        """Device-resident restore of n walks from d_walks, d_carry (waits for the check of the records)."""
+        self.ctx._check(self.ctx.lib.wg_kajita_stream_restore(self.h, WG_MEM_DEVICE, int(n), _ptr(_indices(idx)), _ptr(d_walks),
+                                                              _ptr(d_carry)))
+
+    def copy_from(self, src: "KajitaStream", src_idx=None, dst_idx=None):
+        """Walk src_idx[i] of src -> walk dst_idx[i] of this stream, on the device (wg_kajita_stream_copy); n is the length of
+        the index arrays given, B of this stream when neither is."""
+        si, di = _indices(src_idx), _indices(dst_idx)
+        n = len(di) if di is not None else (len(si) if si is not None else self.B)
+        assert si is None or len(si) == n
+        self.ctx._check(self.ctx.lib.wg_kajita_stream_copy(self.h, n, _ptr(di), src.h, _ptr(si)))
 
     def destroy(self):
         if self.h:

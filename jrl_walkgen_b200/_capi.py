@@ -144,6 +144,17 @@ def kajita_dtypes():
     return step, foot
 
 
+def kajita_stream_walk_dtype():
+    """numpy mirror of wg_kajita_stream_walk (576 B): one whole walk of wg_kajita_stream, its carry rows apart."""
+    np = _np()
+    step, foot = kajita_dtypes()
+    d = np.dtype([("support", "f8", 6), ("prev_support", "f8", 2), ("left", foot), ("right", foot), ("zmp_theta", "f8"),
+                  ("samples_emitted", "i8"), ("final0", "f8", 2), ("last", step), ("hist", "f8", (16, 2)),
+                  ("preview_state", "f8", 8), ("steps_previewed", "i8"), ("open", "i4"), ("pad_", "i4")])
+    assert d.itemsize == 576 and d.fields["hist"][1] == 240 and d.fields["preview_state"][1] == 496
+    return d
+
+
 def pldp_dtypes():
     """numpy mirrors of wg_pldp_state (392 B) and wg_pldp_info (144 B)."""
     np = _np()
@@ -351,6 +362,10 @@ SIGNATURES = {
     "wg_kajita_stream_run": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.c_int]),
     "wg_kajita_stream_state": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "wg_kajita_stream_carry_rows": (C.c_int, [C.c_void_p]),
+    "wg_kajita_stream_save": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "wg_kajita_stream_restore": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "wg_kajita_stream_copy": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "wg_dimitrov_default_params": (None, [C.POINTER(DimitrovParams)]),
     "wg_dimitrov_set_params": (C.c_int, [C.c_void_p, C.POINTER(DimitrovParams)] + [C.c_void_p] * 6),
     "wg_dimitrov_period_count": (C.c_int64, [C.POINTER(DimitrovParams), C.c_int64]),

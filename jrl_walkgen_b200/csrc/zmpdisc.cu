@@ -640,6 +640,175 @@ zmpdisc_stream_kernel(const ZdConsts K, int nwork, const ZsWork *__restrict__ wo
   }
 }
 
+// ---- whole walks (wg_kajita_stream_save / restore / copy) -------------------------------------------------------------
+// A record is ZsRec (31 16-byte words), the preview state (4 words) and {steps_previewed, open, pad} (1 word); a walk's
+// carry is NL-1 words.  One warp per walk, grid-stride; everything moves as 16-byte words.
+constexpr int ZS_WARPS = 8;
+constexpr int ZS_UNROLL = 5;        // carry words in flight per lane: NL = 320 gives 319 words, two rounds of 5 x 32
+constexpr int ZS_REC_V4 = (int)(sizeof(ZsRec) / 16);                                   // 31
+constexpr int ZS_WALK_V4 = (int)(sizeof(wg_kajita_stream_walk) / 16);                  // 36
+constexpr int ZS_STATE_V4 = 4;                                                         // 8 doubles
+constexpr int ZS_F0_V4 = (int)(offsetof(ZdWalk, F0) / 16);                             // {zmp_theta, F0}
+static_assert(sizeof(ZdWalk) == 192 && offsetof(ZdWalk, final0) == 176 && sizeof(ZsRec) == 496, "ZsRec layout");
+static_assert(offsetof(ZsRec, last) == 192 && offsetof(ZsRec, hist) == 240, "ZsRec layout");
+static_assert(sizeof(wg_kajita_stream_walk) == 576 && offsetof(wg_kajita_stream_walk, final0) == offsetof(ZdWalk, final0) &&
+              offsetof(wg_kajita_stream_walk, samples_emitted) == offsetof(ZdWalk, F0) &&
+              offsetof(ZdWalk, F0) == 16 * ZS_F0_V4 + 8 && offsetof(wg_kajita_stream_walk, zmp_theta) == offsetof(ZdWalk, zmp_theta) &&
+              offsetof(wg_kajita_stream_walk, left) == offsetof(ZdWalk, L) && offsetof(wg_kajita_stream_walk, right) == offsetof(ZdWalk, R) &&
+              offsetof(wg_kajita_stream_walk, prev_support) == offsetof(ZdWalk, prev_tx) &&
+              offsetof(wg_kajita_stream_walk, last) == offsetof(ZsRec, last) && offsetof(wg_kajita_stream_walk, hist) == offsetof(ZsRec, hist),
+              "wg_kajita_stream_walk starts with ZsRec");
+static_assert(offsetof(wg_kajita_stream_walk, preview_state) == 16 * ZS_REC_V4 &&
+              offsetof(wg_kajita_stream_walk, steps_previewed) == 16 * (ZS_REC_V4 + ZS_STATE_V4) &&
+              offsetof(wg_kajita_stream_walk, open) == offsetof(wg_kajita_stream_walk, steps_previewed) + 8, "record tail layout");
+
+// A walk's counters, as the host keeps them (emitted, previewed, open), and the walk they belong to.
+struct ZsCounts {
+  int64_t emitted, previewed;
+  int32_t open, b;
+};
+
+// The invariants every run keeps: a run previews max(0, L - NL + 1) of its L = (emitted - previewed) + new samples, so the
+// carry always holds min(emitted, NL-1) of them.
+__host__ __device__ __forceinline__ bool zs_counts_ok(int64_t e, int64_t p, int32_t open, bool pv, int NL1)
+{
+  return (open == 0 || open == 1) && e >= 0 && (open == 0 || e > 0) && p == (pv && e > NL1 ? e - NL1 : 0);
+}
+
+// Words [0, nv) of dst from src, by one warp, with ZS_UNROLL loads of a lane in flight; words from `keep` on are zero.
+__device__ __forceinline__ void zs_move(uint4 *__restrict__ dst, const uint4 *__restrict__ src, int nv, int64_t keep, int lane)
+{
+  if (keep > nv) keep = nv;
+  for (int e0 = 0; e0 < nv; e0 += 32 * ZS_UNROLL) {
+    uint4 v[ZS_UNROLL];
+#pragma unroll
+    for (int u = 0; u < ZS_UNROLL; ++u) {
+      const int e = e0 + 32 * u + lane;
+      v[u] = (e < keep) ? src[e] : make_uint4(0u, 0u, 0u, 0u);
+    }
+#pragma unroll
+    for (int u = 0; u < ZS_UNROLL; ++u) {
+      const int e = e0 + 32 * u + lane;
+      if (e < nv) dst[e] = v[u];
+    }
+  }
+}
+
+// The canonical record of walk cnt[i].b: ZsRec with samples_emitted from the host counter (ZdWalk::F0 stops advancing at
+// EndPhaseOfTheWalking, so it lags a finished walk by the end phase; nothing reads it until the next START), carry rows past
+// emitted - previewed zero, all zero for a walk never started (its ZsRec was never written).
+__global__ void __launch_bounds__(ZS_WARPS * 32)
+stream_save_kernel(int n, const ZsCounts *__restrict__ cnt, const ZsRec *__restrict__ rec, const double *__restrict__ pv_state,
+                   const double2 *__restrict__ carry, int NL1, wg_kajita_stream_walk *__restrict__ out,
+                   double2 *__restrict__ out_carry)
+{
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int i = blockIdx.x * ZS_WARPS + warp; i < n; i += gridDim.x * ZS_WARPS) {
+    const ZsCounts c = cnt[i];
+    const bool live = c.emitted > 0;
+    const uint4 *r = reinterpret_cast<const uint4 *>(rec + c.b);
+    const uint4 *st = pv_state ? reinterpret_cast<const uint4 *>(pv_state + 8 * (int64_t)c.b) : nullptr;
+    uint4 *o = reinterpret_cast<uint4 *>(out + i);
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const int e = lane + 32 * k;
+      if (e >= ZS_WALK_V4) break;
+      uint4 v = make_uint4(0u, 0u, 0u, 0u);
+      if (e < ZS_REC_V4) {
+        if (live) v = r[e];
+      } else if (e < ZS_REC_V4 + ZS_STATE_V4) {
+        if (live && st) v = st[e - ZS_REC_V4];
+      } else {
+        v = make_uint4((unsigned)c.previewed, (unsigned)((uint64_t)c.previewed >> 32), (unsigned)c.open, 0u);
+      }
+      if (e == ZS_F0_V4) { v.z = (unsigned)c.emitted; v.w = (unsigned)((uint64_t)c.emitted >> 32); }
+      o[e] = v;
+    }
+    if (NL1 > 0)
+      zs_move(reinterpret_cast<uint4 *>(out_carry + (int64_t)i * NL1), reinterpret_cast<const uint4 *>(carry + (int64_t)c.b * NL1),
+              NL1, live ? c.emitted - c.previewed : 0, lane);
+  }
+}
+
+// Record in[i] -> walk idx[i]: ZsRec, preview state, carry rows (zero past samples_emitted - steps_previewed) and status 0.
+// The records were validated before this launch.
+__global__ void __launch_bounds__(ZS_WARPS * 32)
+stream_restore_kernel(int n, const int32_t *__restrict__ idx, const wg_kajita_stream_walk *__restrict__ in,
+                      const double2 *__restrict__ in_carry, int NL1, ZsRec *__restrict__ rec, double *__restrict__ pv_state,
+                      double2 *__restrict__ carry, int *__restrict__ status)
+{
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int i = blockIdx.x * ZS_WARPS + warp; i < n; i += gridDim.x * ZS_WARPS) {
+    const int b = idx[i];
+    const uint4 *src = reinterpret_cast<const uint4 *>(in + i);
+    uint4 *r = reinterpret_cast<uint4 *>(rec + b);
+    uint4 *st = pv_state ? reinterpret_cast<uint4 *>(pv_state + 8 * (int64_t)b) : nullptr;
+    uint4 v[2];
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const int e = lane + 32 * k;
+      if (e < ZS_REC_V4 + ZS_STATE_V4) v[k] = src[e];
+    }
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const int e = lane + 32 * k;
+      if (e < ZS_REC_V4) r[e] = v[k];
+      else if (e < ZS_REC_V4 + ZS_STATE_V4 && st) st[e - ZS_REC_V4] = v[k];
+    }
+    if (NL1 > 0)
+      zs_move(reinterpret_cast<uint4 *>(carry + (int64_t)b * NL1), reinterpret_cast<const uint4 *>(in_carry + (int64_t)i * NL1),
+              NL1, in[i].samples_emitted - in[i].steps_previewed, lane);
+    if (lane == 0) status[b] = 0;
+  }
+}
+
+// The invariants of zs_counts_ok over n records from outside the program: *bad = 1 when any record breaks them; the
+// counters of record i go to cnt[i].
+__global__ void __launch_bounds__(ZS_WARPS * 32)
+stream_restore_check_kernel(int n, const wg_kajita_stream_walk *__restrict__ in, int pv, int NL1, int *__restrict__ bad,
+                            ZsCounts *__restrict__ cnt)
+{
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    ZsCounts c;
+    c.emitted = in[i].samples_emitted; c.previewed = in[i].steps_previewed; c.open = in[i].open; c.b = i;
+    if (!zs_counts_ok(c.emitted, c.previewed, c.open, pv != 0, NL1)) *bad = 1;
+    cnt[i] = c;
+  }
+}
+
+// Walk sidx[i] of one stream -> walk didx[i] of another (or of the same, the two index sets disjoint), verbatim; status 0.
+__global__ void __launch_bounds__(ZS_WARPS * 32)
+stream_copy_kernel(int n, const int32_t *__restrict__ didx, const int32_t *__restrict__ sidx, const ZsRec *__restrict__ s_rec,
+                   const double *__restrict__ s_state, const double2 *__restrict__ s_carry, ZsRec *__restrict__ d_rec,
+                   double *__restrict__ d_state, double2 *__restrict__ d_carry, int NL1, int *__restrict__ d_status)
+{
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int i = blockIdx.x * ZS_WARPS + warp; i < n; i += gridDim.x * ZS_WARPS) {
+    const int d = didx[i], s = sidx[i];
+    const uint4 *sr = reinterpret_cast<const uint4 *>(s_rec + s);
+    uint4 *dr = reinterpret_cast<uint4 *>(d_rec + d);
+    const uint4 *ss = s_state ? reinterpret_cast<const uint4 *>(s_state + 8 * (int64_t)s) : nullptr;
+    uint4 *ds = d_state ? reinterpret_cast<uint4 *>(d_state + 8 * (int64_t)d) : nullptr;
+    uint4 v[2];
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const int e = lane + 32 * k;
+      if (e < ZS_REC_V4) v[k] = sr[e];
+      else if (e < ZS_REC_V4 + ZS_STATE_V4 && ss) v[k] = ss[e - ZS_REC_V4];
+    }
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const int e = lane + 32 * k;
+      if (e < ZS_REC_V4) dr[e] = v[k];
+      else if (e < ZS_REC_V4 + ZS_STATE_V4 && ds) ds[e - ZS_REC_V4] = v[k];
+    }
+    if (NL1 > 0)
+      zs_move(reinterpret_cast<uint4 *>(d_carry + (int64_t)d * NL1), reinterpret_cast<const uint4 *>(s_carry + (int64_t)s * NL1),
+              NL1, NL1, lane);
+    if (lane == 0) d_status[d] = 0;
+  }
+}
+
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -1118,6 +1287,9 @@ struct wg_kajita_stream {
   // staging of WG_MEM_HOST runs, grown on demand
   void *d_out[7];
   size_t out_cap[7];
+  // staging of WG_MEM_HOST saves and restores: records, then carry rows
+  void *d_io;
+  size_t io_cap;
 };
 
 // Grow a device buffer to at least `bytes` (half as much again, to amortise).  The old contents are dropped.
@@ -1136,6 +1308,69 @@ static int zs_grow(wg_ctx *ctx, void **p, size_t *cap, size_t bytes)
 
 static size_t zs_align(size_t x) { return (x + 15) / 16 * 16; }
 
+// Make the pinned blob hold at least `bytes`, once the device has read what it last held (ev_staged).  The blob carries the
+// inputs of an append, or, when no append is pending, the indices and counters of a save, restore or copy.
+static int zs_stage_host(wg_kajita_stream *s, size_t bytes)
+{
+  wg_ctx *ctx = s->ctx;
+  WG_CUDA(ctx, cudaEventSynchronize(s->ev_staged));
+  if (bytes > s->h_cap) {
+    cudaFreeHost(s->h_blob);
+    s->h_blob = nullptr;
+    s->h_cap = 0;
+    const size_t want = bytes + bytes / 2;
+    WG_CUDA(ctx, cudaMallocHost(&s->h_blob, want));
+    s->h_cap = want;
+  }
+  return WG_OK;
+}
+
+// Whole walks: the helpers of wg_kajita_stream_save / restore / copy.
+static int zs_carry_rows(const wg_kajita_stream *s) { return s->with_preview ? std::max(0, s->NL - 1) : 0; }
+
+static int zs_refuse(wg_ctx *ctx, const char *call, const char *why)
+{
+  snprintf(ctx->err, sizeof ctx->err, "%s: %s", call, why);
+  return WG_ERR_INVALID;
+}
+
+// Walk indices from the host: NULL = 0..n-1 (needs n <= B); otherwise in [0, B), and unique when `unique`.  Sets mark[b]
+// (B entries, zero on entry) for every walk b named.
+static bool zs_indices_ok(int B, int n, const int32_t *idx, bool unique, std::vector<char> &mark)
+{
+  if (!idx) {
+    if (n > B) return false;
+    for (int i = 0; i < n; ++i) mark[i] = 1;
+    return true;
+  }
+  for (int i = 0; i < n; ++i) {
+    const int32_t b = idx[i];
+    if (b < 0 || b >= B || (unique && mark[b])) return false;
+    mark[b] = 1;
+  }
+  return true;
+}
+
+// The argument checks save and restore share: nullptr when the call may go on, else why it may not.
+static const char *zs_io_refusal(const wg_kajita_stream *s, int mem, int n, const void *walks, const void *carry)
+{
+  if (mem != WG_MEM_HOST && mem != WG_MEM_DEVICE) return "unknown mem";
+  if (n < 0) return "n < 0";
+  if (s->pending) return "an append is pending (run it first)";
+  if (n > 0 && !walks) return "NULL walks";
+  if (s->with_preview ? (n > 0 && !carry) : carry != nullptr) return "carry must be given with preview and NULL without";
+  if (mem == WG_MEM_DEVICE && ((reinterpret_cast<uintptr_t>(walks) | reinterpret_cast<uintptr_t>(carry)) & 15))
+    return "device arrays must be 16-byte aligned";
+  return nullptr;
+}
+
+// Grid of a whole-walk kernel: at most 6 CTAs of ZS_WARPS warps per SM, which all stay resident at up to 40 registers (the
+// kernels take 18 to 38), so the grid-stride loops leave no second wave.
+static int zs_blocks(const wg_ctx *ctx, int n, int per_block)
+{
+  return std::max(1, std::min((n + per_block - 1) / per_block, ctx->sm_count * 6));
+}
+
 extern "C" {
 
 int wg_kajita_stream_destroy(wg_kajita_stream *s)
@@ -1147,7 +1382,7 @@ int wg_kajita_stream_destroy(wg_kajita_stream *s)
   if (s->ev_staged) cudaEventDestroy(s->ev_staged);
   cudaFreeHost(s->h_blob);
   cudaFree(s->d_blob); cudaFree(s->d_rec); cudaFree(s->d_carry); cudaFree(s->d_lead); cudaFree(s->d_pk);
-  cudaFree(s->d_state); cudaFree(s->d_status); cudaFree(s->d_next);
+  cudaFree(s->d_state); cudaFree(s->d_status); cudaFree(s->d_next); cudaFree(s->d_io);
   for (void *p : s->d_out) cudaFree(p);
   delete s;
   return WG_OK;
@@ -1280,15 +1515,8 @@ int wg_kajita_stream_append(wg_kajita_stream *s, const int64_t *step_off, const 
   s->bytes = s->off_order + zs_align(sizeof(int) * s->npv);
   // ---- stage: wait until the device has read the previous blob, then refill it ----
   wg_device_guard guard(ctx->device);
-  WG_CUDA(ctx, cudaEventSynchronize(s->ev_staged));
-  if (s->bytes > s->h_cap) {
-    cudaFreeHost(s->h_blob);
-    s->h_blob = nullptr;
-    s->h_cap = 0;
-    const size_t want = s->bytes + s->bytes / 2;
-    WG_CUDA(ctx, cudaMallocHost(&s->h_blob, want));
-    s->h_cap = want;
-  }
+  int rc = zs_stage_host(s, s->bytes);
+  if (rc != WG_OK) return rc;
   ZsWork *wk = reinterpret_cast<ZsWork *>(s->h_blob);
   wg_rel_step *hs = reinterpret_cast<wg_rel_step *>(s->h_blob + s->off_steps);
   int64_t at = 0;
@@ -1306,7 +1534,7 @@ int wg_kajita_stream_append(wg_kajita_stream *s, const int64_t *step_off, const 
   }
   std::memcpy(s->h_blob + s->off_po, s->co.data(), sizeof(int64_t) * (B + 1));
   if (s->npv) std::memcpy(s->h_blob + s->off_order, pv_order.data(), sizeof(int) * s->npv);
-  int rc = zs_grow(ctx, reinterpret_cast<void **>(&s->d_blob), &s->d_cap, s->bytes);
+  rc = zs_grow(ctx, reinterpret_cast<void **>(&s->d_blob), &s->d_cap, s->bytes);
   if (rc != WG_OK) return rc;
   WG_CUDA(ctx, cudaMemcpyAsync(s->d_blob, s->h_blob, s->bytes, cudaMemcpyHostToDevice, ctx->stream));
   if (s->with_preview && (rc = wgi_preview_plan_set_offsets(s->pv, reinterpret_cast<const int64_t *>(s->h_blob + s->off_po))) != WG_OK)
@@ -1414,6 +1642,161 @@ int wg_kajita_stream_state(wg_kajita_stream *s, int mem, double *preview_state, 
     WG_CUDA(ctx, cudaMemcpyAsync(preview_state, s->d_state, sizeof(double) * 8 * B,
                                  mem == WG_MEM_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, ctx->stream));
     if (mem == WG_MEM_HOST) WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  }
+  return WG_OK;
+}
+
+int wg_kajita_stream_carry_rows(const wg_kajita_stream *s) { return s ? zs_carry_rows(s) : WG_ERR_INVALID; }
+
+int wg_kajita_stream_save(wg_kajita_stream *s, int mem, int n, const int32_t *idx, wg_kajita_stream_walk *walks, double *carry)
+{
+  if (!s) return WG_ERR_INVALID;
+  wg_ctx *ctx = s->ctx;
+  const char *call = "wg_kajita_stream_save";
+  if (const char *why = zs_io_refusal(s, mem, n, walks, carry)) return zs_refuse(ctx, call, why);
+  std::vector<char> mark((size_t)s->B, 0);
+  if (!zs_indices_ok(s->B, n, idx, false, mark)) return zs_refuse(ctx, call, "index out of range, or n > B without indices");
+  if (n == 0) return WG_OK;
+  wg_device_guard guard(ctx->device);
+  const int NL1 = zs_carry_rows(s);
+  const size_t wbytes = sizeof(wg_kajita_stream_walk) * (size_t)n, cbytes = sizeof(double2) * (size_t)NL1 * n;
+  const size_t bytes = sizeof(ZsCounts) * (size_t)n;
+  // the walks' host-side counters and indices, in one H2D copy
+  int rc = zs_stage_host(s, bytes);
+  if (rc != WG_OK) return rc;
+  ZsCounts *c = reinterpret_cast<ZsCounts *>(s->h_blob);
+  for (int i = 0; i < n; ++i) {
+    const int b = idx ? idx[i] : i;
+    c[i].emitted = s->emitted[b]; c[i].previewed = s->previewed[b]; c[i].open = s->open[b]; c[i].b = b;
+  }
+  if ((rc = zs_grow(ctx, reinterpret_cast<void **>(&s->d_blob), &s->d_cap, bytes)) != WG_OK) return rc;
+  WG_CUDA(ctx, cudaMemcpyAsync(s->d_blob, s->h_blob, bytes, cudaMemcpyHostToDevice, ctx->stream));
+  WG_CUDA(ctx, cudaEventRecord(s->ev_staged, ctx->stream));
+  wg_kajita_stream_walk *d_w = walks;
+  double2 *d_c = reinterpret_cast<double2 *>(carry);
+  if (mem == WG_MEM_HOST) {
+    if ((rc = zs_grow(ctx, &s->d_io, &s->io_cap, wbytes + cbytes)) != WG_OK) return rc;
+    d_w = static_cast<wg_kajita_stream_walk *>(s->d_io);
+    d_c = reinterpret_cast<double2 *>(static_cast<unsigned char *>(s->d_io) + wbytes);
+  }
+  wg_prof_start(ctx, WG_K_ZMPDISC);
+  stream_save_kernel<<<zs_blocks(ctx, n, ZS_WARPS), ZS_WARPS * 32, 0, ctx->stream>>>(
+      n, reinterpret_cast<const ZsCounts *>(s->d_blob), s->d_rec, s->d_state, s->d_carry, NL1, d_w, d_c);
+  wg_prof_stop(ctx);
+  WG_LAUNCHED(ctx);
+  if (mem == WG_MEM_DEVICE) return WG_OK;
+  WG_CUDA(ctx, cudaMemcpyAsync(walks, d_w, wbytes, cudaMemcpyDeviceToHost, ctx->stream));
+  if (cbytes) WG_CUDA(ctx, cudaMemcpyAsync(carry, d_c, cbytes, cudaMemcpyDeviceToHost, ctx->stream));
+  WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return WG_OK;
+}
+
+int wg_kajita_stream_restore(wg_kajita_stream *s, int mem, int n, const int32_t *idx, const wg_kajita_stream_walk *walks,
+                             const double *carry)
+{
+  if (!s) return WG_ERR_INVALID;
+  wg_ctx *ctx = s->ctx;
+  const char *call = "wg_kajita_stream_restore";
+  if (const char *why = zs_io_refusal(s, mem, n, walks, carry)) return zs_refuse(ctx, call, why);
+  std::vector<char> mark((size_t)s->B, 0);
+  if (!zs_indices_ok(s->B, n, idx, true, mark))
+    return zs_refuse(ctx, call, "index out of range or repeated, or n > B without indices");
+  const int NL1 = zs_carry_rows(s);
+  const char *bad_record = "a record breaks the invariants of open, samples_emitted and steps_previewed";
+  if (mem == WG_MEM_HOST)
+    for (int i = 0; i < n; ++i)
+      if (!zs_counts_ok(walks[i].samples_emitted, walks[i].steps_previewed, walks[i].open, s->with_preview, NL1))
+        return zs_refuse(ctx, call, bad_record);
+  if (n == 0) return WG_OK;
+  wg_device_guard guard(ctx->device);
+  const size_t wbytes = sizeof(wg_kajita_stream_walk) * (size_t)n, cbytes = sizeof(double2) * (size_t)NL1 * n;
+  // blob: indices | the check kernel's flag | the records' counters, which the check kernel writes (device records)
+  const size_t off_flag = zs_align(sizeof(int32_t) * (size_t)n), off_cnt = off_flag + 16;
+  const size_t bytes = off_cnt + sizeof(ZsCounts) * (size_t)n;
+  int rc = zs_stage_host(s, bytes);
+  if (rc != WG_OK) return rc;
+  int32_t *hi = reinterpret_cast<int32_t *>(s->h_blob);
+  for (int i = 0; i < n; ++i) hi[i] = idx ? idx[i] : i;
+  std::memset(s->h_blob + off_flag, 0, 16);
+  if ((rc = zs_grow(ctx, reinterpret_cast<void **>(&s->d_blob), &s->d_cap, bytes)) != WG_OK) return rc;
+  WG_CUDA(ctx, cudaMemcpyAsync(s->d_blob, s->h_blob, off_cnt, cudaMemcpyHostToDevice, ctx->stream));
+  WG_CUDA(ctx, cudaEventRecord(s->ev_staged, ctx->stream));
+  const wg_kajita_stream_walk *d_w = walks;
+  const double2 *d_c = reinterpret_cast<const double2 *>(carry);
+  const ZsCounts *hc = nullptr;
+  if (mem == WG_MEM_HOST) {
+    if ((rc = zs_grow(ctx, &s->d_io, &s->io_cap, wbytes + cbytes)) != WG_OK) return rc;
+    unsigned char *io = static_cast<unsigned char *>(s->d_io);
+    WG_CUDA(ctx, cudaMemcpyAsync(io, walks, wbytes, cudaMemcpyHostToDevice, ctx->stream));
+    if (cbytes) WG_CUDA(ctx, cudaMemcpyAsync(io + wbytes, carry, cbytes, cudaMemcpyHostToDevice, ctx->stream));
+    d_w = reinterpret_cast<const wg_kajita_stream_walk *>(io);
+    d_c = reinterpret_cast<const double2 *>(io + wbytes);
+  } else {
+    // all or nothing: the records are checked before any walk changes, and the host needs their counters to plan appends
+    wg_prof_start(ctx, WG_K_ZMPDISC);
+    stream_restore_check_kernel<<<zs_blocks(ctx, n, ZS_WARPS * 32), ZS_WARPS * 32, 0, ctx->stream>>>(
+        n, walks, s->with_preview, NL1, reinterpret_cast<int *>(s->d_blob + off_flag), reinterpret_cast<ZsCounts *>(s->d_blob + off_cnt));
+    wg_prof_stop(ctx);
+    WG_LAUNCHED(ctx);
+    WG_CUDA(ctx, cudaMemcpyAsync(s->h_blob + off_flag, s->d_blob + off_flag, bytes - off_flag, cudaMemcpyDeviceToHost, ctx->stream));
+    WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    if (*reinterpret_cast<const int *>(s->h_blob + off_flag)) return zs_refuse(ctx, call, bad_record);
+    hc = reinterpret_cast<const ZsCounts *>(s->h_blob + off_cnt);
+  }
+  wg_prof_start(ctx, WG_K_ZMPDISC);
+  stream_restore_kernel<<<zs_blocks(ctx, n, ZS_WARPS), ZS_WARPS * 32, 0, ctx->stream>>>(
+      n, reinterpret_cast<const int32_t *>(s->d_blob), d_w, d_c, NL1, s->d_rec, s->d_state, s->d_carry, s->d_status);
+  wg_prof_stop(ctx);
+  WG_LAUNCHED(ctx);
+  if (mem == WG_MEM_HOST) WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  for (int i = 0; i < n; ++i) {
+    const int b = hi[i];
+    s->emitted[b] = hc ? hc[i].emitted : walks[i].samples_emitted;
+    s->previewed[b] = hc ? hc[i].previewed : walks[i].steps_previewed;
+    s->open[b] = hc ? hc[i].open : walks[i].open;
+  }
+  return WG_OK;
+}
+
+int wg_kajita_stream_copy(wg_kajita_stream *dst, int n, const int32_t *dst_idx, const wg_kajita_stream *src, const int32_t *src_idx)
+{
+  if (!dst || !src) return WG_ERR_INVALID;
+  wg_ctx *ctx = dst->ctx;
+  const char *call = "wg_kajita_stream_copy";
+  if (n < 0) return zs_refuse(ctx, call, "n < 0");
+  if (src->ctx != ctx) return zs_refuse(ctx, call, "streams of two contexts");
+  if (dst->pending || src->pending) return zs_refuse(ctx, call, "an append is pending (run it first)");
+  if (dst->with_preview != src->with_preview || dst->NL != src->NL) return zs_refuse(ctx, call, "with_preview or NL differ");
+  std::vector<char> dmark((size_t)dst->B, 0), smark((size_t)src->B, 0);
+  if (!zs_indices_ok(dst->B, n, dst_idx, true, dmark) || !zs_indices_ok(src->B, n, src_idx, false, smark))
+    return zs_refuse(ctx, call, "index out of range, repeated destination, or n > B without indices");
+  if (dst == src)
+    for (int b = 0; b < dst->B; ++b)
+      if (dmark[b] && smark[b]) return zs_refuse(ctx, call, "a walk is both source and destination");
+  if (n == 0) return WG_OK;
+  wg_device_guard guard(ctx->device);
+  const size_t off_s = zs_align(sizeof(int32_t) * (size_t)n), bytes = off_s + sizeof(int32_t) * (size_t)n;
+  int rc = zs_stage_host(dst, bytes);
+  if (rc != WG_OK) return rc;
+  int32_t *hd = reinterpret_cast<int32_t *>(dst->h_blob), *hs = reinterpret_cast<int32_t *>(dst->h_blob + off_s);
+  for (int i = 0; i < n; ++i) {
+    hd[i] = dst_idx ? dst_idx[i] : i;
+    hs[i] = src_idx ? src_idx[i] : i;
+  }
+  if ((rc = zs_grow(ctx, reinterpret_cast<void **>(&dst->d_blob), &dst->d_cap, bytes)) != WG_OK) return rc;
+  WG_CUDA(ctx, cudaMemcpyAsync(dst->d_blob, dst->h_blob, bytes, cudaMemcpyHostToDevice, ctx->stream));
+  WG_CUDA(ctx, cudaEventRecord(dst->ev_staged, ctx->stream));
+  wg_prof_start(ctx, WG_K_ZMPDISC);
+  stream_copy_kernel<<<zs_blocks(ctx, n, ZS_WARPS), ZS_WARPS * 32, 0, ctx->stream>>>(
+      n, reinterpret_cast<const int32_t *>(dst->d_blob), reinterpret_cast<const int32_t *>(dst->d_blob + off_s), src->d_rec,
+      src->d_state, src->d_carry, dst->d_rec, dst->d_state, dst->d_carry, zs_carry_rows(dst), dst->d_status);
+  wg_prof_stop(ctx);
+  WG_LAUNCHED(ctx);
+  for (int i = 0; i < n; ++i) {        // the index sets are disjoint when dst == src: no entry is read after it is written
+    const int d = hd[i], s = hs[i];
+    dst->emitted[d] = src->emitted[s];
+    dst->previewed[d] = src->previewed[s];
+    dst->open[d] = src->open[s];
   }
   return WG_OK;
 }
