@@ -56,6 +56,14 @@ def _indices(idx):
     return None if idx is None else np.ascontiguousarray(idx, dtype=np.int32).reshape(-1)
 
 
+def _copy_indices(src_idx, dst_idx, B):
+    """(n, src, dst) of a whole-record copy: n is the length of the index arrays given, B when neither is."""
+    si, di = _indices(src_idx), _indices(dst_idx)
+    n = len(di) if di is not None else (len(si) if si is not None else B)
+    assert si is None or len(si) == n
+    return n, si, di
+
+
 def herdt_default_params(sole_length=0.25, sole_width=0.14) -> HerdtParams:
     """Constants of ZMPVelocityReferencedQP's ctor (ZMPVelocityReferencedQP.cpp:61-118) for a given sole size
     (the reference reads it from the robot model; 0.25 x 0.14 m is the sample robot's, fitted from the datref)."""
@@ -718,9 +726,7 @@ class KajitaStream:
     def copy_from(self, src: "KajitaStream", src_idx=None, dst_idx=None):
         """Walk src_idx[i] of src -> walk dst_idx[i] of this stream, on the device (wg_kajita_stream_copy); n is the length of
         the index arrays given, B of this stream when neither is."""
-        si, di = _indices(src_idx), _indices(dst_idx)
-        n = len(di) if di is not None else (len(si) if si is not None else self.B)
-        assert si is None or len(si) == n
+        n, si, di = _copy_indices(src_idx, dst_idx, self.B)
         self.ctx._check(self.ctx.lib.wg_kajita_stream_copy(self.h, n, _ptr(di), src.h, _ptr(si)))
 
     def destroy(self):
@@ -808,9 +814,7 @@ class HerdtOnline:
     def copy_from(self, src: "HerdtOnline", src_idx=None, dst_idx=None):
         """Robot src_idx[i] of src -> robot dst_idx[i] of this handle, on the device (wg_herdt_online_copy); n is the
         length of the index arrays given, B of this handle when neither is."""
-        si, di = _indices(src_idx), _indices(dst_idx)
-        n = len(di) if di is not None else (len(si) if si is not None else self.B)
-        assert si is None or len(si) == n
+        n, si, di = _copy_indices(src_idx, dst_idx, self.B)
         self.ctx._check(self.ctx.lib.wg_herdt_online_copy(self.h, n, _ptr(di), src.h, _ptr(si)))
 
     def destroy(self):

@@ -12,6 +12,7 @@
 // size-1 at a QP instant (always the 12th, 19th and 20th sample of the previous period), so those three samples
 // are the persistent state (wg_herdt_mpc_state) and full 5 ms rows are an optional output.
 #include "herdt_qp.cuh"
+#include "wg_records.cuh"
 #include <algorithm>
 #include <vector>
 
@@ -769,6 +770,7 @@ online_merge_pop_kernel(int B, const wg_herdt_mpc_state *__restrict__ states, co
 constexpr int ROW_V4 = (int)(sizeof(wg_herdt_tick) / 16);                 // 16
 constexpr int RING_V4 = QCAP * ROW_V4;                                    // 464
 constexpr int RING_ITERS = (RING_V4 + 31) / 32;                           // 15: unrolled, so a lane has all its loads in flight
+constexpr int RING_UNROLL = 8;   // restore and copy: ring words of a lane in flight, the most at 32 registers (16 CTAs per SM)
 constexpr int STATE_LL = (int)(sizeof(wg_herdt_mpc_state) / 8);           // 125
 constexpr int TAIL_V2 = (int)((sizeof(wg_herdt_online_robot) - offsetof(wg_herdt_online_robot, state)) / 16);   // 64
 static_assert(sizeof(wg_herdt_online_robot) == 8448 && offsetof(wg_herdt_online_robot, rows) == 0, "record layout");
@@ -815,12 +817,7 @@ online_restore_kernel(int n, const int32_t *__restrict__ idx, const wg_herdt_onl
   for (int i = blockIdx.x * MPC_WARPS + warp; i < n; i += gridDim.x * MPC_WARPS) {
     const int b = idx ? idx[i] : i;
     const uint4 *src = reinterpret_cast<const uint4 *>(in + i);
-    uint4 *q = reinterpret_cast<uint4 *>(queue + (size_t)b * QCAP);
-#pragma unroll
-    for (int k = 0; k < RING_ITERS; ++k) {
-      const int e = lane + 32 * k;
-      if (e < RING_V4) q[e] = src[e];
-    }
+    wgi_warp_copy16<RING_UNROLL>(reinterpret_cast<uint4 *>(queue + (size_t)b * QCAP), src, RING_V4, RING_V4, lane);
     long long *st = reinterpret_cast<long long *>(states + b);
     const longlong2 *t = reinterpret_cast<const longlong2 *>(src + RING_V4);
     for (int e = lane; e < TAIL_V2; e += 32) {
@@ -853,13 +850,8 @@ online_copy_kernel(int n, const int32_t *__restrict__ didx, const int32_t *__res
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (int i = blockIdx.x * MPC_WARPS + warp; i < n; i += gridDim.x * MPC_WARPS) {
     const int d = didx ? didx[i] : i, s = sidx ? sidx[i] : i;
-    const uint4 *sq = reinterpret_cast<const uint4 *>(s_queue + (size_t)s * QCAP);
-    uint4 *dq = reinterpret_cast<uint4 *>(d_queue + (size_t)d * QCAP);
-#pragma unroll
-    for (int k = 0; k < RING_ITERS; ++k) {
-      const int e = lane + 32 * k;
-      if (e < RING_V4) dq[e] = sq[e];
-    }
+    wgi_warp_copy16<RING_UNROLL>(reinterpret_cast<uint4 *>(d_queue + (size_t)d * QCAP),
+                                 reinterpret_cast<const uint4 *>(s_queue + (size_t)s * QCAP), RING_V4, RING_V4, lane);
     const long long *ss = reinterpret_cast<const long long *>(s_states + s);
     long long *ds = reinterpret_cast<long long *>(d_states + d);
     for (int e = lane; e < STATE_LL; e += 32) ds[e] = ss[e];
@@ -1120,58 +1112,39 @@ struct wg_herdt_online {
   wg_herdt_tick *d_queue = nullptr;    // [B][QCAP]
   OnlineSlot *d_slots = nullptr;       // [B]
   wg_herdt_tick *d_staged = nullptr;   // [B][20]: the rows mpc_post_kernel writes for a robot that fires
-  // staging of start (init states, indices) and of WG_MEM_HOST ticks (commands, rows, running)
-  void *d_init = nullptr, *d_idx = nullptr, *d_cmd = nullptr, *d_rows = nullptr, *d_run = nullptr;
-  size_t cap_init = 0, cap_idx = 0, cap_cmd = 0, cap_rows = 0, cap_run = 0;
-  // staging of WG_MEM_HOST robot records, and the flag of the device-record check
-  void *d_robots = nullptr, *d_flag = nullptr;
-  size_t cap_robots = 0, cap_flag = 0;
+  // staging of WG_MEM_HOST ticks (commands, rows, running) and of WG_MEM_HOST robot records
+  void *d_cmd = nullptr, *d_rows = nullptr, *d_run = nullptr, *d_robots = nullptr;
+  size_t cap_cmd = 0, cap_rows = 0, cap_run = 0, cap_robots = 0;
+  wgi_stage stage;   // start: init states and indices; save, restore, copy: the check flag, and the indices on the device
 };
 
 static void online_free(wg_herdt_online *h)
 {
   cudaFree(h->d_states); cudaFree(h->d_queue); cudaFree(h->d_slots); cudaFree(h->d_staged);
-  cudaFree(h->d_init); cudaFree(h->d_idx); cudaFree(h->d_cmd); cudaFree(h->d_rows); cudaFree(h->d_run);
-  cudaFree(h->d_robots); cudaFree(h->d_flag);
+  cudaFree(h->d_cmd); cudaFree(h->d_rows); cudaFree(h->d_run); cudaFree(h->d_robots);
+  wgi_stage_free(&h->stage);
   delete h;
 }
 
-// Robot indices from the host: NULL = 0..n-1 (needs n <= B); otherwise in [0, B), and unique when `unique`.  Sets mark[b]
-// (B entries, zero on entry) for every robot b named.
-static bool online_indices_ok(int B, int n, const int32_t *idx, bool unique, std::vector<char> &mark)
-{
-  if (!idx) {
-    if (n > B) return false;
-    for (int i = 0; i < n; ++i) mark[i] = 1;
-    return true;
-  }
-  for (int i = 0; i < n; ++i) {
-    const int32_t b = idx[i];
-    if (b < 0 || b >= B || (unique && mark[b])) return false;
-    mark[b] = 1;
-  }
-  return true;
-}
-
-// Upload up to two host index arrays into the handle's index scratch; a NULL array stays NULL.
-static int online_upload_indices(wg_herdt_online *h, int n, const int32_t *a, const int32_t *b, const int32_t **da,
-                                 const int32_t **db)
+// The device mirror of the handle's stage holds a zeroed check flag (an int at its start) when `flag`, then the host index
+// arrays a and b; a NULL array stays NULL on the device.  The flag goes through the pinned blob.  The indices go straight
+// from the caller's pageable arrays: at 10^5 robots and more, packing them into the blob first made the whole call slower.
+static int online_stage(wg_herdt_online *h, int n, bool flag, const int32_t *a, const int32_t *b, const int32_t **da,
+                        const int32_t **db)
 {
   wg_ctx *ctx = h->ctx;
-  const size_t bytes = sizeof(int32_t) * (size_t)n;
+  const size_t ib = sizeof(int32_t) * (size_t)n, off_a = flag ? sizeof(int) : 0, off_b = off_a + (a ? ib : 0);
+  const size_t bytes = off_b + (b ? ib : 0);
+  unsigned char *hb = nullptr;
   int rc;
-  if ((a || b) && (rc = wgi_grow_scratch(ctx, &h->d_idx, &h->cap_idx, bytes * ((a && b) ? 2 : 1))) != WG_OK) return rc;
-  int32_t *d = static_cast<int32_t *>(h->d_idx);
-  *da = nullptr;
-  if (db) *db = nullptr;
-  if (a) { WG_CUDA(ctx, cudaMemcpyAsync(d, a, bytes, cudaMemcpyHostToDevice, ctx->stream)); *da = d; d += n; }
-  if (b) { WG_CUDA(ctx, cudaMemcpyAsync(d, b, bytes, cudaMemcpyHostToDevice, ctx->stream)); *db = d; }
+  if (bytes && (rc = wgi_stage_reserve(ctx, &h->stage, off_a, &hb)) != WG_OK) return rc;
+  if (flag) std::memset(hb, 0, sizeof(int));
+  if (bytes && (rc = wgi_stage_send(ctx, &h->stage, off_a, bytes)) != WG_OK) return rc;
+  if (a) WG_CUDA(ctx, cudaMemcpyAsync(h->stage.d + off_a, a, ib, cudaMemcpyHostToDevice, ctx->stream));
+  if (b) WG_CUDA(ctx, cudaMemcpyAsync(h->stage.d + off_b, b, ib, cudaMemcpyHostToDevice, ctx->stream));
+  *da = a ? reinterpret_cast<const int32_t *>(h->stage.d + off_a) : nullptr;
+  if (db) *db = b ? reinterpret_cast<const int32_t *>(h->stage.d + off_b) : nullptr;
   return WG_OK;
-}
-
-static int online_blocks(wg_ctx *ctx, int n)
-{
-  return std::max(1, std::min((n + MPC_WARPS - 1) / MPC_WARPS, ctx->sm_count * 16));
 }
 
 static int online_ticks(wg_herdt_online *h, MpcState *m, int nticks, const wg_herdt_command *cmd, wg_herdt_tick *rows,
@@ -1186,8 +1159,7 @@ static int online_ticks(wg_herdt_online *h, MpcState *m, int nticks, const wg_he
   wg_herdt_qp_output *out = static_cast<wg_herdt_qp_output *>(m->d_out);
   MpcScratch *scr = static_cast<MpcScratch *>(m->d_scr);
   const herdt::Consts *consts = wg_herdt_device_consts(ctx);
-  const int blocks_tick = std::max(1, std::min((B + 32 * MPC_WARPS - 1) / (32 * MPC_WARPS), ctx->sm_count * 16));
-  const int blocks = std::max(1, std::min((B + MPC_WARPS - 1) / MPC_WARPS, ctx->sm_count * 16));
+  const int blocks_tick = wgi_grid(ctx, B, 32 * MPC_WARPS, 16), blocks = wgi_grid(ctx, B, MPC_WARPS, 16);
   const size_t smem_tick = (sizeof(wg_herdt_qp_input) + sizeof(MpcWarp)) * MPC_WARPS, smem_post = sizeof(MpcWarp) * MPC_WARPS;
   for (int t = 0; t < nticks; ++t) {
     wg_prof_start(ctx, WG_K_HERDT_MPC);
@@ -1256,26 +1228,24 @@ int wg_herdt_online_start(wg_herdt_online *h, int n, const int32_t *idx_host, co
   if (!h || n < 0 || init_stride < 0 || (n > 0 && (!idx_host || !init15_host))) return WG_ERR_INVALID;
   wg_ctx *ctx = h->ctx;
   std::vector<char> seen((size_t)h->B, 0);
-  for (int i = 0; i < n; ++i) {
-    const int32_t b = idx_host[i];
-    if (b < 0 || b >= h->B || seen[b]) return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_start: index out of range or repeated");
-    seen[b] = 1;
-  }
+  if (!wgi_record_indices_ok(h->B, n, idx_host, true, seen))
+    return wg_refuse(ctx, "wg_herdt_online_start", "index out of range or repeated");
   MpcState *m = mpc_of(ctx);
   if (!m->ready) return wg_fail(ctx, WG_ERR_NOT_READY, "wg_herdt_mpc_set_params not called");
   if (n == 0) return WG_OK;
   wg_device_guard guard(ctx->device);
-  std::vector<wg_herdt_mpc_state> init((size_t)n);
-  int rc = mpc_init_impl(ctx, WG_MEM_HOST, n, init15_host, init_stride, init.data(), true);
+  // one H2D copy: the initial states, then the indices
+  const size_t sbytes = sizeof(wg_herdt_mpc_state) * (size_t)n, bytes = sbytes + sizeof(int32_t) * (size_t)n;
+  unsigned char *hb;
+  int rc = wgi_stage_reserve(ctx, &h->stage, bytes, &hb);
   if (rc != WG_OK) return rc;
-  if ((rc = wgi_grow_scratch(ctx, &h->d_init, &h->cap_init, sizeof(wg_herdt_mpc_state) * (size_t)n)) != WG_OK) return rc;
-  if ((rc = wgi_grow_scratch(ctx, &h->d_idx, &h->cap_idx, sizeof(int32_t) * (size_t)n)) != WG_OK) return rc;
-  WG_CUDA(ctx, cudaMemcpyAsync(h->d_init, init.data(), sizeof(wg_herdt_mpc_state) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
-  WG_CUDA(ctx, cudaMemcpyAsync(h->d_idx, idx_host, sizeof(int32_t) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
-  const int blocks = std::max(1, std::min((n + MPC_WARPS - 1) / MPC_WARPS, ctx->sm_count * 16));
-  online_start_kernel<<<blocks, MPC_WARPS * 32, 0, ctx->stream>>>(n, static_cast<const int32_t *>(h->d_idx),
-                                                                  static_cast<const wg_herdt_mpc_state *>(h->d_init),
-                                                                  h->d_states, h->d_queue, h->d_slots);
+  rc = mpc_init_impl(ctx, WG_MEM_HOST, n, init15_host, init_stride, reinterpret_cast<wg_herdt_mpc_state *>(hb), true);
+  if (rc != WG_OK) return rc;
+  std::memcpy(hb + sbytes, idx_host, sizeof(int32_t) * (size_t)n);
+  if ((rc = wgi_stage_send(ctx, &h->stage, bytes)) != WG_OK) return rc;
+  online_start_kernel<<<wgi_grid(ctx, n, MPC_WARPS, 16), MPC_WARPS * 32, 0, ctx->stream>>>(
+      n, reinterpret_cast<const int32_t *>(h->stage.d + sbytes), reinterpret_cast<const wg_herdt_mpc_state *>(h->stage.d),
+      h->d_states, h->d_queue, h->d_slots);
   WG_LAUNCHED(ctx);
   WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return WG_OK;
@@ -1312,11 +1282,10 @@ int wg_herdt_online_save(wg_herdt_online *h, int mem, int n, const int32_t *idx,
 {
   if (!h || n < 0 || (n > 0 && !out) || (mem != WG_MEM_HOST && mem != WG_MEM_DEVICE)) return WG_ERR_INVALID;
   wg_ctx *ctx = h->ctx;
-  if (mem == WG_MEM_DEVICE && reinterpret_cast<uintptr_t>(out) % 16)
-    return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_save: device records must be 16-byte aligned");
+  const char *call = "wg_herdt_online_save";
+  if (mem == WG_MEM_DEVICE && reinterpret_cast<uintptr_t>(out) % 16) return wg_refuse(ctx, call, "device records must be 16-byte aligned");
   std::vector<char> mark((size_t)h->B, 0);
-  if (!online_indices_ok(h->B, n, idx, false, mark))
-    return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_save: index out of range, or n > B without indices");
+  if (!wgi_record_indices_ok(h->B, n, idx, false, mark)) return wg_refuse(ctx, call, "index out of range, or n > B without indices");
   if (n == 0) return WG_OK;
   wg_device_guard guard(ctx->device);
   const size_t bytes = sizeof(wg_herdt_online_robot) * (size_t)n;
@@ -1324,10 +1293,10 @@ int wg_herdt_online_save(wg_herdt_online *h, int mem, int n, const int32_t *idx,
   if (mem == WG_MEM_HOST && (rc = wgi_grow_scratch(ctx, &h->d_robots, &h->cap_robots, bytes)) != WG_OK) return rc;
   wg_herdt_online_robot *d_out = mem == WG_MEM_HOST ? static_cast<wg_herdt_online_robot *>(h->d_robots) : out;
   const int32_t *d_idx;
-  if ((rc = online_upload_indices(h, n, idx, nullptr, &d_idx, nullptr)) != WG_OK) return rc;
+  if ((rc = online_stage(h, n, false, idx, nullptr, &d_idx, nullptr)) != WG_OK) return rc;
   wg_prof_start(ctx, WG_K_HERDT_MPC);
-  online_save_kernel<<<online_blocks(ctx, n), MPC_WARPS * 32, 0, ctx->stream>>>(n, d_idx, h->d_states, h->d_queue, h->d_slots,
-                                                                                d_out);
+  online_save_kernel<<<wgi_grid(ctx, n, MPC_WARPS, 16), MPC_WARPS * 32, 0, ctx->stream>>>(n, d_idx, h->d_states, h->d_queue,
+                                                                                          h->d_slots, d_out);
   wg_prof_stop(ctx);
   WG_LAUNCHED(ctx);
   if (mem == WG_MEM_DEVICE) return WG_OK;
@@ -1345,41 +1314,39 @@ int wg_herdt_online_restore(wg_herdt_online *h, int mem, int n, const int32_t *i
 {
   if (!h || n < 0 || (n > 0 && !in) || (mem != WG_MEM_HOST && mem != WG_MEM_DEVICE)) return WG_ERR_INVALID;
   wg_ctx *ctx = h->ctx;
-  if (mem == WG_MEM_DEVICE && reinterpret_cast<uintptr_t>(in) % 16)
-    return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_restore: device records must be 16-byte aligned");
+  const char *call = "wg_herdt_online_restore";
+  if (mem == WG_MEM_DEVICE && reinterpret_cast<uintptr_t>(in) % 16) return wg_refuse(ctx, call, "device records must be 16-byte aligned");
   std::vector<char> mark((size_t)h->B, 0);
-  if (!online_indices_ok(h->B, n, idx, true, mark))
-    return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_restore: index out of range or repeated, or n > B without indices");
+  if (!wgi_record_indices_ok(h->B, n, idx, true, mark))
+    return wg_refuse(ctx, call, "index out of range or repeated, or n > B without indices");
   if (mem == WG_MEM_HOST)
     for (int i = 0; i < n; ++i)
-      if (!online_record_ok(in[i])) return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_restore: invalid count / running");
+      if (!online_record_ok(in[i])) return wg_refuse(ctx, call, "invalid count / running");
   if (n == 0) return WG_OK;
   wg_device_guard guard(ctx->device);
   const size_t bytes = sizeof(wg_herdt_online_robot) * (size_t)n;
-  const int blocks = online_blocks(ctx, n);
   int rc;
   const wg_herdt_online_robot *d_in = in;
   if (mem == WG_MEM_HOST) {
     if ((rc = wgi_grow_scratch(ctx, &h->d_robots, &h->cap_robots, bytes)) != WG_OK) return rc;
     d_in = static_cast<const wg_herdt_online_robot *>(h->d_robots);
     WG_CUDA(ctx, cudaMemcpyAsync(h->d_robots, in, bytes, cudaMemcpyHostToDevice, ctx->stream));
-  } else {
-    if ((rc = wgi_grow_scratch(ctx, &h->d_flag, &h->cap_flag, sizeof(int))) != WG_OK) return rc;
-    int *flag = static_cast<int *>(h->d_flag), bad = 0;
-    WG_CUDA(ctx, cudaMemsetAsync(flag, 0, sizeof(int), ctx->stream));
+  }
+  // device records: the check flag goes with the indices, and the check kernel runs before any robot changes
+  const int32_t *d_idx;
+  if ((rc = online_stage(h, n, mem == WG_MEM_DEVICE, idx, nullptr, &d_idx, nullptr)) != WG_OK) return rc;
+  if (mem == WG_MEM_DEVICE) {
     wg_prof_start(ctx, WG_K_HERDT_MPC);
-    online_restore_check_kernel<<<std::max(1, std::min((n + MPC_WARPS * 32 - 1) / (MPC_WARPS * 32), ctx->sm_count * 16)),
-                                  MPC_WARPS * 32, 0, ctx->stream>>>(n, in, flag);
+    online_restore_check_kernel<<<wgi_grid(ctx, n, MPC_WARPS * 32, 16), MPC_WARPS * 32, 0, ctx->stream>>>(
+        n, in, reinterpret_cast<int *>(h->stage.d));
     wg_prof_stop(ctx);
     WG_LAUNCHED(ctx);
-    WG_CUDA(ctx, cudaMemcpyAsync(&bad, flag, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    WG_CUDA(ctx, cudaMemcpyAsync(h->stage.h, h->stage.d, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
     WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    if (bad) return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_restore: invalid count / running");
+    if (*reinterpret_cast<const int *>(h->stage.h)) return wg_refuse(ctx, call, "invalid count / running");
   }
-  const int32_t *d_idx;
-  if ((rc = online_upload_indices(h, n, idx, nullptr, &d_idx, nullptr)) != WG_OK) return rc;
   wg_prof_start(ctx, WG_K_HERDT_MPC);
-  online_restore_kernel<<<blocks, MPC_WARPS * 32, 0, ctx->stream>>>(n, d_idx, d_in, h->d_states, h->d_queue, h->d_slots);
+  online_restore_kernel<<<wgi_grid(ctx, n, MPC_WARPS, 16), MPC_WARPS * 32, 0, ctx->stream>>>(n, d_idx, d_in, h->d_states, h->d_queue, h->d_slots);
   wg_prof_stop(ctx);
   WG_LAUNCHED(ctx);
   if (mem == WG_MEM_HOST) WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1391,22 +1358,17 @@ int wg_herdt_online_copy(wg_herdt_online *dst, int n, const int32_t *dst_idx, co
 {
   if (!dst || !src || n < 0) return WG_ERR_INVALID;
   wg_ctx *ctx = dst->ctx;
-  if (src->ctx != ctx) return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_copy: handles of two contexts");
-  std::vector<char> dmark((size_t)dst->B, 0), smark((size_t)src->B, 0);
-  if (!online_indices_ok(dst->B, n, dst_idx, true, dmark) || !online_indices_ok(src->B, n, src_idx, false, smark))
-    return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_copy: index out of range, repeated destination, or n > B without indices");
-  if (dst == src)
-    for (int b = 0; b < dst->B; ++b)
-      if (dmark[b] && smark[b]) return wg_fail(ctx, WG_ERR_INVALID, "wg_herdt_online_copy: a robot is both source and destination");
+  const char *call = "wg_herdt_online_copy";
+  if (src->ctx != ctx) return wg_refuse(ctx, call, "handles of two contexts");
+  if (const char *why = wgi_copy_indices_refusal(n, dst->B, dst_idx, src->B, src_idx, dst == src)) return wg_refuse(ctx, call, why);
   if (n == 0) return WG_OK;
   wg_device_guard guard(ctx->device);
   const int32_t *d_didx, *d_sidx;
-  const int rc = online_upload_indices(dst, n, dst_idx, src_idx, &d_didx, &d_sidx);
+  const int rc = online_stage(dst, n, false, dst_idx, src_idx, &d_didx, &d_sidx);
   if (rc != WG_OK) return rc;
   wg_prof_start(ctx, WG_K_HERDT_MPC);
-  online_copy_kernel<<<online_blocks(ctx, n), MPC_WARPS * 32, 0, ctx->stream>>>(n, d_didx, d_sidx, src->d_states, src->d_queue,
-                                                                                src->d_slots, dst->d_states, dst->d_queue,
-                                                                                dst->d_slots);
+  online_copy_kernel<<<wgi_grid(ctx, n, MPC_WARPS, 16), MPC_WARPS * 32, 0, ctx->stream>>>(
+      n, d_didx, d_sidx, src->d_states, src->d_queue, src->d_slots, dst->d_states, dst->d_queue, dst->d_slots);
   wg_prof_stop(ctx);
   WG_LAUNCHED(ctx);
   return WG_OK;

@@ -1,6 +1,7 @@
 // wg_common.h - internal definitions shared by the CUDA translation units of libwalkgen_b200.so.
 #pragma once
 #include <cuda_runtime.h>
+#include <algorithm>
 #include <cstdio>
 #include <cstring>
 #include <string>
@@ -67,6 +68,13 @@ inline int wg_fail(wg_ctx *ctx, int code, const char *what, cudaError_t e = cuda
   return code;
 }
 
+// Refuse a call's arguments: "<call>: <why>" in ctx->err, WG_ERR_INVALID returned.
+inline int wg_refuse(wg_ctx *ctx, const char *call, const char *why)
+{
+  snprintf(ctx->err, sizeof ctx->err, "%s: %s", call, why);
+  return WG_ERR_INVALID;
+}
+
 #define WG_CUDA(ctx, call)                                                   \
   do {                                                                       \
     cudaError_t e__ = (call);                                                \
@@ -110,6 +118,33 @@ extern "C" int wgi_smem_attr(wg_ctx *ctx, const void *func, size_t bytes);
 // buffer that must grow is freed after the context stream drains (earlier launches may still read it); on return *buf is
 // never null.
 extern "C" int wgi_grow_scratch(wg_ctx *ctx, void **buf, size_t *cap, size_t bytes);
+
+// Host -> device staging of a call's small inputs: a pinned blob, its device mirror, and the event recorded after the copy,
+// which says the device has read the blob.  Reserve waits on that event and grows the blob to `bytes` (*host); send grows the
+// mirror to max(bytes, room), half as much again to amortise (`room`: space that kernels write), copies the first `bytes`
+// into it and records the event.  The host may read the blob after send, and write it again after the next reserve.
+struct wgi_stage {
+  unsigned char *h = nullptr, *d = nullptr;
+  size_t h_cap = 0, d_cap = 0;
+  cudaEvent_t ev = nullptr;   // created by the first reserve
+};
+int wgi_stage_reserve(wg_ctx *ctx, wgi_stage *st, size_t bytes, unsigned char **host);
+int wgi_stage_send(wg_ctx *ctx, wgi_stage *st, size_t bytes, size_t room = 0);
+void wgi_stage_free(wgi_stage *st);   // after the context stream has drained
+
+// Record indices from the host, as the whole-record calls (save / restore / copy) of the on-line generators take them:
+// NULL = 0..n-1 (needs n <= B); otherwise in [0, B), and unique when `unique`.  Sets mark[b] (B entries, zero on entry) for
+// every record b named.
+bool wgi_record_indices_ok(int B, int n, const int32_t *idx, bool unique, std::vector<char> &mark);
+// The index rule of a copy of n records from a handle of sB records into one of dB: destinations unique, sources may
+// repeat, and no index on both sides when the two handles are one.  nullptr when the call may go on, else why it may not.
+const char *wgi_copy_indices_refusal(int n, int dB, const int32_t *dst_idx, int sB, const int32_t *src_idx, bool same);
+
+// Grid of a grid-stride kernel that takes `per_block` items per CTA, at most `per_sm` CTAs per SM, and at least one CTA.
+inline int wgi_grid(const wg_ctx *ctx, int n, int per_block, int per_sm)
+{
+  return std::max(1, std::min((n + per_block - 1) / per_block, ctx->sm_count * per_sm));
+}
 
 // preview.cu internals used by zmpdisc.cu (the footsteps -> CoM pipeline): launch the fused preview kernel over `count`
 // trajectories listed in the device array d_order.

@@ -43,6 +43,65 @@ extern "C" int wgi_grow_scratch(wg_ctx *ctx, void **buf, size_t *cap, size_t byt
   return WG_OK;
 }
 
+int wgi_stage_reserve(wg_ctx *ctx, wgi_stage *st, size_t bytes, unsigned char **host)
+{
+  if (!st->ev) WG_CUDA(ctx, cudaEventCreateWithFlags(&st->ev, cudaEventDisableTiming));
+  else WG_CUDA(ctx, cudaEventSynchronize(st->ev));
+  if (bytes > st->h_cap) {
+    cudaFreeHost(st->h);
+    st->h = nullptr; st->h_cap = 0;
+    WG_CUDA(ctx, cudaMallocHost(&st->h, bytes + bytes / 2));
+    st->h_cap = bytes + bytes / 2;
+  }
+  *host = st->h;
+  return WG_OK;
+}
+
+int wgi_stage_send(wg_ctx *ctx, wgi_stage *st, size_t bytes, size_t room)
+{
+  const size_t need = std::max(bytes, room);
+  int rc;
+  if ((need > st->d_cap || !st->d) &&
+      (rc = wgi_grow_scratch(ctx, reinterpret_cast<void **>(&st->d), &st->d_cap, std::max(need + need / 2, (size_t)256))) != WG_OK)
+    return rc;
+  if (bytes) WG_CUDA(ctx, cudaMemcpyAsync(st->d, st->h, bytes, cudaMemcpyHostToDevice, ctx->stream));
+  WG_CUDA(ctx, cudaEventRecord(st->ev, ctx->stream));
+  return WG_OK;
+}
+
+void wgi_stage_free(wgi_stage *st)
+{
+  if (st->ev) cudaEventDestroy(st->ev);
+  cudaFreeHost(st->h);
+  cudaFree(st->d);
+}
+
+bool wgi_record_indices_ok(int B, int n, const int32_t *idx, bool unique, std::vector<char> &mark)
+{
+  if (!idx) {
+    if (n > B) return false;
+    for (int i = 0; i < n; ++i) mark[i] = 1;
+    return true;
+  }
+  for (int i = 0; i < n; ++i) {
+    const int32_t b = idx[i];
+    if (b < 0 || b >= B || (unique && mark[b])) return false;
+    mark[b] = 1;
+  }
+  return true;
+}
+
+const char *wgi_copy_indices_refusal(int n, int dB, const int32_t *dst_idx, int sB, const int32_t *src_idx, bool same)
+{
+  std::vector<char> dmark((size_t)dB, 0), smark((size_t)sB, 0);
+  if (!wgi_record_indices_ok(dB, n, dst_idx, true, dmark) || !wgi_record_indices_ok(sB, n, src_idx, false, smark))
+    return "index out of range, repeated destination, or n > B without indices";
+  if (same)
+    for (int b = 0; b < dB; ++b)
+      if (dmark[b] && smark[b]) return "an index is both a source and a destination";
+  return nullptr;
+}
+
 extern "C" {
 
 int wg_version(void) { return WG_VERSION; }

@@ -20,6 +20,7 @@
 #include <cmath>
 #include <new>
 #include "wg_common.h"
+#include "wg_records.cuh"
 
 namespace {
 
@@ -675,25 +676,6 @@ __host__ __device__ __forceinline__ bool zs_counts_ok(int64_t e, int64_t p, int3
   return (open == 0 || open == 1) && e >= 0 && (open == 0 || e > 0) && p == (pv && e > NL1 ? e - NL1 : 0);
 }
 
-// Words [0, nv) of dst from src, by one warp, with ZS_UNROLL loads of a lane in flight; words from `keep` on are zero.
-__device__ __forceinline__ void zs_move(uint4 *__restrict__ dst, const uint4 *__restrict__ src, int nv, int64_t keep, int lane)
-{
-  if (keep > nv) keep = nv;
-  for (int e0 = 0; e0 < nv; e0 += 32 * ZS_UNROLL) {
-    uint4 v[ZS_UNROLL];
-#pragma unroll
-    for (int u = 0; u < ZS_UNROLL; ++u) {
-      const int e = e0 + 32 * u + lane;
-      v[u] = (e < keep) ? src[e] : make_uint4(0u, 0u, 0u, 0u);
-    }
-#pragma unroll
-    for (int u = 0; u < ZS_UNROLL; ++u) {
-      const int e = e0 + 32 * u + lane;
-      if (e < nv) dst[e] = v[u];
-    }
-  }
-}
-
 // The canonical record of walk cnt[i].b: ZsRec with samples_emitted from the host counter (ZdWalk::F0 stops advancing at
 // EndPhaseOfTheWalking, so it lags a finished walk by the end phase; nothing reads it until the next START), carry rows past
 // emitted - previewed zero, all zero for a walk never started (its ZsRec was never written).
@@ -725,8 +707,8 @@ stream_save_kernel(int n, const ZsCounts *__restrict__ cnt, const ZsRec *__restr
       o[e] = v;
     }
     if (NL1 > 0)
-      zs_move(reinterpret_cast<uint4 *>(out_carry + (int64_t)i * NL1), reinterpret_cast<const uint4 *>(carry + (int64_t)c.b * NL1),
-              NL1, live ? c.emitted - c.previewed : 0, lane);
+      wgi_warp_copy16<ZS_UNROLL>(reinterpret_cast<uint4 *>(out_carry + (int64_t)i * NL1),
+                                 reinterpret_cast<const uint4 *>(carry + (int64_t)c.b * NL1), NL1, live ? c.emitted - c.previewed : 0, lane);
   }
 }
 
@@ -756,8 +738,9 @@ stream_restore_kernel(int n, const int32_t *__restrict__ idx, const wg_kajita_st
       else if (e < ZS_REC_V4 + ZS_STATE_V4 && st) st[e - ZS_REC_V4] = v[k];
     }
     if (NL1 > 0)
-      zs_move(reinterpret_cast<uint4 *>(carry + (int64_t)b * NL1), reinterpret_cast<const uint4 *>(in_carry + (int64_t)i * NL1),
-              NL1, in[i].samples_emitted - in[i].steps_previewed, lane);
+      wgi_warp_copy16<ZS_UNROLL>(reinterpret_cast<uint4 *>(carry + (int64_t)b * NL1),
+                                 reinterpret_cast<const uint4 *>(in_carry + (int64_t)i * NL1), NL1,
+                                 in[i].samples_emitted - in[i].steps_previewed, lane);
     if (lane == 0) status[b] = 0;
   }
 }
@@ -803,8 +786,8 @@ stream_copy_kernel(int n, const int32_t *__restrict__ didx, const int32_t *__res
       else if (e < ZS_REC_V4 + ZS_STATE_V4 && ds) ds[e - ZS_REC_V4] = v[k];
     }
     if (NL1 > 0)
-      zs_move(reinterpret_cast<uint4 *>(d_carry + (int64_t)d * NL1), reinterpret_cast<const uint4 *>(s_carry + (int64_t)s * NL1),
-              NL1, NL1, lane);
+      wgi_warp_copy16<ZS_UNROLL>(reinterpret_cast<uint4 *>(d_carry + (int64_t)d * NL1),
+                                 reinterpret_cast<const uint4 *>(s_carry + (int64_t)s * NL1), NL1, NL1, lane);
     if (lane == 0) d_status[d] = 0;
   }
 }
@@ -1275,9 +1258,7 @@ struct wg_kajita_stream {
   bool pending;
   int nwork, npv;
   size_t off_steps, off_po, off_order, bytes;
-  unsigned char *h_blob, *d_blob;
-  size_t h_cap, d_cap;
-  cudaEvent_t ev_staged;                        // the device has consumed h_blob
+  wgi_stage stage;                              // an append's blob; when none is pending, a save, restore or copy's
   ZsRec *d_rec;
   double2 *d_carry, *d_lead, *d_pk;
   double *d_state;
@@ -1296,60 +1277,13 @@ struct wg_kajita_stream {
 static int zs_grow(wg_ctx *ctx, void **p, size_t *cap, size_t bytes)
 {
   if (bytes <= *cap && *p) return WG_OK;
-  const size_t want = std::max(bytes + bytes / 2, (size_t)256);
-  WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));   // a kernel of an earlier run may still read the old buffer
-  cudaFree(*p);
-  *p = nullptr;
-  *cap = 0;
-  WG_CUDA(ctx, cudaMalloc(p, want));
-  *cap = want;
-  return WG_OK;
+  return wgi_grow_scratch(ctx, p, cap, std::max(bytes + bytes / 2, (size_t)256));
 }
 
 static size_t zs_align(size_t x) { return (x + 15) / 16 * 16; }
 
-// Make the pinned blob hold at least `bytes`, once the device has read what it last held (ev_staged).  The blob carries the
-// inputs of an append, or, when no append is pending, the indices and counters of a save, restore or copy.
-static int zs_stage_host(wg_kajita_stream *s, size_t bytes)
-{
-  wg_ctx *ctx = s->ctx;
-  WG_CUDA(ctx, cudaEventSynchronize(s->ev_staged));
-  if (bytes > s->h_cap) {
-    cudaFreeHost(s->h_blob);
-    s->h_blob = nullptr;
-    s->h_cap = 0;
-    const size_t want = bytes + bytes / 2;
-    WG_CUDA(ctx, cudaMallocHost(&s->h_blob, want));
-    s->h_cap = want;
-  }
-  return WG_OK;
-}
-
 // Whole walks: the helpers of wg_kajita_stream_save / restore / copy.
 static int zs_carry_rows(const wg_kajita_stream *s) { return s->with_preview ? std::max(0, s->NL - 1) : 0; }
-
-static int zs_refuse(wg_ctx *ctx, const char *call, const char *why)
-{
-  snprintf(ctx->err, sizeof ctx->err, "%s: %s", call, why);
-  return WG_ERR_INVALID;
-}
-
-// Walk indices from the host: NULL = 0..n-1 (needs n <= B); otherwise in [0, B), and unique when `unique`.  Sets mark[b]
-// (B entries, zero on entry) for every walk b named.
-static bool zs_indices_ok(int B, int n, const int32_t *idx, bool unique, std::vector<char> &mark)
-{
-  if (!idx) {
-    if (n > B) return false;
-    for (int i = 0; i < n; ++i) mark[i] = 1;
-    return true;
-  }
-  for (int i = 0; i < n; ++i) {
-    const int32_t b = idx[i];
-    if (b < 0 || b >= B || (unique && mark[b])) return false;
-    mark[b] = 1;
-  }
-  return true;
-}
 
 // The argument checks save and restore share: nullptr when the call may go on, else why it may not.
 static const char *zs_io_refusal(const wg_kajita_stream *s, int mem, int n, const void *walks, const void *carry)
@@ -1366,10 +1300,7 @@ static const char *zs_io_refusal(const wg_kajita_stream *s, int mem, int n, cons
 
 // Grid of a whole-walk kernel: at most 6 CTAs of ZS_WARPS warps per SM, which all stay resident at up to 40 registers (the
 // kernels take 18 to 38), so the grid-stride loops leave no second wave.
-static int zs_blocks(const wg_ctx *ctx, int n, int per_block)
-{
-  return std::max(1, std::min((n + per_block - 1) / per_block, ctx->sm_count * 6));
-}
+constexpr int ZS_CTAS_PER_SM = 6;
 
 extern "C" {
 
@@ -1379,9 +1310,8 @@ int wg_kajita_stream_destroy(wg_kajita_stream *s)
   wg_device_guard guard(s->ctx->device);
   cudaStreamSynchronize(s->ctx->stream);
   if (s->pv) wg_preview_plan_destroy(s->pv);
-  if (s->ev_staged) cudaEventDestroy(s->ev_staged);
-  cudaFreeHost(s->h_blob);
-  cudaFree(s->d_blob); cudaFree(s->d_rec); cudaFree(s->d_carry); cudaFree(s->d_lead); cudaFree(s->d_pk);
+  wgi_stage_free(&s->stage);
+  cudaFree(s->d_rec); cudaFree(s->d_carry); cudaFree(s->d_lead); cudaFree(s->d_pk);
   cudaFree(s->d_state); cudaFree(s->d_status); cudaFree(s->d_next); cudaFree(s->d_io);
   for (void *p : s->d_out) cudaFree(p);
   delete s;
@@ -1407,7 +1337,6 @@ int wg_kajita_stream_create(wg_ctx *ctx, const wg_zmpdisc_params *p, int B, int 
   if (e == cudaSuccess) e = cudaMalloc(&s->d_status, sizeof(int) * B);
   if (e == cudaSuccess) e = cudaMalloc(&s->d_next, sizeof(int));
   if (e == cudaSuccess) e = cudaMalloc(&s->d_lead, sizeof(double2) * (size_t)std::max(1, K.n_lead));
-  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s->ev_staged, cudaEventDisableTiming);
   if (e == cudaSuccess) e = cudaMemsetAsync(s->d_status, 0, sizeof(int) * B, ctx->stream);
   if (e == cudaSuccess && with_preview) e = cudaMalloc(&s->d_state, sizeof(double) * 8 * B);
   if (e == cudaSuccess && with_preview) e = cudaMemsetAsync(s->d_state, 0, sizeof(double) * 8 * B, ctx->stream);
@@ -1416,7 +1345,6 @@ int wg_kajita_stream_create(wg_ctx *ctx, const wg_zmpdisc_params *p, int B, int 
     zmpdisc_lead_kernel<<<(K.n_lead + 127) / 128, 128, 0, ctx->stream>>>(K, s->d_lead);
     e = cudaGetLastError();
   }
-  if (e == cudaSuccess) e = cudaEventRecord(s->ev_staged, ctx->stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
   if (e != cudaSuccess) {
     wg_fail(ctx, WG_ERR_CUDA, "wg_kajita_stream_create", e);
@@ -1515,10 +1443,11 @@ int wg_kajita_stream_append(wg_kajita_stream *s, const int64_t *step_off, const 
   s->bytes = s->off_order + zs_align(sizeof(int) * s->npv);
   // ---- stage: wait until the device has read the previous blob, then refill it ----
   wg_device_guard guard(ctx->device);
-  int rc = zs_stage_host(s, s->bytes);
+  unsigned char *hb;
+  int rc = wgi_stage_reserve(ctx, &s->stage, s->bytes, &hb);
   if (rc != WG_OK) return rc;
-  ZsWork *wk = reinterpret_cast<ZsWork *>(s->h_blob);
-  wg_rel_step *hs = reinterpret_cast<wg_rel_step *>(s->h_blob + s->off_steps);
+  ZsWork *wk = reinterpret_cast<ZsWork *>(hb);
+  wg_rel_step *hs = reinterpret_cast<wg_rel_step *>(hb + s->off_steps);
   int64_t at = 0;
   for (int j = 0; j < nwork; ++j) {
     const int b = work_order[j];
@@ -1532,14 +1461,12 @@ int wg_kajita_stream_append(wg_kajita_stream *s, const int64_t *step_off, const 
     if (ns > 0) std::memcpy(hs + at, steps + step_off[b], sizeof(wg_rel_step) * ns);
     at += ns;
   }
-  std::memcpy(s->h_blob + s->off_po, s->co.data(), sizeof(int64_t) * (B + 1));
-  if (s->npv) std::memcpy(s->h_blob + s->off_order, pv_order.data(), sizeof(int) * s->npv);
-  rc = zs_grow(ctx, reinterpret_cast<void **>(&s->d_blob), &s->d_cap, s->bytes);
-  if (rc != WG_OK) return rc;
-  WG_CUDA(ctx, cudaMemcpyAsync(s->d_blob, s->h_blob, s->bytes, cudaMemcpyHostToDevice, ctx->stream));
-  if (s->with_preview && (rc = wgi_preview_plan_set_offsets(s->pv, reinterpret_cast<const int64_t *>(s->h_blob + s->off_po))) != WG_OK)
+  std::memcpy(hb + s->off_po, s->co.data(), sizeof(int64_t) * (B + 1));
+  if (s->npv) std::memcpy(hb + s->off_order, pv_order.data(), sizeof(int) * s->npv);
+  // the plan copies its offsets from the blob too: before the send, whose event frees the blob
+  if (s->with_preview && (rc = wgi_preview_plan_set_offsets(s->pv, reinterpret_cast<const int64_t *>(hb + s->off_po))) != WG_OK)
     return rc;
-  WG_CUDA(ctx, cudaEventRecord(s->ev_staged, ctx->stream));
+  if ((rc = wgi_stage_send(ctx, &s->stage, s->bytes)) != WG_OK) return rc;
   s->K.cap = (cap + 31) / 32 * 32;
   s->pending = true;
   return WG_OK;
@@ -1587,9 +1514,9 @@ int wg_kajita_stream_run(wg_kajita_stream *s, int mem, double *zmpref_xy, double
     const size_t smem = sizeof(double2) * (size_t)ZD_WARPS * (s->K.cap + 2 * ZD_HIST + ZD_HEAD);
     if (smem > 200 * 1024) return wg_fail(ctx, WG_ERR_INVALID, "step segment too long for the shared-memory buffer");
     WG_SMEM_ATTR(ctx, zmpdisc_stream_kernel, smem);
-    const int grid = std::max(1, std::min((s->nwork + ZD_WARPS - 1) / ZD_WARPS, ctx->sm_count * 3));
-    const ZsWork *wk = reinterpret_cast<const ZsWork *>(s->d_blob);
-    const wg_rel_step *st = reinterpret_cast<const wg_rel_step *>(s->d_blob + s->off_steps);
+    const int grid = wgi_grid(ctx, s->nwork, ZD_WARPS, 3);
+    const ZsWork *wk = reinterpret_cast<const ZsWork *>(s->stage.d);
+    const wg_rel_step *st = reinterpret_cast<const wg_rel_step *>(s->stage.d + s->off_steps);
     WG_CUDA(ctx, cudaMemsetAsync(s->d_next, 0, sizeof(int), ctx->stream));
     wg_prof_start(ctx, WG_K_ZMPDISC);
     zmpdisc_stream_kernel<<<grid, ZD_THREADS, smem, ctx->stream>>>(s->K, s->nwork, wk, st, s->d_rec, o, s->with_preview ? s->d_pk : nullptr,
@@ -1599,7 +1526,7 @@ int wg_kajita_stream_run(wg_kajita_stream *s, int mem, double *zmpref_xy, double
     WG_LAUNCHED(ctx);
   }
   if (s->npv > 0) {
-    const int *order = reinterpret_cast<const int *>(s->d_blob + s->off_order);
+    const int *order = reinterpret_cast<const int *>(s->stage.d + s->off_order);
     if ((rc = wgi_preview_launch_range(ctx, s->pv, order, s->npv, reinterpret_cast<const double *>(s->d_pk), s->d_state,
                                        static_cast<double *>(dev[5]), static_cast<double *>(dev[6]), simulation)) != WG_OK)
       return rc;
@@ -1653,25 +1580,24 @@ int wg_kajita_stream_save(wg_kajita_stream *s, int mem, int n, const int32_t *id
   if (!s) return WG_ERR_INVALID;
   wg_ctx *ctx = s->ctx;
   const char *call = "wg_kajita_stream_save";
-  if (const char *why = zs_io_refusal(s, mem, n, walks, carry)) return zs_refuse(ctx, call, why);
+  if (const char *why = zs_io_refusal(s, mem, n, walks, carry)) return wg_refuse(ctx, call, why);
   std::vector<char> mark((size_t)s->B, 0);
-  if (!zs_indices_ok(s->B, n, idx, false, mark)) return zs_refuse(ctx, call, "index out of range, or n > B without indices");
+  if (!wgi_record_indices_ok(s->B, n, idx, false, mark)) return wg_refuse(ctx, call, "index out of range, or n > B without indices");
   if (n == 0) return WG_OK;
   wg_device_guard guard(ctx->device);
   const int NL1 = zs_carry_rows(s);
   const size_t wbytes = sizeof(wg_kajita_stream_walk) * (size_t)n, cbytes = sizeof(double2) * (size_t)NL1 * n;
   const size_t bytes = sizeof(ZsCounts) * (size_t)n;
   // the walks' host-side counters and indices, in one H2D copy
-  int rc = zs_stage_host(s, bytes);
+  unsigned char *hb;
+  int rc = wgi_stage_reserve(ctx, &s->stage, bytes, &hb);
   if (rc != WG_OK) return rc;
-  ZsCounts *c = reinterpret_cast<ZsCounts *>(s->h_blob);
+  ZsCounts *c = reinterpret_cast<ZsCounts *>(hb);
   for (int i = 0; i < n; ++i) {
     const int b = idx ? idx[i] : i;
     c[i].emitted = s->emitted[b]; c[i].previewed = s->previewed[b]; c[i].open = s->open[b]; c[i].b = b;
   }
-  if ((rc = zs_grow(ctx, reinterpret_cast<void **>(&s->d_blob), &s->d_cap, bytes)) != WG_OK) return rc;
-  WG_CUDA(ctx, cudaMemcpyAsync(s->d_blob, s->h_blob, bytes, cudaMemcpyHostToDevice, ctx->stream));
-  WG_CUDA(ctx, cudaEventRecord(s->ev_staged, ctx->stream));
+  if ((rc = wgi_stage_send(ctx, &s->stage, bytes)) != WG_OK) return rc;
   wg_kajita_stream_walk *d_w = walks;
   double2 *d_c = reinterpret_cast<double2 *>(carry);
   if (mem == WG_MEM_HOST) {
@@ -1680,8 +1606,8 @@ int wg_kajita_stream_save(wg_kajita_stream *s, int mem, int n, const int32_t *id
     d_c = reinterpret_cast<double2 *>(static_cast<unsigned char *>(s->d_io) + wbytes);
   }
   wg_prof_start(ctx, WG_K_ZMPDISC);
-  stream_save_kernel<<<zs_blocks(ctx, n, ZS_WARPS), ZS_WARPS * 32, 0, ctx->stream>>>(
-      n, reinterpret_cast<const ZsCounts *>(s->d_blob), s->d_rec, s->d_state, s->d_carry, NL1, d_w, d_c);
+  stream_save_kernel<<<wgi_grid(ctx, n, ZS_WARPS, ZS_CTAS_PER_SM), ZS_WARPS * 32, 0, ctx->stream>>>(
+      n, reinterpret_cast<const ZsCounts *>(s->stage.d), s->d_rec, s->d_state, s->d_carry, NL1, d_w, d_c);
   wg_prof_stop(ctx);
   WG_LAUNCHED(ctx);
   if (mem == WG_MEM_DEVICE) return WG_OK;
@@ -1697,30 +1623,29 @@ int wg_kajita_stream_restore(wg_kajita_stream *s, int mem, int n, const int32_t 
   if (!s) return WG_ERR_INVALID;
   wg_ctx *ctx = s->ctx;
   const char *call = "wg_kajita_stream_restore";
-  if (const char *why = zs_io_refusal(s, mem, n, walks, carry)) return zs_refuse(ctx, call, why);
+  if (const char *why = zs_io_refusal(s, mem, n, walks, carry)) return wg_refuse(ctx, call, why);
   std::vector<char> mark((size_t)s->B, 0);
-  if (!zs_indices_ok(s->B, n, idx, true, mark))
-    return zs_refuse(ctx, call, "index out of range or repeated, or n > B without indices");
+  if (!wgi_record_indices_ok(s->B, n, idx, true, mark))
+    return wg_refuse(ctx, call, "index out of range or repeated, or n > B without indices");
   const int NL1 = zs_carry_rows(s);
   const char *bad_record = "a record breaks the invariants of open, samples_emitted and steps_previewed";
   if (mem == WG_MEM_HOST)
     for (int i = 0; i < n; ++i)
       if (!zs_counts_ok(walks[i].samples_emitted, walks[i].steps_previewed, walks[i].open, s->with_preview, NL1))
-        return zs_refuse(ctx, call, bad_record);
+        return wg_refuse(ctx, call, bad_record);
   if (n == 0) return WG_OK;
   wg_device_guard guard(ctx->device);
   const size_t wbytes = sizeof(wg_kajita_stream_walk) * (size_t)n, cbytes = sizeof(double2) * (size_t)NL1 * n;
   // blob: indices | the check kernel's flag | the records' counters, which the check kernel writes (device records)
   const size_t off_flag = zs_align(sizeof(int32_t) * (size_t)n), off_cnt = off_flag + 16;
   const size_t bytes = off_cnt + sizeof(ZsCounts) * (size_t)n;
-  int rc = zs_stage_host(s, bytes);
+  unsigned char *hb;
+  int rc = wgi_stage_reserve(ctx, &s->stage, bytes, &hb);
   if (rc != WG_OK) return rc;
-  int32_t *hi = reinterpret_cast<int32_t *>(s->h_blob);
+  int32_t *hi = reinterpret_cast<int32_t *>(hb);
   for (int i = 0; i < n; ++i) hi[i] = idx ? idx[i] : i;
-  std::memset(s->h_blob + off_flag, 0, 16);
-  if ((rc = zs_grow(ctx, reinterpret_cast<void **>(&s->d_blob), &s->d_cap, bytes)) != WG_OK) return rc;
-  WG_CUDA(ctx, cudaMemcpyAsync(s->d_blob, s->h_blob, off_cnt, cudaMemcpyHostToDevice, ctx->stream));
-  WG_CUDA(ctx, cudaEventRecord(s->ev_staged, ctx->stream));
+  std::memset(hb + off_flag, 0, 16);
+  if ((rc = wgi_stage_send(ctx, &s->stage, off_cnt, bytes)) != WG_OK) return rc;
   const wg_kajita_stream_walk *d_w = walks;
   const double2 *d_c = reinterpret_cast<const double2 *>(carry);
   const ZsCounts *hc = nullptr;
@@ -1734,18 +1659,18 @@ int wg_kajita_stream_restore(wg_kajita_stream *s, int mem, int n, const int32_t 
   } else {
     // all or nothing: the records are checked before any walk changes, and the host needs their counters to plan appends
     wg_prof_start(ctx, WG_K_ZMPDISC);
-    stream_restore_check_kernel<<<zs_blocks(ctx, n, ZS_WARPS * 32), ZS_WARPS * 32, 0, ctx->stream>>>(
-        n, walks, s->with_preview, NL1, reinterpret_cast<int *>(s->d_blob + off_flag), reinterpret_cast<ZsCounts *>(s->d_blob + off_cnt));
+    stream_restore_check_kernel<<<wgi_grid(ctx, n, ZS_WARPS * 32, ZS_CTAS_PER_SM), ZS_WARPS * 32, 0, ctx->stream>>>(
+        n, walks, s->with_preview, NL1, reinterpret_cast<int *>(s->stage.d + off_flag), reinterpret_cast<ZsCounts *>(s->stage.d + off_cnt));
     wg_prof_stop(ctx);
     WG_LAUNCHED(ctx);
-    WG_CUDA(ctx, cudaMemcpyAsync(s->h_blob + off_flag, s->d_blob + off_flag, bytes - off_flag, cudaMemcpyDeviceToHost, ctx->stream));
+    WG_CUDA(ctx, cudaMemcpyAsync(hb + off_flag, s->stage.d + off_flag, bytes - off_flag, cudaMemcpyDeviceToHost, ctx->stream));
     WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    if (*reinterpret_cast<const int *>(s->h_blob + off_flag)) return zs_refuse(ctx, call, bad_record);
-    hc = reinterpret_cast<const ZsCounts *>(s->h_blob + off_cnt);
+    if (*reinterpret_cast<const int *>(hb + off_flag)) return wg_refuse(ctx, call, bad_record);
+    hc = reinterpret_cast<const ZsCounts *>(hb + off_cnt);
   }
   wg_prof_start(ctx, WG_K_ZMPDISC);
-  stream_restore_kernel<<<zs_blocks(ctx, n, ZS_WARPS), ZS_WARPS * 32, 0, ctx->stream>>>(
-      n, reinterpret_cast<const int32_t *>(s->d_blob), d_w, d_c, NL1, s->d_rec, s->d_state, s->d_carry, s->d_status);
+  stream_restore_kernel<<<wgi_grid(ctx, n, ZS_WARPS, ZS_CTAS_PER_SM), ZS_WARPS * 32, 0, ctx->stream>>>(
+      n, reinterpret_cast<const int32_t *>(s->stage.d), d_w, d_c, NL1, s->d_rec, s->d_state, s->d_carry, s->d_status);
   wg_prof_stop(ctx);
   WG_LAUNCHED(ctx);
   if (mem == WG_MEM_HOST) WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1763,32 +1688,26 @@ int wg_kajita_stream_copy(wg_kajita_stream *dst, int n, const int32_t *dst_idx, 
   if (!dst || !src) return WG_ERR_INVALID;
   wg_ctx *ctx = dst->ctx;
   const char *call = "wg_kajita_stream_copy";
-  if (n < 0) return zs_refuse(ctx, call, "n < 0");
-  if (src->ctx != ctx) return zs_refuse(ctx, call, "streams of two contexts");
-  if (dst->pending || src->pending) return zs_refuse(ctx, call, "an append is pending (run it first)");
-  if (dst->with_preview != src->with_preview || dst->NL != src->NL) return zs_refuse(ctx, call, "with_preview or NL differ");
-  std::vector<char> dmark((size_t)dst->B, 0), smark((size_t)src->B, 0);
-  if (!zs_indices_ok(dst->B, n, dst_idx, true, dmark) || !zs_indices_ok(src->B, n, src_idx, false, smark))
-    return zs_refuse(ctx, call, "index out of range, repeated destination, or n > B without indices");
-  if (dst == src)
-    for (int b = 0; b < dst->B; ++b)
-      if (dmark[b] && smark[b]) return zs_refuse(ctx, call, "a walk is both source and destination");
+  if (n < 0) return wg_refuse(ctx, call, "n < 0");
+  if (src->ctx != ctx) return wg_refuse(ctx, call, "streams of two contexts");
+  if (dst->pending || src->pending) return wg_refuse(ctx, call, "an append is pending (run it first)");
+  if (dst->with_preview != src->with_preview || dst->NL != src->NL) return wg_refuse(ctx, call, "with_preview or NL differ");
+  if (const char *why = wgi_copy_indices_refusal(n, dst->B, dst_idx, src->B, src_idx, dst == src)) return wg_refuse(ctx, call, why);
   if (n == 0) return WG_OK;
   wg_device_guard guard(ctx->device);
   const size_t off_s = zs_align(sizeof(int32_t) * (size_t)n), bytes = off_s + sizeof(int32_t) * (size_t)n;
-  int rc = zs_stage_host(dst, bytes);
+  unsigned char *hb;
+  int rc = wgi_stage_reserve(ctx, &dst->stage, bytes, &hb);
   if (rc != WG_OK) return rc;
-  int32_t *hd = reinterpret_cast<int32_t *>(dst->h_blob), *hs = reinterpret_cast<int32_t *>(dst->h_blob + off_s);
+  int32_t *hd = reinterpret_cast<int32_t *>(hb), *hs = reinterpret_cast<int32_t *>(hb + off_s);
   for (int i = 0; i < n; ++i) {
     hd[i] = dst_idx ? dst_idx[i] : i;
     hs[i] = src_idx ? src_idx[i] : i;
   }
-  if ((rc = zs_grow(ctx, reinterpret_cast<void **>(&dst->d_blob), &dst->d_cap, bytes)) != WG_OK) return rc;
-  WG_CUDA(ctx, cudaMemcpyAsync(dst->d_blob, dst->h_blob, bytes, cudaMemcpyHostToDevice, ctx->stream));
-  WG_CUDA(ctx, cudaEventRecord(dst->ev_staged, ctx->stream));
+  if ((rc = wgi_stage_send(ctx, &dst->stage, bytes)) != WG_OK) return rc;
   wg_prof_start(ctx, WG_K_ZMPDISC);
-  stream_copy_kernel<<<zs_blocks(ctx, n, ZS_WARPS), ZS_WARPS * 32, 0, ctx->stream>>>(
-      n, reinterpret_cast<const int32_t *>(dst->d_blob), reinterpret_cast<const int32_t *>(dst->d_blob + off_s), src->d_rec,
+  stream_copy_kernel<<<wgi_grid(ctx, n, ZS_WARPS, ZS_CTAS_PER_SM), ZS_WARPS * 32, 0, ctx->stream>>>(
+      n, reinterpret_cast<const int32_t *>(dst->stage.d), reinterpret_cast<const int32_t *>(dst->stage.d + off_s), src->d_rec,
       src->d_state, src->d_carry, dst->d_rec, dst->d_state, dst->d_carry, zs_carry_rows(dst), dst->d_status);
   wg_prof_stop(ctx);
   WG_LAUNCHED(ctx);
