@@ -885,6 +885,90 @@ int wg_kajita_stream_copy(wg_kajita_stream *dst, int n, const int32_t *dst_idx, 
                           const int32_t *src_idx);
 
 /* ------------------------------------------------------------------------------------------------
+ * Kajita2003 on-line generator, one 5 ms control tick at a time, for B walks
+ *   replaces PatternGeneratorInterface::RunOneStepOfTheControlLoop, Kajita branch (PatternGeneratorInterfacePrivate.cpp:
+ *            1283-1314): the refill of the ZMP / CoM / feet queues from the step stack and the pop of one row per tick;
+ *            :StartOnLineStepSequencing (InitOnLine), :addstandardonlinestep (StepStackHandler::AddStandardOnLineStep),
+ *            :StopOnLineStepSequencing (StepStackHandler::StopOnLineStep) and StepStackHandler::AddStepInTheStack between
+ *            ticks.
+ * Every walk keeps its own queue, step stack, support-foot parity (m_KeepLastCorrectSupportFoot) and clock.  One tick of
+ * walk b is what one RunOneStepOfTheControlLoop does for that walk alone:
+ *   1. its command of this tick is applied (see wg_kajita_command);
+ *   2. while the walk is on line and its queue holds <= 2*NL+1 samples: an empty stack first takes the default step
+ *      (0, keep*0.19, 0, t_single, t_double) and keep flips; the front step is popped and its segment emitted
+ *      (OnLineAddFoot).  It is the last step when the stack is then empty after a STOP: the end phase follows
+ *      (EndPhaseOfTheWalking) and the walk goes off line;
+ *   3. when the queue holds <= 2*NL samples the walk stops for good (running 0 until it is started again);
+ *   4. otherwise the front row is popped into rows[t][b] and running[t][b] = 1.
+ * A walk that is not started, or has stopped, ignores its commands: its running entry is 0 and its row is untouched with
+ * WG_MEM_DEVICE, zero with WG_MEM_HOST.  Samples are the ones wg_kajita_stream emits (bitwise the off-line plan of the
+ * walk's realised step list), the CoM is its preview with simulation = 1.  NL is the preview gains' at create.
+ *
+ * Every refill is decided on the host from host-known values (queue = emitted - popped, the stacks, the commands), so the
+ * device is never read back.  A call of nticks <= WG_KAJITA_ONLINE_CHUNK ticks is at most four launches: one
+ * wg_kajita_stream run (front end + preview) for all the refills of the call, a scatter of the new rows into the walks'
+ * queues, a gather of rows[t][b]; a call without refills is the gather alone.  Longer calls are split into chunks of
+ * WG_KAJITA_ONLINE_CHUNK ticks.  With WG_MEM_DEVICE a tick call does not synchronise, and once its buffers exist it
+ * allocates nothing.
+ *
+ * Memory: walk b's queue is a ring of R wg_kajita_tick rows (224 B each) in device memory,
+ *   R = 2*NL + 1 + round(max_step_time/T) + round(t_double/(2T)) + 3*NL + WG_KAJITA_ONLINE_CHUNK - 1
+ * (wg_kajita_online_ring_rows): a refill happens at <= 2*NL+1 queued samples and adds at most one segment and the end
+ * phase, and the rows of a chunk are all written before its first pop, so up to CHUNK-1 rows popped earlier in the chunk
+ * are still held.  Every call checks the bound.  NL = 320, max_step_time = 0.8 s: 1922 rows, 430 KB per walk.
+ * ---------------------------------------------------------------------------------------------- */
+#define WG_KAJITA_ONLINE_CHUNK 160
+enum { WG_KAJITA_PUSH = 1, WG_KAJITA_STANDARD = 2, WG_KAJITA_STOP = 4 };
+
+typedef struct wg_kajita_command {     /* one walk, one tick; applied before that tick; ignored by a walk that is not on line */
+  wg_rel_step step;                    /* PUSH: pushed onto the back of the stack as given (AddStepInTheStack);         */
+                                       /* STANDARD: sx, sy, theta of :addstandardonlinestep: (sx, sy + keep*0.19,      */
+                                       /*   theta, t_single, t_double) is pushed and keep flips                         */
+  int32_t flags;                       /* WG_KAJITA_PUSH or WG_KAJITA_STANDARD, or WG_KAJITA_STOP (:StopOnLineStep-    */
+                                       /*   Sequencing: keep flips when the stack holds an even number of steps, the    */
+                                       /*   stack is cleared, the next step that empties it is the last); 0 = none      */
+  int32_t pad_[3];
+} wg_kajita_command;                   /* 64 bytes */
+
+typedef struct wg_kajita_tick {        /* one popped row                                                                */
+  double com_x[3], com_y[3];           /* COMState x, y: preview CoM (position, velocity, acceleration)                 */
+  double com_z, com_yaw;               /* com_height of the handle; ZMP theta (degrees)                                 */
+  double zmp_px, zmp_py, zmp_theta;    /* ZMPPosition: filtered ZMP reference, theta (degrees)                          */
+  double zmp_time;                     /*   the walk's clock: T accumulated sample by sample from its start             */
+  double zmp_out[2];                   /* cart-table ZMP of the preview                                                 */
+  wg_foot_sample left, right;
+  int32_t step_type[3];                /* stepType of the ZMP, left-foot and right-foot samples                         */
+  int32_t pad_;
+} wg_kajita_tick;                      /* 224 bytes, a multiple of 16 */
+
+typedef struct wg_kajita_online wg_kajita_online;
+/* Needs preview gains on the context (WG_ERR_NOT_READY otherwise).  com_height goes into every row's com_z.  A step
+ * whose round((SS+DS)/T) exceeds round(max_step_time/T) is refused by start and tick; the default step timing of p must
+ * fit. */
+int wg_kajita_online_create(wg_ctx *ctx, const wg_zmpdisc_params *p, int B, double com_height, double max_step_time,
+                            wg_kajita_online **out);
+int wg_kajita_online_destroy(wg_kajita_online *h);
+int wg_kajita_online_ring_rows(const wg_kajita_online *h);   /* R above */
+/* :StartOnLineStepSequencing for the n walks idx_host[0..n): walk idx[i] (re)starts with the steps [off[i], off[i+1]) of
+ * steps_host (step_offsets_host has n+1 entries), init_feet_host[i] as in wg_kajita_plan_create, keep = keep_last_host[i]
+ * (+1 or -1; NULL: +1 for all).  The steps go through the stream with WG_STREAM_START: the 2*NL lead-in, then one segment
+ * per step after the first (the support-foot step), all queued; the stack starts empty; the walk is on line and running.
+ * Walks not listed keep running.  Refused with WG_ERR_INVALID, nothing changed: n < 0, an index out of [0, B) or
+ * repeated, NULL arrays with n > 0, a walk without steps, keep not +-1, a step timing the stream refuses or longer than
+ * max_step_time, more samples than the ring holds. */
+int wg_kajita_online_start(wg_kajita_online *h, int n, const int32_t *idx_host, const int64_t *step_offsets_host,
+                           const wg_rel_step *steps_host, const double *init_feet_host, const int32_t *keep_last_host);
+/* nticks control ticks for every started walk.  commands_host [nticks][B] (HOST memory, may be NULL); in `mem`, each may
+ * be NULL: rows [nticks][B], running [nticks][B] (1 = RunOneStepOfTheControlLoop returned true).  Refused with
+ * WG_ERR_INVALID, nothing changed: nticks < 0, an unknown mem, unaligned device rows, unknown flags, STOP together with
+ * a step, PUSH together with STANDARD, a pushed step whose timing the stream refuses or that is longer than
+ * max_step_time; WG_ERR_NOT_READY when the context's preview gains no longer have the handle's NL. */
+int wg_kajita_online_tick(wg_kajita_online *h, int mem, int nticks, const wg_kajita_command *commands_host,
+                          wg_kajita_tick *rows, int8_t *running);
+/* Host arrays of B entries, any may be NULL: samples queued, steps on the stack, running, on line. */
+int wg_kajita_online_state(wg_kajita_online *h, int64_t *queued, int32_t *stacked, int32_t *running, int32_t *online);
+
+/* ------------------------------------------------------------------------------------------------
  * Dimitrov2008 front to back: feet trajectories -> support polygons -> per-period constraint matrices ->
  * PLDP solve -> LIPM, closed loop on the device (one warp owns one walk for its whole duration)
  *   replaces ComputeConvexHull::DoComputeConvexHull                     (src/Mathematics/ConvexHull.cpp:87-203)

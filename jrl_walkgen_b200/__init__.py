@@ -22,6 +22,9 @@ ACTIVE_SET_DTYPE = _capi.herdt_active_set_dtype()
 PLDP_STATE_DTYPE, PLDP_INFO_DTYPE = _capi.pldp_dtypes()
 REL_STEP_DTYPE, KAJITA_FOOT_DTYPE = _capi.kajita_dtypes()
 KAJITA_STREAM_WALK_DTYPE = _capi.kajita_stream_walk_dtype()
+KAJITA_TICK_DTYPE, KAJITA_COMMAND_DTYPE = _capi.kajita_online_dtypes()
+KAJITA_PUSH, KAJITA_STANDARD, KAJITA_STOP = _capi.WG_KAJITA_PUSH, _capi.WG_KAJITA_STANDARD, _capi.WG_KAJITA_STOP
+KAJITA_ONLINE_CHUNK = _capi.KAJITA_ONLINE_CHUNK
 LCI_DTYPE, DIMITROV_PERIOD_DTYPE = _capi.dimitrov_dtypes()
 HERDT_COMMAND_DTYPE = _capi.herdt_command_dtype()
 CMD_VEL, CMD_STOP = _capi.WG_CMD_VEL, _capi.WG_CMD_STOP
@@ -32,6 +35,8 @@ HERDT_INIT15 = (0.0316055, 0.0, 0.0, 0.0, 0.0, 0.0, 0.7116911, 0.0, 0.0, 0.0, 0.
 DimitrovParams = _capi.DimitrovParams
 
 __all__ = ["MultiContext", "LCI_DTYPE", "DIMITROV_PERIOD_DTYPE", "DimitrovParams", "dimitrov_default_params", "Context", "PreviewPlan", "KajitaPlan", "KajitaStream", "HerdtOnline",
+           "KajitaOnline", "KAJITA_TICK_DTYPE", "KAJITA_COMMAND_DTYPE", "KAJITA_PUSH", "KAJITA_STANDARD", "KAJITA_STOP",
+           "KAJITA_ONLINE_CHUNK",
            "HERDT_COMMAND_DTYPE", "CMD_VEL", "CMD_STOP", "HERDT_ONLINE_QUEUE", "ONLINE_ROBOT_DTYPE", "HERDT_INIT15",
            "STREAM_START", "STREAM_FINISH", "zmpdisc_default_params", "REL_STEP_DTYPE", "KAJITA_FOOT_DTYPE", "KAJITA_STREAM_WALK_DTYPE", "preview_gains", "herdt_default_params", "herdt_mpc_default_params", "HerdtParams", "HerdtMpcParams",
            "PLDP_STATE_DTYPE", "PLDP_INFO_DTYPE", "FOOT_DTYPE", "TICK_DTYPE", "MPC_STATE_DTYPE", "MPC_STEP_DTYPE", "TICKS_PER_STEP", "QP_INPUT_DTYPE",
@@ -238,6 +243,11 @@ class Context:
     def kajita_stream(self, B, params=None, with_preview=True) -> "KajitaStream":
         """B walks whose footsteps arrive while they run (wg_kajita_stream_create)."""
         return KajitaStream(self, B, params, with_preview)
+
+    def kajita_online(self, B, params=None, com_height=0.814, max_step_time=0.8) -> "KajitaOnline":
+        """B walks driven one 5 ms control tick at a time, each refilling its queues from its own step stack
+        (wg_kajita_online_create); needs preview gains on the context."""
+        return KajitaOnline(self, B, params, com_height, max_step_time)
 
     def preview_one_iteration(self, x, y, sx, sy, window_xy, simulation=True):
         """PreviewControl::OneIterationOfPreview for one instance (host buffers)."""
@@ -732,6 +742,65 @@ class KajitaStream:
     def destroy(self):
         if self.h:
             self.ctx.lib.wg_kajita_stream_destroy(self.h)
+            self.h = None
+
+
+class KajitaOnline:
+    """On-line Kajita2003 generator for B walks: RunOneStepOfTheControlLoop's Kajita branch batched, each walk with its own
+    start tick, step stack, commands (PUSH, :addstandardonlinestep, :StopOnLineStepSequencing) and queues
+    (wg_kajita_online_*)."""
+
+    def __init__(self, ctx: Context, B, params=None, com_height=0.814, max_step_time=0.8):
+        self.ctx = ctx
+        self.B = int(B)
+        self.params = params if params is not None else zmpdisc_default_params()
+        h = C.c_void_p()
+        ctx._check(ctx.lib.wg_kajita_online_create(ctx.h, C.byref(self.params), self.B, float(com_height), float(max_step_time),
+                                                   C.byref(h)))
+        self.h = h
+        self.ring_rows = int(ctx.lib.wg_kajita_online_ring_rows(h))
+
+    def start(self, idx, steps, init_feet, keep_last=None):
+        """:StartOnLineStepSequencing for the walks idx: steps is one REL_STEP_DTYPE list per walk (its first step the
+        support-foot step), init_feet [len(idx)][6], keep_last [len(idx)] of +-1 or None (+1)."""
+        idx = np.ascontiguousarray(idx, dtype=np.int32).reshape(-1)
+        lists = [np.asarray(s, dtype=REL_STEP_DTYPE).reshape(-1) for s in steps]
+        assert len(lists) == len(idx)
+        off = np.concatenate([[0], np.cumsum([len(s) for s in lists])]).astype(np.int64)
+        st = np.ascontiguousarray(np.concatenate(lists) if lists else np.zeros(0, dtype=REL_STEP_DTYPE))
+        feet = np.ascontiguousarray(init_feet, dtype=np.float64).reshape(len(idx), 6)
+        keep = None if keep_last is None else np.ascontiguousarray(keep_last, dtype=np.int32).reshape(len(idx))
+        self.ctx._check(self.ctx.lib.wg_kajita_online_start(self.h, len(idx), idx.ctypes.data, off.ctypes.data_as(_capi.c_i64_p),
+                                                            st.ctypes.data, feet.ctypes.data, _ptr(keep)))
+
+    def tick(self, nticks, commands=None, rows=True, running=True):
+        """nticks ticks on host arrays: commands [nticks][B] of KAJITA_COMMAND_DTYPE or None -> (rows [nticks][B] of
+        KAJITA_TICK_DTYPE, running [nticks][B] int8), each None when not asked for."""
+        n = int(nticks)
+        cmd = None if commands is None else np.ascontiguousarray(commands, dtype=KAJITA_COMMAND_DTYPE)
+        assert cmd is None or cmd.shape == (n, self.B)
+        r = np.zeros((n, self.B), dtype=KAJITA_TICK_DTYPE) if rows else None
+        run = np.zeros((n, self.B), dtype=np.int8) if running else None
+        self.ctx._check(self.ctx.lib.wg_kajita_online_tick(self.h, WG_MEM_HOST, n, _ptr(cmd), _ptr(r), _ptr(run)))
+        return r, run
+
+    def tick_device(self, nticks, commands=None, d_rows=None, d_running=None):
+        """Device-resident rows and running flags (asynchronous on the context stream); commands stay a host array."""
+        cmd = None if commands is None else np.ascontiguousarray(commands, dtype=KAJITA_COMMAND_DTYPE)
+        assert cmd is None or cmd.shape == (int(nticks), self.B)
+        self.ctx._check(self.ctx.lib.wg_kajita_online_tick(self.h, WG_MEM_DEVICE, int(nticks), _ptr(cmd), _ptr(d_rows),
+                                                           _ptr(d_running)))
+
+    def state(self):
+        """-> (queued int64 [B], stacked int32 [B], running int32 [B], online int32 [B])."""
+        q = np.zeros(self.B, dtype=np.int64)
+        s, r, o = (np.zeros(self.B, dtype=np.int32) for _ in range(3))
+        self.ctx._check(self.ctx.lib.wg_kajita_online_state(self.h, q.ctypes.data, s.ctypes.data, r.ctypes.data, o.ctypes.data))
+        return q, s, r, o
+
+    def destroy(self):
+        if self.h:
+            self.ctx.lib.wg_kajita_online_destroy(self.h)
             self.h = None
 
 

@@ -164,6 +164,24 @@ def pldp_dtypes():
     return state, info
 
 
+KAJITA_ONLINE_CHUNK = 160
+WG_KAJITA_PUSH = 1
+WG_KAJITA_STANDARD = 2
+WG_KAJITA_STOP = 4
+
+
+def kajita_online_dtypes():
+    """numpy mirrors of wg_kajita_tick (224 B) and wg_kajita_command (64 B)."""
+    np = _np()
+    step, foot = kajita_dtypes()
+    tick = np.dtype([("com_x", "f8", 3), ("com_y", "f8", 3), ("com_z", "f8"), ("com_yaw", "f8"), ("zmp_px", "f8"),
+                     ("zmp_py", "f8"), ("zmp_theta", "f8"), ("zmp_time", "f8"), ("zmp_out", "f8", 2), ("left", foot),
+                     ("right", foot), ("step_type", "i4", 3), ("pad_", "i4")])
+    cmd = np.dtype([("step", step), ("flags", "i4"), ("pad_", "i4", 3)])
+    assert tick.itemsize == 224 and cmd.itemsize == 64
+    return tick, cmd
+
+
 HERDT_N = 16
 HERDT_TICKS_PER_STEP = 20
 HERDT_MAX_VARS = 36
@@ -366,6 +384,13 @@ SIGNATURES = {
     "wg_kajita_stream_save": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "wg_kajita_stream_restore": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "wg_kajita_stream_copy": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "wg_kajita_online_create": (C.c_int, [C.c_void_p, C.POINTER(ZmpDiscParams), C.c_int, C.c_double, C.c_double,
+                                          C.POINTER(C.c_void_p)]),
+    "wg_kajita_online_destroy": (C.c_int, [C.c_void_p]),
+    "wg_kajita_online_ring_rows": (C.c_int, [C.c_void_p]),
+    "wg_kajita_online_start": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, c_i64_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "wg_kajita_online_tick": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "wg_kajita_online_state": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "wg_dimitrov_default_params": (None, [C.POINTER(DimitrovParams)]),
     "wg_dimitrov_set_params": (C.c_int, [C.c_void_p, C.POINTER(DimitrovParams)] + [C.c_void_p] * 6),
     "wg_dimitrov_period_count": (C.c_int64, [C.POINTER(DimitrovParams), C.c_int64]),
