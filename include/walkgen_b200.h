@@ -968,6 +968,57 @@ int wg_kajita_online_tick(wg_kajita_online *h, int mem, int nticks, const wg_kaj
 /* Host arrays of B entries, any may be NULL: samples queued, steps on the stack, running, on line. */
 int wg_kajita_online_state(wg_kajita_online *h, int64_t *queued, int32_t *stacked, int32_t *running, int32_t *online);
 
+/* Whole walks: checkpoints, rewinds, forks (footstep lookahead: fork a walk, push one candidate step per branch, tick the
+ * branches, keep the winner) and migration.  A walk is one wg_kajita_online_walk record and, beside it in `mem`, its
+ * preview carry carry[n][NL-1][2] (the stream contract: wg_kajita_online_carry_rows rows) and its queue
+ * queue[n][R][wg_kajita_tick] (R = wg_kajita_online_ring_rows), front first.  Its step stack is host state and travels in a
+ * HOST array: the stacks of walks 0..n-1 concatenated in record order, walk i owning the next walks[i].stacked steps.
+ *
+ * Records are canonical: two walks with the same history since their START save to the same bytes, whatever their ring
+ * held before and whatever indices they live at.  Queue rows past queued = stream.samples_emitted - popped are zero; the
+ * CoM words (com_x, com_y, zmp_out) of the last stream.samples_emitted - stream.steps_previewed queued rows, which the
+ * preview has not written yet, are zero; pad_ is zero.  A walk never started saves as zeros with keep = +1.
+ *
+ * Index arrays are HOST pointers; NULL means walks 0..n-1 and needs n <= B.  Every call runs on the context stream, in order
+ * with ticks.  A refused call returns WG_ERR_INVALID and changes no walk, on the device or on the host.  Device arrays must
+ * be 16-byte aligned.  All three refuse n < 0 and n above B for a NULL index array; save and restore refuse an unknown mem
+ * and NULL walks, carry or queue with n > 0.
+ *
+ * wg_kajita_online_save: walk idx[i] -> walks[i], carry[i], queue[i] and its stack into stack_host; repeats allowed;
+ *   *stack_len (may be NULL) = the steps written.  Refused when the stacks hold more than stack_cap steps
+ *   (wg_kajita_online_state reports them).  WG_MEM_DEVICE: one H2D copy of the indices and host-side fields, two launches,
+ *   no synchronisation.  WG_MEM_HOST: the same, then the D2H copies and a synchronise.
+ * wg_kajita_online_restore: walks[i], carry[i], queue[i] and the stacks -> walk idx[i]; indices unique.  Every record is
+ *   validated before any walk changes: the stream's invariants (wg_kajita_stream_restore), stream.open == online; running,
+ *   online and transition each 0 or 1; online implies running, transition implies online, !online implies stacked == 0;
+ *   keep = +-1; 0 <= popped <= samples_emitted, queued <= R, running implies queued >= 2*NL; stacked >= 0 and the stacks
+ *   together hold exactly stack_len steps, each one a step a PUSH command would accept.  The clock and the walk state
+ *   proper are not validated.  Queue row j goes to ring row (popped + j) mod R.  WG_MEM_HOST: the H2D copies, two launches,
+ *   a synchronise.  WG_MEM_DEVICE: the n records are read back in one D2H copy (one synchronise: the host replays the tick
+ *   rules from their fields), then two launches.
+ * wg_kajita_online_copy: walk src_idx[i] of src -> walk dst_idx[i] of dst, device to device: the stream part through
+ *   wg_kajita_stream_copy, the queued rows and clock in one more launch (two launches, no synchronisation), the host-side
+ *   state and stack on the host.  src_idx may repeat (fork one walk into K); dst_idx must be unique.  Refused: handles of
+ *   two contexts, handles whose NL or R differ, dst == src with an index that is both a source and a destination.
+ * Records are meaningful only under the zmpdisc parameters and com_height they were saved with; those are not checked. */
+typedef struct wg_kajita_online_walk {
+  wg_kajita_stream_walk stream;  /* the owned stream's walk, exactly as wg_kajita_stream_save writes it                   */
+  int64_t popped;                /* samples popped since START; queued = stream.samples_emitted - popped                 */
+  double clock;                  /* ZMPPosition::time of the walk's next sample                                          */
+  int32_t keep;                  /* m_KeepLastCorrectSupportFoot, +1 or -1                                               */
+  int32_t running, online, transition;  /* m_Running, m_KajitaOnLine, m_TransitionFinishOnLine                          */
+  int32_t stacked;               /* steps on the stack; they travel in the stack array, front first                      */
+  int32_t pad_[3];
+} wg_kajita_online_walk;         /* 624 bytes, a multiple of 16 */
+
+int wg_kajita_online_carry_rows(const wg_kajita_online *h);   /* NL-1 */
+int wg_kajita_online_save(wg_kajita_online *h, int mem, int n, const int32_t *idx, wg_kajita_online_walk *walks, double *carry,
+                          wg_kajita_tick *queue, wg_rel_step *stack_host, int64_t stack_cap, int64_t *stack_len);
+int wg_kajita_online_restore(wg_kajita_online *h, int mem, int n, const int32_t *idx, const wg_kajita_online_walk *walks,
+                             const double *carry, const wg_kajita_tick *queue, const wg_rel_step *stack_host, int64_t stack_len);
+int wg_kajita_online_copy(wg_kajita_online *dst, int n, const int32_t *dst_idx, const wg_kajita_online *src,
+                          const int32_t *src_idx);
+
 /* ------------------------------------------------------------------------------------------------
  * Dimitrov2008 front to back: feet trajectories -> support polygons -> per-period constraint matrices ->
  * PLDP solve -> LIPM, closed loop on the device (one warp owns one walk for its whole duration)

@@ -23,6 +23,7 @@ PLDP_STATE_DTYPE, PLDP_INFO_DTYPE = _capi.pldp_dtypes()
 REL_STEP_DTYPE, KAJITA_FOOT_DTYPE = _capi.kajita_dtypes()
 KAJITA_STREAM_WALK_DTYPE = _capi.kajita_stream_walk_dtype()
 KAJITA_TICK_DTYPE, KAJITA_COMMAND_DTYPE = _capi.kajita_online_dtypes()
+KAJITA_ONLINE_WALK_DTYPE = _capi.kajita_online_walk_dtype()
 KAJITA_PUSH, KAJITA_STANDARD, KAJITA_STOP = _capi.WG_KAJITA_PUSH, _capi.WG_KAJITA_STANDARD, _capi.WG_KAJITA_STOP
 KAJITA_ONLINE_CHUNK = _capi.KAJITA_ONLINE_CHUNK
 LCI_DTYPE, DIMITROV_PERIOD_DTYPE = _capi.dimitrov_dtypes()
@@ -35,7 +36,7 @@ HERDT_INIT15 = (0.0316055, 0.0, 0.0, 0.0, 0.0, 0.0, 0.7116911, 0.0, 0.0, 0.0, 0.
 DimitrovParams = _capi.DimitrovParams
 
 __all__ = ["MultiContext", "LCI_DTYPE", "DIMITROV_PERIOD_DTYPE", "DimitrovParams", "dimitrov_default_params", "Context", "PreviewPlan", "KajitaPlan", "KajitaStream", "HerdtOnline",
-           "KajitaOnline", "KAJITA_TICK_DTYPE", "KAJITA_COMMAND_DTYPE", "KAJITA_PUSH", "KAJITA_STANDARD", "KAJITA_STOP",
+           "KajitaOnline", "KAJITA_ONLINE_WALK_DTYPE", "KAJITA_TICK_DTYPE", "KAJITA_COMMAND_DTYPE", "KAJITA_PUSH", "KAJITA_STANDARD", "KAJITA_STOP",
            "KAJITA_ONLINE_CHUNK",
            "HERDT_COMMAND_DTYPE", "CMD_VEL", "CMD_STOP", "HERDT_ONLINE_QUEUE", "ONLINE_ROBOT_DTYPE", "HERDT_INIT15",
            "STREAM_START", "STREAM_FINISH", "zmpdisc_default_params", "REL_STEP_DTYPE", "KAJITA_FOOT_DTYPE", "KAJITA_STREAM_WALK_DTYPE", "preview_gains", "herdt_default_params", "herdt_mpc_default_params", "HerdtParams", "HerdtMpcParams",
@@ -759,6 +760,7 @@ class KajitaOnline:
                                                    C.byref(h)))
         self.h = h
         self.ring_rows = int(ctx.lib.wg_kajita_online_ring_rows(h))
+        self.carry_rows = int(ctx.lib.wg_kajita_online_carry_rows(h))   # NL-1
 
     def start(self, idx, steps, init_feet, keep_last=None):
         """:StartOnLineStepSequencing for the walks idx: steps is one REL_STEP_DTYPE list per walk (its first step the
@@ -797,6 +799,74 @@ class KajitaOnline:
         s, r, o = (np.zeros(self.B, dtype=np.int32) for _ in range(3))
         self.ctx._check(self.ctx.lib.wg_kajita_online_state(self.h, q.ctypes.data, s.ctypes.data, r.ctypes.data, o.ctypes.data))
         return q, s, r, o
+
+    def _stack_buffer(self, idx):
+        """A host array for the stacks of the walks idx (all B when None), sized from state()."""
+        stacked = self.state()[1]
+        cap = int(stacked.sum() if idx is None else stacked[np.asarray(idx, dtype=np.int64)].sum())
+        return np.zeros(max(cap, 1), dtype=REL_STEP_DTYPE), cap
+
+    @staticmethod
+    def _split_stacks(walks, buf):
+        ends = np.cumsum(walks["stacked"].astype(np.int64))
+        return [buf[e - k:e].copy() for e, k in zip(ends, walks["stacked"].astype(np.int64))]
+
+    def save(self, idx=None):
+        """-> (walks [n] of KAJITA_ONLINE_WALK_DTYPE, carry [n][carry_rows][2], queue [n][ring_rows] of KAJITA_TICK_DTYPE,
+        stacks: one REL_STEP_DTYPE array per walk, front first) of the walks idx (all B when None)."""
+        ia = _indices(idx)
+        n = self.B if ia is None else len(ia)
+        walks = np.zeros(n, dtype=KAJITA_ONLINE_WALK_DTYPE)
+        carry = np.zeros((n, self.carry_rows, 2))
+        queue = np.zeros((n, self.ring_rows), dtype=KAJITA_TICK_DTYPE)
+        buf, cap = self._stack_buffer(ia)
+        ln = C.c_int64()
+        self.ctx._check(self.ctx.lib.wg_kajita_online_save(self.h, WG_MEM_HOST, n, _ptr(ia), walks.ctypes.data, carry.ctypes.data,
+                                                           queue.ctypes.data, buf.ctypes.data, cap, C.byref(ln)))
+        return walks, carry, queue, self._split_stacks(walks, buf)
+
+    @staticmethod
+    def _join_stacks(stacks):
+        lists = [np.asarray(s, dtype=REL_STEP_DTYPE).reshape(-1) for s in stacks]
+        buf = np.ascontiguousarray(np.concatenate(lists) if lists else np.zeros(0, dtype=REL_STEP_DTYPE))
+        return buf, len(buf)
+
+    def restore(self, walks, carry, queue, stacks, idx=None):
+        """Write host records, carry rows, queues and stacks into the walks idx (0..len(walks)-1 when None); all or nothing."""
+        rec = np.ascontiguousarray(walks, dtype=KAJITA_ONLINE_WALK_DTYPE).reshape(-1)
+        n = len(rec)
+        c = np.ascontiguousarray(carry, dtype=np.float64)
+        q = np.ascontiguousarray(queue, dtype=KAJITA_TICK_DTYPE)
+        assert c.shape == (n, self.carry_rows, 2) and q.shape == (n, self.ring_rows)
+        ia = _indices(idx)
+        assert ia is None or len(ia) == n
+        buf, ln = self._join_stacks(stacks)
+        self.ctx._check(self.ctx.lib.wg_kajita_online_restore(self.h, WG_MEM_HOST, n, _ptr(ia), rec.ctypes.data, c.ctypes.data,
+                                                              q.ctypes.data, buf.ctypes.data if ln else None, ln))
+
+    def save_device(self, n, d_walks, d_carry, d_queue, idx=None):
+        """Device-resident save of n walks into d_walks, d_carry, d_queue (asynchronous on the context stream) -> the stacks,
+        one REL_STEP_DTYPE array per walk."""
+        ia = _indices(idx)
+        buf, cap = self._stack_buffer(ia)
+        k = self.state()[1][np.arange(int(n)) if ia is None else ia].astype(np.int64)
+        ln = C.c_int64()
+        self.ctx._check(self.ctx.lib.wg_kajita_online_save(self.h, WG_MEM_DEVICE, int(n), _ptr(ia), _ptr(d_walks), _ptr(d_carry),
+                                                           _ptr(d_queue), buf.ctypes.data, cap, C.byref(ln)))
+        ends = np.cumsum(k)
+        return [buf[e - m:e].copy() for e, m in zip(ends, k)]
+
+    def restore_device(self, n, d_walks, d_carry, d_queue, stacks, idx=None):
+        """Device-resident restore of n walks from d_walks, d_carry, d_queue and the host stacks (reads the records back)."""
+        buf, ln = self._join_stacks(stacks)
+        self.ctx._check(self.ctx.lib.wg_kajita_online_restore(self.h, WG_MEM_DEVICE, int(n), _ptr(_indices(idx)), _ptr(d_walks),
+                                                              _ptr(d_carry), _ptr(d_queue), buf.ctypes.data if ln else None, ln))
+
+    def copy_from(self, src: "KajitaOnline", src_idx=None, dst_idx=None):
+        """Walk src_idx[i] of src -> walk dst_idx[i] of this handle, on the device (wg_kajita_online_copy); n is the length of
+        the index arrays given, B of this handle when neither is."""
+        n, si, di = _copy_indices(src_idx, dst_idx, self.B)
+        self.ctx._check(self.ctx.lib.wg_kajita_online_copy(self.h, n, _ptr(di), src.h, _ptr(si)))
 
     def destroy(self):
         if self.h:

@@ -182,6 +182,15 @@ def kajita_online_dtypes():
     return tick, cmd
 
 
+def kajita_online_walk_dtype():
+    """numpy mirror of wg_kajita_online_walk (624 B): one whole walk of wg_kajita_online, its carry, queue and stack apart."""
+    np = _np()
+    d = np.dtype([("stream", kajita_stream_walk_dtype()), ("popped", "i8"), ("clock", "f8"), ("keep", "i4"), ("running", "i4"),
+                  ("online", "i4"), ("transition", "i4"), ("stacked", "i4"), ("pad_", "i4", 3)])
+    assert d.itemsize == 624 and d.fields["popped"][1] == 576
+    return d
+
+
 HERDT_N = 16
 HERDT_TICKS_PER_STEP = 20
 HERDT_MAX_VARS = 36
@@ -391,6 +400,12 @@ SIGNATURES = {
     "wg_kajita_online_start": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, c_i64_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "wg_kajita_online_tick": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "wg_kajita_online_state": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "wg_kajita_online_carry_rows": (C.c_int, [C.c_void_p]),
+    "wg_kajita_online_save": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_void_p, C.c_int64, C.POINTER(C.c_int64)]),
+    "wg_kajita_online_restore": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_int64]),
+    "wg_kajita_online_copy": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "wg_dimitrov_default_params": (None, [C.POINTER(DimitrovParams)]),
     "wg_dimitrov_set_params": (C.c_int, [C.c_void_p, C.POINTER(DimitrovParams)] + [C.c_void_p] * 6),
     "wg_dimitrov_period_count": (C.c_int64, [C.POINTER(DimitrovParams), C.c_int64]),

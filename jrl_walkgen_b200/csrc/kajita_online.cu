@@ -9,6 +9,7 @@
 #include <deque>
 #include <new>
 #include "wg_common.h"
+#include "wg_records.cuh"
 
 namespace {
 
@@ -101,6 +102,101 @@ kajita_online_gather_kernel(int B, const int32_t *__restrict__ first, const int3
   }
 }
 
+// ---- whole walks (wg_kajita_online_save / restore / copy) -------------------------------------------------------------
+// One warp per walk, grid-stride; rows move as 16-byte words.  The stream part of a record (its first 36 words) is the
+// stream's, moved by its own strided kernels (zmpdisc.cu); these kernels move the queue, the clock and the handle's words.
+constexpr int KO_UNROLL = 8;
+constexpr int KO_CTAS_PER_SM = 6;   // all resident at up to 40 registers (the kernels take 36 to 40): no second wave
+constexpr int KO_STREAM_V4 = (int)(sizeof(wg_kajita_stream_walk) / 16);   // 36
+constexpr int KO_WALK_V4 = (int)(sizeof(wg_kajita_online_walk) / 16);     // 39
+static_assert(sizeof(wg_kajita_online_walk) == 624 && offsetof(wg_kajita_online_walk, popped) == 576 &&
+              offsetof(wg_kajita_online_walk, clock) == 584 && offsetof(wg_kajita_online_walk, keep) == 592 &&
+              offsetof(wg_kajita_online_walk, stacked) == 608, "wg_kajita_online_walk words");
+
+// Walk b's queued span: q rows from ring row `first` on (wrapping at R), the first nc of them with their CoM.
+struct KoSpan {
+  int32_t b, first, q, nc;
+};
+
+// A save's host-side words of record i: its span, and record words 36..38 (word 36's clock half is the device's).
+struct KoSave {
+  KoSpan sp;
+  uint4 tail[3];
+};
+
+// A copy of walk s's queued span and clock to walk d, at the same ring rows.
+struct KoPair {
+  int32_t d, s, first, q;
+};
+
+// Record words 36..38 and queue rows of walks in[i].sp.b, front first: the q queued rows, the CoM words (0..2 and 6) of
+// rows nc..q-1 zero (the preview has not written them: they hold whatever an earlier walk left), rows past q zero.
+__global__ void __launch_bounds__(KO_WARPS * 32)
+kajita_online_save_kernel(int n, const KoSave *__restrict__ in, int R, const uint4 *__restrict__ ring,
+                          const double *__restrict__ clock, uint4 *__restrict__ walks, uint4 *__restrict__ queue)
+{
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int i = blockIdx.x * KO_WARPS + warp; i < n; i += gridDim.x * KO_WARPS) {
+    const KoSpan sp = in[i].sp;
+    if (lane < 3) {
+      uint4 v = in[i].tail[lane];
+      if (lane == 0) {
+        const unsigned long long c = (unsigned long long)__double_as_longlong(clock[sp.b]);
+        v.z = (unsigned)c; v.w = (unsigned)(c >> 32);
+      }
+      walks[(int64_t)i * KO_WALK_V4 + KO_STREAM_V4 + lane] = v;
+    }
+    const uint4 *rb = ring + (size_t)sp.b * R * KO_WORDS;
+    uint4 *oq = queue + (size_t)i * R * KO_WORDS;
+    const int a = min(sp.nc, R - sp.first);          // whole rows before the wrap
+    wgi_warp_copy16<KO_UNROLL>(oq, rb + (size_t)sp.first * KO_WORDS, a * KO_WORDS, a * KO_WORDS, lane);
+    wgi_warp_copy16<KO_UNROLL>(oq + (size_t)a * KO_WORDS, rb, (sp.nc - a) * KO_WORDS, (sp.nc - a) * KO_WORDS, lane);
+    for (int e = sp.nc * KO_WORDS + lane; e < sp.q * KO_WORDS; e += 32) {
+      const int j = e / KO_WORDS, w = e - j * KO_WORDS;
+      int s = sp.first + j;
+      if (s >= R) s -= R;
+      oq[e] = (w < 3 || w == 6) ? make_uint4(0u, 0u, 0u, 0u) : rb[(size_t)s * KO_WORDS + w];
+    }
+    wgi_warp_copy16<KO_UNROLL>(oq + (size_t)sp.q * KO_WORDS, rb, (R - sp.q) * KO_WORDS, 0, lane);
+  }
+}
+
+// Queue rows of record i -> ring rows first.. of walk sp[i].b (wrapping at R), its clock -> clock[b].  Ring rows past the
+// queued span are left as they are: nothing reads them before a refill writes them.
+__global__ void __launch_bounds__(KO_WARPS * 32)
+kajita_online_restore_kernel(int n, const KoSpan *__restrict__ span, const wg_kajita_online_walk *__restrict__ walks,
+                             const uint4 *__restrict__ queue, int R, uint4 *__restrict__ ring, double *__restrict__ clock)
+{
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int i = blockIdx.x * KO_WARPS + warp; i < n; i += gridDim.x * KO_WARPS) {
+    const KoSpan sp = span[i];
+    if (lane == 0) clock[sp.b] = walks[i].clock;
+    const uint4 *iq = queue + (size_t)i * R * KO_WORDS;
+    uint4 *rb = ring + (size_t)sp.b * R * KO_WORDS;
+    const int a = min(sp.q, R - sp.first);
+    wgi_warp_copy16<KO_UNROLL>(rb + (size_t)sp.first * KO_WORDS, iq, a * KO_WORDS, a * KO_WORDS, lane);
+    wgi_warp_copy16<KO_UNROLL>(rb, iq + (size_t)a * KO_WORDS, (sp.q - a) * KO_WORDS, (sp.q - a) * KO_WORDS, lane);
+  }
+}
+
+// Walk pair[i].s of one handle -> walk pair[i].d of another (or of the same, the index sets disjoint): the queued span at
+// the same ring rows, and the clock.
+__global__ void __launch_bounds__(KO_WARPS * 32)
+kajita_online_copy_kernel(int n, const KoPair *__restrict__ pair, int R, const uint4 *__restrict__ s_ring,
+                          const double *__restrict__ s_clock, uint4 *__restrict__ d_ring, double *__restrict__ d_clock)
+{
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int i = blockIdx.x * KO_WARPS + warp; i < n; i += gridDim.x * KO_WARPS) {
+    const KoPair p = pair[i];
+    if (lane == 0) d_clock[p.d] = s_clock[p.s];
+    const uint4 *sb = s_ring + (size_t)p.s * R * KO_WORDS;
+    uint4 *db = d_ring + (size_t)p.d * R * KO_WORDS;
+    const int a = min(p.q, R - p.first);
+    wgi_warp_copy16<KO_UNROLL>(db + (size_t)p.first * KO_WORDS, sb + (size_t)p.first * KO_WORDS, a * KO_WORDS, a * KO_WORDS, lane);
+    wgi_warp_copy16<KO_UNROLL>(db, sb, (p.q - a) * KO_WORDS, (p.q - a) * KO_WORDS, lane);
+  }
+}
+
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -124,7 +220,8 @@ struct wg_kajita_online {
   double2 *d_ring = nullptr;          // [B][R] rows
   double *d_clock = nullptr;          // [B] time of the walk's next sample
   void *d_run = nullptr, *d_rows = nullptr, *d_flags = nullptr;   // run outputs; WG_MEM_HOST staging of rows, running
-  size_t cap_run = 0, cap_rows = 0, cap_flags = 0;
+  void *d_io = nullptr;               // WG_MEM_HOST staging of whole walks: records, carry, queues
+  size_t cap_run = 0, cap_rows = 0, cap_flags = 0, cap_io = 0;
   wgi_stage stage;                    // a chunk's scatter work, then first[B], npop[B]
   KoRun run;                          // where the last run's outputs are
   // the run being planned: per walk the steps it appends and its flags
@@ -162,7 +259,7 @@ static wg_rel_step ko_standard(const wg_zmpdisc_params &P, double sx, double sy,
 static void ko_free(wg_kajita_online *h)
 {
   if (h->s) wg_kajita_stream_destroy(h->s);
-  cudaFree(h->d_ring); cudaFree(h->d_clock); cudaFree(h->d_run); cudaFree(h->d_rows); cudaFree(h->d_flags);
+  cudaFree(h->d_ring); cudaFree(h->d_clock); cudaFree(h->d_run); cudaFree(h->d_rows); cudaFree(h->d_flags); cudaFree(h->d_io);
   wgi_stage_free(&h->stage);
   delete h;
 }
@@ -480,6 +577,224 @@ int wg_kajita_online_state(wg_kajita_online *h, int64_t *queued, int32_t *stacke
     if (running) running[b] = w.running;
     if (online) online[b] = w.online;
   }
+  return WG_OK;
+}
+
+}  // extern "C"
+
+// ---- whole walks ------------------------------------------------------------------------------------------------------
+// The argument checks save and restore share: nullptr when the call may go on, else why it may not.
+static const char *ko_io_refusal(const wg_kajita_online *h, int mem, int n, const void *walks, const void *carry, const void *queue)
+{
+  if (mem != WG_MEM_HOST && mem != WG_MEM_DEVICE) return "unknown mem";
+  if (n < 0) return "n < 0";
+  if (n > 0 && (!walks || !queue || (!carry && h->NL > 1))) return "NULL walks, carry or queue with n > 0";
+  if (mem == WG_MEM_DEVICE &&
+      ((reinterpret_cast<uintptr_t>(walks) | reinterpret_cast<uintptr_t>(carry) | reinterpret_cast<uintptr_t>(queue)) & 15))
+    return "device arrays must be 16-byte aligned";
+  return nullptr;
+}
+
+// The invariants every tick keeps, over a record from outside the program: nullptr when it keeps them, else which it breaks.
+static const char *ko_record_refusal(const wg_kajita_online *h, const wg_kajita_online_walk &r)
+{
+  if (!wgi_kajita_stream_record_ok(h->s, &r.stream))
+    return "a record breaks the stream's invariants of open, samples_emitted and steps_previewed";
+  if ((r.running | r.online | r.transition) & ~1) return "running, online and transition must be 0 or 1";
+  if (r.stream.open != r.online) return "stream.open differs from online";
+  if ((r.online && !r.running) || (r.transition && !r.online) || (!r.online && r.stacked != 0))
+    return "online without running, transition without online, or a stack on a walk off line";
+  if (r.keep != 1 && r.keep != -1) return "keep must be +1 or -1";
+  const int64_t q = r.stream.samples_emitted - r.popped;
+  if (r.popped < 0 || q < 0 || q > h->R) return "popped out of [0, samples_emitted], or more queued rows than the ring holds";
+  if (r.running && q < 2 * (int64_t)h->NL) return "a running walk with fewer than 2 NL queued samples";
+  if (r.stacked < 0) return "stacked < 0";
+  return nullptr;
+}
+
+// Device arrays of n records in the handle's WG_MEM_HOST staging: records, carry, queues.
+static int ko_io(wg_kajita_online *h, int n, wg_kajita_online_walk **w, double **c, wg_kajita_tick **q)
+{
+  const size_t wb = sizeof(wg_kajita_online_walk) * (size_t)n, cb = ko_align(sizeof(double2) * (size_t)(h->NL - 1) * n);
+  const int rc = wgi_grow_scratch(h->ctx, &h->d_io, &h->cap_io, wb + cb + sizeof(wg_kajita_tick) * (size_t)h->R * n);
+  if (rc != WG_OK) return rc;
+  unsigned char *base = static_cast<unsigned char *>(h->d_io);
+  *w = reinterpret_cast<wg_kajita_online_walk *>(base);
+  *c = reinterpret_cast<double *>(base + wb);
+  *q = reinterpret_cast<wg_kajita_tick *>(base + wb + cb);
+  return WG_OK;
+}
+
+extern "C" {
+
+int wg_kajita_online_carry_rows(const wg_kajita_online *h) { return h ? h->NL - 1 : WG_ERR_INVALID; }
+
+int wg_kajita_online_save(wg_kajita_online *h, int mem, int n, const int32_t *idx, wg_kajita_online_walk *walks, double *carry,
+                          wg_kajita_tick *queue, wg_rel_step *stack_host, int64_t stack_cap, int64_t *stack_len)
+{
+  if (!h) return WG_ERR_INVALID;
+  wg_ctx *ctx = h->ctx;
+  const char *call = "wg_kajita_online_save";
+  if (const char *why = ko_io_refusal(h, mem, n, walks, carry, queue)) return wg_refuse(ctx, call, why);
+  std::vector<char> mark((size_t)h->B, 0);
+  if (!wgi_record_indices_ok(h->B, n, idx, false, mark)) return wg_refuse(ctx, call, "index out of range, or n > B without indices");
+  int64_t total = 0;
+  for (int i = 0; i < n; ++i) total += (int64_t)h->walks[idx ? idx[i] : i].stack.size();
+  if (total > stack_cap) return wg_refuse(ctx, call, "the stacks hold more than stack_cap steps");
+  if (total > 0 && !stack_host) return wg_refuse(ctx, call, "NULL stack_host with steps to save");
+  if (stack_len) *stack_len = total;
+  if (n == 0) return WG_OK;
+  wg_device_guard guard(ctx->device);
+  // the stream's counters, then the handle's words and spans, in one H2D copy
+  const size_t cb = ko_align(wgi_kajita_stream_counts(h->s, n, idx, nullptr)), bytes = cb + sizeof(KoSave) * (size_t)n;
+  unsigned char *hb;
+  int rc = wgi_stage_reserve(ctx, &h->stage, bytes, &hb);
+  if (rc != WG_OK) return rc;
+  wgi_kajita_stream_counts(h->s, n, idx, hb);
+  KoSave *ks = reinterpret_cast<KoSave *>(hb + cb);
+  const int64_t NL1 = h->NL - 1;
+  int64_t at = 0;
+  for (int i = 0; i < n; ++i) {
+    const int b = idx ? idx[i] : i;
+    const KoWalk &w = h->walks[b];
+    const int64_t q = w.emitted - w.popped;
+    KoSave &k = ks[i];
+    k.sp = KoSpan{b, (int32_t)(w.popped % h->R), (int32_t)q, (int32_t)std::max<int64_t>(0, q - std::min(w.emitted, NL1))};
+    k.tail[0] = make_uint4((unsigned)w.popped, (unsigned)((uint64_t)w.popped >> 32), 0u, 0u);
+    k.tail[1] = make_uint4((unsigned)w.keep, w.running, w.online, w.transition);
+    k.tail[2] = make_uint4((unsigned)w.stack.size(), 0u, 0u, 0u);
+    std::copy(w.stack.begin(), w.stack.end(), stack_host + at);
+    at += (int64_t)w.stack.size();
+  }
+  if ((rc = wgi_stage_send(ctx, &h->stage, bytes)) != WG_OK) return rc;
+  wg_kajita_online_walk *d_w = walks;
+  double *d_c = carry;
+  wg_kajita_tick *d_q = queue;
+  if (mem == WG_MEM_HOST && (rc = ko_io(h, n, &d_w, &d_c, &d_q)) != WG_OK) return rc;
+  if ((rc = wgi_kajita_stream_save_strided(h->s, n, h->stage.d, d_w, sizeof(wg_kajita_online_walk), d_c)) != WG_OK) return rc;
+  wg_prof_start(ctx, WG_K_ZMPDISC);
+  kajita_online_save_kernel<<<wgi_grid(ctx, n, KO_WARPS, KO_CTAS_PER_SM), KO_WARPS * 32, 0, ctx->stream>>>(
+      n, reinterpret_cast<const KoSave *>(h->stage.d + cb), h->R, reinterpret_cast<const uint4 *>(h->d_ring), h->d_clock,
+      reinterpret_cast<uint4 *>(d_w), reinterpret_cast<uint4 *>(d_q));
+  wg_prof_stop(ctx);
+  WG_LAUNCHED(ctx);
+  if (mem == WG_MEM_DEVICE) return WG_OK;
+  WG_CUDA(ctx, cudaMemcpyAsync(walks, d_w, sizeof(wg_kajita_online_walk) * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+  if (NL1 > 0) WG_CUDA(ctx, cudaMemcpyAsync(carry, d_c, sizeof(double2) * NL1 * n, cudaMemcpyDeviceToHost, ctx->stream));
+  WG_CUDA(ctx, cudaMemcpyAsync(queue, d_q, sizeof(wg_kajita_tick) * (size_t)h->R * n, cudaMemcpyDeviceToHost, ctx->stream));
+  WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return WG_OK;
+}
+
+int wg_kajita_online_restore(wg_kajita_online *h, int mem, int n, const int32_t *idx, const wg_kajita_online_walk *walks,
+                             const double *carry, const wg_kajita_tick *queue, const wg_rel_step *stack_host, int64_t stack_len)
+{
+  if (!h) return WG_ERR_INVALID;
+  wg_ctx *ctx = h->ctx;
+  const char *call = "wg_kajita_online_restore";
+  if (const char *why = ko_io_refusal(h, mem, n, walks, carry, queue)) return wg_refuse(ctx, call, why);
+  std::vector<char> mark((size_t)h->B, 0);
+  if (!wgi_record_indices_ok(h->B, n, idx, true, mark))
+    return wg_refuse(ctx, call, "index out of range or repeated, or n > B without indices");
+  if (stack_len < 0 || (stack_len > 0 && !stack_host)) return wg_refuse(ctx, call, "stack_len < 0, or NULL stack_host with steps");
+  if (n == 0) return stack_len == 0 ? WG_OK : wg_refuse(ctx, call, "the stacks hold other than stack_len steps");
+  wg_device_guard guard(ctx->device);
+  // blob: indices | spans | (device records) the records read back
+  const size_t ib = ko_align(sizeof(int32_t) * (size_t)n), sb = ib + sizeof(KoSpan) * (size_t)n;
+  const size_t bytes = sb + (mem == WG_MEM_DEVICE ? sizeof(wg_kajita_online_walk) * (size_t)n : 0);
+  unsigned char *hb;
+  int rc = wgi_stage_reserve(ctx, &h->stage, bytes, &hb);
+  if (rc != WG_OK) return rc;
+  const wg_kajita_online_walk *rec = walks;
+  if (mem == WG_MEM_DEVICE) {       // the host replays the tick rules from these fields: read them back once
+    WG_CUDA(ctx, cudaMemcpyAsync(hb + sb, walks, bytes - sb, cudaMemcpyDeviceToHost, ctx->stream));
+    WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    rec = reinterpret_cast<const wg_kajita_online_walk *>(hb + sb);
+  }
+  int64_t total = 0;
+  for (int i = 0; i < n; ++i) {
+    if (const char *why = ko_record_refusal(h, rec[i])) return wg_refuse(ctx, call, why);
+    total += rec[i].stacked;
+  }
+  if (total != stack_len) return wg_refuse(ctx, call, "the stacks hold other than stack_len steps");
+  for (int64_t k = 0; k < stack_len; ++k)
+    if (!ko_step_ok(h, stack_host[k])) return wg_refuse(ctx, call, "a stacked step timing out of range or longer than max_step_time");
+  int32_t *hi = reinterpret_cast<int32_t *>(hb);
+  KoSpan *hs = reinterpret_cast<KoSpan *>(hb + ib);
+  for (int i = 0; i < n; ++i) {
+    hi[i] = idx ? idx[i] : i;
+    hs[i] = KoSpan{hi[i], (int32_t)(rec[i].popped % h->R), (int32_t)(rec[i].stream.samples_emitted - rec[i].popped), 0};
+  }
+  if ((rc = wgi_stage_send(ctx, &h->stage, sb)) != WG_OK) return rc;
+  const wg_kajita_online_walk *d_w = walks;
+  const double *d_c = carry;
+  const wg_kajita_tick *d_q = queue;
+  if (mem == WG_MEM_HOST) {
+    wg_kajita_online_walk *w;
+    double *c;
+    wg_kajita_tick *q;
+    if ((rc = ko_io(h, n, &w, &c, &q)) != WG_OK) return rc;
+    WG_CUDA(ctx, cudaMemcpyAsync(w, walks, sizeof(wg_kajita_online_walk) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+    if (h->NL > 1)
+      WG_CUDA(ctx, cudaMemcpyAsync(c, carry, sizeof(double2) * (size_t)(h->NL - 1) * n, cudaMemcpyHostToDevice, ctx->stream));
+    WG_CUDA(ctx, cudaMemcpyAsync(q, queue, sizeof(wg_kajita_tick) * (size_t)h->R * n, cudaMemcpyHostToDevice, ctx->stream));
+    d_w = w; d_c = c; d_q = q;
+  }
+  wg_prof_start(ctx, WG_K_ZMPDISC);
+  kajita_online_restore_kernel<<<wgi_grid(ctx, n, KO_WARPS, KO_CTAS_PER_SM), KO_WARPS * 32, 0, ctx->stream>>>(
+      n, reinterpret_cast<const KoSpan *>(h->stage.d + ib), d_w, reinterpret_cast<const uint4 *>(d_q), h->R,
+      reinterpret_cast<uint4 *>(h->d_ring), h->d_clock);
+  wg_prof_stop(ctx);
+  WG_LAUNCHED(ctx);
+  if ((rc = wgi_kajita_stream_restore_strided(h->s, n, hi, reinterpret_cast<const int32_t *>(h->stage.d), rec, d_w,
+                                              sizeof(wg_kajita_online_walk), d_c)) != WG_OK)
+    return rc;
+  if (mem == WG_MEM_HOST) WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  int64_t at = 0;
+  for (int i = 0; i < n; ++i) {
+    const wg_kajita_online_walk &r = rec[i];
+    KoWalk &w = h->walks[hi[i]];
+    w.stack.assign(stack_host + at, stack_host + at + r.stacked);
+    at += r.stacked;
+    w.emitted = r.stream.samples_emitted;
+    w.popped = r.popped;
+    w.keep = r.keep;
+    w.running = r.running; w.online = r.online; w.transition = r.transition;
+  }
+  return WG_OK;
+}
+
+int wg_kajita_online_copy(wg_kajita_online *dst, int n, const int32_t *dst_idx, const wg_kajita_online *src, const int32_t *src_idx)
+{
+  if (!dst || !src) return WG_ERR_INVALID;
+  wg_ctx *ctx = dst->ctx;
+  const char *call = "wg_kajita_online_copy";
+  if (n < 0) return wg_refuse(ctx, call, "n < 0");
+  if (src->ctx != ctx) return wg_refuse(ctx, call, "handles of two contexts");
+  if (dst->NL != src->NL || dst->R != src->R) return wg_refuse(ctx, call, "NL or ring rows differ");
+  if (const char *why = wgi_copy_indices_refusal(n, dst->B, dst_idx, src->B, src_idx, dst == src)) return wg_refuse(ctx, call, why);
+  if (n == 0) return WG_OK;
+  wg_device_guard guard(ctx->device);
+  int rc = wg_kajita_stream_copy(dst->s, n, dst_idx, src->s, src_idx);
+  if (rc != WG_OK) return rc;
+  const size_t bytes = sizeof(KoPair) * (size_t)n;
+  unsigned char *hb;
+  if ((rc = wgi_stage_reserve(ctx, &dst->stage, bytes, &hb)) != WG_OK) return rc;
+  KoPair *hp = reinterpret_cast<KoPair *>(hb);
+  for (int i = 0; i < n; ++i) {
+    const int d = dst_idx ? dst_idx[i] : i, s = src_idx ? src_idx[i] : i;
+    const KoWalk &w = src->walks[s];
+    hp[i] = KoPair{d, s, (int32_t)(w.popped % src->R), (int32_t)(w.emitted - w.popped)};
+  }
+  if ((rc = wgi_stage_send(ctx, &dst->stage, bytes)) != WG_OK) return rc;
+  wg_prof_start(ctx, WG_K_ZMPDISC);
+  kajita_online_copy_kernel<<<wgi_grid(ctx, n, KO_WARPS, KO_CTAS_PER_SM), KO_WARPS * 32, 0, ctx->stream>>>(
+      n, reinterpret_cast<const KoPair *>(dst->stage.d), dst->R, reinterpret_cast<const uint4 *>(src->d_ring), src->d_clock,
+      reinterpret_cast<uint4 *>(dst->d_ring), dst->d_clock);
+  wg_prof_stop(ctx);
+  WG_LAUNCHED(ctx);
+  for (int i = 0; i < n; ++i)          // the index sets are disjoint when dst == src: no entry is read after it is written
+    dst->walks[hp[i].d] = src->walks[hp[i].s];
   return WG_OK;
 }
 

@@ -172,6 +172,20 @@ extern "C" int wgi_qld_set_generator_hessian(wg_ctx *ctx, int n, int nmax, const
 extern "C" int wgi_qld_solve_generator(wg_ctx *ctx, int B, const wg_qld_batch *q, const double *A0, const double *A1,
                                        const unsigned char *sample, long long row_stride, const double *uz_dev, int N);
 
+// zmpdisc.cu internals used by kajita_online.cu: the stream part of wg_kajita_online's whole-walk records, which hold a
+// wg_kajita_stream_walk at offset 0 and are `stride` bytes apart (a multiple of 16).  The stream must have no append pending.
+//   wgi_kajita_stream_counts: the host-side counters of walks idx[0..n) (NULL: 0..n-1) as the save kernel reads them, into
+//     `host` when not NULL; returns their size in bytes.  Staged by the caller, read by wgi_kajita_stream_save_strided.
+//   wgi_kajita_stream_save_strided: one launch, as wg_kajita_stream_save's, of the staged counters d_counts.
+//   wgi_kajita_stream_record_ok: the invariants wg_kajita_stream_restore checks.
+//   wgi_kajita_stream_restore_strided: one launch, as wg_kajita_stream_restore's, of records already validated: d_walks on the
+//     device, walks_host their host copy, from which the host-side counters of walks idx[i] (host) / d_idx[i] (device) are set.
+size_t wgi_kajita_stream_counts(const wg_kajita_stream *s, int n, const int32_t *idx, void *host);
+int wgi_kajita_stream_save_strided(wg_kajita_stream *s, int n, const void *d_counts, void *d_walks, size_t stride, double *d_carry);
+bool wgi_kajita_stream_record_ok(const wg_kajita_stream *s, const wg_kajita_stream_walk *w);
+int wgi_kajita_stream_restore_strided(wg_kajita_stream *s, int n, const int32_t *idx, const int32_t *d_idx, const void *walks_host,
+                                      const void *d_walks, size_t stride, const double *d_carry);
+
 struct wg_device_guard {
   int prev = -1;
   explicit wg_device_guard(int dev) { cudaGetDevice(&prev); if (prev != dev) cudaSetDevice(dev); else prev = -1; }

@@ -759,6 +759,74 @@ stream_restore_check_kernel(int n, const wg_kajita_stream_walk *__restrict__ in,
   }
 }
 
+// stream_save_kernel and stream_restore_kernel for records stride_v4 16-byte words apart that hold the stream's record at
+// their offset 0 (wg_kajita_online_walk).  Restatements rather than a shared body, so that the two kernels above keep their
+// code.
+__global__ void __launch_bounds__(ZS_WARPS * 32)
+stream_save_strided_kernel(int n, const ZsCounts *__restrict__ cnt, const ZsRec *__restrict__ rec, const double *__restrict__ pv_state,
+                           const double2 *__restrict__ carry, int NL1, uint4 *__restrict__ out, int stride_v4,
+                           double2 *__restrict__ out_carry)
+{
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int i = blockIdx.x * ZS_WARPS + warp; i < n; i += gridDim.x * ZS_WARPS) {
+    const ZsCounts c = cnt[i];
+    const bool live = c.emitted > 0;
+    const uint4 *r = reinterpret_cast<const uint4 *>(rec + c.b);
+    const uint4 *st = pv_state ? reinterpret_cast<const uint4 *>(pv_state + 8 * (int64_t)c.b) : nullptr;
+    uint4 *o = out + (int64_t)i * stride_v4;
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const int e = lane + 32 * k;
+      if (e >= ZS_WALK_V4) break;
+      uint4 v = make_uint4(0u, 0u, 0u, 0u);
+      if (e < ZS_REC_V4) {
+        if (live) v = r[e];
+      } else if (e < ZS_REC_V4 + ZS_STATE_V4) {
+        if (live && st) v = st[e - ZS_REC_V4];
+      } else {
+        v = make_uint4((unsigned)c.previewed, (unsigned)((uint64_t)c.previewed >> 32), (unsigned)c.open, 0u);
+      }
+      if (e == ZS_F0_V4) { v.z = (unsigned)c.emitted; v.w = (unsigned)((uint64_t)c.emitted >> 32); }
+      o[e] = v;
+    }
+    if (NL1 > 0)
+      wgi_warp_copy16<ZS_UNROLL>(reinterpret_cast<uint4 *>(out_carry + (int64_t)i * NL1),
+                                 reinterpret_cast<const uint4 *>(carry + (int64_t)c.b * NL1), NL1, live ? c.emitted - c.previewed : 0, lane);
+  }
+}
+
+__global__ void __launch_bounds__(ZS_WARPS * 32)
+stream_restore_strided_kernel(int n, const int32_t *__restrict__ idx, const uint4 *__restrict__ in, int stride_v4,
+                              const double2 *__restrict__ in_carry, int NL1, ZsRec *__restrict__ rec, double *__restrict__ pv_state,
+                              double2 *__restrict__ carry, int *__restrict__ status)
+{
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int i = blockIdx.x * ZS_WARPS + warp; i < n; i += gridDim.x * ZS_WARPS) {
+    const int b = idx[i];
+    const uint4 *src = in + (int64_t)i * stride_v4;
+    const wg_kajita_stream_walk *w = reinterpret_cast<const wg_kajita_stream_walk *>(src);
+    uint4 *r = reinterpret_cast<uint4 *>(rec + b);
+    uint4 *st = pv_state ? reinterpret_cast<uint4 *>(pv_state + 8 * (int64_t)b) : nullptr;
+    uint4 v[2];
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const int e = lane + 32 * k;
+      if (e < ZS_REC_V4 + ZS_STATE_V4) v[k] = src[e];
+    }
+#pragma unroll
+    for (int k = 0; k < 2; ++k) {
+      const int e = lane + 32 * k;
+      if (e < ZS_REC_V4) r[e] = v[k];
+      else if (e < ZS_REC_V4 + ZS_STATE_V4 && st) st[e - ZS_REC_V4] = v[k];
+    }
+    if (NL1 > 0)
+      wgi_warp_copy16<ZS_UNROLL>(reinterpret_cast<uint4 *>(carry + (int64_t)b * NL1),
+                                 reinterpret_cast<const uint4 *>(in_carry + (int64_t)i * NL1), NL1,
+                                 w->samples_emitted - w->steps_previewed, lane);
+    if (lane == 0) status[b] = 0;
+  }
+}
+
 // Walk sidx[i] of one stream -> walk didx[i] of another (or of the same, the two index sets disjoint), verbatim; status 0.
 __global__ void __launch_bounds__(ZS_WARPS * 32)
 stream_copy_kernel(int n, const int32_t *__restrict__ didx, const int32_t *__restrict__ sidx, const ZsRec *__restrict__ s_rec,
@@ -1721,3 +1789,51 @@ int wg_kajita_stream_copy(wg_kajita_stream *dst, int n, const int32_t *dst_idx, 
 }
 
 }  // extern "C"
+
+// ---- the stream part of wg_kajita_online's whole-walk records (kajita_online.cu) -------------------------------------
+size_t wgi_kajita_stream_counts(const wg_kajita_stream *s, int n, const int32_t *idx, void *host)
+{
+  ZsCounts *c = static_cast<ZsCounts *>(host);
+  for (int i = 0; c && i < n; ++i) {
+    const int b = idx ? idx[i] : i;
+    c[i].emitted = s->emitted[b]; c[i].previewed = s->previewed[b]; c[i].open = s->open[b]; c[i].b = b;
+  }
+  return sizeof(ZsCounts) * (size_t)n;
+}
+
+int wgi_kajita_stream_save_strided(wg_kajita_stream *s, int n, const void *d_counts, void *d_walks, size_t stride, double *d_carry)
+{
+  wg_ctx *ctx = s->ctx;
+  wg_prof_start(ctx, WG_K_ZMPDISC);
+  stream_save_strided_kernel<<<wgi_grid(ctx, n, ZS_WARPS, ZS_CTAS_PER_SM), ZS_WARPS * 32, 0, ctx->stream>>>(
+      n, static_cast<const ZsCounts *>(d_counts), s->d_rec, s->d_state, s->d_carry, zs_carry_rows(s), static_cast<uint4 *>(d_walks),
+      (int)(stride / 16), reinterpret_cast<double2 *>(d_carry));
+  wg_prof_stop(ctx);
+  WG_LAUNCHED(ctx);
+  return WG_OK;
+}
+
+bool wgi_kajita_stream_record_ok(const wg_kajita_stream *s, const wg_kajita_stream_walk *w)
+{
+  return zs_counts_ok(w->samples_emitted, w->steps_previewed, w->open, s->with_preview, zs_carry_rows(s));
+}
+
+int wgi_kajita_stream_restore_strided(wg_kajita_stream *s, int n, const int32_t *idx, const int32_t *d_idx, const void *walks_host,
+                                      const void *d_walks, size_t stride, const double *d_carry)
+{
+  wg_ctx *ctx = s->ctx;
+  wg_prof_start(ctx, WG_K_ZMPDISC);
+  stream_restore_strided_kernel<<<wgi_grid(ctx, n, ZS_WARPS, ZS_CTAS_PER_SM), ZS_WARPS * 32, 0, ctx->stream>>>(
+      n, d_idx, static_cast<const uint4 *>(d_walks), (int)(stride / 16), reinterpret_cast<const double2 *>(d_carry), zs_carry_rows(s),
+      s->d_rec, s->d_state, s->d_carry, s->d_status);
+  wg_prof_stop(ctx);
+  WG_LAUNCHED(ctx);
+  for (int i = 0; i < n; ++i) {
+    const int b = idx ? idx[i] : i;
+    const wg_kajita_stream_walk *w = reinterpret_cast<const wg_kajita_stream_walk *>(static_cast<const unsigned char *>(walks_host) + i * stride);
+    s->emitted[b] = w->samples_emitted;
+    s->previewed[b] = w->steps_previewed;
+    s->open[b] = w->open;
+  }
+  return WG_OK;
+}
