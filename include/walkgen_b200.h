@@ -496,6 +496,53 @@ int wg_herdt_online_tick(wg_herdt_online *h, int mem, int nticks, const wg_herdt
 /* The B state records in DEVICE memory (plain data, editable between calls as wg_herdt_mpc_run_batch's are). */
 wg_herdt_mpc_state *wg_herdt_online_states(wg_herdt_online *h);
 
+/* Plans: the MPC solution of a robot at the tick it fires, expanded over its horizon (ZMPVelocityReferencedQP::Solution():
+ * Solution_vec, SupportStates_deq, SupportOrientations_deq, ZMPVelocityReferencedQP.hh:126).  The horizon is the reference's
+ * own prediction: previewed sample k (k = 1..N, index k-1 of the prw_ arrays) lies k T after the QP instant, T the QP period
+ * wg_herdt_params.T, and is S_k x^ + U_k u with x^ = com_x (com_y), u = jerk_x (jerk_y) and the matrices of
+ * RigidBodySystem::compute_dyn_cjerk (rigid-body-system.cpp:377-452): position, velocity, acceleration, and the CoP of the
+ * QP's model height wg_herdt_params.com_height with g = 9.81 (not the state's com_height).
+ * Rows: the QP fires at the tick of clock `time`.  The period it computes is sample j = 0..20, the CoM j Ts after the instant
+ * of com_x under jerk_x[0] / jerk_y[0] (Ts = wg_herdt_mpc_params.Ts, so j = 20 is previewed sample 1).  Sample j is the row
+ * popped 8 + j ticks after the firing tick, at clock time + (8 + j) Ts; j = 0 is the deques' inherited back row, which takes
+ * the period's feet, and j = 20 is popped as the next period's j = 0.  At a robot's first QP after its start the deques hold
+ * 8 rows instead of 9, and every row comes one tick earlier: 7 + j ticks after the firing tick.
+ * The plan is the QP's solution: at the end of a walk with wg_herdt_mpc_params.return_to_centre = 1, the jerk the period
+ * applies is the return-to-centre jerk, not jerk_x[0] / jerk_y[0], and then the state's CoM leaves the previewed one.
+ * A plan is not part of a robot (wg_herdt_online_robot): after a restore or a copy, the caller's entry still describes the
+ * robot's earlier history until the robot fires again. */
+typedef struct wg_herdt_plan {                 /* the QP of one firing robot, expanded over its horizon                 */
+  double time;                                 /* clock at which the QP fired (what wg_herdt_mpc_step.time reports)     */
+  double com_x[3], com_y[3];                   /* CoM_ at the QP instant: the horizon's initial state (QP input)        */
+  double jerk_x[WG_HERDT_N], jerk_y[WG_HERDT_N];             /* Solution_vec[0..2N)                                     */
+  double prw_com_x[WG_HERDT_N][3], prw_com_y[WG_HERDT_N][3]; /* CoM (pos, vel, acc) at previewed samples k = 1..N        */
+  double prw_cop_x[WG_HERDT_N], prw_cop_y[WG_HERDT_N];       /* CoP at previewed samples k = 1..N                       */
+  double sup_x[WG_HERDT_N + 1], sup_y[WG_HERDT_N + 1], sup_yaw[WG_HERDT_N + 1]; /* SupportStates_deq[0..N]              */
+  double step_x[2], step_y[2], step_yaw[2];    /* previewed footsteps s < n_steps: Solution_vec[2N+s], [2N+ns+s], and
+                                                  the support yaw of the sample where step s starts; 0 beyond n_steps    */
+  int8_t sup_foot[WG_HERDT_N + 1], sup_phase[WG_HERDT_N + 1], sup_step[WG_HERDT_N + 1], sup_changed[WG_HERDT_N + 1];
+  int8_t step_sample[2], step_foot[2];         /* previewed sample (1..N) where step s starts, and its foot; 0 = none    */
+  int32_t n_steps, fail, iterations, qp_count; /* ns; QLD ifail convention; active-set changes; the robot's qp_count
+                                                  counting this QP (its state's qp_count right after the tick)          */
+  int32_t pad_[2];
+} wg_herdt_plan;                               /* 1888 bytes, a multiple of 16                                           */
+
+/* wg_herdt_online_tick, and the plan of every robot that fires.  commands, rows, running and mem mean what they mean for
+ * wg_herdt_online_tick, and rows, running flags and states come out bitwise as wg_herdt_online_tick leaves them.  In `mem`,
+ * each may be NULL:
+ *   plans     [B]   robot b's entry is written at every tick of the call at which b fires, so the last firing of the call
+ *                   wins; the entries of robots that do not fire in the call are left untouched (both memory modes).  The
+ *                   caller owns the array, so a plan outlives the call and the handle's scratch.
+ *   plan_tick [B]   the index t within the call of b's last firing, or -1.
+ * With both NULL the call is wg_herdt_online_tick: the same four launches per tick and the same work.  Otherwise a tick is
+ * five launches: the plan kernel runs after the period.  WG_MEM_DEVICE: no synchronisation and, once the handle's buffers
+ * exist, no allocation.  WG_MEM_HOST: plans are uploaded (so untouched entries keep their bytes), ticked as on the device and
+ * copied back with plan_tick.
+ * Refused with WG_ERR_INVALID, nothing changed: what wg_herdt_online_tick refuses, and device plans that are not 16-byte
+ * aligned (records are stored as 16-byte words). */
+int wg_herdt_online_tick_plan(wg_herdt_online *h, int mem, int nticks, const wg_herdt_command *commands, wg_herdt_tick *rows,
+                              int8_t *running, wg_herdt_plan *plans, int32_t *plan_tick);
+
 /* Whole robots: save, restore and copy, for checkpoints, lookahead branches and migration between handles, processes or GPUs.
  *
  * A robot of wg_herdt_online is its state record, its deques and its {count, running} slot: everything the next tick of that

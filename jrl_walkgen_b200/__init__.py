@@ -31,6 +31,7 @@ HERDT_COMMAND_DTYPE = _capi.herdt_command_dtype()
 CMD_VEL, CMD_STOP = _capi.WG_CMD_VEL, _capi.WG_CMD_STOP
 HERDT_ONLINE_QUEUE = _capi.HERDT_ONLINE_QUEUE
 ONLINE_ROBOT_DTYPE = _capi.herdt_online_robot_dtype()
+HERDT_PLAN_DTYPE = _capi.herdt_plan_dtype()
 # init15 of the TestHerdt2010 start at rest: CoM (x, dx, ddx, y, dy, ddy, z), trunk yaw and rate, left and right foot (x, y, theta)
 HERDT_INIT15 = (0.0316055, 0.0, 0.0, 0.0, 0.0, 0.0, 0.7116911, 0.0, 0.0, 0.0, 0.09, 0.0, 0.0, -0.09, 0.0)
 DimitrovParams = _capi.DimitrovParams
@@ -38,7 +39,7 @@ DimitrovParams = _capi.DimitrovParams
 __all__ = ["MultiContext", "LCI_DTYPE", "DIMITROV_PERIOD_DTYPE", "DimitrovParams", "dimitrov_default_params", "Context", "PreviewPlan", "KajitaPlan", "KajitaStream", "HerdtOnline",
            "KajitaOnline", "KAJITA_ONLINE_WALK_DTYPE", "KAJITA_TICK_DTYPE", "KAJITA_COMMAND_DTYPE", "KAJITA_PUSH", "KAJITA_STANDARD", "KAJITA_STOP",
            "KAJITA_ONLINE_CHUNK",
-           "HERDT_COMMAND_DTYPE", "CMD_VEL", "CMD_STOP", "HERDT_ONLINE_QUEUE", "ONLINE_ROBOT_DTYPE", "HERDT_INIT15",
+           "HERDT_COMMAND_DTYPE", "CMD_VEL", "CMD_STOP", "HERDT_ONLINE_QUEUE", "ONLINE_ROBOT_DTYPE", "HERDT_PLAN_DTYPE", "HERDT_INIT15",
            "STREAM_START", "STREAM_FINISH", "zmpdisc_default_params", "REL_STEP_DTYPE", "KAJITA_FOOT_DTYPE", "KAJITA_STREAM_WALK_DTYPE", "preview_gains", "herdt_default_params", "herdt_mpc_default_params", "HerdtParams", "HerdtMpcParams",
            "PLDP_STATE_DTYPE", "PLDP_INFO_DTYPE", "FOOT_DTYPE", "TICK_DTYPE", "MPC_STATE_DTYPE", "MPC_STEP_DTYPE", "TICKS_PER_STEP", "QP_INPUT_DTYPE",
            "QP_OUTPUT_DTYPE", "ACTIVE_SET_DTYPE", "WalkgenError", "device_count",
@@ -908,6 +909,27 @@ class HerdtOnline:
         """Device-resident form (asynchronous on the context stream)."""
         self.ctx._check(self.ctx.lib.wg_herdt_online_tick(self.h, WG_MEM_DEVICE, int(nticks), _ptr(d_commands), _ptr(d_rows),
                                                           _ptr(d_running)))
+
+    def tick_plan(self, nticks, plans, commands=None, rows=True, running=True):
+        """tick(), and the plan of every robot that fires (wg_herdt_online_tick_plan): plans, a host array [B] of
+        HERDT_PLAN_DTYPE, is updated in place for the robots that fire (the last firing of the call wins), the other
+        entries keep their bytes -> (rows, running, plan_tick [B] int32: index of the last firing in the call, or -1)."""
+        n = int(nticks)
+        cmd = None if commands is None else np.ascontiguousarray(commands, dtype=HERDT_COMMAND_DTYPE)
+        assert cmd is None or cmd.shape == (n, self.B)
+        assert plans is None or (plans.dtype == HERDT_PLAN_DTYPE and plans.shape == (self.B,) and plans.flags["C_CONTIGUOUS"])
+        r = np.zeros((n, self.B), dtype=TICK_DTYPE) if rows else None
+        run = np.zeros((n, self.B), dtype=np.int8) if running else None
+        pt = np.full(self.B, -1, dtype=np.int32)
+        self.ctx._check(self.ctx.lib.wg_herdt_online_tick_plan(self.h, WG_MEM_HOST, n, _ptr(cmd), _ptr(r), _ptr(run),
+                                                               _ptr(plans), _ptr(pt)))
+        return r, run, pt
+
+    def tick_plan_device(self, nticks, d_plans, d_commands=None, d_rows=None, d_running=None, d_plan_tick=None):
+        """Device-resident form of tick_plan (asynchronous on the context stream)."""
+        self.ctx._check(self.ctx.lib.wg_herdt_online_tick_plan(self.h, WG_MEM_DEVICE, int(nticks), _ptr(d_commands),
+                                                               _ptr(d_rows), _ptr(d_running), _ptr(d_plans),
+                                                               _ptr(d_plan_tick)))
 
     @property
     def d_states(self) -> int:

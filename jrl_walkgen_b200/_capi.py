@@ -285,6 +285,21 @@ def herdt_online_robot_dtype():
     return d
 
 
+def herdt_plan_dtype():
+    """numpy mirror of wg_herdt_plan (1888 B): the QP of one firing robot of wg_herdt_online, expanded over its horizon."""
+    np = _np()
+    N = HERDT_N
+    d = np.dtype([("time", "f8"), ("com_x", "f8", 3), ("com_y", "f8", 3), ("jerk_x", "f8", N), ("jerk_y", "f8", N),
+                  ("prw_com_x", "f8", (N, 3)), ("prw_com_y", "f8", (N, 3)), ("prw_cop_x", "f8", N), ("prw_cop_y", "f8", N),
+                  ("sup_x", "f8", N + 1), ("sup_y", "f8", N + 1), ("sup_yaw", "f8", N + 1),
+                  ("step_x", "f8", 2), ("step_y", "f8", 2), ("step_yaw", "f8", 2),
+                  ("sup_foot", "i1", N + 1), ("sup_phase", "i1", N + 1), ("sup_step", "i1", N + 1),
+                  ("sup_changed", "i1", N + 1), ("step_sample", "i1", 2), ("step_foot", "i1", 2),
+                  ("n_steps", "i4"), ("fail", "i4"), ("iterations", "i4"), ("qp_count", "i4"), ("pad_", "i4", 2)])
+    assert d.itemsize == 1888
+    return d
+
+
 # name -> (restype, argtypes); also the list checked against include/walkgen_b200.h by the tests
 SIGNATURES = {
     "wg_version": (C.c_int, []),
@@ -426,6 +441,8 @@ SIGNATURES = {
     "wg_herdt_online_start": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
     "wg_herdt_online_tick": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "wg_herdt_online_states": (C.c_void_p, [C.c_void_p]),
+    "wg_herdt_online_tick_plan": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_void_p]),
     "wg_herdt_online_save": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "wg_herdt_online_restore": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "wg_herdt_online_copy": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -859,6 +859,91 @@ online_copy_kernel(int n, const int32_t *__restrict__ didx, const int32_t *__res
   }
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Plans (wg_herdt_online_tick_plan): after the period, the QP record and solution of each robot that fired this tick,
+// expanded over the horizon, one warp per robot.  The record is assembled in shared memory and stored as 16-byte words.
+// ---------------------------------------------------------------------------------------------------------------
+constexpr int PLAN_V4 = (int)(sizeof(wg_herdt_plan) / 16);   // 118
+static_assert(sizeof(wg_herdt_plan) == 1888 && sizeof(wg_herdt_plan) % 16 == 0, "plan layout");
+static_assert(offsetof(wg_herdt_plan, sup_changed) - offsetof(wg_herdt_plan, sup_foot) ==
+                  offsetof(wg_herdt_qp_input, sup_changed) - offsetof(wg_herdt_qp_input, sup_foot), "plan support bytes");
+
+// plan_tick[b] = t for a robot that fires at tick t of the call; tick 0 writes -1 for the others.  plans[b] of a robot that
+// does not fire is not touched.
+__global__ void __launch_bounds__(MPC_WARPS * 32)
+online_plan_kernel(int B, int t, const herdt::Consts *__restrict__ Cp, const wg_herdt_mpc_state *__restrict__ states,
+                   const MpcScratch *__restrict__ scratch, const wg_herdt_qp_input *__restrict__ qp_rec,
+                   const wg_herdt_qp_output *__restrict__ qp_out, wg_herdt_plan *__restrict__ plans,
+                   int32_t *__restrict__ plan_tick)
+{
+  __shared__ __align__(16) wg_herdt_plan sp[MPC_WARPS];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const herdt::Consts &C = *Cp;
+  const double T = C.P.T;
+  wg_herdt_plan &p = sp[warp];
+  for (int b = blockIdx.x * MPC_WARPS + warp; b < B; b += gridDim.x * MPC_WARPS) {
+    const int fire = scratch[b].fire;
+    if (plan_tick && lane == 0 && (fire || t == 0)) plan_tick[b] = fire ? t : -1;
+    if (!fire || !plans) continue;
+    const wg_herdt_qp_input &in = qp_rec[b];
+    const wg_herdt_qp_output &o = qp_out[b];
+    uint4 *pv = reinterpret_cast<uint4 *>(&p);
+    for (int e = lane; e < PLAN_V4; e += 32) pv[e] = make_uint4(0u, 0u, 0u, 0u);
+    __syncwarp();
+    // sample k = i + 1 of axis lane / 16: S_k x^ + U_k u, U lower triangular (rigid-body-system.cpp:377-452)
+    const int axis = lane >> 4, i = lane & 15;
+    const double *cv = axis ? in.com_y : in.com_x;
+    const double c0 = cv[0], c1 = cv[1], c2 = cv[2];
+    const double u = o.x[axis * N + i];
+    const double kT = (i + 1) * T;
+    double pos = c0 + kT * c1 + kT * kT * 0.5 * c2, vel = c1 + kT * c2, acc = c2;
+    double cop = C.Sz[i][0] * c0 + C.Sz[i][1] * c1 + C.Sz[i][2] * c2;
+#pragma unroll 1
+    for (int j = 0; j < N; ++j) {
+      const double uj = __shfl_sync(0xffffffffu, u, (axis << 4) + j);
+      if (j <= i) {
+        const int d = i - j;
+        pos = fma((1 + 3 * d + 3 * d * d) * T * T * T / 6.0, uj, pos);
+        vel = fma((2 * d + 1) * T * T * 0.5, uj, vel);
+        acc = fma(T, uj, acc);
+        cop = fma(C.uz[d], uj, cop);
+      }
+    }
+    double *pc = axis ? &p.prw_com_y[i][0] : &p.prw_com_x[i][0];
+    pc[0] = pos; pc[1] = vel; pc[2] = acc;
+    (axis ? p.prw_cop_y : p.prw_cop_x)[i] = cop;
+    (axis ? p.jerk_y : p.jerk_x)[i] = u;
+    if (lane < N + 1) { p.sup_x[lane] = in.sup_x[lane]; p.sup_y[lane] = in.sup_y[lane]; p.sup_yaw[lane] = in.sup_yaw[lane]; }
+    {
+      const int8_t *sb = in.sup_foot;
+      int8_t *db = p.sup_foot;
+      for (int e = lane; e < 4 * (N + 1); e += 32) db[e] = sb[e];
+    }
+    const int ns = (o.n_vars - 2 * N) / 2;
+    if (lane < 2 && lane < ns && ns <= WG_HERDT_MAX_STEPS) {
+      // step s starts at the first previewed sample of StepNumber s + 1 (generator-vel-ref.cpp:106-128)
+      int k = N;
+      for (int kk = N; kk >= 1; --kk)
+        if (in.sup_step[kk] == lane + 1) k = kk;
+      p.step_x[lane] = o.x[2 * N + lane];
+      p.step_y[lane] = o.x[2 * N + ns + lane];
+      p.step_yaw[lane] = in.sup_yaw[k];
+      p.step_sample[lane] = (int8_t)k;
+      p.step_foot[lane] = in.sup_foot[k];
+    }
+    if (lane == 0) {
+      p.time = states[b].clock;
+      p.qp_count = states[b].qp_count;
+      p.n_steps = ns; p.fail = o.fail; p.iterations = o.iterations;
+    }
+    if (lane < 3) { p.com_x[lane] = in.com_x[lane]; p.com_y[lane] = in.com_y[lane]; }
+    __syncwarp();
+    uint4 *dst = reinterpret_cast<uint4 *>(plans + b);
+    for (int e = lane; e < PLAN_V4; e += 32) dst[e] = pv[e];
+    __syncwarp();
+  }
+}
+
 }  // namespace
 
 const herdt::Consts *wg_herdt_device_consts(wg_ctx *ctx);
@@ -1115,6 +1200,8 @@ struct wg_herdt_online {
   // staging of WG_MEM_HOST ticks (commands, rows, running) and of WG_MEM_HOST robot records
   void *d_cmd = nullptr, *d_rows = nullptr, *d_run = nullptr, *d_robots = nullptr;
   size_t cap_cmd = 0, cap_rows = 0, cap_run = 0, cap_robots = 0;
+  void *d_plans = nullptr, *d_plan_tick = nullptr;   // staging of WG_MEM_HOST plans
+  size_t cap_plans = 0, cap_plan_tick = 0;
   wgi_stage stage;   // start: init states and indices; save, restore, copy: the check flag, and the indices on the device
 };
 
@@ -1122,6 +1209,7 @@ static void online_free(wg_herdt_online *h)
 {
   cudaFree(h->d_states); cudaFree(h->d_queue); cudaFree(h->d_slots); cudaFree(h->d_staged);
   cudaFree(h->d_cmd); cudaFree(h->d_rows); cudaFree(h->d_run); cudaFree(h->d_robots);
+  cudaFree(h->d_plans); cudaFree(h->d_plan_tick);
   wgi_stage_free(&h->stage);
   delete h;
 }
@@ -1148,7 +1236,7 @@ static int online_stage(wg_herdt_online *h, int n, bool flag, const int32_t *a, 
 }
 
 static int online_ticks(wg_herdt_online *h, MpcState *m, int nticks, const wg_herdt_command *cmd, wg_herdt_tick *rows,
-                        int8_t *running)
+                        int8_t *running, wg_herdt_plan *plans, int32_t *plan_tick)
 {
   wg_ctx *ctx = h->ctx;
   const int B = h->B;
@@ -1179,6 +1267,12 @@ static int online_ticks(wg_herdt_online *h, MpcState *m, int nticks, const wg_he
                                                                         running ? running + (size_t)t * nb : nullptr);
     wg_prof_stop(ctx);
     WG_LAUNCHED(ctx);
+    if (plans || plan_tick) {
+      wg_prof_start(ctx, WG_K_HERDT_MPC);
+      online_plan_kernel<<<blocks, MPC_WARPS * 32, 0, ctx->stream>>>(B, t, consts, h->d_states, scr, rec, out, plans, plan_tick);
+      wg_prof_stop(ctx);
+      WG_LAUNCHED(ctx);
+    }
   }
   return WG_OK;
 }
@@ -1251,31 +1345,53 @@ int wg_herdt_online_start(wg_herdt_online *h, int n, const int32_t *idx_host, co
   return WG_OK;
 }
 
-int wg_herdt_online_tick(wg_herdt_online *h, int mem, int nticks, const wg_herdt_command *commands, wg_herdt_tick *rows,
-                         int8_t *running)
+static int online_tick_call(wg_herdt_online *h, int mem, int nticks, const wg_herdt_command *commands, wg_herdt_tick *rows,
+                            int8_t *running, wg_herdt_plan *plans, int32_t *plan_tick)
 {
   if (!h || nticks < 0 || (mem != WG_MEM_HOST && mem != WG_MEM_DEVICE)) return WG_ERR_INVALID;
   wg_ctx *ctx = h->ctx;
+  if (mem == WG_MEM_DEVICE && reinterpret_cast<uintptr_t>(plans) % 16)
+    return wg_refuse(ctx, "wg_herdt_online_tick_plan", "device plans must be 16-byte aligned");
   MpcState *m = mpc_of(ctx);
   if (!m->ready || !wg_herdt_device_consts(ctx))
     return wg_fail(ctx, WG_ERR_NOT_READY, "wg_herdt_set_params / wg_herdt_mpc_set_params not called");
   if (h->B == 0 || nticks == 0) return WG_OK;
   wg_device_guard guard(ctx->device);
-  if (mem == WG_MEM_DEVICE) return online_ticks(h, m, nticks, commands, rows, running);
-  const size_t n = (size_t)h->B * nticks;
+  if (mem == WG_MEM_DEVICE) return online_ticks(h, m, nticks, commands, rows, running, plans, plan_tick);
+  const size_t n = (size_t)h->B * nticks, nb = (size_t)h->B;
   int rc;
   if (commands && (rc = wgi_grow_scratch(ctx, &h->d_cmd, &h->cap_cmd, sizeof(wg_herdt_command) * n)) != WG_OK) return rc;
   if (rows && (rc = wgi_grow_scratch(ctx, &h->d_rows, &h->cap_rows, sizeof(wg_herdt_tick) * n)) != WG_OK) return rc;
   if (running && (rc = wgi_grow_scratch(ctx, &h->d_run, &h->cap_run, sizeof(int8_t) * n)) != WG_OK) return rc;
+  if (plans && (rc = wgi_grow_scratch(ctx, &h->d_plans, &h->cap_plans, sizeof(wg_herdt_plan) * nb)) != WG_OK) return rc;
+  if (plan_tick && (rc = wgi_grow_scratch(ctx, &h->d_plan_tick, &h->cap_plan_tick, sizeof(int32_t) * nb)) != WG_OK) return rc;
   if (commands) WG_CUDA(ctx, cudaMemcpyAsync(h->d_cmd, commands, sizeof(wg_herdt_command) * n, cudaMemcpyHostToDevice, ctx->stream));
   if (rows) WG_CUDA(ctx, cudaMemsetAsync(h->d_rows, 0, sizeof(wg_herdt_tick) * n, ctx->stream));
+  if (plans) WG_CUDA(ctx, cudaMemcpyAsync(h->d_plans, plans, sizeof(wg_herdt_plan) * nb, cudaMemcpyHostToDevice, ctx->stream));
   rc = online_ticks(h, m, nticks, commands ? static_cast<const wg_herdt_command *>(h->d_cmd) : nullptr,
-                    rows ? static_cast<wg_herdt_tick *>(h->d_rows) : nullptr, running ? static_cast<int8_t *>(h->d_run) : nullptr);
+                    rows ? static_cast<wg_herdt_tick *>(h->d_rows) : nullptr, running ? static_cast<int8_t *>(h->d_run) : nullptr,
+                    plans ? static_cast<wg_herdt_plan *>(h->d_plans) : nullptr,
+                    plan_tick ? static_cast<int32_t *>(h->d_plan_tick) : nullptr);
   if (rc != WG_OK) return rc;
   if (rows) WG_CUDA(ctx, cudaMemcpyAsync(rows, h->d_rows, sizeof(wg_herdt_tick) * n, cudaMemcpyDeviceToHost, ctx->stream));
   if (running) WG_CUDA(ctx, cudaMemcpyAsync(running, h->d_run, sizeof(int8_t) * n, cudaMemcpyDeviceToHost, ctx->stream));
+  if (plans) WG_CUDA(ctx, cudaMemcpyAsync(plans, h->d_plans, sizeof(wg_herdt_plan) * nb, cudaMemcpyDeviceToHost, ctx->stream));
+  if (plan_tick)
+    WG_CUDA(ctx, cudaMemcpyAsync(plan_tick, h->d_plan_tick, sizeof(int32_t) * nb, cudaMemcpyDeviceToHost, ctx->stream));
   WG_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return WG_OK;
+}
+
+int wg_herdt_online_tick(wg_herdt_online *h, int mem, int nticks, const wg_herdt_command *commands, wg_herdt_tick *rows,
+                         int8_t *running)
+{
+  return online_tick_call(h, mem, nticks, commands, rows, running, nullptr, nullptr);
+}
+
+int wg_herdt_online_tick_plan(wg_herdt_online *h, int mem, int nticks, const wg_herdt_command *commands, wg_herdt_tick *rows,
+                              int8_t *running, wg_herdt_plan *plans, int32_t *plan_tick)
+{
+  return online_tick_call(h, mem, nticks, commands, rows, running, plans, plan_tick);
 }
 
 int wg_herdt_online_save(wg_herdt_online *h, int mem, int n, const int32_t *idx, wg_herdt_online_robot *out)
